@@ -29,6 +29,10 @@ data-path collective: the path has no exchange step.
             on this box's host cores, on a bounded prefix of the same users.
   parity    the metric rows the CPU baseline computed for that prefix against the rows the timed e2e call wrote for the
             same users: {users, rows compared, mismatches beyond 1e-6 / NaN pattern, largest difference}.
+
+`--dump-outputs DIR` writes the metric rows of the last timed step as DIR/<metric>.npy, the defined values, and
+DIR/<metric>_defined.npy, where they are defined (see dump_outputs), so that two builds can be compared output for output:
+with the same arguments the inputs are the same from run to run.
 """
 import argparse
 import hashlib
@@ -43,10 +47,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 from tools import synth  # noqa: E402
 
 METRIC = "evaluated_users_per_sec"
 UNIT = "users/s"
+DUMP_BYTES = 60 << 20      # --dump-outputs: array bytes of all files, under 64 MB with the .npy headers
 METRIC_FLAGS = dict(p="precision", tp="trunc_precision", r="recall", ap="average_precision",
                     tap="trunc_average_precision", ndcg="ndcg", hit="hit", rr="rr", roc="roc_auc", pr="pr_auc")
 
@@ -60,6 +66,25 @@ def env_int(name, default):
 
 def workload_name(cfg, users_total, gpus, scaling):
     return "%s; %d users in all, block-partitioned over %d GPU(s) (%s scaling)" % (cfg.name, users_total, gpus, scaling)
+
+
+def dump_outputs(out_dir, rows, rank, world):
+    """Write this rank's metric rows (name -> (users,) or (users, K) array) to out_dir, every file finite: a metric is NaN
+    where the reference leaves it undefined (a user without test items or with too few candidates), so <name>.npy holds
+    the defined values in user order and <name>_defined.npy (float32, the rows' shape) 1 where a value is defined and 0
+    where the caller gets NaN.  Under torchrun the names end in _rank<r>.  The ranks share DUMP_BYTES; when the files
+    would be larger, the same seeded sample of users is kept in every file."""
+    os.makedirs(out_dir, exist_ok=True)
+    m = next(iter(rows.values())).shape[0]
+    row_bytes = sum((v.nbytes + 4 * v.size) // max(m, 1) for v in rows.values())
+    keep = min(m, DUMP_BYTES // world // max(row_bytes, 1))
+    users = None if keep == m else np.sort(np.random.default_rng(12345 + rank).choice(m, keep, replace=False))
+    tail = "" if world == 1 else "_rank%d" % rank
+    for name, v in rows.items():
+        v = v if users is None else v[users]
+        defined = np.isfinite(v)
+        np.save(os.path.join(out_dir, name + tail + ".npy"), v[defined])
+        np.save(os.path.join(out_dir, name + "_defined" + tail + ".npy"), defined.astype(np.float32))
 
 
 # ----------------------------------------------------------------------------- CPU arms
@@ -297,6 +322,10 @@ def product_arm(args, cfg, rank, world, local_rank):
     e1.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # the rows the last timed step wrote (the e2e and pageable legs below write their own buffers)
+        dump_outputs(args.dump_outputs, {METRIC_FLAGS[q]: v.cpu().numpy().reshape(m, -1) if cfg.cumulative and q in _capi.TOPK_METRICS
+                                         else v.cpu().numpy() for q, v in douts.items()}, rank, world)
     dev_ms = e0.elapsed_time(e1)
     per_rank = None
     if world > 1:
@@ -337,7 +366,7 @@ def product_arm(args, cfg, rank, world, local_rank):
     call_pageable()
     barrier()
     t0 = time.perf_counter()
-    pg_steps = min(args.steps, 3)
+    pg_steps = args.steps
     for _ in range(pg_steps):
         call_pageable()
     barrier()
@@ -537,7 +566,15 @@ def main():
     ap.add_argument("--items", type=int, default=0, help="items (default: the configuration's n)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--zero-users", type=float, default=0.0, help="fraction of users whose factors are set to zero (robustness line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the metric rows of the last timed step as DIR/<metric>.npy (the defined values) and "
+                         "DIR/<metric>_defined.npy (1 where defined, 0 where NaN); at most 64 MB in all: larger outputs "
+                         "as a fixed seeded sample of users")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what this repository's CUDA path computed (--impl b200)")
 
     cfg = synth.CONFIGS[args.config]
     args.users = args.users or cfg.m

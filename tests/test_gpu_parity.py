@@ -507,14 +507,13 @@ print("AFTER", int(np.isfinite(r.metrics["ROC_AUC"][:2000]).sum() > 0))
 """
 
 
-def test_sigint_stops_the_call_between_user_batches(scoring_path):
+def test_sigint_stops_the_call_between_user_batches():
     """Ctrl-C (reference: SignalSwitcher, src/recometrics.hpp:114-174 -- drain the loop, restore the handler, re-raise, throw):
     a SIGINT sent while calls are running ends them within a batch or two with KeyboardInterrupt / "procedure was
-    interrupted", the previous handler is back in place, and the library keeps working."""
+    interrupted", the previous handler is back in place, and the library keeps working.  The probe process inherits
+    RMB200_PATH from the scoring_path fixture: it runs once with the library's choice and once with RMB200_PATH=fma."""
     import subprocess
     import sys
-    if scoring_path != "auto":
-        pytest.skip("one run is enough (the probe is a process of its own; rank counting runs the FMA tiles either way)")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     run = subprocess.run([sys.executable, "-c", _SIGINT_PROBE, root], capture_output=True, text=True, timeout=600)
     assert run.returncode == 0, run.stdout + run.stderr
