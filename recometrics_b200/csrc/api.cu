@@ -157,6 +157,8 @@ struct DevBuf {
         }                                                                                \
     } while (0)
 
+#define TRY(expr) do { const int rc_ = (expr); if (rc_ != RMB200_OK) return rc_; } while (0)   // int return codes
+
 inline int round_up(int x, int q) { return (x + q - 1) / q * q; }
 
 struct PhaseTimer {
@@ -599,250 +601,315 @@ struct ResultStream {
     }
 };
 
-template <typename T>
-int stage_rows(const T* src, size_t ld, int rows, int cols, bool on_dev, DevBuf& staging,
-               const T** dev_src, size_t* dev_ld, cudaStream_t st, rmb200_timing_t& tm)
+inline const rmb200_extra_t* ex_or_default(const rmb200_extra_t* ex)
 {
-    if (on_dev) { *dev_src = src; *dev_ld = ld; return RMB200_OK; }
-    CK(upload_rows(staging.p, src, ld * sizeof(T), (size_t)cols * sizeof(T), (size_t)rows, st));
-    tm.h2d_bytes += (int64_t)rows * cols * (int64_t)sizeof(T);
-    *dev_src = staging.as<T>();
-    *dev_ld = (size_t)cols;
+    static const rmb200_extra_t dflt = []() {
+        rmb200_extra_t e;
+        std::memset(&e, 0, sizeof(e));
+        e.struct_size = (int32_t)sizeof(e);
+        e.device = -1;
+        return e;
+    }();
+    return ex ? ex : &dflt;
+}
+
+// The users [*ub, *ue) of a call: rmb200_extra_t::user_begin / user_end; 0, 0 = all m users, user_end < 0 = none.
+int user_range(const rmb200_extra_t* ex, int m, int* ub, int* ue)
+{
+    *ub = 0; *ue = ex->user_end < 0 ? 0 : m;                             // user_end < 0: explicit empty block
+    if (ex->user_end >= 0 && (ex->user_begin != 0 || ex->user_end != 0)) { *ub = ex->user_begin; *ue = ex->user_end; }
+    if (*ub < 0 || *ue > m || *ub > *ue) { set_err("bad argument", "user range outside [0, m]"); return RMB200_ERR_BAD_ARG; }
     return RMB200_OK;
 }
 
-template <typename T>
-int run_call(const CallArgs<T>& a)
+#ifndef RMB_F_CMID
+#define RMB_F_CMID 512              // candidate buffer of the tensor path for 32 < k_metrics <= 128
+#endif
+
+// per-batch counters of a -DRMB_F_STATS=1 build's filter (filter_select.cuh); nothing in a production build
+void print_filter_stats(const int* over_retry, int nb, int nb_pad, int sample_tiles, int sample_stride, int sample_rank)
 {
-    using namespace rmb;
-    const auto t_begin = std::chrono::steady_clock::now();
-    const rmb200_extra_t* ex = a.ex;
-    const bool on_dev = ex && ex->inputs_on_device;
+#if RMB_F_STATS
+    std::fprintf(stderr, "[rmb200 stats] users %d: appends/user %.1f cuts/user %.2f slow-path entries/user %.1f cursor moves/user %.1f retries %d handed back %d (sample tiles %d stride %d rank %d)\n",
+                 nb, over_retry[2] / (double)nb, over_retry[3] / (double)nb, over_retry[4] / (double)nb, over_retry[5] / (double)nb,
+                 over_retry[1], over_retry[0], sample_tiles, sample_stride, sample_rank);
+    const unsigned long long* ck = reinterpret_cast<const unsigned long long*>(over_retry + 8);
+    const double nc = (double)(nb_pad / rmb::BM);
+    for (int ps = 0; ps < 2; ps++)
+        std::fprintf(stderr, "[rmb200 stats]   pass %d, one epilogue warp, kcycles per CTA: wait acc %.0f, ld+fast %.0f, append %.0f, cursor %.0f, meet+cut %.0f, total %.0f\n",
+                     ps, ck[ps * 6 + 0] / nc / 1e3, ck[ps * 6 + 1] / nc / 1e3, ck[ps * 6 + 2] / nc / 1e3, ck[ps * 6 + 3] / nc / 1e3, ck[ps * 6 + 4] / nc / 1e3, ck[ps * 6 + 5] / nc / 1e3);
+#endif
+}
+
+// One evaluation call on one device.  plan() makes every decision that needs only the arguments and the device; the resident
+// steps (csr_slices .. batch_buffers) put on the device what every batch reads; run_batch() evaluates one batch of UB users.
+// All of it runs on the legacy default stream `st`, but the uploads of host inputs (PrefetchStream) and result copies (ResultStream).
+template <typename T>
+struct Call {
+    static constexpr int BN = rmb::NumTraits<T>::BN;
+    struct Batch {   // users [b0, b0 + nb) of the call; slot: staging buffer of their factors (host inputs) and result set (host outputs)
+        int b0, nb, nb_pad, slot; bool prefetched = false;
+        const T* Asrc = nullptr; size_t Ald = 0;     // the batch's user factors, row-major on the device
+    };
+    const CallArgs<T>& a;
+    const rmb200_extra_t* ex;
+    const bool on_dev, nested;                  // nested: one device's share of a multi-GPU call (run_multi)
+    const int dev, ub, mr, K;                   // mr users from ub ("shard"); device-side rows are shard-local
+    cudaStream_t st = nullptr;                  // legacy default stream: ordered after the caller's default-stream work
+    PhaseTimer pt{st}, pk{st};                  // phases; the dominant scoring kernel alone
     rmb200_timing_t tm;
-    std::memset(&tm, 0, sizeof(tm));
-
-    // ---- argument checks (shape errors are the binding's job in the reference,
-    //      recometrics/wrapper.pyx:261-268; here they become RMB200_ERR_BAD_ARG) ----
-    if (a.m <= 0 || a.n <= 0 || a.k <= 0 || a.K <= 0) { set_err("bad argument", "m, n, k and k_metrics must be positive"); return RMB200_ERR_BAD_ARG; }
-    if (!a.A || !a.B || !a.trp || !a.tep) { set_err("bad argument", "A, B, Xtrain_csr_p and Xtest_csr_p are required"); return RMB200_ERR_BAD_ARG; }
-    if (a.lda < (size_t)a.k || a.ldb < (size_t)a.k) { set_err("bad argument", "lda/ldb smaller than k"); return RMB200_ERR_BAD_ARG; }
-    if (a.out[5] && !a.tev) { set_err("bad argument", "NDCG requested but Xtest_csr (values) is NULL"); return RMB200_ERR_BAD_ARG; }
-    if (ex && ex->struct_size != (int32_t)sizeof(rmb200_extra_t)) { set_err("bad argument", "rmb200_extra_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
-    bool any_out = false;
-    for (int q = 0; q < 10; q++) any_out |= (a.out[q] != nullptr);
-    const bool want_means = ex && (ex->metric_means || ex->metric_counts);
-    const bool want_extras = ex && (ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status);
-    const bool want_filter_stats = (ex && ex->filter_stats) || std::getenv("RMB200_FILTER_STATS") != nullptr;
-    if (!any_out && !want_extras && !want_means) return RMB200_OK;
-
-    int ub = 0, ue = a.m;
-    if (ex && ex->user_end < 0) return RMB200_OK;                        // explicit empty block
-    if (ex && (ex->user_begin != 0 || ex->user_end != 0)) { ub = ex->user_begin; ue = ex->user_end; }
-    if (ub < 0 || ue > a.m || ub > ue) { set_err("bad argument", "user range outside [0, m]"); return RMB200_ERR_BAD_ARG; }
-    const int mr = ue - ub;   // users of this call ("shard"); device-side rows are shard-local
-    if (mr == 0) return RMB200_OK;
-
-    // ---- device ----
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        set_err("no CUDA device", "librecometrics_b200 has no CPU fallback");
-        return RMB200_ERR_NO_DEVICE;
-    }
-    int dev = -1;
-    if (ex && ex->device >= 0) dev = ex->device;
-    else if (const char* env = std::getenv("RMB200_DEVICE")) dev = std::atoi(env);
-    if (dev < 0) CK(cudaGetDevice(&dev));
-    if (dev >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
-    CK(cudaSetDevice(dev));
-
-    const bool nested = a.mc != nullptr;                   // one device's share of a multi-GPU call: run_multi() holds the mutex and the latch
-    std::unique_lock<std::mutex> lock(g_call_mutex, std::defer_lock);
-    if (!nested) lock.lock();
-    SignalLatch latch(!nested);
-    cudaStream_t st = nullptr;   // legacy default stream: ordered after the caller's default-stream work
-    PhaseTimer pt(st), pk(st);   // phases; the dominant scoring kernel alone
-
-    // hpp:391-393
-    int mip = a.min_items_pool < a.K ? a.K : a.min_items_pool;
-    if (mip < 2) mip = 2;
-    int mpt = a.min_pos_test;
-    if (!(ex && ex->strict_min_pos_test)) mpt = mpt < 1 ? mpt : 1;   // std::min(min_pos_test, 1): quirk Q1
-
-    // what a "NaN" written into the outputs looks like: a quiet NaN, or the caller's bit pattern (R: NA_REAL, hpp:75-80)
+    // ---- the plan ----
+    int mip = 0, mpt = 0, C = 0, p_pad = 0, n_pad = 0, n_pad128 = 0, KB = 0, f_stages = 0, nsm = 148, UB = 0, fma_slices = 1, mean_W = 1;
+    size_t rs = 1;
     T nan_value = std::numeric_limits<T>::quiet_NaN();
-    if (ex && ex->has_nan_bits) {
-        if (sizeof(T) == 8) { const uint64_t b = ex->nan_bits; std::memcpy(&nan_value, &b, 8); }
-        else { const uint32_t b = (uint32_t)ex->nan_bits; std::memcpy(&nan_value, &b, 4); }
-        if (nan_value == nan_value) { set_err("bad argument", "rmb200_extra_t::nan_bits is not a NaN"); return RMB200_ERR_BAD_ARG; }
-    }
-
-    const int K = a.K;
-    // candidate buffer: K kept + 128 appended per tile + head-room between two cuts (the tensor-core filter keeps
-    // the slack band below the K-th best as well: about 2.5 K entries on Gaussian scores, so it gets more room)
-    int C = (K <= 64) ? 256 : (K <= 192 ? 512 : 1024);
-    const bool want_roc = a.out[8] != nullptr, want_pr = a.out[9] != nullptr;
-    const bool count_ranks = want_roc || want_pr || (ex && ex->pos_rank);
-    const int p_pad = round_up(a.k, KPAD);
-    constexpr int BN = NumTraits<T>::BN;
-    const int n_pad = round_up(a.n, BN);
-    const size_t rs = a.cumulative ? (size_t)K : 1;
-
-    // ---- which scoring path: tensor-core filter + exact re-scoring (top-K only), or FMA tiles ----
-    int path_req = ex ? ex->scoring_path : 0;                       // 0 auto, 1 fma, 2 tensor
-    if (path_req == 0) if (const char* env = std::getenv("RMB200_PATH")) {
-        if (!std::strcmp(env, "fma")) path_req = 1; else if (!std::strcmp(env, "tensor")) path_req = 2; else if (!std::strcmp(env, "full")) path_req = 3;
-    }
-    // k_metrics beyond what the selection kernels' candidate buffers hold: the full-order path (full_order.cu)
-    bool use_full = path_req == 3 || K > RMB200_MAX_K;
-    if (use_full && ex && (ex->scoring_path == 1 || ex->scoring_path == 2)) { set_err("unsupported", "scoring_path fma / tensor need k_metrics <= RMB200_MAX_K (384)"); return RMB200_ERR_UNSUPPORTED; }
-    if (use_full) path_req = 3;                                      // (an RMB200_PATH preference does not apply)
-    const int KB = round_up(a.k + (a.bias ? 1 : 0), 16);            // fp16 factors per row (bias = one more factor)
-    int f_stages = 0;
+    bool want_roc = false, want_pr = false, count_ranks = false, want_means = false, want_filter_stats = false;
+    bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
+    int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
+    int fo_chunk = 0; size_t fo_bytes = 0;
+    int auc_dbg = 0, filter_dbg = 0;            // developer: RMB200_AUC_DBG / RMB200_DBG timing experiments (wrong results)
+    // ---- resident state ----
+    int lo_hi[4] = {0, 0, 0, 0};                // trp[ub], trp[ue], tep[ub], tep[ue]
+    size_t nnz_tr = 0, nnz_te = 0;
+    const int *trp_d = nullptr, *tep_d = nullptr, *tri_d = nullptr, *tei_d = nullptr;
+    const T *tev_d = nullptr, *bias_d = nullptr, *Bsrc = nullptr; size_t Bld = 0;    // Bsrc: item factors, row-major on the device
+    long long* pos_rank_d = nullptr;
+    bool have_Bt = false; int mean_block0 = 0;
+    DevBuf d_trp, d_tri, d_tep, d_tei, d_tev, d_Arow[2];
+    DevBuf d_Bt, d_bias, d_Brow, d_Bb, d_maxbn, d_chunkn;
+    DevBuf d_status, d_flags, d_umin, d_pos_raw, d_pos_sorted, d_pos_perm, d_pos_item, d_auc, d_log2, d_pos_rank;
+    DevBuf d_fo, d_near, d_nz_mark, d_nz_list, d_nz_cnt, d_At_nz;
+    DevBuf d_At, d_cs, d_ci, d_cc, d_out[2][10], d_tki[2], d_tks[2], d_stat_out[2], d_Ab, d_anorm;
+    DevBuf d_capx, d_overflow, d_fb_list, d_At_fb;
+    DevBuf d_psum, d_pcnt, d_means, d_mcounts;
+    PrefetchStream pf;                          // (declared after the buffers they fill or read: destroyed, i.e. drained, before them)
+    ResultStream rsx;
+    Call(const CallArgs<T>& args, int device, int user_begin, int users) : a(args), ex(args.ex), on_dev(args.ex->inputs_on_device != 0),
+        nested(args.mc != nullptr), dev(device), ub(user_begin), mr(users), K(args.K) { std::memset(&tm, 0, sizeof(tm)); }
+    int plan()
     {
+        using namespace rmb;
+        // hpp:391-393
+        mip = a.min_items_pool < K ? K : a.min_items_pool;
+        if (mip < 2) mip = 2;
+        mpt = a.min_pos_test;
+        if (!ex->strict_min_pos_test) mpt = mpt < 1 ? mpt : 1;   // std::min(min_pos_test, 1): quirk Q1
+        // what a "NaN" written into the outputs looks like: a quiet NaN, or the caller's bit pattern (R: NA_REAL, hpp:75-80)
+        if (ex->has_nan_bits) {
+            if (sizeof(T) == 8) { const uint64_t b = ex->nan_bits; std::memcpy(&nan_value, &b, 8); }
+            else { const uint32_t b = (uint32_t)ex->nan_bits; std::memcpy(&nan_value, &b, 4); }
+            if (nan_value == nan_value) { set_err("bad argument", "rmb200_extra_t::nan_bits is not a NaN"); return RMB200_ERR_BAD_ARG; }
+        }
+        // candidate buffer: K kept + 128 appended per tile + head-room between two cuts (the tensor-core filter keeps
+        // the slack band below the K-th best as well: about 2.5 K entries on Gaussian scores, so it gets more room)
+        C = (K <= 64) ? 256 : (K <= 192 ? 512 : 1024);
+        want_roc = a.out[8] != nullptr; want_pr = a.out[9] != nullptr;
+        count_ranks = want_roc || want_pr || ex->pos_rank;
+        want_means = ex->metric_means || ex->metric_counts;
+        want_filter_stats = ex->filter_stats || std::getenv("RMB200_FILTER_STATS") != nullptr;
+        p_pad = round_up(a.k, KPAD);
+        n_pad = round_up(a.n, BN);
+        rs = a.cumulative ? (size_t)K : 1;
+        mean_W = a.cumulative ? K : 1;
+        if (const char* env = std::getenv("RMB200_AUC_DBG")) auc_dbg = std::atoi(env);
+        if (const char* env = std::getenv("RMB200_DBG")) filter_dbg = std::atoi(env);
+        // ---- which scoring path: tensor-core filter + exact re-scoring (top-K only), or FMA tiles ----
+        int path_req = ex->scoring_path;                                 // 0 auto, 1 fma, 2 tensor
+        if (path_req == 0) if (const char* env = std::getenv("RMB200_PATH")) {
+            if (!std::strcmp(env, "fma")) path_req = 1; else if (!std::strcmp(env, "tensor")) path_req = 2; else if (!std::strcmp(env, "full")) path_req = 3;
+        }
+        // k_metrics beyond what the selection kernels' candidate buffers hold: the full-order path (full_order.cu)
+        use_full = path_req == 3 || K > RMB200_MAX_K;
+        if (use_full && (ex->scoring_path == 1 || ex->scoring_path == 2)) { set_err("unsupported", "scoring_path fma / tensor need k_metrics <= RMB200_MAX_K (384)"); return RMB200_ERR_UNSUPPORTED; }
+        if (use_full) path_req = 3;                                      // (an RMB200_PATH preference does not apply)
+        KB = round_up(a.k + (a.bias ? 1 : 0), 16);                       // fp16 factors per row (bias = one more factor)
         // A tile + ring stages + barriers + row state within the 227 KB a CTA can have
         const long long tile = (long long)KB * 256, budget = 227 * 1024 - (long long)filter_smem_fixed_bytes();
         f_stages = (int)(budget / tile) - 1;
         if (f_stages > F_MAX_STAGES) f_stages = F_MAX_STAGES;
         if (const char* env = std::getenv("RMB200_STAGES")) { const int v = std::atoi(env); if (v >= 2 && v < f_stages) f_stages = v; }   // developer: shallower ring
-    }
-    // With rank counting (ROC/PR-AUC) every score has to be exact: the FMA tiles do everything.  Exception: with the
-    // reference's tie-breaking noise the ranked top-K comes from the tensor path as well (its exact stage is where the
-    // noise is applied, tie_noise.cuh), after the FMA pass has counted the ranks.
-    const bool tensor_shape_ok = f_stages >= 2 && K <= 256 && !use_full;
-    const bool tensor_ok = tensor_shape_ok && (!count_ranks || a.noise);
-    if (path_req == 2 && !tensor_ok) { set_err("unsupported", "scoring_path=tensor needs no ROC/PR-AUC (rank counting), k <= ~400 and k_metrics <= 256"); return RMB200_ERR_UNSUPPORTED; }
-    const bool use_tensor = tensor_ok && path_req != 1;
-    // break_ties_with_noise (the reference's default) where the tensor path's exact stage cannot apply it -- shapes only the FMA
-    // tiles handle (k_metrics 257..384, more than ~400 factors) or an RMB200_PATH=fma preference: the full-order path, which
-    // adds every candidate's draw before sorting.  Only an explicit scoring_path = 1 keeps the FMA tiles (noise-free order).
-    if (a.noise && !use_tensor && !use_full && !(ex && ex->scoring_path == 1)) { use_full = true; path_req = 3; }
-    const bool fma_counts_first = use_tensor && count_ranks;
-    // ... and inside the rank counts (ROC/PR-AUC with the noise): the FMA tiles count on the noise-free scores and report, per
-    // held-out item, the candidates within the noise's reach; users for whom the noise decides a rank are handed to the full-order path
-    const bool noise_handback = a.noise && count_ranks && !use_full;
-    tm.scoring_path = use_full ? 3 : (use_tensor ? 2 : 1);
-#ifndef RMB_F_CMID
-#define RMB_F_CMID 512
-#endif
-    if (use_tensor) C = (K <= 32) ? 256 : (K <= 128 ? RMB_F_CMID : 1024);
-    if (use_tensor) if (const char* env = std::getenv("RMB200_FILTER_C")) { const int v = std::atoi(env); if ((v == 256 || v == 512 || v == 1024) && v >= C) C = v; }   // developer
-    if (use_full) C = round_up(K < a.n ? K : a.n, 32);              // row pitch of the ranked lists
-
-    // ---- CSR slices of users [ub, ue), index pointers re-based to the slice ----
-    int lo_hi[4];   // trp[ub], trp[ue], tep[ub], tep[ue]
-    if (!on_dev) {
-        lo_hi[0] = a.trp[ub]; lo_hi[1] = a.trp[ue]; lo_hi[2] = a.tep[ub]; lo_hi[3] = a.tep[ue];
-    } else {
-        CK(cudaMemcpy(&lo_hi[0], a.trp + ub, sizeof(int), cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(&lo_hi[1], a.trp + ue, sizeof(int), cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(&lo_hi[2], a.tep + ub, sizeof(int), cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(&lo_hi[3], a.tep + ue, sizeof(int), cudaMemcpyDeviceToHost));
-    }
-    if (lo_hi[1] < lo_hi[0] || lo_hi[3] < lo_hi[2]) { set_err("bad argument", "CSR index pointers decrease"); return RMB200_ERR_BAD_ARG; }
-    const size_t nnz_tr = (size_t)(lo_hi[1] - lo_hi[0]);
-    const size_t nnz_te = (size_t)(lo_hi[3] - lo_hi[2]);
-    if ((nnz_tr && !a.tri) || (nnz_te && !a.tei)) { set_err("bad argument", "CSR indices missing"); return RMB200_ERR_BAD_ARG; }
-
-    DevBuf d_trp, d_tri, d_tep, d_tei, d_tev, d_Arow[2];
-    PrefetchStream pf;                                     // (declared after the buffers it fills: destroyed, i.e. drained, before them)
-    if (!on_dev) CK(pf.init());
-    CK(d_trp.alloc((size_t)(mr + 1) * sizeof(int)));
-    CK(d_tep.alloc((size_t)(mr + 1) * sizeof(int)));
-    const int* tri_d = nullptr; const int* tei_d = nullptr; const T* tev_d = nullptr;
-    pt.start();
-    if (!on_dev) {
-        std::vector<int> tmp1((size_t)mr + 1), tmp2((size_t)mr + 1);
-        for (int i = 0; i <= mr; i++) { tmp1[i] = a.trp[ub + i] - lo_hi[0]; tmp2[i] = a.tep[ub + i] - lo_hi[2]; }
-        CK(cudaMemcpyAsync(d_trp.p, tmp1.data(), tmp1.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(d_tep.p, tmp2.data(), tmp2.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-        CK(d_tri.alloc(nnz_tr * sizeof(int)));
-        CK(d_tei.alloc(nnz_te * sizeof(int)));
-        if (nnz_tr) CK(upload_rows(d_tri.p, a.tri + lo_hi[0], nnz_tr * sizeof(int), nnz_tr * sizeof(int), 1, st));
-        // the held-out rows are not needed before the first batch's metrics (rank counting: its first scoring step): they
-        // go up on the prefetch stream, behind the item factors on the link instead of in front of them
-        if (nnz_te) CK(upload_rows(d_tei.p, a.tei + lo_hi[2], nnz_te * sizeof(int), nnz_te * sizeof(int), 1, pf.s));
-        if (a.tev) {
-            CK(d_tev.alloc(nnz_te * sizeof(T)));
-            if (nnz_te) CK(upload_rows(d_tev.p, a.tev + lo_hi[2], nnz_te * sizeof(T), nnz_te * sizeof(T), 1, pf.s));
-            tev_d = d_tev.as<T>();
+        // With rank counting (ROC/PR-AUC) every score has to be exact: the FMA tiles do everything.  Exception: with the
+        // reference's tie-breaking noise the ranked top-K comes from the tensor path as well (its exact stage is where the
+        // noise is applied, tie_noise.cuh), after the FMA pass has counted the ranks.
+        const bool tensor_shape_ok = f_stages >= 2 && K <= 256 && !use_full;
+        const bool tensor_ok = tensor_shape_ok && (!count_ranks || a.noise);
+        if (path_req == 2 && !tensor_ok) { set_err("unsupported", "scoring_path=tensor needs no ROC/PR-AUC (rank counting), k <= ~400 and k_metrics <= 256"); return RMB200_ERR_UNSUPPORTED; }
+        use_tensor = tensor_ok && path_req != 1;
+        // break_ties_with_noise (the reference's default) where the tensor path's exact stage cannot apply it -- shapes only the FMA
+        // tiles handle (k_metrics 257..384, more than ~400 factors) or an RMB200_PATH=fma preference: the full-order path, which
+        // adds every candidate's draw before sorting.  Only an explicit scoring_path = 1 keeps the FMA tiles (noise-free order).
+        if (a.noise && !use_tensor && !use_full && ex->scoring_path != 1) use_full = true;
+        fma_counts_first = use_tensor && count_ranks;
+        // ... and inside the rank counts (ROC/PR-AUC with the noise): the FMA tiles count on the noise-free scores and report, per
+        // held-out item, the candidates within the noise's reach; users for whom the noise decides a rank are handed to the full-order path
+        noise_handback = a.noise && count_ranks && !use_full;
+        tm.scoring_path = use_full ? 3 : (use_tensor ? 2 : 1);
+        if (use_tensor) C = (K <= 32) ? 256 : (K <= 128 ? RMB_F_CMID : 1024);
+        if (use_tensor) if (const char* env = std::getenv("RMB200_FILTER_C")) { const int v = std::atoi(env); if ((v == 256 || v == 512 || v == 1024) && v >= C) C = v; }   // developer
+        if (use_full) C = round_up(K < a.n ? K : a.n, 32);              // row pitch of the ranked lists
+        n_pad128 = round_up(a.n, 128);
+        // ---- user batches ----
+        cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+        const int wave_users = nsm * BM;                       // one CTA (128 users) per SM
+        UB = 8 * wave_users;                                   // users per batch: 8 full waves ...
+        // ... 4 when the filter's item image is much larger than the L2 (256 MB at 1M items x 128 factors): the CTAs of a longer
+        // launch drift further apart and re-stream the item tiles from HBM (cfg4: 3.16 M users/s at 4 waves, 3.10 at 8, 2.96 at
+        // 16, 2.76 with all 1M users in one launch; smaller catalogues prefer 8; profiles/r02_batch_size.txt)
+        if (use_tensor && (size_t)n_pad128 * KB * sizeof(__half) > (size_t)160 << 20) UB = 4 * wave_users;
+        if (const char* env = std::getenv("RMB200_BATCH_USERS")) { const int v = std::atoi(env); if (v > 0) UB = round_up(v, BM); }
+        if (use_full) {
+            // ranked lists (K entries per user) and cumulative rows (K columns per metric) of a batch within ~2 GB
+            const long long per_user = (long long)C * (long long)(sizeof(T) + 4) + (a.cumulative ? 8ll * K * (long long)sizeof(T) : 0);
+            long long cap = (2ll << 30) / (per_user > 0 ? per_user : 1);
+            cap = cap / BM * BM;
+            if (cap < BM) cap = BM;
+            if (UB > cap) UB = (int)cap;
         }
-        CK(cudaEventRecord(pf.test_rows, pf.s));
-        pf.test_rows_pending = true;
-        CK(cudaStreamSynchronize(st));   // tmp1/tmp2 go out of scope
-        tri_d = d_tri.as<int>(); tei_d = d_tei.as<int>();
-        tm.h2d_bytes += (int64_t)(2 * (size_t)(mr + 1) * sizeof(int) + (nnz_tr + nnz_te) * sizeof(int) + (a.tev ? nnz_te * sizeof(T) : 0));
-        pt.stop(tm.h2d_ms);
-    } else {
-        rebase_indptr_kernel<<<(mr + 1 + 255) / 256, 256, 0, st>>>(a.trp + ub, lo_hi[0], d_trp.as<int>(), mr + 1);
-        rebase_indptr_kernel<<<(mr + 1 + 255) / 256, 256, 0, st>>>(a.tep + ub, lo_hi[2], d_tep.as<int>(), mr + 1);
-        CK(cudaGetLastError());
-        tm.kernel_launches += 2;
-        tri_d = a.tri ? a.tri + lo_hi[0] : nullptr;
-        tei_d = a.tei ? a.tei + lo_hi[2] : nullptr;
-        tev_d = a.tev ? a.tev + lo_hi[2] : nullptr;
-        pt.stop(tm.prep_ms);
-    }
-    const int* trp_d = d_trp.as<int>();
-    const int* tep_d = d_tep.as<int>();
-
-    // ---- item factors: row-major staging copy, then the operand image of the chosen path ----
-    DevBuf d_Bt, d_bias, d_Brow, d_Bb, d_maxbn, d_chunkn;
-    const T* Bsrc = nullptr; size_t Bld = 0;
-    if (!on_dev) {
-        CK(d_Brow.alloc((size_t)a.n * a.k * sizeof(T)));
-        pt.start();
-        if (!nested) {
-            int rc = stage_rows<T>(a.B, a.ldb, a.n, a.k, false, d_Brow, &Bsrc, &Bld, st, tm);
-            if (rc) return rc;
-        } else {
-            // this device's slice of the rows from the host, the other slices from the peers' copies (see MultiCtx)
-            MultiCtx& mc = *a.mc;
-            const int G = mc.G, g = a.mc_rank;
-            auto slice = [&](int h) { return (long long)a.n * h / G; };
-            const size_t row_bytes = (size_t)a.k * sizeof(T);
-            unsigned char* base = static_cast<unsigned char*>(d_Brow.p);
-            if (slice(g + 1) > slice(g))
-                CK(upload_rows(base + (size_t)slice(g) * row_bytes, a.B + (size_t)slice(g) * a.ldb, a.ldb * sizeof(T), row_bytes,
-                               (size_t)(slice(g + 1) - slice(g)), st));
-            tm.h2d_bytes += (int64_t)(slice(g + 1) - slice(g)) * (int64_t)row_bytes;
-            CK(cudaStreamSynchronize(st));
-            mc.Bptr[g] = d_Brow.p; mc.Bdev[g] = dev;
-            if (!mc.meet(0)) { set_err("multi-GPU call", "another device failed"); return RMB200_ERR_CUDA; }
-            for (int h = 1; h < G; h++) {
-                const int src = (g + h) % G;
-                const size_t off = (size_t)slice(src) * row_bytes, bytes = (size_t)(slice(src + 1) - slice(src)) * row_bytes;
-                if (bytes) CK(cudaMemcpyPeerAsync(base + off, dev, static_cast<unsigned char*>(mc.Bptr[src]) + off, mc.Bdev[src], bytes, st));
+        if (UB > round_up(mr, BM)) UB = round_up(mr, BM);
+        if (use_full) full_order_plan(a.n, (int)sizeof(T), UB, &fo_chunk, &fo_bytes);
+        // sampled threshold guess of the filter (filter_select.cuh, pass 0): every stride-th item tile, about 7/K of the
+        // catalogue (1/16 .. 1/8); the guess is the r-th best of the sample with r = the smallest rank for which
+        // P(Poisson(K * sample / n) >= r) <= 1e-6, i.e. fewer than K items of the whole catalogue reach it about once
+        // in a million users (those users' CTAs walk the catalogue a second time; results never depend on the guess)
+        if (use_tensor) {
+            const int NT = (a.n + 127) / 128;
+            int min_tiles = 512;
+            if (const char* env = std::getenv("RMB200_SAMPLE_MIN_TILES")) { const int v = std::atoi(env); if (v >= 16) min_tiles = v; }   // developer
+            bool on = NT >= min_tiles;
+            if (const char* env = std::getenv("RMB200_SAMPLE")) on = on && std::atoi(env) != 0;
+            if (on) {
+                double frac = 7.0 / K;
+                if (frac < 1.0 / 16) frac = 1.0 / 16;
+                if (frac > 1.0 / 8) frac = 1.0 / 8;
+                int stride = (int)(1.0 / frac);
+                if (const char* env = std::getenv("RMB200_SAMPLE_STRIDE")) { const int v = std::atoi(env); if (v >= 2) stride = v; }
+                const int ns = NT / stride;                                  // tiles 0, stride, ..., (ns-1)*stride: all full tiles
+                const double lam = (double)K * ((double)ns * 128.0) / (double)a.n;
+                double term = std::exp(-lam), cdf = 0.0;                     // P(X <= r-1), X ~ Poisson(lam)
+                int r = 0;
+                while (r < 4096) { cdf += term; r++; term *= lam / r; if (1.0 - cdf <= 1e-6) break; }
+                if (const char* env = std::getenv("RMB200_SAMPLE_RANK")) { const int v = std::atoi(env); if (v >= 1) r = v; }
+                // (the guess is the r-th largest of up to min(C / 4, 128) group maxima of the sample, filter_select.cuh)
+                const int groups = (C / 4 < 128 ? C / 4 : 128) < ns ? (C / 4 < 128 ? C / 4 : 128) : ns;
+                if (ns >= 8 && 2 * r <= groups) { f_sample_tiles = ns; f_sample_stride = stride; f_sample_rank = r; }
             }
-            CK(cudaStreamSynchronize(st));
-            if (!mc.meet(1)) { set_err("multi-GPU call", "another device failed"); return RMB200_ERR_CUDA; }   // nobody frees its copy before everybody has fetched
-            Bsrc = d_Brow.as<T>(); Bld = (size_t)a.k;
         }
-        pt.stop(tm.h2d_ms);
-    } else { Bsrc = a.B; Bld = a.ldb; }
-    bool have_Bt = false;
-    auto pack_Bt = [&]() -> int {          // operand image of the FMA path (the tensor path needs it only as a fall-back)
+        // A call with fewer user tiles than SMs (small m) cuts the catalogue into item ranges on the FMA tiles: one CTA per (user tile,
+        // range), every range keeping its own best K, joined afterwards (merge_slices_kernel); rank counts are added atomically.
+        if (!use_full) {
+            const int tiles = UB / BM, NT_all = (a.n + BN - 1) / BN;
+            int sl = tiles > 0 ? nsm / tiles : 1;
+            if (sl > NT_all / 8) sl = NT_all / 8;                       // (at least eight item tiles per range)
+            if (sl > C / K) sl = C / K;                                 // the joined heads fit one row ...
+            if (sl > 512 / K) sl = 512 / K;                             // ... and the final sort
+            if (const char* env = std::getenv("RMB200_SLICES")) { const int v = std::atoi(env); if (v >= 1 && v < sl) sl = v; }      // developer
+            if (sl > 1) fma_slices = sl;
+        }
+        return RMB200_OK;
+    }
+    // CSR slices of users [ub, ue), index pointers re-based to the slice
+    int csr_slices()
+    {
+        const int* ends[4] = {a.trp + ub, a.trp + ub + mr, a.tep + ub, a.tep + ub + mr};
+        for (int i = 0; i < 4; i++)
+            if (on_dev) CK(cudaMemcpy(&lo_hi[i], ends[i], sizeof(int), cudaMemcpyDeviceToHost)); else lo_hi[i] = *ends[i];
+        if (lo_hi[1] < lo_hi[0] || lo_hi[3] < lo_hi[2]) { set_err("bad argument", "CSR index pointers decrease"); return RMB200_ERR_BAD_ARG; }
+        nnz_tr = (size_t)(lo_hi[1] - lo_hi[0]);
+        nnz_te = (size_t)(lo_hi[3] - lo_hi[2]);
+        if ((nnz_tr && !a.tri) || (nnz_te && !a.tei)) { set_err("bad argument", "CSR indices missing"); return RMB200_ERR_BAD_ARG; }
+        if (!on_dev) CK(pf.init());
+        CK(d_trp.alloc((size_t)(mr + 1) * sizeof(int)));
+        CK(d_tep.alloc((size_t)(mr + 1) * sizeof(int)));
+        pt.start();
+        if (!on_dev) {
+            std::vector<int> tmp1((size_t)mr + 1), tmp2((size_t)mr + 1);
+            for (int i = 0; i <= mr; i++) { tmp1[i] = a.trp[ub + i] - lo_hi[0]; tmp2[i] = a.tep[ub + i] - lo_hi[2]; }
+            CK(cudaMemcpyAsync(d_trp.p, tmp1.data(), tmp1.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(d_tep.p, tmp2.data(), tmp2.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+            CK(d_tri.alloc(nnz_tr * sizeof(int)));
+            CK(d_tei.alloc(nnz_te * sizeof(int)));
+            if (nnz_tr) CK(upload_rows(d_tri.p, a.tri + lo_hi[0], nnz_tr * sizeof(int), nnz_tr * sizeof(int), 1, st));
+            // the held-out rows are not needed before the first batch's metrics (rank counting: its first scoring step): they
+            // go up on the prefetch stream, behind the item factors on the link instead of in front of them
+            if (nnz_te) CK(upload_rows(d_tei.p, a.tei + lo_hi[2], nnz_te * sizeof(int), nnz_te * sizeof(int), 1, pf.s));
+            if (a.tev) {
+                CK(d_tev.alloc(nnz_te * sizeof(T)));
+                if (nnz_te) CK(upload_rows(d_tev.p, a.tev + lo_hi[2], nnz_te * sizeof(T), nnz_te * sizeof(T), 1, pf.s));
+                tev_d = d_tev.as<T>();
+            }
+            CK(cudaEventRecord(pf.test_rows, pf.s));
+            pf.test_rows_pending = true;
+            CK(cudaStreamSynchronize(st));   // tmp1/tmp2 go out of scope
+            tri_d = d_tri.as<int>(); tei_d = d_tei.as<int>();
+            tm.h2d_bytes += (int64_t)(2 * (size_t)(mr + 1) * sizeof(int) + (nnz_tr + nnz_te) * sizeof(int) + (a.tev ? nnz_te * sizeof(T) : 0));
+            pt.stop(tm.h2d_ms);
+        } else {
+            rebase_indptr_kernel<<<(mr + 1 + 255) / 256, 256, 0, st>>>(a.trp + ub, lo_hi[0], d_trp.as<int>(), mr + 1);
+            rebase_indptr_kernel<<<(mr + 1 + 255) / 256, 256, 0, st>>>(a.tep + ub, lo_hi[2], d_tep.as<int>(), mr + 1);
+            TRY(launched(2));
+            tri_d = a.tri ? a.tri + lo_hi[0] : nullptr;
+            tei_d = a.tei ? a.tei + lo_hi[2] : nullptr;
+            tev_d = a.tev ? a.tev + lo_hi[2] : nullptr;
+            pt.stop(tm.prep_ms);
+        }
+        trp_d = d_trp.as<int>(); tep_d = d_tep.as<int>();
+        return RMB200_OK;
+    }
+    // item factors: row-major on the device, then the operand image of the FMA path where it scores
+    int item_factors()
+    {
+        if (!on_dev) {
+            CK(d_Brow.alloc((size_t)a.n * a.k * sizeof(T)));
+            pt.start();
+            TRY(upload_item_rows());
+            pt.stop(tm.h2d_ms);
+            Bsrc = d_Brow.as<T>(); Bld = (size_t)a.k;
+        } else { Bsrc = a.B; Bld = a.ldb; }
+        if (!use_tensor || fma_counts_first) TRY(ensure_Bt());
+        if (!use_tensor) { d_Brow.release(); if (!on_dev) Bsrc = nullptr; }     // the FMA path reads only the tiled copy
+        return RMB200_OK;
+    }
+    long long item_slice(int h) const { return (long long)a.n * h / (nested ? a.mc->G : 1); }
+    // the host's item factors into d_Brow; one device of a multi-GPU call uploads its slice of the rows and fetches the other
+    // slices from the peers' copies (see MultiCtx)
+    int upload_item_rows()
+    {
+        const int g = a.mc_rank;
+        const size_t row_bytes = (size_t)a.k * sizeof(T);
+        unsigned char* base = static_cast<unsigned char*>(d_Brow.p);
+        if (item_slice(g + 1) > item_slice(g))
+            CK(upload_rows(base + (size_t)item_slice(g) * row_bytes, a.B + (size_t)item_slice(g) * a.ldb, a.ldb * sizeof(T), row_bytes,
+                           (size_t)(item_slice(g + 1) - item_slice(g)), st));
+        tm.h2d_bytes += (int64_t)(item_slice(g + 1) - item_slice(g)) * (int64_t)row_bytes;
+        if (!nested) return RMB200_OK;
+        MultiCtx& mc = *a.mc;
+        CK(cudaStreamSynchronize(st));
+        mc.Bptr[g] = d_Brow.p; mc.Bdev[g] = dev;
+        if (!mc.meet(0)) { set_err("multi-GPU call", "another device failed"); return RMB200_ERR_CUDA; }
+        for (int h = 1; h < mc.G; h++) {
+            const int src = (g + h) % mc.G;
+            const size_t off = (size_t)item_slice(src) * row_bytes, bytes = (size_t)(item_slice(src + 1) - item_slice(src)) * row_bytes;
+            if (bytes) CK(cudaMemcpyPeerAsync(base + off, dev, static_cast<unsigned char*>(mc.Bptr[src]) + off, mc.Bdev[src], bytes, st));
+        }
+        CK(cudaStreamSynchronize(st));
+        if (!mc.meet(1)) { set_err("multi-GPU call", "another device failed"); return RMB200_ERR_CUDA; }   // nobody frees its copy before everybody has fetched
+        return RMB200_OK;
+    }
+    // operand image of the FMA path (the tensor path needs it only for a hand-back)
+    int ensure_Bt()
+    {
         if (have_Bt) return RMB200_OK;
         CK(d_Bt.alloc((size_t)p_pad * n_pad * sizeof(T)));
         pt.start();
         dim3 grid(n_pad / 32, (p_pad + 31) / 32), block(32, 8);
-        pack_tiles_kernel<T, BN><<<grid, block, 0, st>>>(Bsrc, Bld, a.n, a.k, d_Bt.as<T>(), n_pad, p_pad);
-        CK(cudaGetLastError());
-        tm.kernel_launches++;
+        rmb::pack_tiles_kernel<T, BN><<<grid, block, 0, st>>>(Bsrc, Bld, a.n, a.k, d_Bt.as<T>(), n_pad, p_pad);
+        TRY(launched());
         pt.stop(tm.prep_ms);   // (synchronises)
         have_Bt = true;
         return RMB200_OK;
-    };
-    if (!use_tensor || fma_counts_first) {
-        int rc = pack_Bt();
-        if (rc) return rc;
-        if (!use_tensor) {
-            d_Brow.release();      // the FMA path reads only the tiled copy
-            if (!on_dev) Bsrc = nullptr;
-        }
     }
-    const T* bias_d = nullptr;
-    if (a.bias) {
+    int item_bias()
+    {
+        if (!a.bias) return RMB200_OK;
         CK(d_bias.alloc((size_t)n_pad * sizeof(T)));
         DevBuf d_braw;
         const T* bsrc = a.bias;
@@ -855,14 +922,17 @@ int run_call(const CallArgs<T>& a)
             bsrc = d_braw.as<T>();
         }
         pt.start();
-        pad_copy_kernel<T><<<(n_pad + 255) / 256, 256, 0, st>>>(bsrc, a.n, d_bias.as<T>(), n_pad);
-        CK(cudaGetLastError());
-        tm.kernel_launches++;
+        rmb::pad_copy_kernel<T><<<(n_pad + 255) / 256, 256, 0, st>>>(bsrc, a.n, d_bias.as<T>(), n_pad);
+        TRY(launched());
         pt.stop(tm.prep_ms);
         bias_d = d_bias.as<T>();
+        return RMB200_OK;
     }
-    const int n_pad128 = round_up(a.n, 128);
-    if (use_tensor) {
+    // the tensor path's fp16 item image and the norms its error bound uses
+    int item_image()
+    {
+        using namespace rmb;
+        if (!use_tensor) return RMB200_OK;
         CK(d_Bb.alloc((size_t)n_pad128 * KB * sizeof(__half)));
         CK(d_maxbn.alloc(4 * sizeof(unsigned)));                    // [0] max_j ||b_j||, [1] largest observed error / bound ratio (statistic)
         CK(d_chunkn.alloc((size_t)(n_pad128 / 32) * sizeof(float)));
@@ -875,41 +945,37 @@ int run_call(const CallArgs<T>& a)
         CK(cudaGetLastError());
         pack_f16_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(Bsrc, Bld, a.n, a.k, bias_d, 0, nullptr, d_maxbn.as<unsigned>(),
                                                                             d_Bb.as<__half>(), n_pad128, KB);
-        CK(cudaGetLastError());
-        tm.kernel_launches += 2;
+        TRY(launched(2));
         pt.stop(tm.prep_ms);
+        return RMB200_OK;
     }
-
-    // ---- per-user state ----
-    DevBuf d_status, d_flags, d_umin, d_pos_raw, d_pos_sorted, d_pos_perm, d_pos_item, d_auc, d_log2, d_pos_rank;
-    CK(d_status.alloc((size_t)mr * sizeof(int)));
-    CK(d_flags.alloc((size_t)mr * sizeof(int)));
-    if (count_ranks) {
-        CK(d_umin.alloc((size_t)mr * sizeof(unsigned long long)));
-        CK(d_pos_raw.alloc(nnz_te * sizeof(T)));
-        CK(d_pos_sorted.alloc(nnz_te * sizeof(T)));
-        CK(d_pos_perm.alloc(nnz_te * sizeof(int)));
-        CK(d_pos_item.alloc(nnz_te * sizeof(int)));
-        CK(d_auc.alloc(nnz_te * sizeof(unsigned int)));
-        CK(cudaMemsetAsync(d_auc.p, 0, nnz_te * sizeof(unsigned int) + (nnz_te ? 0 : 16), st));
-        CK(cudaMemsetAsync(d_pos_sorted.p, 0, nnz_te * sizeof(T) + (nnz_te ? 0 : 16), st));
-        CK(cudaMemsetAsync(d_pos_perm.p, 0, nnz_te * sizeof(int) + (nnz_te ? 0 : 16), st));
-        CK(cudaMemsetAsync(d_pos_item.p, 0, nnz_te * sizeof(int) + (nnz_te ? 0 : 16), st));
-    }
-    long long* pos_rank_d = nullptr;
-    if (ex && ex->pos_rank) {
-        if (on_dev) pos_rank_d = reinterpret_cast<long long*>(ex->pos_rank) + lo_hi[2];
-        else { CK(d_pos_rank.alloc(nnz_te * sizeof(long long))); pos_rank_d = d_pos_rank.as<long long>(); }
-        CK(cudaMemsetAsync(pos_rank_d, 0, nnz_te * sizeof(long long), st));
-    }
+    int user_state()
     {
+        using namespace rmb;
+        CK(d_status.alloc((size_t)mr * sizeof(int)));
+        CK(d_flags.alloc((size_t)mr * sizeof(int)));
+        if (count_ranks) {
+            CK(d_umin.alloc((size_t)mr * sizeof(unsigned long long)));
+            CK(d_pos_raw.alloc(nnz_te * sizeof(T)));
+            CK(d_pos_sorted.alloc(nnz_te * sizeof(T)));
+            CK(d_pos_perm.alloc(nnz_te * sizeof(int)));
+            CK(d_pos_item.alloc(nnz_te * sizeof(int)));
+            CK(d_auc.alloc(nnz_te * sizeof(unsigned int)));
+            CK(cudaMemsetAsync(d_auc.p, 0, nnz_te * sizeof(unsigned int) + (nnz_te ? 0 : 16), st));
+            CK(cudaMemsetAsync(d_pos_sorted.p, 0, nnz_te * sizeof(T) + (nnz_te ? 0 : 16), st));
+            CK(cudaMemsetAsync(d_pos_perm.p, 0, nnz_te * sizeof(int) + (nnz_te ? 0 : 16), st));
+            CK(cudaMemsetAsync(d_pos_item.p, 0, nnz_te * sizeof(int) + (nnz_te ? 0 : 16), st));
+        }
+        if (ex->pos_rank) {
+            if (on_dev) pos_rank_d = reinterpret_cast<long long*>(ex->pos_rank) + lo_hi[2];
+            else { CK(d_pos_rank.alloc(nnz_te * sizeof(long long))); pos_rank_d = d_pos_rank.as<long long>(); }
+            CK(cudaMemsetAsync(pos_rank_d, 0, nnz_te * sizeof(long long), st));
+        }
         std::vector<double> l2((size_t)K);
         for (int i = 0; i < K; i++) l2[i] = std::log2((double)(i + 2));   // hpp:620 std::log2(ix+2)
         CK(d_log2.alloc((size_t)K * sizeof(double)));
         CK(cudaMemcpy(d_log2.p, l2.data(), (size_t)K * sizeof(double), cudaMemcpyHostToDevice));
-    }
-    pt.start();
-    {
+        pt.start();
         StatusParams sp;
         sp.trp = trp_d; sp.tep = tep_d; sp.n = a.n; sp.K = K; sp.user_begin = 0; sp.user_end = mr;
         sp.has_ndcg = a.out[5] != nullptr;
@@ -918,510 +984,457 @@ int run_call(const CallArgs<T>& a)
         sp.ustatus = d_status.as<int>(); sp.uflags = d_flags.as<int>();
         sp.umin = count_ranks ? d_umin.as<unsigned long long>() : nullptr;
         user_status_kernel<<<(mr + 255) / 256, 256, 0, st>>>(sp);
-        CK(cudaGetLastError());
-        tm.kernel_launches++;
+        TRY(launched());
+        pt.stop(tm.prep_ms);
+        return RMB200_OK;
     }
-    pt.stop(tm.prep_ms);
-
-    // ---- user batches ----
-    int nsm = 148;
-    cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-    const int wave_users = nsm * BM;                       // one CTA (128 users) per SM
-    int UB = 8 * wave_users;                               // users per batch: 8 full waves ...
-    // ... 4 when the filter's item image is much larger than the L2 (256 MB at 1M items x 128 factors): the CTAs of a longer
-    // launch drift further apart and re-stream the item tiles from HBM (cfg4: 3.16 M users/s at 4 waves, 3.10 at 8, 2.96 at
-    // 16, 2.76 with all 1M users in one launch; smaller catalogues prefer 8; profiles/r02_batch_size.txt)
-    if (use_tensor && (size_t)round_up(a.n, 128) * KB * sizeof(__half) > (size_t)160 << 20) UB = 4 * wave_users;
-    if (const char* env = std::getenv("RMB200_BATCH_USERS")) { const int v = std::atoi(env); if (v > 0) UB = round_up(v, BM); }
-    int fo_chunk = 0; size_t fo_bytes = 0;
-    if (use_full) {
-        // ranked lists (K entries per user) and cumulative rows (K columns per metric) of a batch within ~2 GB
-        const long long per_user = (long long)C * (long long)(sizeof(T) + 4) + (a.cumulative ? 8ll * K * (long long)sizeof(T) : 0);
-        long long cap = (2ll << 30) / (per_user > 0 ? per_user : 1);
-        cap = cap / BM * BM;
-        if (cap < BM) cap = BM;
-        if (UB > cap) UB = (int)cap;
-    }
-    if (UB > round_up(mr, BM)) UB = round_up(mr, BM);
-    DevBuf d_fo, d_near, d_nz_mark, d_nz_list, d_nz_cnt, d_At_nz;
-    if (use_full) {
-        full_order_plan(a.n, (int)sizeof(T), UB, &fo_chunk, &fo_bytes);
-        CK(d_fo.alloc(fo_bytes));
-    }
-    if (noise_handback) {
-        CK(d_near.alloc(nnz_te * sizeof(unsigned)));
-        CK(cudaMemsetAsync(d_near.p, 0, nnz_te * sizeof(unsigned) + (nnz_te ? 0 : 16), st));
-        CK(d_nz_mark.alloc((size_t)UB * sizeof(int)));
-        CK(d_nz_list.alloc((size_t)UB * sizeof(int)));
-        CK(d_nz_cnt.alloc(16));
-    }
-
-    DevBuf d_At, d_cs, d_ci, d_cc, d_out[2][10], d_tki[2], d_tks[2], d_stat_out[2], d_Ab, d_anorm;
-    ResultStream rsx;                                     // (declared after the buffers it reads: drained before they are freed)
-    if (!on_dev) CK(rsx.init());
-    CK(d_At.alloc((size_t)p_pad * UB * sizeof(T)));
-    DevBuf d_capx, d_overflow, d_fb_list, d_At_fb;
-    // sampled threshold guess of the filter (filter_select.cuh, pass 0): every stride-th item tile, about 7/K of the
-    // catalogue (1/16 .. 1/8); the guess is the r-th best of the sample with r = the smallest rank for which
-    // P(Poisson(K * sample / n) >= r) <= 1e-6, i.e. fewer than K items of the whole catalogue reach it about once
-    // in a million users (those users' CTAs walk the catalogue a second time; results never depend on the guess)
-    int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
-    if (use_tensor) {
-        const int NT = (a.n + 127) / 128;
-        int min_tiles = 512;
-        if (const char* env = std::getenv("RMB200_SAMPLE_MIN_TILES")) { const int v = std::atoi(env); if (v >= 16) min_tiles = v; }   // developer
-        bool on = NT >= min_tiles;
-        if (const char* env = std::getenv("RMB200_SAMPLE")) on = on && std::atoi(env) != 0;
-        if (on) {
-            double frac = 7.0 / K;
-            if (frac < 1.0 / 16) frac = 1.0 / 16;
-            if (frac > 1.0 / 8) frac = 1.0 / 8;
-            int stride = (int)(1.0 / frac);
-            if (const char* env = std::getenv("RMB200_SAMPLE_STRIDE")) { const int v = std::atoi(env); if (v >= 2) stride = v; }
-            const int ns = NT / stride;                                  // tiles 0, stride, ..., (ns-1)*stride: all full tiles
-            const double lam = (double)K * ((double)ns * 128.0) / (double)a.n;
-            double term = std::exp(-lam), cdf = 0.0;                     // P(X <= r-1), X ~ Poisson(lam)
-            int r = 0;
-            while (r < 4096) { cdf += term; r++; term *= lam / r; if (1.0 - cdf <= 1e-6) break; }
-            if (const char* env = std::getenv("RMB200_SAMPLE_RANK")) { const int v = std::atoi(env); if (v >= 1) r = v; }
-            // (the guess is the r-th largest of up to min(C / 4, 128) group maxima of the sample, filter_select.cuh)
-            const int groups = (C / 4 < 128 ? C / 4 : 128) < ns ? (C / 4 < 128 ? C / 4 : 128) : ns;
-            if (ns >= 8 && 2 * r <= groups) { f_sample_tiles = ns; f_sample_stride = stride; f_sample_rank = r; }
+    // buffers of one batch (two sets of the staging buffers for host inputs and outputs); the first batch's users go up
+    int batch_buffers()
+    {
+        if (use_full) CK(d_fo.alloc(fo_bytes));
+        if (noise_handback) {
+            CK(d_near.alloc(nnz_te * sizeof(unsigned)));
+            CK(cudaMemsetAsync(d_near.p, 0, nnz_te * sizeof(unsigned) + (nnz_te ? 0 : 16), st));
+            CK(d_nz_mark.alloc((size_t)UB * sizeof(int)));
+            CK(d_nz_list.alloc((size_t)UB * sizeof(int)));
+            CK(d_nz_cnt.alloc(16));
         }
-    }
-    if (use_tensor) {
-        CK(d_Ab.alloc((size_t)UB * KB * sizeof(__half)));
-        CK(d_anorm.alloc((size_t)UB * sizeof(float)));
-        CK(d_capx.alloc((size_t)UB * C * sizeof(uint2)));
-        CK(d_overflow.alloc(40 * sizeof(int)));    // [0] users handed back to the FMA path, [1] users that took the retry pass, [6] length of the hand-back list, [8..] cycle counters (stats builds)
-        CK(d_fb_list.alloc((size_t)UB * sizeof(int)));
+        if (!on_dev) CK(rsx.init());
+        CK(d_At.alloc((size_t)p_pad * UB * sizeof(T)));
+        if (use_tensor) {
+            CK(d_Ab.alloc((size_t)UB * KB * sizeof(__half)));
+            CK(d_anorm.alloc((size_t)UB * sizeof(float)));
+            CK(d_capx.alloc((size_t)UB * C * sizeof(uint2)));
+            CK(d_overflow.alloc(40 * sizeof(int)));    // [0] users handed back to the FMA path, [1] users that took the retry pass, [6] length of the hand-back list, [8..] cycle counters (stats builds)
+            CK(d_fb_list.alloc((size_t)UB * sizeof(int)));
+        }
+        if (!on_dev) {
+            CK(d_Arow[0].alloc((size_t)UB * a.k * sizeof(T)));
+            if (UB < mr) CK(d_Arow[1].alloc((size_t)UB * a.k * sizeof(T)));
+            TRY(upload_users(0, 0));
+        }
+        CK(d_cs.alloc((size_t)UB * fma_slices * C * sizeof(T)));
+        CK(d_ci.alloc((size_t)UB * fma_slices * C * sizeof(int)));
+        CK(d_cc.alloc((size_t)UB * fma_slices * sizeof(int)));
+        for (int set = 0; !on_dev && set < (UB < mr ? 2 : 1); set++) {
+            for (int q = 0; q < 10; q++)
+                if (a.out[q]) CK(d_out[set][q].alloc((size_t)UB * (q < 8 ? rs : 1) * sizeof(T)));
+            if (ex->topk_items) CK(d_tki[set].alloc((size_t)UB * K * sizeof(int)));
+            if (ex->topk_scores) CK(d_tks[set].alloc((size_t)UB * K * sizeof(T)));
+            if (ex->status) CK(d_stat_out[set].alloc((size_t)UB * sizeof(int)));
+        }
+        // per-metric means over the users of the call (extension): partial sums per 256 users, added up in order at the end
+        if (want_means) {
+            int mean_blocks_total = 0;
+            for (int b0 = 0; b0 < mr; b0 += UB) mean_blocks_total += (((mr - b0) < UB ? (mr - b0) : UB) + rmb::MEAN_CHUNK - 1) / rmb::MEAN_CHUNK;
+            CK(d_psum.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(double)));
+            CK(d_pcnt.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(int)));
+        }
+        return RMB200_OK;
     }
     // upload of users [b0, b0 + UB) into staging buffer `slot`, on the prefetch stream
-    auto upload_users = [&](int b0, int slot) -> int {
+    int upload_users(int b0, int slot)
+    {
         const int nb = (mr - b0) < UB ? (mr - b0) : UB;
         if (pf.freed_valid[slot]) CK(cudaStreamWaitEvent(pf.s, pf.freed[slot], 0));
         CK(upload_rows(d_Arow[slot].p, a.A + (size_t)(ub + b0) * a.lda, a.lda * sizeof(T), (size_t)a.k * sizeof(T), (size_t)nb, pf.s));
         tm.h2d_bytes += (int64_t)nb * a.k * (int64_t)sizeof(T);
         CK(cudaEventRecord(pf.ready[slot], pf.s));
         return RMB200_OK;
-    };
-    if (!on_dev) {
-        CK(d_Arow[0].alloc((size_t)UB * a.k * sizeof(T)));
-        if (UB < mr) CK(d_Arow[1].alloc((size_t)UB * a.k * sizeof(T)));
-        int rc = upload_users(0, 0);
-        if (rc) return rc;
     }
-    // A call with fewer user tiles than SMs (small m) cuts the catalogue into item ranges on the FMA tiles: one CTA per (user tile,
-    // range), every range keeping its own best K, joined afterwards (merge_slices_kernel); rank counts are added atomically.
-    int fma_slices = 1;
-    if (!use_full) {
-        const int tiles = UB / BM, NT_all = (a.n + BN - 1) / BN;
-        int sl = tiles > 0 ? nsm / tiles : 1;
-        if (sl > NT_all / 8) sl = NT_all / 8;                       // (at least eight item tiles per range)
-        if (sl > C / K) sl = C / K;                                 // the joined heads fit one row ...
-        if (sl > 512 / K) sl = 512 / K;                             // ... and the final sort
-        if (const char* env = std::getenv("RMB200_SLICES")) { const int v = std::atoi(env); if (v >= 1 && v < sl) sl = v; }      // developer
-        if (sl > 1) fma_slices = sl;
+    // the kernels reading the staged rows are queued: mark the buffer; once the scoring kernel is queued as well, the
+    // next batch's rows go up into the other buffer (pageable sources keep this thread busy copying meanwhile)
+    int staged_rows_consumed(const Batch& b)
+    {
+        if (!on_dev) { CK(cudaEventRecord(pf.freed[b.slot], st)); pf.freed_valid[b.slot] = true; }
+        return RMB200_OK;
     }
-    CK(d_cs.alloc((size_t)UB * fma_slices * C * sizeof(T)));
-    CK(d_ci.alloc((size_t)UB * fma_slices * C * sizeof(int)));
-    CK(d_cc.alloc((size_t)UB * fma_slices * sizeof(int)));
-    if (!on_dev) {
-        for (int set = 0; set < (UB < mr ? 2 : 1); set++) {
-            for (int q = 0; q < 10; q++)
-                if (a.out[q]) CK(d_out[set][q].alloc((size_t)UB * (q < 8 ? rs : 1) * sizeof(T)));
-            if (ex && ex->topk_items) CK(d_tki[set].alloc((size_t)UB * K * sizeof(int)));
-            if (ex && ex->topk_scores) CK(d_tks[set].alloc((size_t)UB * K * sizeof(T)));
-            if (ex && ex->status) CK(d_stat_out[set].alloc((size_t)UB * sizeof(int)));
-        }
+    int prefetch_next_users(Batch& b)
+    {
+        if (on_dev || b.prefetched || b.b0 + UB >= mr) return RMB200_OK;
+        b.prefetched = true;
+        return upload_users(b.b0 + UB, b.slot ^ 1);
     }
-
-    // per-metric means over the users of the call (extension): partial sums per 256 users, added up in order at the end
-    DevBuf d_psum, d_pcnt, d_means, d_mcounts;
-    const int mean_W = a.cumulative ? K : 1;
-    int mean_blocks_total = 0, mean_block0 = 0;
-    if (want_means) {
-        for (int b0 = 0; b0 < mr; b0 += UB) mean_blocks_total += (((mr - b0) < UB ? (mr - b0) : UB) + MEAN_CHUNK - 1) / MEAN_CHUNK;
-        CK(d_psum.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(double)));
-        CK(d_pcnt.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(int)));
-    }
-
-    for (int b0 = 0; b0 < mr; b0 += UB) {
-        if (g_interrupt.load()) break;                     // hpp:488-489
+    int launched(int n = 1) { CK(cudaGetLastError()); tm.kernel_launches += n; return RMB200_OK; }   // the kernels just queued
+    int wait_test_rows() { if (pf.test_rows_pending) { CK(cudaStreamWaitEvent(st, pf.test_rows, 0)); pf.test_rows_pending = false; } return RMB200_OK; }
+    int run_batch(int b0)
+    {
         const int nb = (mr - b0) < UB ? (mr - b0) : UB;
-        const int nb_pad = round_up(nb, BM);
-        const int a_slot = (b0 / UB) & 1;                  // staging buffer holding this batch's user factors (host inputs)
-        const int r_set = (b0 / UB) & 1;                   // set of result staging buffers of this batch (host outputs)
-        // the kernels reading the staged rows are queued: mark the buffer; once the scoring kernel is queued as well, the
-        // next batch's rows go up into the other buffer (pageable sources keep this thread busy copying meanwhile)
-        auto staged_rows_consumed = [&]() -> int {
-            if (on_dev) return RMB200_OK;
-            CK(cudaEventRecord(pf.freed[a_slot], st));
-            pf.freed_valid[a_slot] = true;
-            return RMB200_OK;
-        };
-        bool prefetched = false;
-        auto prefetch_next_users = [&]() -> int {
-            if (on_dev || prefetched || b0 + UB >= mr) return RMB200_OK;
-            prefetched = true;
-            return upload_users(b0 + UB, a_slot ^ 1);
-        };
-
-        // user factors of the batch -> k-major
-        const T* Asrc = nullptr; size_t Ald = 0;
+        Batch b{b0, nb, round_up(nb, rmb::BM), (b0 / UB) & 1};
+        TRY(stage_users(b));
+        TRY(score(b));
+        TRY(rank_fixups(b));
+        pt.stop(tm.score_select_ms);                       // (the span score() opened)
+        float ms = 0;                                      // (every path's dominant kernel is wrapped in pk)
+        cudaEventElapsedTime(&ms, pk.a, pk.b);
+        tm.dominant_kernel_ms += ms;
+        TRY(metrics(b));
+        return send_results(b);
+    }
+    // user factors of the batch -> k-major; with rank counting, the held-out items' scores, sorted per user
+    int stage_users(Batch& b)
+    {
+        using namespace rmb;
         if (!on_dev) {
             pt.start();
-            CK(cudaStreamWaitEvent(st, pf.ready[a_slot], 0));     // uploaded one batch ahead: only what is still exposed is timed
-            Asrc = d_Arow[a_slot].as<T>(); Ald = (size_t)a.k;
+            CK(cudaStreamWaitEvent(st, pf.ready[b.slot], 0));     // uploaded one batch ahead: only what is still exposed is timed
+            b.Asrc = static_cast<const T*>(d_Arow[b.slot].p); b.Ald = (size_t)a.k;
             pt.stop(tm.h2d_ms);
-        } else { Asrc = a.A + (size_t)(ub + b0) * a.lda; Ald = a.lda; }
+        } else { b.Asrc = a.A + (size_t)(ub + b.b0) * a.lda; b.Ald = a.lda; }
         pt.start();
-        {
-            dim3 grid(nb_pad / 32, (p_pad + 31) / 32), block(32, 8);
-            pack_tiles_kernel<T, BM><<<grid, block, 0, st>>>(Asrc, Ald, nb, a.k, d_At.as<T>(), nb_pad, p_pad);
-            CK(cudaGetLastError());
-            tm.kernel_launches++;
-
-            if (!use_tensor) { int rc = staged_rows_consumed(); if (rc) return rc; }
-        }
+        dim3 grid(b.nb_pad / 32, (p_pad + 31) / 32), block(32, 8);
+        pack_tiles_kernel<T, BM><<<grid, block, 0, st>>>(b.Asrc, b.Ald, b.nb, a.k, d_At.as<T>(), b.nb_pad, p_pad);
+        TRY(launched());
+        if (!use_tensor) TRY(staged_rows_consumed(b));
         if (count_ranks && !use_full) {
-            if (pf.test_rows_pending) { CK(cudaStreamWaitEvent(st, pf.test_rows, 0)); pf.test_rows_pending = false; }
-            const int blocks = (nb + 7) / 8 < 8 * nsm ? (nb + 7) / 8 : 8 * nsm;
-            score_entries_kernel<T, BM><<<blocks, 256, 0, st>>>(d_At.as<T>(), d_Bt.as<T>(), bias_d, p_pad, b0, nb,
+            TRY(wait_test_rows());
+            const int blocks = (b.nb + 7) / 8 < 8 * nsm ? (b.nb + 7) / 8 : 8 * nsm;
+            score_entries_kernel<T, BM><<<blocks, 256, 0, st>>>(d_At.as<T>(), d_Bt.as<T>(), bias_d, p_pad, b.b0, b.nb,
                                                              tep_d, tei_d, d_status.as<int>(), d_pos_raw.as<T>());
             CK(cudaGetLastError());
-            sort_positives_kernel<T><<<blocks, 256, 0, st>>>(b0, nb, tep_d, tei_d, d_status.as<int>(), d_pos_raw.as<T>(),
+            sort_positives_kernel<T><<<blocks, 256, 0, st>>>(b.b0, b.nb, tep_d, tei_d, d_status.as<int>(), d_pos_raw.as<T>(),
                                                               d_pos_sorted.as<T>(), d_pos_perm.as<int>(), d_pos_item.as<int>());
-            CK(cudaGetLastError());
-            tm.kernel_launches += 2;
+            TRY(launched(2));
         }
         pt.stop(tm.prep_ms);
-
-        bool pk_pending = false;
-        // fused score / exclude / select (/ rank counting) on the FMA pipe: the whole batch, or (umap) the listed users only
-        auto run_fma = [&](const T* At_ptr, int n_rows, const int* umap, bool with_counts, bool timed) -> int {
-            ScoreSelectParams<T> sp = ScoreSelectParams<T>();       // (every field defined: optional ones stay null)
-            sp.At = At_ptr; sp.Bt = d_Bt.as<T>(); sp.bias = bias_d;
-            sp.p_pad = p_pad; sp.n = a.n; sp.mb = n_rows; sp.user0 = b0;
-            sp.trp = trp_d; sp.tri = tri_d; sp.tep = tep_d; sp.ustatus = d_status.as<int>();
-            sp.cand_score = d_cs.as<T>(); sp.cand_item = d_ci.as<int>(); sp.cand_count = d_cc.as<int>();
-            sp.uflags = d_flags.as<int>(); sp.K = K;
-            sp.pos_sorted = with_counts ? d_pos_sorted.as<T>() : nullptr;
-            sp.auc_cnt = with_counts ? d_auc.as<unsigned int>() : nullptr;
-            sp.pos_item = with_counts ? d_pos_item.as<int>() : nullptr;
-            sp.auc_near = (with_counts && noise_handback) ? d_near.as<unsigned>() : nullptr;
-            sp.umin = with_counts ? d_umin.as<unsigned long long>() : nullptr;
-            sp.umap = umap;
-            const int slices = (umap == nullptr && !use_tensor) ? fma_slices : 1;
-            sp.slice_rows = slices > 1 ? UB : 0;
-            if (const char* env = std::getenv("RMB200_AUC_DBG")) sp.dbg = std::atoi(env);      // developer: timing experiments (wrong results)
-            if (timed) cudaEventRecord(pk.a, st);
-            CK(launch_score_select<T>(sp, C, with_counts, n_rows, slices, st));
-            if (timed) { cudaEventRecord(pk.b, st); pk_pending = true; }
-            tm.kernel_launches++;
-            if (slices > 1) {
-                merge_slices_kernel<T><<<(n_rows + 7) / 8, 256, 0, st>>>(d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, n_rows, slices, UB);
-                CK(cudaGetLastError());
-                tm.kernel_launches++;
-            }
-            return RMB200_OK;
-        };
-        auto run_fma_batch = [&]() -> int {
-            int rc = run_fma(d_At.as<T>(), nb, nullptr, count_ranks, true);
-            if (rc) return rc;
-            return prefetch_next_users();
-        };
+        return RMB200_OK;
+    }
+    // the batch's candidates on its path; opens the scoring span (run_batch closes it)
+    int score(Batch& b)
+    {
         if (fma_counts_first) {            // rank counts (and the smallest candidate score) from the FMA tiles; its top-K is replaced below
             pt.start();
-            int rc = run_fma_batch();
-            if (rc) return rc;
+            TRY(run_fma(b, d_At.as<T>(), b.nb, nullptr, count_ranks, true));
+            TRY(prefetch_next_users(b));
             pt.stop(tm.score_select_ms);
         }
-        if (use_tensor) {
-            // norms + fp16 operand image of the batch's users, then the tensor-core filter and the exact re-scoring
-            pt.start();
-            const long long total = (long long)nb_pad * (KB / 8);
-            row_norm_kernel<T><<<(nb + NORM_ROWS_PER_BLOCK - 1) / NORM_ROWS_PER_BLOCK, 256, 0, st>>>(Asrc, Ald, nb, a.k, (const T*)nullptr, a.bias ? 1 : 0,
-                                                                                               d_anorm.as<float>(), nullptr, nullptr);
-            CK(cudaGetLastError());
-            pack_f16_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(Asrc, Ald, nb, a.k, (const T*)nullptr, a.bias ? 1 : 0,
-                                                                                d_anorm.as<float>(), nullptr, d_Ab.as<__half>(), nb_pad, KB);
-            CK(cudaGetLastError());
-            CK(cudaMemsetAsync(d_overflow.p, 0, 40 * sizeof(int), st));
-            tm.kernel_launches += 2;
-            pt.stop(tm.prep_ms);
-            pt.start();
-            const FilterErrCoef ec = filter_err_coefs(KB);
-            FilterParams fp;
-            fp.Ab = d_Ab.as<__half>(); fp.Bb = d_Bb.as<__half>(); fp.KB = KB; fp.stages = f_stages;
-            fp.c_rel = ec.c_rel; fp.c_abs = ec.c_abs; fp.c_const = ec.c_const;
-            fp.n = a.n; fp.mb = nb; fp.user0 = b0;
-            fp.anorm = d_anorm.as<float>(); fp.maxbn = d_maxbn.as<unsigned>(); fp.chunk_norm = d_chunkn.as<float>();
-            fp.trp = trp_d; fp.tri = tri_d; fp.ustatus = d_status.as<int>();
-            fp.cand = d_capx.as<uint2>(); fp.cand_count = d_cc.as<int>();
-            fp.overflow = d_overflow.as<int>(); fp.uflags = d_flags.as<int>(); fp.K = K;
-            fp.sample_tiles = f_sample_tiles; fp.sample_stride = f_sample_stride; fp.sample_rank = f_sample_rank;
-            fp.retries = d_overflow.as<int>() + 1;
-            fp.noise_band = a.noise ? 2.02e-12f : 0.f;
-            fp.dbg = 0; if (const char* env = std::getenv("RMB200_DBG")) fp.dbg = std::atoi(env);
-            cudaEventRecord(pk.a, st);
-            CK(launch_filter_select(fp, C, nb_pad / BM, st));
-            cudaEventRecord(pk.b, st);
-            pk_pending = true;
-            tm.kernel_launches++;
-            // the exact stage reads the staged user factors (through d_At) and the filter is queued: the next batch's rows can go up
-            { int rc = staged_rows_consumed(); if (rc) return rc; }
-            { int rc = prefetch_next_users(); if (rc) return rc; }
-            NoiseArgs nz;
-            nz.on = a.noise; nz.seed_user0 = (unsigned long long)a.seed + (unsigned long long)(ub + b0); nz.trp = trp_d; nz.tri = tri_d; nz.n = a.n;
-            FilterErrStat es;
-            es.anorm = d_anorm.as<float>(); es.maxbn = d_maxbn.as<unsigned>(); es.chunk_norm = d_chunkn.as<float>();
-            es.c_rel = ec.c_rel; es.c_abs = ec.c_abs; es.c_const = ec.c_const;
-            es.max_ratio_bits = want_filter_stats ? d_maxbn.as<unsigned>() + 1 : nullptr;
-            CK(launch_exact_topk<T>(d_capx.as<uint2>(), d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, nb, b0, d_At.as<T>(), p_pad, a.k,
-                                    Bsrc, Bld, bias_d, d_flags.as<int>(), K, nz, es, st));
-            tm.kernel_launches++;
-            int over_retry[40] = {0};
-            CK(cudaMemcpyAsync(over_retry, d_overflow.p, 40 * sizeof(int), cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-#if RMB_F_STATS
-            std::fprintf(stderr, "[rmb200 stats] users %d: appends/user %.1f cuts/user %.2f slow-path entries/user %.1f cursor moves/user %.1f retries %d handed back %d (sample tiles %d stride %d rank %d)\n",
-                         nb, over_retry[2] / (double)nb, over_retry[3] / (double)nb, over_retry[4] / (double)nb, over_retry[5] / (double)nb,
-                         over_retry[1], over_retry[0], f_sample_tiles, f_sample_stride, f_sample_rank);
-            {
-                const unsigned long long* ck = reinterpret_cast<const unsigned long long*>(over_retry + 8);
-                const double nc = (double)(nb_pad / BM);
-                for (int ps = 0; ps < 2; ps++)
-                    std::fprintf(stderr, "[rmb200 stats]   pass %d, one epilogue warp, kcycles per CTA: wait acc %.0f, ld+fast %.0f, append %.0f, cursor %.0f, meet+cut %.0f, total %.0f\n",
-                                 ps, ck[ps * 6 + 0] / nc / 1e3, ck[ps * 6 + 1] / nc / 1e3, ck[ps * 6 + 2] / nc / 1e3, ck[ps * 6 + 3] / nc / 1e3, ck[ps * 6 + 4] / nc / 1e3, ck[ps * 6 + 5] / nc / 1e3);
-            }
-#endif
-            const int n_over = over_retry[0];
-            tm.filter_retry_rows += over_retry[1];
-            if (n_over > 0) {
-                // some users' kept band did not fit their candidate buffer (near-constant scores) or their factors cannot be scaled
-                // into fp16 range: THOSE users are re-run on the FMA tiles (same results), everybody else keeps the filter's result
-                tm.filter_fallback_batches++;
-                tm.filter_fallback_users += n_over;
-                pt.stop(tm.score_select_ms);
-                int rc = pack_Bt();
-                if (rc) return rc;
-                pt.start();
-                const int n_over_pad = round_up(n_over, BM);
-                CK(d_At_fb.alloc((size_t)p_pad * n_over_pad * sizeof(T)));
-                collect_flagged_kernel<<<1, 1024, 0, st>>>(d_cc.as<int>(), nb, d_fb_list.as<int>(), d_overflow.as<int>() + 6);
-                CK(cudaGetLastError());
-                dim3 grid(n_over_pad / 32, (p_pad + 31) / 32), block(32, 8);
-                pack_tiles_gather_kernel<T, BM><<<grid, block, 0, st>>>(Asrc, Ald, d_fb_list.as<int>(), n_over, a.k, d_At_fb.as<T>(), n_over_pad, p_pad);
-                CK(cudaGetLastError());
-                tm.kernel_launches += 2;
-                { int rc2 = staged_rows_consumed(); if (rc2) return rc2; }      // (the gather read the staged rows once more)
-                if (n_over <= 2048 && a.n >= 32768) {
-                    // a few users of a large catalogue: the full-order path (every candidate scored by item-parallel blocks, one
-                    // segmented sort) -- on the FMA tiles ONE CTA walked the whole catalogue for them (78 ms at 1M items for a
-                    // single user, profiles/r02v: two of four ranks of a strong-scaling run ran at half speed for it)
-                    int chunk = 0; size_t bytes = 0;
-                    full_order_plan(a.n, (int)sizeof(T), n_over, &chunk, &bytes);
-                    CK(d_fo.alloc(bytes));
-                    FullOrderArgs<T> fo;
-                    fo.At = d_At_fb.as<T>(); fo.Bt = d_Bt.as<T>(); fo.bias = bias_d; fo.p_pad = p_pad; fo.n = a.n; fo.K = K; fo.C = C;
-                    fo.user0 = b0; fo.nb = n_over; fo.umap = d_fb_list.as<int>();
-                    fo.trp = trp_d; fo.tri = tri_d; fo.tep = tep_d; fo.tei = tei_d; fo.ustatus = d_status.as<int>(); fo.uflags = d_flags.as<int>();
-                    fo.cand_score = d_cs.as<T>(); fo.cand_item = d_ci.as<int>(); fo.cand_count = d_cc.as<int>();
-                    fo.umin = count_ranks ? d_umin.as<unsigned long long>() : nullptr;
-                    fo.auc_cnt = count_ranks ? d_auc.as<unsigned int>() : nullptr;
-                    fo.pos_perm = count_ranks ? d_pos_perm.as<int>() : nullptr;
-                    fo.noise = a.noise; fo.seed_user0 = (unsigned long long)a.seed + (unsigned long long)(ub + b0);
-                    fo.scratch = d_fo.p; fo.scratch_bytes = bytes; fo.chunk_users = chunk;
-                    if (pf.test_rows_pending && count_ranks) { CK(cudaStreamWaitEvent(st, pf.test_rows, 0)); pf.test_rows_pending = false; }
-                    long long nl = 0;
-                    CK(full_order_run<T>(fo, st, &nl));
-                    tm.kernel_launches += nl;
-                } else {
-                    rc = run_fma(d_At_fb.as<T>(), n_over, d_fb_list.as<int>(), false, false);
-                    if (rc) return rc;
-                }
-            }
-        } else if (use_full) {
-            // every candidate scored, (noise,) sorted: ranked top-K, smallest candidate score and held-out ranks off the sorted lists
-            pt.start();
-            if (pf.test_rows_pending) { CK(cudaStreamWaitEvent(st, pf.test_rows, 0)); pf.test_rows_pending = false; }
-            FullOrderArgs<T> fo;
-            fo.At = d_At.as<T>(); fo.Bt = d_Bt.as<T>(); fo.bias = bias_d; fo.p_pad = p_pad; fo.n = a.n; fo.K = K; fo.C = C;
-            fo.user0 = b0; fo.nb = nb; fo.umap = nullptr;
-            fo.trp = trp_d; fo.tri = tri_d; fo.tep = tep_d; fo.tei = tei_d; fo.ustatus = d_status.as<int>(); fo.uflags = d_flags.as<int>();
-            fo.cand_score = d_cs.as<T>(); fo.cand_item = d_ci.as<int>(); fo.cand_count = d_cc.as<int>();
-            fo.umin = count_ranks ? d_umin.as<unsigned long long>() : nullptr;
-            fo.auc_cnt = count_ranks ? d_auc.as<unsigned int>() : nullptr;
-            fo.pos_perm = count_ranks ? d_pos_perm.as<int>() : nullptr;
-            fo.noise = a.noise; fo.seed_user0 = (unsigned long long)a.seed + (unsigned long long)(ub + b0);
-            fo.scratch = d_fo.p; fo.scratch_bytes = fo_bytes; fo.chunk_users = fo_chunk;
-            cudaEventRecord(pk.a, st);
-            long long nl = 0;
-            CK(full_order_run<T>(fo, st, &nl));
-            cudaEventRecord(pk.b, st);
-            pk_pending = true;
-            tm.kernel_launches += nl;
-            { int rc = prefetch_next_users(); if (rc) return rc; }
-        } else {
-            pt.start();
-            int rc = run_fma_batch();
-            if (rc) return rc;
+        if (use_tensor) return score_tensor(b);
+        pt.start();
+        if (!use_full) TRY(run_fma(b, d_At.as<T>(), b.nb, nullptr, count_ranks, true));
+        else {    // every candidate scored, (noise,) sorted: ranked top-K, smallest candidate score and held-out ranks off the sorted lists
+            TRY(wait_test_rows());
+            TRY(run_full_order(b, d_At.as<T>(), b.nb, nullptr, fo_chunk, fo_bytes, true));
         }
-        if (!use_full) {
-            CK(launch_rank_topk<T>(d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, nb, use_tensor ? K : K * fma_slices, st));
-            tm.kernel_launches++;
-        }
+        return prefetch_next_users(b);
+    }
+    // fused score / exclude / select (/ rank counting) on the FMA pipe: the whole batch, or (umap) the listed users only
+    int run_fma(Batch& b, const T* At_ptr, int n_rows, const int* umap, bool with_counts, bool timed)
+    {
+        using namespace rmb;
+        ScoreSelectParams<T> sp = ScoreSelectParams<T>();       // (every field defined: optional ones stay null)
+        sp.At = At_ptr; sp.Bt = d_Bt.as<T>(); sp.bias = bias_d;
+        sp.p_pad = p_pad; sp.n = a.n; sp.mb = n_rows; sp.user0 = b.b0;
+        sp.trp = trp_d; sp.tri = tri_d; sp.tep = tep_d; sp.ustatus = d_status.as<int>();
+        sp.cand_score = d_cs.as<T>(); sp.cand_item = d_ci.as<int>(); sp.cand_count = d_cc.as<int>();
+        sp.uflags = d_flags.as<int>(); sp.K = K;
+        sp.pos_sorted = with_counts ? d_pos_sorted.as<T>() : nullptr;
+        sp.auc_cnt = with_counts ? d_auc.as<unsigned int>() : nullptr;
+        sp.pos_item = with_counts ? d_pos_item.as<int>() : nullptr;
+        sp.auc_near = (with_counts && noise_handback) ? d_near.as<unsigned>() : nullptr;
+        sp.umin = with_counts ? d_umin.as<unsigned long long>() : nullptr;
+        sp.umap = umap;
+        const int slices = (umap == nullptr && !use_tensor) ? fma_slices : 1;
+        sp.slice_rows = slices > 1 ? UB : 0;
+        sp.dbg = auc_dbg;
+        if (timed) cudaEventRecord(pk.a, st);
+        CK(launch_score_select<T>(sp, C, with_counts, n_rows, slices, st));
+        if (timed) cudaEventRecord(pk.b, st);
+        tm.kernel_launches++;
+        if (slices > 1) { merge_slices_kernel<T><<<(n_rows + 7) / 8, 256, 0, st>>>(d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, n_rows, slices, UB); TRY(launched()); }
+        return RMB200_OK;
+    }
+    // the full-order path over n_users rows of At (umap: their batch-local users), with scratch of full_order_plan()
+    int run_full_order(Batch& b, const T* At, int n_users, const int* umap, int chunk, size_t bytes, bool timed)
+    {
+        rmb::FullOrderArgs<T> fo;
+        fo.At = At; fo.Bt = d_Bt.as<T>(); fo.bias = bias_d; fo.p_pad = p_pad; fo.n = a.n; fo.K = K; fo.C = C;
+        fo.user0 = b.b0; fo.nb = n_users; fo.umap = umap;
+        fo.trp = trp_d; fo.tri = tri_d; fo.tep = tep_d; fo.tei = tei_d; fo.ustatus = d_status.as<int>(); fo.uflags = d_flags.as<int>();
+        fo.cand_score = d_cs.as<T>(); fo.cand_item = d_ci.as<int>(); fo.cand_count = d_cc.as<int>();
+        fo.umin = count_ranks ? d_umin.as<unsigned long long>() : nullptr;
+        fo.auc_cnt = count_ranks ? d_auc.as<unsigned int>() : nullptr;
+        fo.pos_perm = count_ranks ? d_pos_perm.as<int>() : nullptr;
+        fo.noise = a.noise; fo.seed_user0 = (unsigned long long)a.seed + (unsigned long long)(ub + b.b0);
+        fo.scratch = d_fo.p; fo.scratch_bytes = bytes; fo.chunk_users = chunk;
+        if (timed) cudaEventRecord(pk.a, st);
+        long long nl = 0;
+        CK(rmb::full_order_run<T>(fo, st, &nl));
+        if (timed) cudaEventRecord(pk.b, st);
+        tm.kernel_launches += nl;
+        return RMB200_OK;
+    }
+    // Re-scores n listed users of the batch on their own: their staged rows gathered into `tile`, then the full-order path, or
+    // (on_fma) the FMA tiles over the list.  With `flags`, the list and its length (*list_len) are collected from them first.
+    int hand_back(Batch& b, DevBuf& tile, int* list, int n, const int* flags, int* list_len, bool on_fma)
+    {
+        using namespace rmb;
+        TRY(ensure_Bt());
+        const int n_pad_u = round_up(n, BM);
+        CK(tile.alloc((size_t)p_pad * n_pad_u * sizeof(T)));
+        if (flags) { collect_flagged_kernel<<<1, 1024, 0, st>>>(flags, b.nb, list, list_len); TRY(launched()); }
+        dim3 grid(n_pad_u / 32, (p_pad + 31) / 32), block(32, 8);
+        pack_tiles_gather_kernel<T, BM><<<grid, block, 0, st>>>(b.Asrc, b.Ald, list, n, a.k, tile.as<T>(), n_pad_u, p_pad);
+        TRY(launched());
+        TRY(staged_rows_consumed(b));      // (the gather read the staged rows once more)
+        if (on_fma) return run_fma(b, tile.as<T>(), n, list, false, false);
+        int chunk = 0; size_t bytes = 0;
+        full_order_plan(a.n, (int)sizeof(T), n, &chunk, &bytes);
+        CK(d_fo.alloc(bytes));
+        if (count_ranks) TRY(wait_test_rows());
+        return run_full_order(b, tile.as<T>(), n, list, chunk, bytes, false);
+    }
+    // norms + fp16 operand image of the batch's users, then the tensor-core filter and the exact re-scoring
+    int score_tensor(Batch& b)
+    {
+        using namespace rmb;
+        pt.start();
+        const long long total = (long long)b.nb_pad * (KB / 8);
+        row_norm_kernel<T><<<(b.nb + NORM_ROWS_PER_BLOCK - 1) / NORM_ROWS_PER_BLOCK, 256, 0, st>>>(b.Asrc, b.Ald, b.nb, a.k, (const T*)nullptr, a.bias ? 1 : 0,
+                                                                                                 d_anorm.as<float>(), nullptr, nullptr);
+        CK(cudaGetLastError());
+        pack_f16_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(b.Asrc, b.Ald, b.nb, a.k, (const T*)nullptr, a.bias ? 1 : 0,
+                                                                            d_anorm.as<float>(), nullptr, d_Ab.as<__half>(), b.nb_pad, KB);
+        TRY(launched(2));
+        CK(cudaMemsetAsync(d_overflow.p, 0, 40 * sizeof(int), st));
+        pt.stop(tm.prep_ms);
+        pt.start();
+        const FilterErrCoef ec = filter_err_coefs(KB);
+        FilterParams fp;
+        fp.Ab = d_Ab.as<__half>(); fp.Bb = d_Bb.as<__half>(); fp.KB = KB; fp.stages = f_stages;
+        fp.c_rel = ec.c_rel; fp.c_abs = ec.c_abs; fp.c_const = ec.c_const;
+        fp.n = a.n; fp.mb = b.nb; fp.user0 = b.b0;
+        fp.anorm = d_anorm.as<float>(); fp.maxbn = d_maxbn.as<unsigned>(); fp.chunk_norm = d_chunkn.as<float>();
+        fp.trp = trp_d; fp.tri = tri_d; fp.ustatus = d_status.as<int>();
+        fp.cand = d_capx.as<uint2>(); fp.cand_count = d_cc.as<int>();
+        fp.overflow = d_overflow.as<int>(); fp.uflags = d_flags.as<int>(); fp.K = K;
+        fp.sample_tiles = f_sample_tiles; fp.sample_stride = f_sample_stride; fp.sample_rank = f_sample_rank;
+        fp.retries = d_overflow.as<int>() + 1;
+        fp.noise_band = a.noise ? 2.02e-12f : 0.f;
+        fp.dbg = filter_dbg;
+        cudaEventRecord(pk.a, st);
+        CK(launch_filter_select(fp, C, b.nb_pad / BM, st));
+        cudaEventRecord(pk.b, st);
+        tm.kernel_launches++;
+        // the exact stage reads the staged user factors (through d_At) and the filter is queued: the next batch's rows can go up
+        TRY(staged_rows_consumed(b));
+        TRY(prefetch_next_users(b));
+        NoiseArgs nz;
+        nz.on = a.noise; nz.seed_user0 = (unsigned long long)a.seed + (unsigned long long)(ub + b.b0); nz.trp = trp_d; nz.tri = tri_d; nz.n = a.n;
+        FilterErrStat es;
+        es.anorm = d_anorm.as<float>(); es.maxbn = d_maxbn.as<unsigned>(); es.chunk_norm = d_chunkn.as<float>();
+        es.c_rel = ec.c_rel; es.c_abs = ec.c_abs; es.c_const = ec.c_const;
+        es.max_ratio_bits = want_filter_stats ? d_maxbn.as<unsigned>() + 1 : nullptr;
+        CK(launch_exact_topk<T>(d_capx.as<uint2>(), d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, b.nb, b.b0, d_At.as<T>(), p_pad, a.k,
+                                Bsrc, Bld, bias_d, d_flags.as<int>(), K, nz, es, st));
+        tm.kernel_launches++;
+        int over_retry[40] = {0};
+        CK(cudaMemcpyAsync(over_retry, d_overflow.p, 40 * sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        print_filter_stats(over_retry, b.nb, b.nb_pad, f_sample_tiles, f_sample_stride, f_sample_rank);
+        const int n_over = over_retry[0];
+        tm.filter_retry_rows += over_retry[1];
+        if (n_over == 0) return RMB200_OK;
+        // some users' kept band did not fit their candidate buffer (near-constant scores) or their factors cannot be scaled
+        // into fp16 range: THOSE users are re-run on the FMA tiles (same results), everybody else keeps the filter's result
+        tm.filter_fallback_batches++;
+        tm.filter_fallback_users += n_over;
+        pt.stop(tm.score_select_ms);
+        TRY(ensure_Bt());
+        pt.start();
+        // a few users of a large catalogue go to the full-order path (every candidate scored by item-parallel blocks, one
+        // segmented sort) -- on the FMA tiles ONE CTA walked the whole catalogue for them (78 ms at 1M items for a
+        // single user, profiles/r02v: two of four ranks of a strong-scaling run ran at half speed for it)
+        return hand_back(b, d_At_fb, d_fb_list.as<int>(), n_over, d_cc.as<int>(), d_overflow.as<int>() + 6, n_over > 2048 || a.n < 32768);
+    }
+    // the selected candidates ranked; the noise hand-back; the all-equal check of the FMA tiles under the noise
+    int rank_fixups(Batch& b)
+    {
+        using namespace rmb;
+        if (!use_full) { CK(launch_rank_topk<T>(d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, b.nb, use_tensor ? K : K * fma_slices, st)); tm.kernel_launches++; }
         if (noise_handback) {
             // users for whom the tie-breaking noise decides a rank: their ranked top-K and ranks from the full-order path
-            mark_noise_users_kernel<<<(nb + 255) / 256, 256, 0, st>>>(tep_d, d_near.as<unsigned>(), d_status.as<int>(), b0, nb, d_nz_mark.as<int>());
+            mark_noise_users_kernel<<<(b.nb + 255) / 256, 256, 0, st>>>(tep_d, d_near.as<unsigned>(), d_status.as<int>(), b.b0, b.nb, d_nz_mark.as<int>());
             CK(cudaGetLastError());
             CK(cudaMemsetAsync(d_nz_cnt.p, 0, 16, st));
-            collect_flagged_kernel<<<1, 1024, 0, st>>>(d_nz_mark.as<int>(), nb, d_nz_list.as<int>(), d_nz_cnt.as<int>());
-            CK(cudaGetLastError());
-            tm.kernel_launches += 2;
+            collect_flagged_kernel<<<1, 1024, 0, st>>>(d_nz_mark.as<int>(), b.nb, d_nz_list.as<int>(), d_nz_cnt.as<int>());
+            TRY(launched(2));
             int n_nz = 0;
             CK(cudaMemcpyAsync(&n_nz, d_nz_cnt.p, sizeof(int), cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
             if (n_nz > 0) {
                 tm.noise_handback_users += n_nz;
-                int rc = pack_Bt();
-                if (rc) return rc;
-                const int n_pad_u = round_up(n_nz, BM);
-                CK(d_At_nz.alloc((size_t)p_pad * n_pad_u * sizeof(T)));
-                dim3 grid(n_pad_u / 32, (p_pad + 31) / 32), block(32, 8);
-                pack_tiles_gather_kernel<T, BM><<<grid, block, 0, st>>>(Asrc, Ald, d_nz_list.as<int>(), n_nz, a.k, d_At_nz.as<T>(), n_pad_u, p_pad);
-                CK(cudaGetLastError());
-                tm.kernel_launches++;
-                { int rc2 = staged_rows_consumed(); if (rc2) return rc2; }
-                int chunk = 0; size_t bytes = 0;
-                full_order_plan(a.n, (int)sizeof(T), n_nz, &chunk, &bytes);
-                CK(d_fo.alloc(bytes));
-                FullOrderArgs<T> fo;
-                fo.At = d_At_nz.as<T>(); fo.Bt = d_Bt.as<T>(); fo.bias = bias_d; fo.p_pad = p_pad; fo.n = a.n; fo.K = K; fo.C = C;
-                fo.user0 = b0; fo.nb = n_nz; fo.umap = d_nz_list.as<int>();
-                fo.trp = trp_d; fo.tri = tri_d; fo.tep = tep_d; fo.tei = tei_d; fo.ustatus = d_status.as<int>(); fo.uflags = d_flags.as<int>();
-                fo.cand_score = d_cs.as<T>(); fo.cand_item = d_ci.as<int>(); fo.cand_count = d_cc.as<int>();
-                fo.umin = d_umin.as<unsigned long long>(); fo.auc_cnt = d_auc.as<unsigned int>(); fo.pos_perm = d_pos_perm.as<int>();
-                fo.noise = 1; fo.seed_user0 = (unsigned long long)a.seed + (unsigned long long)(ub + b0);
-                fo.scratch = d_fo.p; fo.scratch_bytes = bytes; fo.chunk_users = chunk;
-                long long nl = 0;
-                CK(full_order_run<T>(fo, st, &nl));
-                tm.kernel_launches += nl;
+                TRY(hand_back(b, d_At_nz, d_nz_list.as<int>(), n_nz, nullptr, nullptr, false));
             }
         }
         if (a.noise && !use_tensor && !use_full && !count_ranks) {
-            all_equal_check_kernel<T><<<nb, 128, 0, st>>>(d_cs.as<T>(), d_cc.as<int>(), C, b0, K, a.n, trp_d, tri_d, d_status.as<int>(),
-                                                           d_At.as<T>(), d_Bt.as<T>(), bias_d, p_pad, d_flags.as<int>());
-            CK(cudaGetLastError());
-            tm.kernel_launches++;
+            all_equal_check_kernel<T><<<b.nb, 128, 0, st>>>(d_cs.as<T>(), d_cc.as<int>(), C, b.b0, K, a.n, trp_d, tri_d, d_status.as<int>(),
+                                                             d_At.as<T>(), d_Bt.as<T>(), bias_d, p_pad, d_flags.as<int>());
+            TRY(launched());
         }
-        pt.stop(tm.score_select_ms);
-        if (pk_pending) { float ms = 0; cudaEventElapsedTime(&ms, pk.a, pk.b); tm.dominant_kernel_ms += ms; }
-
-        // per-user metrics
+        return RMB200_OK;
+    }
+    // per-user metrics (and the partial sums of their means) into the caller's rows, or into the batch's result set
+    int metrics(Batch& b)
+    {
+        using namespace rmb;
         pt.start();
-        {
-            MetricsParams<T> mp;
-            mp.n = a.n; mp.K = K; mp.C = C; mp.user0 = b0; mp.mb = nb; mp.cumulative = a.cumulative;
-            mp.want_roc = want_roc; mp.want_pr = want_pr; mp.count_ranks = count_ranks; mp.noise = a.noise;
-            mp.trp = trp_d; mp.tep = tep_d; mp.tei = tei_d; mp.tev = tev_d;
-            mp.ustatus = d_status.as<int>(); mp.uflags = d_flags.as<int>();
-            mp.cand_score = d_cs.as<T>(); mp.cand_item = d_ci.as<int>(); mp.cand_count = d_cc.as<int>();
-            mp.auc_cnt = d_auc.as<unsigned int>(); mp.umin = d_umin.as<unsigned long long>();
-            mp.pos_perm = d_pos_perm.as<int>(); mp.log2tab = d_log2.as<double>();
-            mp.nan_value = nan_value;
-            T* outs[10];
-            if (!on_dev && rsx.copied_valid[r_set]) CK(cudaStreamWaitEvent(st, rsx.copied[r_set], 0));      // the set's previous rows have left
-            for (int q = 0; q < 10; q++) {
-                const size_t stride = q < 8 ? rs : 1;
-                if (!a.out[q]) outs[q] = nullptr;
-                else if (on_dev) outs[q] = a.out[q] + (size_t)(ub + b0) * stride;
-                else outs[q] = d_out[r_set][q].as<T>();
-            }
-            mp.p = outs[0]; mp.tp = outs[1]; mp.r = outs[2]; mp.ap = outs[3]; mp.tap = outs[4];
-            mp.ndcg = outs[5]; mp.hit = outs[6]; mp.rr = outs[7]; mp.roc = outs[8]; mp.pr = outs[9];
-            mp.status_out = nullptr; mp.topk_items = nullptr; mp.topk_scores = nullptr;
-            if (ex && ex->status) mp.status_out = on_dev ? ex->status + ub + b0 : d_stat_out[r_set].as<int>();
-            if (ex && ex->topk_items) mp.topk_items = on_dev ? ex->topk_items + (size_t)(ub + b0) * K : d_tki[r_set].as<int>();
-            if (ex && ex->topk_scores) mp.topk_scores = on_dev ? reinterpret_cast<T*>(ex->topk_scores) + (size_t)(ub + b0) * K : d_tks[r_set].as<T>();
-            mp.pos_rank = pos_rank_d;
-            if (pf.test_rows_pending) { CK(cudaStreamWaitEvent(st, pf.test_rows, 0)); pf.test_rows_pending = false; }
-            user_metrics_kernel<T><<<(nb + METRICS_WARPS - 1) / METRICS_WARPS, METRICS_WARPS * 32, 0, st>>>(mp);
-            CK(cudaGetLastError());
-            tm.kernel_launches++;
-            if (want_means) {
-                MeanParams<T> qp;
-                for (int q = 0; q < 10; q++) qp.out[q] = outs[q];
-                qp.nb = nb; qp.W = mean_W; qp.part_sum = d_psum.as<double>(); qp.part_cnt = d_pcnt.as<int>(); qp.block0 = mean_block0;
-                const int blocks = (nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
-                metric_partial_kernel<T><<<dim3(blocks, 10), MEAN_CHUNK, 0, st>>>(qp);
-                CK(cudaGetLastError());
-                tm.kernel_launches++;
-                mean_block0 += blocks;
-            }
+        MetricsParams<T> mp;
+        mp.n = a.n; mp.K = K; mp.C = C; mp.user0 = b.b0; mp.mb = b.nb; mp.cumulative = a.cumulative;
+        mp.want_roc = want_roc; mp.want_pr = want_pr; mp.count_ranks = count_ranks; mp.noise = a.noise;
+        mp.trp = trp_d; mp.tep = tep_d; mp.tei = tei_d; mp.tev = tev_d;
+        mp.ustatus = d_status.as<int>(); mp.uflags = d_flags.as<int>();
+        mp.cand_score = d_cs.as<T>(); mp.cand_item = d_ci.as<int>(); mp.cand_count = d_cc.as<int>();
+        mp.auc_cnt = d_auc.as<unsigned int>(); mp.umin = d_umin.as<unsigned long long>();
+        mp.pos_perm = d_pos_perm.as<int>(); mp.log2tab = d_log2.as<double>();
+        mp.nan_value = nan_value;
+        T* outs[10];
+        if (!on_dev && rsx.copied_valid[b.slot]) CK(cudaStreamWaitEvent(st, rsx.copied[b.slot], 0));      // the set's previous rows have left
+        const size_t row = (size_t)(ub + b.b0);
+        const int slot = b.slot;
+        for (int q = 0; q < 10; q++) {
+            const size_t stride = q < 8 ? rs : 1;
+            if (!a.out[q]) outs[q] = nullptr;
+            else if (on_dev) outs[q] = a.out[q] + row * stride;
+            else outs[q] = d_out[slot][q].as<T>();
+        }
+        mp.p = outs[0]; mp.tp = outs[1]; mp.r = outs[2]; mp.ap = outs[3]; mp.tap = outs[4];
+        mp.ndcg = outs[5]; mp.hit = outs[6]; mp.rr = outs[7]; mp.roc = outs[8]; mp.pr = outs[9];
+        mp.status_out = !ex->status ? nullptr : on_dev ? ex->status + row : d_stat_out[slot].as<int>();
+        mp.topk_items = !ex->topk_items ? nullptr : on_dev ? ex->topk_items + row * K : d_tki[slot].as<int>();
+        mp.topk_scores = !ex->topk_scores ? nullptr : on_dev ? reinterpret_cast<T*>(ex->topk_scores) + row * K : d_tks[slot].as<T>();
+        mp.pos_rank = pos_rank_d;
+        TRY(wait_test_rows());
+        user_metrics_kernel<T><<<(b.nb + METRICS_WARPS - 1) / METRICS_WARPS, METRICS_WARPS * 32, 0, st>>>(mp);
+        TRY(launched());
+        if (want_means) {
+            MeanParams<T> qp;
+            for (int q = 0; q < 10; q++) qp.out[q] = outs[q];
+            qp.nb = b.nb; qp.W = mean_W; qp.part_sum = d_psum.as<double>(); qp.part_cnt = d_pcnt.as<int>(); qp.block0 = mean_block0;
+            const int blocks = (b.nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
+            metric_partial_kernel<T><<<dim3(blocks, 10), MEAN_CHUNK, 0, st>>>(qp);
+            TRY(launched());
+            mean_block0 += blocks;
         }
         pt.stop(tm.metrics_ms);
-
-        // results of the batch -> caller's arrays at the shard's row offset (no gather collective:
-        // every shard writes its own disjoint rows)
-        if (!on_dev) {
-            CK(cudaEventRecord(rsx.ready[r_set], st));
-            CK(cudaStreamWaitEvent(rsx.s, rsx.ready[r_set], 0));
-            for (int q = 0; q < 10; q++) {
-                if (!a.out[q] || (ex && ex->skip_row_copy)) continue;
-                const size_t stride = q < 8 ? rs : 1;
-                const size_t bytes = (size_t)nb * stride * sizeof(T);
-                CK(cudaMemcpyAsync(a.out[q] + (size_t)(ub + b0) * stride, d_out[r_set][q].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
-                tm.d2h_bytes += (int64_t)bytes;
+        return RMB200_OK;
+    }
+    // results of the batch -> caller's arrays at the shard's row offset (no gather collective: every shard writes its own
+    // disjoint rows)
+    int send_results(const Batch& b)
+    {
+        if (on_dev) return RMB200_OK;
+        const size_t row = (size_t)(ub + b.b0), nb = (size_t)b.nb;
+        CK(cudaEventRecord(rsx.ready[b.slot], st));
+        CK(cudaStreamWaitEvent(rsx.s, rsx.ready[b.slot], 0));
+        for (int q = 0; q < 10; q++) {
+            if (!a.out[q] || ex->skip_row_copy) continue;
+            const size_t stride = q < 8 ? rs : 1;
+            const size_t bytes = (size_t)nb * stride * sizeof(T);
+            CK(cudaMemcpyAsync(a.out[q] + row * stride, d_out[b.slot][q].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
+            tm.d2h_bytes += (int64_t)bytes;
+        }
+        if (ex->status) { CK(cudaMemcpyAsync(ex->status + row, d_stat_out[b.slot].p, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * 4; }
+        if (ex->topk_items) { CK(cudaMemcpyAsync(ex->topk_items + row * K, d_tki[b.slot].p, (size_t)nb * K * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * 4; }
+        if (ex->topk_scores) { CK(cudaMemcpyAsync(reinterpret_cast<T*>(ex->topk_scores) + row * K, d_tks[b.slot].p, (size_t)nb * K * sizeof(T), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * (int64_t)sizeof(T); }
+        CK(cudaEventRecord(rsx.copied[b.slot], rsx.s));
+        rsx.copied_valid[b.slot] = true;
+        return RMB200_OK;
+    }
+    // ---- after the last batch: what is still in flight, held-out ranks, metric means, the filter's error statistic ----
+    int finish()
+    {
+        if (!on_dev) {                                        // what is still exposed of the result copies
+            const auto t_d = std::chrono::steady_clock::now();
+            CK(cudaStreamSynchronize(rsx.s));
+            tm.d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_d).count();
+        }
+        if (!on_dev && ex->pos_rank && !g_interrupt.load()) {
+            pt.start();
+            CK(cudaMemcpyAsync(ex->pos_rank + lo_hi[2], pos_rank_d, nnz_te * sizeof(long long), cudaMemcpyDeviceToHost, st));
+            tm.d2h_bytes += (int64_t)(nnz_te * sizeof(long long));
+            pt.stop(tm.d2h_ms);
+        }
+        if (want_means && !g_interrupt.load()) {
+            double* means_d = nullptr; long long* counts_d = nullptr;
+            const size_t cells = (size_t)10 * mean_W;
+            if (on_dev) { means_d = ex->metric_means; counts_d = reinterpret_cast<long long*>(ex->metric_counts); }
+            else {
+                if (ex->metric_means) { CK(d_means.alloc(cells * sizeof(double))); means_d = d_means.as<double>(); }
+                if (ex->metric_counts) { CK(d_mcounts.alloc(cells * sizeof(long long))); counts_d = d_mcounts.as<long long>(); }
             }
-            if (ex && ex->status) { CK(cudaMemcpyAsync(ex->status + ub + b0, d_stat_out[r_set].p, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * 4; }
-            if (ex && ex->topk_items) { CK(cudaMemcpyAsync(ex->topk_items + (size_t)(ub + b0) * K, d_tki[r_set].p, (size_t)nb * K * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * 4; }
-            if (ex && ex->topk_scores) { CK(cudaMemcpyAsync(reinterpret_cast<T*>(ex->topk_scores) + (size_t)(ub + b0) * K, d_tks[r_set].p, (size_t)nb * K * sizeof(T), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * (int64_t)sizeof(T); }
-            CK(cudaEventRecord(rsx.copied[r_set], rsx.s));
-            rsx.copied_valid[r_set] = true;
+            pt.start();
+            rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_psum.as<double>(), d_pcnt.as<int>(), mean_block0, mean_W, means_d, counts_d);
+            TRY(launched());
+            pt.stop(tm.metrics_ms);
+            if (!on_dev) {
+                if (ex->metric_means) { CK(cudaMemcpyAsync(ex->metric_means, means_d, cells * sizeof(double), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(double)); }
+                if (ex->metric_counts) { CK(cudaMemcpyAsync(ex->metric_counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
+            }
         }
-    }
-    if (!on_dev) {                                        // what is still exposed of the result copies
-        const auto t_d = std::chrono::steady_clock::now();
-        CK(cudaStreamSynchronize(rsx.s));
-        tm.d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_d).count();
-    }
-    if (!on_dev && ex && ex->pos_rank && !g_interrupt.load()) {
-        pt.start();
-        CK(cudaMemcpyAsync(ex->pos_rank + lo_hi[2], pos_rank_d, nnz_te * sizeof(long long), cudaMemcpyDeviceToHost, st));
-        tm.d2h_bytes += (int64_t)(nnz_te * sizeof(long long));
-        pt.stop(tm.d2h_ms);
-    }
-    if (want_means && !g_interrupt.load()) {
-        double* means_d = nullptr; long long* counts_d = nullptr;
-        const size_t cells = (size_t)10 * mean_W;
-        if (on_dev) { means_d = ex->metric_means; counts_d = reinterpret_cast<long long*>(ex->metric_counts); }
-        else {
-            if (ex->metric_means) { CK(d_means.alloc(cells * sizeof(double))); means_d = d_means.as<double>(); }
-            if (ex->metric_counts) { CK(d_mcounts.alloc(cells * sizeof(long long))); counts_d = d_mcounts.as<long long>(); }
+        if (use_tensor && want_filter_stats) {
+            float ratio = 0.f;
+            CK(cudaMemcpyAsync(&ratio, d_maxbn.as<unsigned>() + 1, sizeof(float), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            tm.filter_err_ratio_max = (double)ratio;
         }
-        pt.start();
-        metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_psum.as<double>(), d_pcnt.as<int>(), mean_block0, mean_W, means_d, counts_d);
-        CK(cudaGetLastError());
-        tm.kernel_launches++;
-        pt.stop(tm.metrics_ms);
-        if (!on_dev) {
-            if (ex->metric_means) { CK(cudaMemcpyAsync(ex->metric_means, means_d, cells * sizeof(double), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(double)); }
-            if (ex->metric_counts) { CK(cudaMemcpyAsync(ex->metric_counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
-        }
-    }
-    if (use_tensor && want_filter_stats) {
-        float ratio = 0.f;
-        CK(cudaMemcpyAsync(&ratio, d_maxbn.as<unsigned>() + 1, sizeof(float), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        tm.filter_err_ratio_max = (double)ratio;
+        return RMB200_OK;
     }
-    CK(cudaStreamSynchronize(st));
+};
 
-    tm.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    tm.devices_used = 1;
-    if (ex && ex->timing) *ex->timing = tm;
+template <typename T>
+int run_call(const CallArgs<T>& a)
+{
+    const auto t_begin = std::chrono::steady_clock::now();
+    const rmb200_extra_t* ex = a.ex;
+    // ---- argument checks (shape errors are the binding's job in the reference,
+    //      recometrics/wrapper.pyx:261-268; here they become RMB200_ERR_BAD_ARG) ----
+    if (a.m <= 0 || a.n <= 0 || a.k <= 0 || a.K <= 0) { set_err("bad argument", "m, n, k and k_metrics must be positive"); return RMB200_ERR_BAD_ARG; }
+    if (!a.A || !a.B || !a.trp || !a.tep) { set_err("bad argument", "A, B, Xtrain_csr_p and Xtest_csr_p are required"); return RMB200_ERR_BAD_ARG; }
+    if (a.lda < (size_t)a.k || a.ldb < (size_t)a.k) { set_err("bad argument", "lda/ldb smaller than k"); return RMB200_ERR_BAD_ARG; }
+    if (a.out[5] && !a.tev) { set_err("bad argument", "NDCG requested but Xtest_csr (values) is NULL"); return RMB200_ERR_BAD_ARG; }
+    if (ex->struct_size != (int32_t)sizeof(rmb200_extra_t)) { set_err("bad argument", "rmb200_extra_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
+    bool any_out = ex->metric_means || ex->metric_counts || ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status;
+    for (int q = 0; q < 10; q++) any_out |= (a.out[q] != nullptr);
+    if (!any_out) return RMB200_OK;
+    int ub = 0, ue = 0;
+    TRY(user_range(ex, a.m, &ub, &ue));
+    if (ue == ub) return RMB200_OK;
+
+    // ---- device ----
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+        cudaGetLastError();
+        set_err("no CUDA device", "librecometrics_b200 has no CPU fallback");
+        return RMB200_ERR_NO_DEVICE;
+    }
+    int dev = -1;
+    if (ex->device >= 0) dev = ex->device;
+    else if (const char* env = std::getenv("RMB200_DEVICE")) dev = std::atoi(env);
+    if (dev < 0) CK(cudaGetDevice(&dev));
+    if (dev >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
+    CK(cudaSetDevice(dev));
+
+    const bool nested = a.mc != nullptr;                   // run_multi() holds the mutex and the latch
+    std::unique_lock<std::mutex> lock(g_call_mutex, std::defer_lock);
+    if (!nested) lock.lock();
+    SignalLatch latch(!nested);
+    Call<T> c(a, dev, ub, ue - ub);
+    TRY(c.plan());
+    TRY(c.csr_slices());
+    TRY(c.item_factors());
+    TRY(c.item_bias());
+    TRY(c.item_image());
+    TRY(c.user_state());
+    TRY(c.batch_buffers());
+    for (int b0 = 0; b0 < c.mr; b0 += c.UB) {
+        if (g_interrupt.load()) break;                     // hpp:488-489
+        TRY(c.run_batch(b0));
+    }
+    TRY(c.finish());
+    c.tm.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    c.tm.devices_used = 1;
+    if (ex->timing) *ex->timing = c.tm;
 
     if (g_interrupt.load()) {   // hpp:167-173: restore the handler, re-raise, report
         latch.restore();
@@ -1430,18 +1443,6 @@ int run_call(const CallArgs<T>& a)
         return RMB200_ERR_INTERRUPTED;
     }
     return RMB200_OK;
-}
-
-inline const rmb200_extra_t* ex_or_default(const rmb200_extra_t* ex)
-{
-    static const rmb200_extra_t dflt = []() {
-        rmb200_extra_t e;
-        std::memset(&e, 0, sizeof(e));
-        e.struct_size = (int32_t)sizeof(e);
-        e.device = -1;
-        return e;
-    }();
-    return ex ? ex : &dflt;
 }
 
 // Which GPUs the call runs on: rmb200_extra_t::devices, else (no explicit `device`) env RMB200_DEVICES = "all" | "0,1,2,...".
@@ -1496,10 +1497,8 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     const auto t_begin = std::chrono::steady_clock::now();
     const rmb200_extra_t* ex = ex_or_default(a0.ex);
     if (a0.m <= 0) { set_err("bad argument", "m, n, k and k_metrics must be positive"); return RMB200_ERR_BAD_ARG; }
-    int ub = 0, ue = a0.m;
-    if (ex->user_end < 0) return RMB200_OK;
-    if (ex->user_begin != 0 || ex->user_end != 0) { ub = ex->user_begin; ue = ex->user_end; }
-    if (ub < 0 || ue > a0.m || ub > ue) { set_err("bad argument", "user range outside [0, m]"); return RMB200_ERR_BAD_ARG; }
+    int ub = 0, ue = 0;
+    TRY(user_range(ex, a0.m, &ub, &ue));
     // contiguous blocks in units of one CTA's 128 users; devices left without a unit sit the call out
     const int units = (ue - ub + rmb::BM - 1) / rmb::BM;
     std::vector<int> devs, lo, hi;
@@ -1619,14 +1618,13 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
     T* outs[10] = {p, tp, r, ap, tap, ndcg, hit, rr, roc, pr};
     for (int q = 0; q < 10; q++) a.out[q] = outs[q];
     a.consider_cold_start = ccs ? 1 : 0; a.min_items_pool = mip; a.min_pos_test = mpt; a.seed = seed;
-    a.bias = bias; a.ex = ex;
+    a.bias = bias; a.ex = ex_or_default(ex);
     try {
         std::vector<int> devs;
-        int rc = resolve_devices(ex, devs);
-        if (rc) return rc;
+        TRY(resolve_devices(a.ex, devs));
         if (devs.size() > 1) return run_multi<T>(a, devs);
         if (devs.size() == 1) {                 // a list of one: that device
-            rmb200_extra_t one = *ex_or_default(ex);
+            rmb200_extra_t one = *a.ex;
             one.device = devs[0]; one.devices = nullptr; one.n_devices = 0;
             a.ex = &one;
             return run_call<T>(a);
