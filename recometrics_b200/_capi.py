@@ -9,7 +9,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# RMB200_LIB: developer override used by tools/variants.sh to time alternative builds of the same library
+# RMB200_LIB: developer override, loads another build of the same library (e.g. to time two builds side by side)
 LIB_PATH = os.environ.get("RMB200_LIB") or os.path.join(_HERE, "librecometrics_b200.so")
 
 OK, ERR_BAD_ARG, ERR_NO_DEVICE, ERR_CUDA, ERR_OOM, ERR_INTERRUPTED, ERR_UNSUPPORTED, ERR_RUNTIME = range(8)

@@ -281,8 +281,7 @@ cudaError_t launch_exact_topk_inst(const uint2* capx, T* cs, int* ci, int* cc, i
     if (staging + mt_bytes <= 100 * 1024) {       // two blocks per SM
         // 16-byte copies when every factor row starts on a 16-byte boundary and is a multiple of 16 bytes long
         constexpr int V = 16 / (int)sizeof(T);
-        bool vec = (p % V == 0) && (ldb % V == 0) && ((reinterpret_cast<uintptr_t>(Brow) & 15) == 0);
-        if (const char* env = std::getenv("RMB200_EXACT_VEC")) vec = vec && std::atoi(env) != 0;      // developer: element-wise staging
+        const bool vec = (p % V == 0) && (ldb % V == 0) && ((reinterpret_cast<uintptr_t>(Brow) & 15) == 0);
         auto kern = vec ? rmb::exact_topk_kernel<T, C, 2> : rmb::exact_topk_kernel<T, C, 1>;
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(staging + mt_bytes));
         if (e != cudaSuccess) return e;
@@ -622,31 +621,14 @@ int user_range(const rmb200_extra_t* ex, int m, int* ub, int* ue)
     return RMB200_OK;
 }
 
-#ifndef RMB_F_CMID
-#define RMB_F_CMID 512              // candidate buffer of the tensor path for 32 < k_metrics <= 128
-#endif
-
-// per-batch counters of a -DRMB_F_STATS=1 build's filter (filter_select.cuh); nothing in a production build
-void print_filter_stats(const int* over_retry, int nb, int nb_pad, int sample_tiles, int sample_stride, int sample_rank)
-{
-#if RMB_F_STATS
-    std::fprintf(stderr, "[rmb200 stats] users %d: appends/user %.1f cuts/user %.2f slow-path entries/user %.1f cursor moves/user %.1f retries %d handed back %d (sample tiles %d stride %d rank %d)\n",
-                 nb, over_retry[2] / (double)nb, over_retry[3] / (double)nb, over_retry[4] / (double)nb, over_retry[5] / (double)nb,
-                 over_retry[1], over_retry[0], sample_tiles, sample_stride, sample_rank);
-    const unsigned long long* ck = reinterpret_cast<const unsigned long long*>(over_retry + 8);
-    const double nc = (double)(nb_pad / rmb::BM);
-    for (int ps = 0; ps < 2; ps++)
-        std::fprintf(stderr, "[rmb200 stats]   pass %d, one epilogue warp, kcycles per CTA: wait acc %.0f, ld+fast %.0f, append %.0f, cursor %.0f, meet+cut %.0f, total %.0f\n",
-                     ps, ck[ps * 6 + 0] / nc / 1e3, ck[ps * 6 + 1] / nc / 1e3, ck[ps * 6 + 2] / nc / 1e3, ck[ps * 6 + 3] / nc / 1e3, ck[ps * 6 + 4] / nc / 1e3, ck[ps * 6 + 5] / nc / 1e3);
-#endif
-}
-
 // One evaluation call on one device.  plan() makes every decision that needs only the arguments and the device; the resident
 // steps (csr_slices .. batch_buffers) put on the device what every batch reads; run_batch() evaluates one batch of UB users.
 // All of it runs on the legacy default stream `st`, but the uploads of host inputs (PrefetchStream) and result copies (ResultStream).
 template <typename T>
 struct Call {
     static constexpr int BN = rmb::NumTraits<T>::BN;
+    // filter counters (d_overflow): [0] users handed back to the FMA path, [1] users that took the retry pass, [6] length of the hand-back list
+    static constexpr int OVERFLOW_INTS = 7;
     struct Batch {   // users [b0, b0 + nb) of the call; slot: staging buffer of their factors (host inputs) and result set (host outputs)
         int b0, nb, nb_pad, slot; bool prefetched = false;
         const T* Asrc = nullptr; size_t Ald = 0;     // the batch's user factors, row-major on the device
@@ -666,7 +648,6 @@ struct Call {
     bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
     int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
     int fo_chunk = 0; size_t fo_bytes = 0;
-    int auc_dbg = 0, filter_dbg = 0;            // developer: RMB200_AUC_DBG / RMB200_DBG timing experiments (wrong results)
     // ---- resident state ----
     int lo_hi[4] = {0, 0, 0, 0};                // trp[ub], trp[ue], tep[ub], tep[ue]
     size_t nnz_tr = 0, nnz_te = 0;
@@ -705,13 +686,11 @@ struct Call {
         want_roc = a.out[8] != nullptr; want_pr = a.out[9] != nullptr;
         count_ranks = want_roc || want_pr || ex->pos_rank;
         want_means = ex->metric_means || ex->metric_counts;
-        want_filter_stats = ex->filter_stats || std::getenv("RMB200_FILTER_STATS") != nullptr;
+        want_filter_stats = ex->filter_stats != 0;
         p_pad = round_up(a.k, KPAD);
         n_pad = round_up(a.n, BN);
         rs = a.cumulative ? (size_t)K : 1;
         mean_W = a.cumulative ? K : 1;
-        if (const char* env = std::getenv("RMB200_AUC_DBG")) auc_dbg = std::atoi(env);
-        if (const char* env = std::getenv("RMB200_DBG")) filter_dbg = std::atoi(env);
         // ---- which scoring path: tensor-core filter + exact re-scoring (top-K only), or FMA tiles ----
         int path_req = ex->scoring_path;                                 // 0 auto, 1 fma, 2 tensor
         if (path_req == 0) if (const char* env = std::getenv("RMB200_PATH")) {
@@ -726,7 +705,6 @@ struct Call {
         const long long tile = (long long)KB * 256, budget = 227 * 1024 - (long long)filter_smem_fixed_bytes();
         f_stages = (int)(budget / tile) - 1;
         if (f_stages > F_MAX_STAGES) f_stages = F_MAX_STAGES;
-        if (const char* env = std::getenv("RMB200_STAGES")) { const int v = std::atoi(env); if (v >= 2 && v < f_stages) f_stages = v; }   // developer: shallower ring
         // With rank counting (ROC/PR-AUC) every score has to be exact: the FMA tiles do everything.  Exception: with the
         // reference's tie-breaking noise the ranked top-K comes from the tensor path as well (its exact stage is where the
         // noise is applied, tie_noise.cuh), after the FMA pass has counted the ranks.
@@ -743,8 +721,7 @@ struct Call {
         // held-out item, the candidates within the noise's reach; users for whom the noise decides a rank are handed to the full-order path
         noise_handback = a.noise && count_ranks && !use_full;
         tm.scoring_path = use_full ? 3 : (use_tensor ? 2 : 1);
-        if (use_tensor) C = (K <= 32) ? 256 : (K <= 128 ? RMB_F_CMID : 1024);
-        if (use_tensor) if (const char* env = std::getenv("RMB200_FILTER_C")) { const int v = std::atoi(env); if ((v == 256 || v == 512 || v == 1024) && v >= C) C = v; }   // developer
+        if (use_tensor) C = (K <= 32) ? 256 : (K <= 128 ? 512 : 1024);
         if (use_full) C = round_up(K < a.n ? K : a.n, 32);              // row pitch of the ranked lists
         n_pad128 = round_up(a.n, 128);
         // ---- user batches ----
@@ -772,16 +749,11 @@ struct Call {
         // in a million users (those users' CTAs walk the catalogue a second time; results never depend on the guess)
         if (use_tensor) {
             const int NT = (a.n + 127) / 128;
-            int min_tiles = 512;
-            if (const char* env = std::getenv("RMB200_SAMPLE_MIN_TILES")) { const int v = std::atoi(env); if (v >= 16) min_tiles = v; }   // developer
-            bool on = NT >= min_tiles;
-            if (const char* env = std::getenv("RMB200_SAMPLE")) on = on && std::atoi(env) != 0;
-            if (on) {
+            if (NT >= 512) {                                                  // (64K items and up)
                 double frac = 7.0 / K;
                 if (frac < 1.0 / 16) frac = 1.0 / 16;
                 if (frac > 1.0 / 8) frac = 1.0 / 8;
-                int stride = (int)(1.0 / frac);
-                if (const char* env = std::getenv("RMB200_SAMPLE_STRIDE")) { const int v = std::atoi(env); if (v >= 2) stride = v; }
+                const int stride = (int)(1.0 / frac);
                 const int ns = NT / stride;                                  // tiles 0, stride, ..., (ns-1)*stride: all full tiles
                 const double lam = (double)K * ((double)ns * 128.0) / (double)a.n;
                 double term = std::exp(-lam), cdf = 0.0;                     // P(X <= r-1), X ~ Poisson(lam)
@@ -801,7 +773,6 @@ struct Call {
             if (sl > NT_all / 8) sl = NT_all / 8;                       // (at least eight item tiles per range)
             if (sl > C / K) sl = C / K;                                 // the joined heads fit one row ...
             if (sl > 512 / K) sl = 512 / K;                             // ... and the final sort
-            if (const char* env = std::getenv("RMB200_SLICES")) { const int v = std::atoi(env); if (v >= 1 && v < sl) sl = v; }      // developer
             if (sl > 1) fma_slices = sl;
         }
         return RMB200_OK;
@@ -1005,7 +976,7 @@ struct Call {
             CK(d_Ab.alloc((size_t)UB * KB * sizeof(__half)));
             CK(d_anorm.alloc((size_t)UB * sizeof(float)));
             CK(d_capx.alloc((size_t)UB * C * sizeof(uint2)));
-            CK(d_overflow.alloc(40 * sizeof(int)));    // [0] users handed back to the FMA path, [1] users that took the retry pass, [6] length of the hand-back list, [8..] cycle counters (stats builds)
+            CK(d_overflow.alloc(OVERFLOW_INTS * sizeof(int)));
             CK(d_fb_list.alloc((size_t)UB * sizeof(int)));
         }
         if (!on_dev) {
@@ -1135,7 +1106,6 @@ struct Call {
         sp.umap = umap;
         const int slices = (umap == nullptr && !use_tensor) ? fma_slices : 1;
         sp.slice_rows = slices > 1 ? UB : 0;
-        sp.dbg = auc_dbg;
         if (timed) cudaEventRecord(pk.a, st);
         CK(launch_score_select<T>(sp, C, with_counts, n_rows, slices, st));
         if (timed) cudaEventRecord(pk.b, st);
@@ -1195,7 +1165,7 @@ struct Call {
         pack_f16_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(b.Asrc, b.Ald, b.nb, a.k, (const T*)nullptr, a.bias ? 1 : 0,
                                                                             d_anorm.as<float>(), nullptr, d_Ab.as<__half>(), b.nb_pad, KB);
         TRY(launched(2));
-        CK(cudaMemsetAsync(d_overflow.p, 0, 40 * sizeof(int), st));
+        CK(cudaMemsetAsync(d_overflow.p, 0, OVERFLOW_INTS * sizeof(int), st));
         pt.stop(tm.prep_ms);
         pt.start();
         const FilterErrCoef ec = filter_err_coefs(KB);
@@ -1210,7 +1180,6 @@ struct Call {
         fp.sample_tiles = f_sample_tiles; fp.sample_stride = f_sample_stride; fp.sample_rank = f_sample_rank;
         fp.retries = d_overflow.as<int>() + 1;
         fp.noise_band = a.noise ? 2.02e-12f : 0.f;
-        fp.dbg = filter_dbg;
         cudaEventRecord(pk.a, st);
         CK(launch_filter_select(fp, C, b.nb_pad / BM, st));
         cudaEventRecord(pk.b, st);
@@ -1227,10 +1196,9 @@ struct Call {
         CK(launch_exact_topk<T>(d_capx.as<uint2>(), d_cs.as<T>(), d_ci.as<int>(), d_cc.as<int>(), C, b.nb, b.b0, d_At.as<T>(), p_pad, a.k,
                                 Bsrc, Bld, bias_d, d_flags.as<int>(), K, nz, es, st));
         tm.kernel_launches++;
-        int over_retry[40] = {0};
-        CK(cudaMemcpyAsync(over_retry, d_overflow.p, 40 * sizeof(int), cudaMemcpyDeviceToHost, st));
+        int over_retry[OVERFLOW_INTS] = {0};
+        CK(cudaMemcpyAsync(over_retry, d_overflow.p, OVERFLOW_INTS * sizeof(int), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        print_filter_stats(over_retry, b.nb, b.nb_pad, f_sample_tiles, f_sample_stride, f_sample_rank);
         const int n_over = over_retry[0];
         tm.filter_retry_rows += over_retry[1];
         if (n_over == 0) return RMB200_OK;

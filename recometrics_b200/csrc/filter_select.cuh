@@ -51,61 +51,19 @@ namespace rmb {
 
 constexpr int FN = 128;                  // items per MMA tile = TMEM columns per accumulator buffer
 constexpr int F_EPI_WARPS = 16;          // warp w reads TMEM lanes (user rows) 32*(w%4)..+31, column chunk w/4 of every tile
-#ifndef RMB_F_MMA_WARPS
-#define RMB_F_MMA_WARPS 2                // MMA-issuing warps, taking turns tile by tile: one warp's per-tile barrier waits and commits
-#endif                                   // (~300 cycles in which it issues nothing) overlap with the other warp's MMAs
-constexpr int F_MMA_WARPS = RMB_F_MMA_WARPS;
+constexpr int F_MMA_WARPS = 2;           // MMA-issuing warps, taking turns tile by tile: one warp's per-tile barrier waits and commits
+                                         // (~300 cycles in which it issues nothing) overlap with the other warp's MMAs
 constexpr int F_THREADS = (F_EPI_WARPS + 1 + F_MMA_WARPS) * 32;   // + TMA producer warp + MMA warps
-#ifndef RMB_F_ACCBUFS
-#define RMB_F_ACCBUFS 4                  // TMEM accumulator buffers (2 or 4): slack between the MMA warp and the slowest epilogue warp
-#endif
-constexpr int F_ACCBUFS = RMB_F_ACCBUFS;
-constexpr int F_ACCSHIFT = F_ACCBUFS == 4 ? 2 : 1;
+constexpr int F_ACCBUFS = 4;             // TMEM accumulator buffers: slack between the MMA warp and the slowest epilogue warp
+constexpr int F_ACCSHIFT = 2;            // log2(F_ACCBUFS): a buffer's phase parity flips every F_ACCBUFS iterations
 constexpr int F_TMEM_COLS = F_ACCBUFS * FN;
 constexpr int F_MAX_STAGES = 6;              // ring depth: as many B tiles as fit next to the A tile (5 at 128 factors)
 constexpr int F_CHUNK = 32;              // TMEM columns per tcgen05.ld
-#ifndef RMB_F_CUT_MARGIN
-#define RMB_F_CUT_MARGIN 48               // a row's regions are cut back together once they hold this many more than the last cut kept
-#endif
-constexpr int F_CUT_MARGIN = RMB_F_CUT_MARGIN;
-#ifndef RMB_F_MAIN_MARGIN
-#define RMB_F_MAIN_MARGIN 250              // ... in the pass that starts from the sampled guess: its thresholds are tight from the first tile on, a cut
-                                           // (which stalls its warp and soon the CTA's pipeline) buys little there (A/B on B200: 52 -> 47.4 ms per batch)
-#endif
-constexpr int F_MAIN_MARGIN = RMB_F_MAIN_MARGIN;
-#ifndef RMB_F_COMPACT_AT
-#define RMB_F_COMPACT_AT 0                // a cut compacts the row's regions only when one of them holds more than this (0: every cut compacts)
-#endif
-constexpr int F_COMPACT_AT = RMB_F_COMPACT_AT;
-#ifndef RMB_F_MAX_MEET
-#define RMB_F_MAX_MEET 64                 // most item tiles between two meetings of a quarter's warps
-#endif
-constexpr int F_MAX_MEET = RMB_F_MAX_MEET;
-
-#ifndef RMB_F_FAST_APPEND
-#define RMB_F_FAST_APPEND 1              // predicated in-line appends on the common slow path (0: always the out-of-line group function)
-#endif
-#ifndef RMB_F_NO_CN
-#define RMB_F_NO_CN 0
-#endif
-#ifndef RMB_F_DBG
-#define RMB_F_DBG 0                      // developer build: honour FilterParams::dbg (env RMB200_DBG) inside the tile loop
-#endif
-#ifndef RMB_F_STATS
-#define RMB_F_STATS 0                    // developer build: count appends / cuts / slow-path entries / cursor moves into FilterParams::retries[1..4]
-#endif
-#if RMB_F_STATS
-#define F_STAT(i, v) atomicAdd(&rs->stat[i], (v))
-#define F_CLK(var) const long long var = clock64()
-#define F_CLK_ADD(i, a, b) do { if (warp == RMB_F_STAT_WARP && lane == 0) clk[i] += (b) - (a); } while (0)
-#else
-#define F_STAT(i, v) do { } while (0)
-#define F_CLK(var) do { } while (0)
-#define F_CLK_ADD(i, a, b) do { } while (0)
-#endif
-#ifndef RMB_F_STAT_WARP
-#define RMB_F_STAT_WARP 5
-#endif
+constexpr int F_CUT_MARGIN = 48;         // a row's regions are cut back together once they hold this many more than the last cut kept
+constexpr int F_MAIN_MARGIN = 250;       // ... in the pass that starts from the sampled guess: its thresholds are tight from the first tile on, a cut
+                                         // (which stalls its warp and soon the CTA's pipeline) buys little there (A/B on B200: 52 -> 47.4 ms per batch)
+constexpr int F_MAX_MEET = 64;           // most item tiles between two meetings of a quarter's warps
+constexpr int F_CUT_BITS = 10;           // bisection steps of the cuts at the meetings (the cut at the end of a pass is exact: 32)
 
 struct FilterParams {
     const __half* __restrict__ Ab;          // [user tiles][KB/8][128][8]  fp16 user factors (+1.0 bias column), each row scaled by pow2_scale_for(||a_u||)
@@ -128,7 +86,6 @@ struct FilterParams {
     int K;
     int sample_tiles, sample_stride, sample_rank;   // pass 0 (see filter_pass_tile); sample_tiles == 0: no sampling
     int* retries;                           // rows that needed the retry pass (statistics; may be nullptr)
-    int dbg;                                // developer switch (env RMB200_DBG): 1 = skip the scan (pipeline ceiling), 2 = no row is ranked (fast path only), 4 = no meetings, 8 = no tcgen05.ld, 16 = no TMA after the first ring round, 32 = half of the k steps (bits honoured only in -DRMB_F_DBG=1 builds)
 };
 
 struct FilterRowState {      // per user row of the CTA, shared by the four epilogue warps of its TMEM lane quarter
@@ -146,7 +103,6 @@ struct FilterRowState {      // per user row of the CTA, shared by the four epil
     int tot_prev[4][BM];             // per warp: row total after the previous meeting (the same value in the quarter's four warps)
     int interval[F_EPI_WARPS];       // per warp: tiles between its last two meetings
     int retry;                       // some row of the CTA needs the retry pass
-    int stat[4];                     // RMB_F_STATS: appends, cuts, slow-path entries (8-column groups), cursor moves
 };
 
 
@@ -230,24 +186,20 @@ __device__ __forceinline__ float filter_err(const float ca, const float cn, cons
 
 // One warp: cut a row's candidates back to those that can still belong to the exact top K.  Every candidate carries the
 // LOWER bound lb = approx - e of its exact score (e from its item's chunk norm); its upper bound is lb + 2e.
-// tau' = the K-th best lower bound; kept: KEEP_LB ? lb >= tau' (sample pass: the K best lower bounds themselves) :
-// ub >= tau' (whatever can still reach the exact top K).  The row's buffer is four regions of C/4 entries (one per
-// epilogue warp of the quarter), region s holding cnt4[s] entries; all of them are read into registers first, so the
-// survivors can be written back in place: CONTIG ? packed at the head of the buffer : dealt round-robin over the regions.
+// tau' = the K-th best lower bound; kept: ub >= tau' (whatever can still reach the exact top K).  The row's buffer is
+// four regions of C/4 entries (one per epilogue warp of the quarter), region s holding cnt4[s] entries; all of them are
+// read into registers first, so the survivors can be written back in place: CONTIG ? packed at the head of the buffer :
+// dealt round-robin over the regions.
 // tau' is found by bisection on the order-preserving keys: BITS halvings of [min key, max key], each one a count of the
 // keys at or above the probe (compare + warp REDUX).  The interval's lower end always satisfies #(lb key >= lo) >= K,
 // so it is a valid (slightly low: interval width = key range / 2^BITS) stand-in for tau'; BITS = 32 makes it exact.
 // A cut stalls its warp -- and, once the four accumulator buffers have run full, the whole CTA -- for its duration:
 // one load phase, no shared-memory traffic, no shuffles inside the search.  K <= total entries is required.
-// compact = false: only the bound is refreshed, the regions stay as they are.
 // Returns the number kept; *tau_out = (the stand-in for) tau'.
-#ifndef RMB_F_CUT_BITS
-#define RMB_F_CUT_BITS 10
-#endif
 template <int C, int BITS, bool CONTIG>
 __device__ __noinline__ int cut_regions(uint2* cd, const int c0, const int c1, const int c2, const int c3, const int K,
-                                        const float ca, const float efl, const float* __restrict__ chunk_norm, const bool keep_lb,
-                                        const bool compact, const int lane, float* tau_out)
+                                        const float ca, const float efl, const float* __restrict__ chunk_norm,
+                                        const int lane, float* tau_out)
 {
     constexpr int E = C / 32, RC = C / 4, EPR = E / 4;      // entries per lane, region capacity, per-lane entries per region
     const int ns = (max(max(c0, c1), max(c2, c3)) + 31) >> 5;      // occupied 32-entry slots per region (warp-uniform): the rest is skipped
@@ -283,17 +235,16 @@ __device__ __noinline__ int cut_regions(uint2* cd, const int c0, const int c1, c
     }
     const float tau = NumTraits<float>::from_orderable((u64)lo);
     *tau_out = tau;
-    if (!compact) { __syncwarp(); return c0 + c1 + c2 + c3; }      // bound refreshed, the regions stay as they are
     const unsigned cut = (tau == tau) ? lo : 1u;               // NaN bound (K NaN scores): keep everything
     // write-back: an entry whose lower bound reaches the cut stays; one below it stays iff its UPPER bound lb + 2e does
-    // (sample pass: lower bounds only) -- only those look their error bound up.
+    // -- only those look their error bound up.
     int base = 0;
     __syncwarp();
 #pragma unroll
     for (int e = 0; e < E; e++) {
         if ((e % EPR) < ns) {
             bool keep = lbk[e] != 0u && lbk[e] >= cut;
-            if (!keep && !keep_lb && lbk[e] != 0u) {
+            if (!keep && lbk[e] != 0u) {
                 const float er = filter_err(ca, chunk_norm[(unsigned)it[e] >> 5], efl);
                 const float ub = __fadd_ru(NumTraits<float>::from_orderable((u64)lbk[e]), __fadd_ru(er, er));
                 keep = NumTraits<float>::key(ub) >= cut;
@@ -388,7 +339,6 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
         mbar_init(bar_a, 1);
         mbar_fence_init();
         rs->retry = 0;
-        for (int i = 0; i < 4; i++) rs->stat[i] = 0;
     }
     if (warp == F_EPI_WARPS + 1) {      // the MMA warp owns the tensor-memory allocation
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"((unsigned)F_TMEM_COLS));
@@ -413,14 +363,9 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
             for (int j = 0; j < ntiles; j++) {
                 mbar_wait(bar_empty + 8 * s, ph ^ 1);                         // first round passes immediately
                 if (elect_one()) {
-#if RMB_F_DBG
-                    if ((P.dbg & 16) && it0 + j >= S) { mbar_arrive(bar_full + 8 * s); } else       // 16: no TMA after the first round (stale tiles)
-#endif
-                    {
                     mbar_arrive_expect_tx(bar_full + 8 * s, tile_bytes);
                     tma_bulk_g2s(smem_u32(b_ring) + (unsigned)s * tile_bytes, P.Bb + (size_t)filter_pass_tile(P, pass, j) * KB * 128,
                                  tile_bytes, bar_full + 8 * s);
-                    }
                 }
                 __syncwarp();
                 if (++s == S) { s = 0; ph ^= 1; }
@@ -430,10 +375,7 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
             // D fp32 (bit 4), A and B fp16 (format 0 at bits 7 and 10), both K-major, N=128 (>>3 at bit 17), M=128 (>>4 at bit 24)
             const unsigned idesc = (1u << 4) | ((unsigned)(FN >> 3) << 17) | ((128u >> 4) << 24);
             const uint64_t adesc0 = umma_desc(smem_u32(a_tile)), bdesc0 = umma_desc(smem_u32(b_ring));
-            int ksteps = KB / 16;                                             // K=16 per MMA = two 16-byte k chunks of 2048 B
-#if RMB_F_DBG
-            if (P.dbg & 32) ksteps = ksteps / 2 > 0 ? ksteps / 2 : 1;         // 32: half of the k steps
-#endif
+            const int ksteps = KB / 16;                                       // K=16 per MMA = two 16-byte k chunks of 2048 B
             const int w = warp - (F_EPI_WARPS + 1);
             mbar_wait(bar_a, 0);
             int j = (w - it0 % F_MMA_WARPS + F_MMA_WARPS) % F_MMA_WARPS;      // first iteration of this pass that is this warp's
@@ -465,9 +407,8 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
             const int ul = tile_u0 + row;
             const unsigned qbar = 1 + q;                    // named barrier of the quarter's four warps
             const int Kp = pass == 0 ? P.sample_rank : P.K; // how many best candidates the pass keeps track of
-            const bool keep_lb = pass == 0;
             if (slot == 0) {
-                bool ranked = (ul < P.mb) && (P.ustatus[P.user0 + ul] == 0) && !(RMB_F_DBG && (P.dbg & 2));
+                bool ranked = (ul < P.mb) && (P.ustatus[P.user0 + ul] == 0);
                 if (pass < 2 && (pass == 0 || P.sample_tiles == 0)) {            // first pass of the CTA: the row's error-bound terms
                     int fl = 0;
                     float ca = 0.f, efl = 0.f;
@@ -533,9 +474,6 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                 int item_base = slot * F_CHUNK;
                 const int item_step = P.sample_stride * FN;
                 const unsigned taddr0 = tmem_base + ((unsigned)(q * 32) << 16) + (unsigned)(slot * F_CHUNK);
-#if RMB_F_STATS
-                const long long clk_pass0 = clock64();
-#endif
 #pragma unroll 1
                 for (int left = ntiles; left > 0; left--, item_base += item_step) {
                     const int tile_end = item_base - slot * F_CHUNK + FN;
@@ -608,53 +546,30 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                     }
                 }
                 asm volatile("bar.sync %0, 128;" ::"r"(qbar) : "memory");
-#if RMB_F_STATS
-                if (warp == RMB_F_STAT_WARP && lane == 0 && P.retries)
-                    atomicAdd(reinterpret_cast<unsigned long long*>(P.retries + 7) + 5, (unsigned long long)(clock64() - clk_pass0));
-#endif
             } else {
-            // error bound in the tile loop: the sample pass compares the approximate scores themselves (the cut then keeps
-            // the best LOWER bounds); the other passes test upper bounds, approx + e >= tau'
-            const float ca_l = pass == 0 ? 0.f : rs->ca[row];
-            float tau_m = pass == 0 ? tau : __fsub_rd(tau, rs->efl[row]);          // tau' minus the row's constant error term
+            // error bound in the tile loop: candidates pass on their upper bounds, approx + e >= tau'
+            const float ca_l = rs->ca[row];
+            float tau_m = __fsub_rd(tau, rs->efl[row]);     // tau' minus the row's constant error term
             int meet_in = 0;                                // tiles until the next meeting
-#if RMB_F_STATS
-            long long clk[6] = {0, 0, 0, 0, 0, 0};          // one warp's cycles: waiting for the accumulator, tcgen05.ld + fast path, appends, cursor moves, meetings + cuts, pass total
-            const long long clk_pass0 = clock64();
-#endif
             // loop-carried pipeline state, kept incrementally (no per-tile index arithmetic): accumulator buffer and its phase
-            // parity, first item id of this warp's 32-column chunk, the item step between two tiles of the pass
+            // parity, first item id of this warp's 32-column chunk
             int buf = it0 & (F_ACCBUFS - 1);
             unsigned par = (unsigned)(it0 >> F_ACCSHIFT) & 1u;
             int item_base = slot * F_CHUNK;
-            const int item_step = (pass == 0 ? P.sample_stride : 1) * FN;
             const unsigned taddr0 = tmem_base + ((unsigned)(q * 32) << 16) + (unsigned)(slot * F_CHUNK);
 
 #pragma unroll 1
-            for (int left = ntiles; left > 0; left--, item_base += item_step) {
+            for (int left = ntiles; left > 0; left--, item_base += FN) {
                 const int tile_end = item_base - slot * F_CHUNK + FN;
-#if RMB_F_NO_CN
-                const float cn = __uint_as_float(*P.maxbn);                    // developer: one bound for the whole catalogue (timing experiments)
-#else
                 const float cn = __ldg(P.chunk_norm + (item_base >> 5));       // largest item norm of this chunk (in flight while the warp waits)
-#endif
-                F_CLK(t_a);
                 mbar_wait(bar_accf + 8 * buf, par);
                 tc_fence_after();
-                F_CLK(t_b);
-                F_CLK_ADD(0, t_a, t_b);
                 unsigned v[32];
-#if RMB_F_DBG
-                if (!(P.dbg & 8))
-#endif
                 tmem_ld32(taddr0 + (unsigned)(buf * FN), v);
                 tc_fence_before();                      // this warp's part of the accumulator is in registers
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_acce + 8 * buf);
                 if (++buf == F_ACCBUFS) { buf = 0; par ^= 1u; }
-#if RMB_F_DBG
-                if (P.dbg & 1) continue;
-#endif
                 const bool has_train = t_nxt < tile_end;
                 // NaN-propagating max of each group of 8 columns; one compare for the whole chunk, groups only when it passes
                 float gm[4];
@@ -667,65 +582,40 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                     gm[g] = max_nan(max_nan(m01, m23), max_nan(m45, m67));
                 }
                 const float thr = __fmaf_rd(-ca_l, cn, tau_m);                     // approx < thr: the upper bound stays below tau'
-                F_CLK(t_c);
                 if (!(max_nan(max_nan(gm[0], gm[1]), max_nan(gm[2], gm[3])) < thr)) {
                     uint2* cd = P.cand + ((size_t)ul * C + slot * RC);            // this warp's region of the row's buffer
                     asm volatile("" : "+l"(cd));                                  // (one pointer, indexed by the fill: keeps the address math to one IMAD.WIDE per store)
                     const float err = filter_err(rs->ca[row], cn, rs->efl[row]);  // candidates are stored with their lower bound
-#if RMB_F_FAST_APPEND
                     if (!has_train && tile_end <= P.n && mycnt <= RC - F_CHUNK) {
                         // common case (no train item of the row in this tile, no padding column, room for the whole chunk):
                         // predicated appends, no calls, no loops
 #pragma unroll
                         for (int g = 0; g < 4; g++) {
                             if (!(gm[g] < thr)) {
-                                F_STAT(2, 1);
-                                const int before = mycnt;
 #pragma unroll
                                 for (int e8 = 0; e8 < 8; e8++) {
-#if RMB_F_FAST_APPEND == 2
-                                    // branch-free: every score of the group is stored at the region's end, the fill only moves
-                                    // past the ones that pass (what lies beyond the fill is never read; the region has room for
-                                    // the whole chunk).  A divergent branch costs this warp more than seven wasted stores.
-                                    const float sc = __uint_as_float(v[8 * g + e8]);
-                                    cd[mycnt] = make_uint2(__float_as_uint(__fsub_rd(sc, err)), (unsigned)(item_base + 8 * g + e8));
-                                    mycnt += (sc < thr) ? 0 : 1;
-#else
                                     if (!(__uint_as_float(v[8 * g + e8]) < thr)) {
                                         cd[mycnt] = make_uint2(__float_as_uint(__fsub_rd(__uint_as_float(v[8 * g + e8]), err)), (unsigned)(item_base + 8 * g + e8));
                                         mycnt++;
                                     }
-#endif
                                 }
-                                F_STAT(0, mycnt - before);
-                                (void)before;
                             }
                         }
-                    } else
-#endif
-                    {
+                    } else {
 #pragma unroll
-                    for (int g = 0; g < 4; g++) {
-                        if (!(gm[g] < thr)) {
-                            F_STAT(2, 1);
-                            const int before = mycnt;
-                            const int t_cur = rs->tcur[slot][row];
-                            mycnt = filter_append_group<RC>(__uint_as_float(v[8 * g + 0]), __uint_as_float(v[8 * g + 1]), __uint_as_float(v[8 * g + 2]),
-                                                            __uint_as_float(v[8 * g + 3]), __uint_as_float(v[8 * g + 4]), __uint_as_float(v[8 * g + 5]),
-                                                            __uint_as_float(v[8 * g + 6]), __uint_as_float(v[8 * g + 7]), thr, err, item_base + 8 * g, P.n,
-                                                            P.tri, t_cur, has_train ? rs->tend[row] : t_cur, cd, mycnt, row);
-                            F_STAT(0, mycnt - before);
-                            (void)before;
+                        for (int g = 0; g < 4; g++) {
+                            if (!(gm[g] < thr)) {
+                                const int t_cur = rs->tcur[slot][row];
+                                mycnt = filter_append_group<RC>(__uint_as_float(v[8 * g + 0]), __uint_as_float(v[8 * g + 1]), __uint_as_float(v[8 * g + 2]),
+                                                                __uint_as_float(v[8 * g + 3]), __uint_as_float(v[8 * g + 4]), __uint_as_float(v[8 * g + 5]),
+                                                                __uint_as_float(v[8 * g + 6]), __uint_as_float(v[8 * g + 7]), thr, err, item_base + 8 * g, P.n,
+                                                                P.tri, t_cur, has_train ? rs->tend[row] : t_cur, cd, mycnt, row);
+                            }
                         }
                     }
-                    }
                 }
-                F_CLK(t_d);
-                F_CLK_ADD(1, t_b, t_c);
-                F_CLK_ADD(2, t_c, t_d);
                 // move the train cursor past this tile: the id after t_nxt was prefetched into shared memory when the cursor last moved
                 if (has_train) {
-                    F_STAT(3, 1);
                     asm volatile("cp.async.wait_all;" ::: "memory");
                     int nxt = rs->nxt2_train[slot][row];
                     int t_cur = rs->tcur[slot][row] + 1;
@@ -737,12 +627,7 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                         asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(&rs->nxt2_train[slot][row])), "l"(P.tri + t_cur + 1) : "memory");
                     else rs->nxt2_train[slot][row] = INT_MAX;
                 }
-                F_CLK(t_e);
-                F_CLK_ADD(3, t_d, t_e);
                 if (--meet_in >= 0 && left > 1) continue;
-#if RMB_F_DBG
-                if (P.dbg & 4) continue;
-#endif
 
                 // ---- meeting point of the quarter's four warps: publish the region fills, cut rows that grew past their trigger
                 rs->cnt4[slot][row] = mycnt;
@@ -759,21 +644,16 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                         if ((r & 3) != slot) continue;                         // the quarter's warps share the work
                         const int rr = q * 32 + r;
                         float tau_r;
-                        // compact only when the regions run short of room; otherwise just refresh the row's bound
-                        const bool compact = max(max(rs->cnt4[0][rr], rs->cnt4[1][rr]), max(rs->cnt4[2][rr], rs->cnt4[3][rr])) > F_COMPACT_AT;
-                        const int kept = cut_regions<C, RMB_F_CUT_BITS, false>(P.cand + (size_t)(tile_u0 + rr) * C, rs->cnt4[0][rr], rs->cnt4[1][rr],
-                                                                                  rs->cnt4[2][rr], rs->cnt4[3][rr], Kp, rs->ca[rr], rs->efl[rr], P.chunk_norm,
-                                                                                  keep_lb, compact, lane, &tau_r);
+                        const int kept = cut_regions<C, F_CUT_BITS, false>(P.cand + (size_t)(tile_u0 + rr) * C, rs->cnt4[0][rr], rs->cnt4[1][rr],
+                                                                              rs->cnt4[2][rr], rs->cnt4[3][rr], Kp, rs->ca[rr], rs->efl[rr], P.chunk_norm,
+                                                                              lane, &tau_r);
                         if (lane == 0) {
-                            F_STAT(1, 1);
                             float t_new = fmaxf(tau_r, rs->tau[rr]);            // an earlier (valid) bound may be the sharper one; a NaN bound is ignored
-                            if (compact && kept > 4 * (RC - 32)) { rs->flags[rr] |= 2; t_new = CUDART_INF_F; }     // the kept band does not fit
+                            if (kept > 4 * (RC - 32)) { rs->flags[rr] |= 2; t_new = CUDART_INF_F; }     // the kept band does not fit
                             rs->tau[rr] = t_new;
                             rs->trig[rr] = kept + (pass == 1 && P.sample_tiles > 0 ? F_MAIN_MARGIN : F_CUT_MARGIN);
-                            if (compact) {
 #pragma unroll
-                                for (int sgm = 0; sgm < 4; sgm++) rs->cnt4[sgm][rr] = (kept + 3 - sgm) >> 2;
-                            }
+                            for (int sgm = 0; sgm < 4; sgm++) rs->cnt4[sgm][rr] = (kept + 3 - sgm) >> 2;
                         }
                     }
                     asm volatile("bar.sync %0, 128;" ::"r"(qbar) : "memory");
@@ -783,7 +663,7 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                 }
                 tau = rs->tau[row];
                 if (rs->flags[row] & 2) { mycnt = 0; tau = CUDART_INF_F; if (slot == 0) rs->tau[row] = CUDART_INF_F; }     // the row is closed: whatever it holds is void
-                tau_m = pass == 0 ? tau : __fsub_rd(tau, rs->efl[row]);
+                tau_m = __fsub_rd(tau, rs->efl[row]);
                 const int interval = rs->interval[warp];
                 // next meeting: far enough that barriers are rare, close enough that no region can fill up at twice the
                 // append rate just seen (all of it into one region); a burst beyond that closes the row (flag 2)
@@ -792,8 +672,6 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                 nxt_iv = __reduce_min_sync(FULL, nxt_iv);
                 nxt_iv = nxt_iv < 1 ? 1 : (nxt_iv > F_MAX_MEET ? F_MAX_MEET : nxt_iv);
                 meet_in = nxt_iv - 1;
-                F_CLK(t_f);
-                F_CLK_ADD(4, t_e, t_f);
                 rs->tot_prev[slot][row] = tot;
                 if (lane == 0) rs->interval[warp] = nxt_iv;
             }
@@ -808,27 +686,16 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                 const bool have_k = nv >= Kp && !(rs->flags[rr] & 2);
                 if (nv > 0 && !(rs->flags[rr] & 2)) {
                     const int kept = cut_regions<C, 32, true>(P.cand + (size_t)(tile_u0 + rr) * C, c0, c1, c2, c3, have_k ? Kp : nv, rs->ca[rr], rs->efl[rr],
-                                                             P.chunk_norm, keep_lb, true, lane, &tau_r);
-                    if (lane == 0 && pass > 0) rs->cnt[rr] = kept;      // last cut: the exact stage gets only what can still be in the top K
+                                                             P.chunk_norm, lane, &tau_r);
+                    if (lane == 0) rs->cnt[rr] = kept;                  // last cut: the exact stage gets only what can still be in the top K
                 }
-                if (lane == 0) {
-                    if (pass == 0) {
-                        rs->guess[rr] = (have_k && tau_r == tau_r) ? tau_r : -CUDART_INF_F;   // too small a sample / overflow: no guess
-                        rs->flags[rr] &= ~2;
-                    } else if (pass == 1 && !(rs->flags[rr] & 2)) {
-                        const float g = rs->guess[rr];
-                        const bool ok = (g == -CUDART_INF_F) || (have_k && !(tau_r < g));     // >= K kept lower bounds reach the guess (a NaN bound: everything was kept)
-                        if (!ok) { rs->flags[rr] |= 4; rs->retry = 1; }
-                    }
+                if (lane == 0 && pass == 1 && !(rs->flags[rr] & 2)) {
+                    const float g = rs->guess[rr];
+                    const bool ok = (g == -CUDART_INF_F) || (have_k && !(tau_r < g));     // >= K kept lower bounds reach the guess (a NaN bound: everything was kept)
+                    if (!ok) { rs->flags[rr] |= 4; rs->retry = 1; }
                 }
             }
             asm volatile("bar.sync %0, 128;" ::"r"(qbar) : "memory");
-#if RMB_F_STATS
-            if (warp == RMB_F_STAT_WARP && lane == 0 && P.retries) {
-                clk[5] = clock64() - clk_pass0;
-                for (int i = 0; i < 6; i++) atomicAdd(reinterpret_cast<unsigned long long*>(P.retries + 7) + (pass == 0 ? 0 : 6) + i, (unsigned long long)clk[i]);
-            }
-#endif
             }   // (passes 1 and 2)
         }
         it0 += ntiles;
@@ -851,9 +718,6 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
 
     tc_fence_before();
     __syncthreads();
-#if RMB_F_STATS
-    if (tid < 4 && P.retries) atomicAdd(P.retries + 1 + tid, rs->stat[tid]);
-#endif
     if (warp == F_EPI_WARPS + 1)
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((unsigned)F_TMEM_COLS));
 }

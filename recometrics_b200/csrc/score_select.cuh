@@ -44,17 +44,6 @@
 #include <limits.h>
 #include <string.h>
 
-// build-time tuning knobs of the FMA loop (tools/variants.sh times the alternatives)
-#ifndef RMB_SWPIPE
-#define RMB_SWPIPE 0        // 1: explicit register double buffering of the operand fragments
-#endif
-#ifndef RMB_UNROLL
-#define RMB_UNROLL 8        // factors per unrolled block of the FMA loop (multiple of KPAD)
-#endif
-#ifndef RMB_EARLYTRY
-#define RMB_EARLYTRY 0      // 1: probe the next stage's mbarrier one block before it is needed
-#endif
-
 namespace rmb {
 
 constexpr int BM = 128;             // users per CTA tile (items per tile: NumTraits<T>::BN)
@@ -206,8 +195,6 @@ struct ScoreSelectParams {
     int slice_rows;                     // item slices (gridDim.y > 1: a call with fewer user tiles than SMs cuts the catalogue into ranges, one CTA per
                                         // (user tile, range)): rows of cand_score / cand_item / cand_count per slice -- slice y keeps the best K of its
                                         // range in rows [y * slice_rows, ...), merge_slices_kernel joins them; rank counts are then added atomically
-    int dbg;                            // developer (RMB200_AUC_DBG, timing experiments only -- results are wrong): 1 counting warps skip the
-                                        // counting, 2 they skip masking / minima as well, 4 no hand-over of score blocks at all, 8 the FMA warps do a quarter of their FMAs
     const int* __restrict__ umap;       // optional [mb]: row r of this launch is batch-local user umap[r] (CSR rows, status, flags and
                                         // candidate buffers are those of the mapped user; At holds the launch's rows in order).  Used
                                         // to re-run only the users the tensor-core filter handed back (api.cu)
@@ -242,17 +229,6 @@ __device__ __forceinline__ void mbar_wait(const unsigned bar, const unsigned par
             "selp.u32 %0, 1, 0, p;\n\t}"
             : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
     } while (!ok);
-}
-// non-blocking probe (the result arrives ~90 cycles later: issue it early, test it late)
-__device__ __forceinline__ unsigned mbar_try(const unsigned bar, const unsigned parity)
-{
-    unsigned ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok;
 }
 // global -> shared bulk copy executed by the TMA unit, completion counted on an mbarrier
 __device__ __forceinline__ void tma_bulk_g2s(const unsigned dst, const void* src, const unsigned bytes, const unsigned bar)
@@ -764,7 +740,7 @@ __device__ __noinline__ void auc_count_role(const ScoreSelectParams<T>& P, RowSt
     }
     T rmin = NumTraits<T>::inf();
     // (pointers of the parameter block in registers: through the reference every use is a load from the parameter space)
-    const int dbg = P.dbg, n_items = P.n;
+    const int n_items = P.n;
     const int* const tri_g = P.tri;
     unsigned int* const cnt_g = P.auc_cnt;
     const unsigned int* const near_g = P.auc_near;
@@ -772,89 +748,84 @@ __device__ __noinline__ void auc_count_role(const ScoreSelectParams<T>& P, RowSt
     const int* const item_g = P.pos_item;
     count_sync();                                                // (the staged entries are visible)
 
-    if (dbg & 4) return;
     for (int tile = 0; tile < NT; tile++) {
         const int item0 = (t_begin + tile) * BN;
         mbar_wait(bar_blkf + 8 * cw, (unsigned)tile & 1u);
-        if (!(dbg & 2)) {
-            if (lane < 16) {
-                T* dst = blk + (size_t)lane * BNP;
-                while (t_nxt < item0 + BN) {
-                    dst[t_nxt - item0] = NumTraits<T>::nan();
-                    t_cur++;
-                    t_nxt = t_cur < t_end ? tri_g[t_cur] : INT_MAX;
-                }
-                if (item0 + BN > n_items)
-                    for (int x = (n_items > item0 ? n_items - item0 : 0); x < BN; x++) dst[x] = NumTraits<T>::nan();
+        if (lane < 16) {
+            T* dst = blk + (size_t)lane * BNP;
+            while (t_nxt < item0 + BN) {
+                dst[t_nxt - item0] = NumTraits<T>::nan();
+                t_cur++;
+                t_nxt = t_cur < t_end ? tri_g[t_cur] : INT_MAX;
             }
-            __syncwarp();
-            const T* src = blk + (size_t)(lane >> 1) * BNP + (lane & 1) * (BN / 2);
-            constexpr int VEC = 16 / (int)sizeof(T);
-            T m0 = NumTraits<T>::inf(), m1 = NumTraits<T>::inf();
-#pragma unroll 4
-            for (int x = 0; x < BN / 2; x += 2 * VEC) {
-                T v[VEC], w[VEC];
-                lds_vec(src + x, v);
-                lds_vec(src + x + VEC, w);
-#pragma unroll
-                for (int e = 0; e < VEC; e++) { m0 = fmin(m0, v[e]); m1 = fmin(m1, w[e]); }     // fmin ignores NaN
-            }
-            rmin = fmin(rmin, fmin(m0, m1));
+            if (item0 + BN > n_items)
+                for (int x = (n_items > item0 ? n_items - item0 : 0); x < BN; x++) dst[x] = NumTraits<T>::nan();
         }
+        __syncwarp();
+        const T* half_row = blk + (size_t)(lane >> 1) * BNP + (lane & 1) * (BN / 2);
+        constexpr int VEC = 16 / (int)sizeof(T);
+        T m0 = NumTraits<T>::inf(), m1 = NumTraits<T>::inf();
+#pragma unroll 4
+        for (int x = 0; x < BN / 2; x += 2 * VEC) {
+            T v[VEC], w[VEC];
+            lds_vec(half_row + x, v);
+            lds_vec(half_row + x + VEC, w);
+#pragma unroll
+            for (int e = 0; e < VEC; e++) { m0 = fmin(m0, v[e]); m1 = fmin(m1, w[e]); }     // fmin ignores NaN
+        }
+        rmin = fmin(rmin, fmin(m0, m1));
         count_sync();                                            // all 128 rows of the tile are staged and masked
-        if (!(dbg & 3)) {
-            for (int j = 0, u = tc; u < n_units; j++, u += NCT) {
-                int row;
-                if (j < 4) row = j == 0 ? unit_row[0] : (j == 1 ? unit_row[1] : (j == 2 ? unit_row[2] : unit_row[3]));
-                else {
-                    int lo = 0, hi = BM - 1;
-                    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (upref[mid] <= u) lo = mid; else hi = mid - 1; }
-                    row = lo;
-                }
-                const int q = pref[row] + UN * (u - upref[row]);                   // first entry of the unit
-                const int run = min(pref[row + 1] - q, UN);
-                const size_t e0 = (size_t)rs->tp0[row] + (size_t)(q - pref[row]);
-                const T* src = blk_all + (size_t)row * BNP;
-                // the unit's counters, scores and item ids: unconditional loads (entries past the unit's end re-read its first
-                // one), all in flight together -- the counters come from L2, a dependent load per entry cost more than the counting
-                unsigned before[UN];
-                T thr[UN], eff[UN];
-                int col[UN];
+        for (int j = 0, u = tc; u < n_units; j++, u += NCT) {
+            int row;
+            if (j < 4) row = j == 0 ? unit_row[0] : (j == 1 ? unit_row[1] : (j == 2 ? unit_row[2] : unit_row[3]));
+            else {
+                int lo = 0, hi = BM - 1;
+                while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (upref[mid] <= u) lo = mid; else hi = mid - 1; }
+                row = lo;
+            }
+            const int q = pref[row] + UN * (u - upref[row]);                   // first entry of the unit
+            const int run = min(pref[row + 1] - q, UN);
+            const size_t e0 = (size_t)rs->tp0[row] + (size_t)(q - pref[row]);
+            const T* src = blk_all + (size_t)row * BNP;
+            // the unit's counters, scores and item ids: unconditional loads (entries past the unit's end re-read its first
+            // one), all in flight together -- the counters come from L2, a dependent load per entry cost more than the counting
+            unsigned before[UN];
+            T thr[UN], eff[UN];
+            int col[UN];
 #pragma unroll
-                for (int t = 0; t < UN; t++) before[t] = sliced ? 0u : cnt_g[e0 + (t < run ? t : 0)];
-                if (q + UN <= PCAP) {
+            for (int t = 0; t < UN; t++) before[t] = sliced ? 0u : cnt_g[e0 + (t < run ? t : 0)];
+            if (q + UN <= PCAP) {
 #pragma unroll
-                    for (int t = 0; t < UN; t++) { thr[t] = pthr[q + t]; col[t] = pitem[q + t] - item0; }
-                } else {
+                for (int t = 0; t < UN; t++) { thr[t] = pthr[q + t]; col[t] = pitem[q + t] - item0; }
+            } else {
 #pragma unroll
-                    for (int t = 0; t < UN; t++) { thr[t] = sorted_g[e0 + (t < run ? t : 0)]; col[t] = item_g[e0 + (t < run ? t : 0)] - item0; }
-                }
-                unsigned banded = 0;                                          // entries within the noise's reach of other candidates: below
+                for (int t = 0; t < UN; t++) { thr[t] = sorted_g[e0 + (t < run ? t : 0)]; col[t] = item_g[e0 + (t < run ? t : 0)] - item0; }
+            }
+            unsigned banded = 0;                                          // entries within the noise's reach of other candidates: below
 #pragma unroll
-                for (int t = 0; t < UN; t++) {
-                    bool on = t < run;
-                    if (on && near_g != nullptr && noise_reach(thr[t]) > (T)0) { banded |= 1u << t; on = false; }
-                    if (!on) col[t] = 0;
-                    eff[t] = !on ? NumTraits<T>::inf() : (col[t] >= BN ? next_below<T>(thr[t]) : thr[t]);
-                }
-                unsigned c[UN];
-                count_above<UN>(src, eff, c);
+            for (int t = 0; t < UN; t++) {
+                bool on = t < run;
+                if (on && near_g != nullptr && noise_reach(thr[t]) > (T)0) { banded |= 1u << t; on = false; }
+                if (!on) col[t] = 0;
+                eff[t] = !on ? NumTraits<T>::inf() : (col[t] >= BN ? next_below<T>(thr[t]) : thr[t]);
+            }
+            unsigned c[UN];
+            count_above<UN>(src, eff, c);
 #pragma unroll
-                for (int t = 0; t < UN; t++) {
-                    if (t < run && !((banded >> t) & 1u)) {
-                        unsigned ct = c[t];
-                        if (col[t] > 0 && col[t] < BN)
-                            for (int x = 0; x < col[t]; x++) ct += (src[x] == thr[t]);
-                        if (!sliced) cnt_g[e0 + t] = before[t] + ct;
-                        else if (ct) atomicAdd(&cnt_g[e0 + t], ct);
-                    }
+            for (int t = 0; t < UN; t++) {
+                if (t < run && !((banded >> t) & 1u)) {
+                    unsigned ct = c[t];
+                    if (col[t] > 0 && col[t] < BN)
+                        for (int x = 0; x < col[t]; x++) ct += (src[x] == thr[t]);
+                    if (!sliced) cnt_g[e0 + t] = before[t] + ct;
+                    else if (ct) atomicAdd(&cnt_g[e0 + t], ct);
                 }
-                while (banded) {
-                    const int t = __ffs(banded) - 1;
-                    banded &= banded - 1;
-                    auc_count_banded<T>(P, src, e0 + t, t == 0 ? thr[0] : (t == 1 ? thr[1] : (UN > 2 && t == 2 ? thr[UN > 2 ? 2 : 0] : thr[UN - 1])),
-                                        (q + t < PCAP ? pitem[q + t] : item_g[e0 + t]) - item0);
-                }
+            }
+            while (banded) {
+                const int t = __ffs(banded) - 1;
+                banded &= banded - 1;
+                auc_count_banded<T>(P, src, e0 + t, t == 0 ? thr[0] : (t == 1 ? thr[1] : (UN > 2 && t == 2 ? thr[UN > 2 ? 2 : 0] : thr[UN - 1])),
+                                    (q + t < PCAP ? pitem[q + t] : item_g[e0 + t]) - item0);
             }
         }
         __syncwarp();
@@ -960,48 +931,25 @@ score_select_kernel(const __grid_constant__ ScoreSelectParams<T> P)
     const int wrow0 = warp * 16;                    // first CTA row of this warp
     T* blk = reinterpret_cast<T*>(smem_raw + L::blk_off) + (size_t)warp * 16 * BNP;   // AUC only: [16][BNP]
     MicroTile<T> mt;
-    typename MicroTile<T>::Frag frag[2];            // operand registers, double buffered across k
+    typename MicroTile<T>::Frag frag;               // operand registers of one k step
     int it = 0;
-    unsigned ready = mbar_try(bar_full, 0);         // probe of the stage about to be consumed
     for (int tile = 0; tile < NT; tile++) {
         const int item0 = (t_begin + tile) * BN;
         mt.zero();
         for (int kc = 0; kc < KC; kc++, it++) {
             const int s = it % S;
-            if (!ready) mbar_wait(bar_full + 8 * s, (it / S) & 1);
+            mbar_wait(bar_full + 8 * s, (it / S) & 1);
             const int k0 = kc * BK;
-            const int kcount = (P.p_pad - k0) < BK ? (P.p_pad - k0) : BK;
+            const int kcount = (P.p_pad - k0) < BK ? (P.p_pad - k0) : BK;      // a multiple of KPAD
             const T* sA = As + (size_t)s * BK * UM + wrow0;
             const T* sB = Bs + (size_t)s * BK * BN;
-#if RMB_SWPIPE
-            MicroTile<T>::load(frag[0], sA, sB, ly, lx);
             for (int kk0 = 0; kk0 < kcount; kk0 += KPAD) {
-                if (kk0 + KPAD >= kcount) {          // last block of the stage: probe the next stage now
-                    const int nit = it + 1;
-                    ready = (nit < total) ? mbar_try(bar_full + 8 * (nit % S), (nit / S) & 1) : 1u;
-                }
 #pragma unroll
                 for (int kk = 0; kk < KPAD; kk++) {
-                    if (kk + 1 < KPAD || kk0 + KPAD < kcount)
-                        MicroTile<T>::load(frag[(kk + 1) & 1], sA + (kk0 + kk + 1) * UM, sB + (kk0 + kk + 1) * BN, ly, lx);
-                    mt.compute(frag[kk & 1]);
+                    MicroTile<T>::load(frag, sA + (kk0 + kk) * UM, sB + (kk0 + kk) * BN, ly, lx);
+                    mt.compute(frag);
                 }
             }
-#else
-            for (int kk0 = 0; kk0 < ((AUC && (P.dbg & 8) && kc > 0) ? 0 : kcount); kk0 += RMB_UNROLL) {     // (developer, dbg & 8: a quarter of the FMAs -- the counting warps set the pace)
-                if (RMB_EARLYTRY && kk0 + RMB_UNROLL >= kcount) {   // last block of the stage: probe the next stage now
-                    const int nit = it + 1;
-                    ready = (nit < total) ? mbar_try(bar_full + 8 * (nit % S), (nit / S) & 1) : 1u;
-                }
-#pragma unroll
-                for (int kk = 0; kk < RMB_UNROLL; kk++) {
-                    if (RMB_UNROLL > KPAD && kk0 + kk >= kcount) break;     // only the tail chunk of a k that is not a multiple of the unroll
-                    MicroTile<T>::load(frag[0], sA + (kk0 + kk) * UM, sB + (kk0 + kk) * BN, ly, lx);
-                    mt.compute(frag[0]);
-                }
-            }
-            if (!RMB_EARLYTRY) ready = 0;
-#endif
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_empty + 8 * s);
         }
@@ -1013,7 +961,7 @@ score_select_kernel(const __grid_constant__ ScoreSelectParams<T> P)
             for (int c = 0; c < NC; c++) biasv[c] = P.bias[item0 + lx * 4 + (c & 3) + (c >> 2) * 64];
         }
         bool inserted = false;
-        if (AUC && tile > 0 && !(P.dbg & 4)) mbar_wait(bar_blke + 8 * warp, (unsigned)(tile - 1) & 1u);      // the counting warp is done with the previous block
+        if (AUC && tile > 0) mbar_wait(bar_blke + 8 * warp, (unsigned)(tile - 1) & 1u);      // the counting warp is done with the previous block
 #pragma unroll
         for (int i = 0; i < 8; i++) {
             const int row_l = ly * 4 + (i & 3) + (i >> 2) * 8;
@@ -1035,14 +983,14 @@ score_select_kernel(const __grid_constant__ ScoreSelectParams<T> P)
                     row_slow<T>(rs, cs, ci, P.tri, P.n, tau, row, item0 + 64 + lx * 4, item0 + BN, s[NC - 4], s[NC - 3], s[NC - 2], s[NC - 1]);
                 inserted = true;
             }
-            if (AUC && !(P.dbg & 4)) {
+            if (AUC) {
                 T* dst = blk + (size_t)row_l * BNP + lx * 4;
                 sts4(dst, &s[0]);
                 if (NC == 8) sts4(dst + 64, &s[NC - 4]);
             }
         }
         __syncwarp();
-        if (AUC && lane == 0 && !(P.dbg & 4)) mbar_arrive(bar_blkf + 8 * warp);      // the tile's score block is the counting warp's now
+        if (AUC && lane == 0) mbar_arrive(bar_blkf + 8 * warp);      // the tile's score block is the counting warp's now
 
         // advance the train cursors of the warp's rows past this tile (lanes 0..15, rare)
         if (lane < 16) {

@@ -12,7 +12,3 @@ timeout 300 ncu --set full --import-source on --clock-control none -k regex:scor
     python tools/run_once.py --config 3 --users 37888 --reps 1 > gpurun_out/ncu_auc_${TAG}.log 2>&1
 fi
 cat gpurun_out/quick_tests_${TAG}.txt | cut -c1-300; cat gpurun_out/quick_bench_cfg3_${TAG}.log | cut -c1-900
-if [ -n "$CFG2" ]; then
-( for v in 512 128 64 32; do echo "== RMB200_SAMPLE_MIN_TILES=$v"; RMB200_SAMPLE_MIN_TILES=$v timeout 120 python tools/run_once.py --config 2 --users 138493 --reps 3 2>&1 | tail -1 | cut -c1-330; done ) > gpurun_out/cfg2_sample_${TAG}.log 2>&1
-cat gpurun_out/cfg2_sample_${TAG}.log
-fi
