@@ -183,6 +183,56 @@ RMB200_API int rmb200_calc_metrics_ex_f64(
     int32_t nthreads, uint64_t seed,
     const double *item_biases, const rmb200_extra_t *extra);
 
+/* Item exposure of the ranked top-K lists of one call (zero-initialise, then set struct_size = sizeof(rmb200_exposure_t)).
+ * Counted are the users of the call ([user_begin, user_end), every device of a multi-GPU call) whose ranked list is defined
+ * (status 0: exactly the users whose topk_items row the call writes); each adds its min(k_metrics, candidates) listed items.
+ * item_counts[j] = how many counted users have item j in their list = numpy.bincount(topk_items[topk_items >= 0], minlength=n).
+ * The statistics depend only on the integer counts and are computed by rmb200_exposure_stats, on the host:
+ *   coverage = items_covered / n;  gini = sum_i (2i - n - 1) c_(i) / (n * entries) over ALL n items, c ascending (RecBole's
+ *   GiniIndex: one item holding everything gives (n - 1) / n, uniform exposure 0);  entropy_bits = -sum_{c_j > 0} p_j log2 p_j,
+ *   p_j = c_j / entries.  With entries = 0: coverage 0, gini and entropy_bits NaN.  Statistics at k_metrics only (also
+ *   when cumulative). */
+typedef struct rmb200_exposure {
+    int32_t struct_size;          /* = sizeof(rmb200_exposure_t)                                                          */
+    int32_t reserved0;            /* padding                                                                              */
+    int64_t *item_counts;         /* optional out [n]; a device pointer when extra->inputs_on_device                     */
+    int64_t users, entries, items_covered;     /* out: counted users, listed entries (sum of item_counts), items with a count > 0 */
+    double  coverage, gini, entropy_bits;      /* out                                                                     */
+} rmb200_exposure_t;
+
+/* rmb200_calc_metrics_ex_f32 / _f64 plus the item exposure of the call's ranked lists; exposure == NULL is exactly the _ex
+ * call.  Requesting it counts as an output (a call with only `exposure` computes the ranked lists).  An interrupted call writes
+ * nothing into `exposure`; an empty user block gives zero counts and the statistics of no entry. */
+RMB200_API int rmb200_calc_metrics_exposure_f32(
+    const float *A, size_t lda, const float *B, size_t ldb,
+    int32_t m, int32_t n, int32_t k,
+    const int32_t *Xtrain_csr_p, const int32_t *Xtrain_csr_i,
+    const int32_t *Xtest_csr_p, const int32_t *Xtest_csr_i, const float *Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    float *p_at_k, float *tp_at_k, float *r_at_k, float *ap_at_k, float *tap_at_k,
+    float *ndcg_at_k, float *hit_at_k, float *rr_at_k, float *roc_auc, float *pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test,
+    int32_t nthreads, uint64_t seed,
+    const float *item_biases, const rmb200_extra_t *extra, rmb200_exposure_t *exposure);
+
+RMB200_API int rmb200_calc_metrics_exposure_f64(
+    const double *A, size_t lda, const double *B, size_t ldb,
+    int32_t m, int32_t n, int32_t k,
+    const int32_t *Xtrain_csr_p, const int32_t *Xtrain_csr_i,
+    const int32_t *Xtest_csr_p, const int32_t *Xtest_csr_i, const double *Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    double *p_at_k, double *tp_at_k, double *r_at_k, double *ap_at_k, double *tap_at_k,
+    double *ndcg_at_k, double *hit_at_k, double *rr_at_k, double *roc_auc, double *pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test,
+    int32_t nthreads, uint64_t seed,
+    const double *item_biases, const rmb200_extra_t *extra, rmb200_exposure_t *exposure);
+
+/* Host only, needs no GPU: entries, items_covered, coverage, gini and entropy_bits of `out` from counts[n] -- the function the
+ * library itself uses after every call, so that counts summed over shards give the statistics of the whole run.  users and
+ * item_counts are left alone.  RMB200_ERR_BAD_ARG for n <= 0, a negative count, a total beyond int64 or a wrong struct_size. */
+RMB200_API int rmb200_exposure_stats(const int64_t *counts, int32_t n, rmb200_exposure_t *out);
+RMB200_API int rmb200_sizeof_exposure(void);
+
 /* Number of usable CUDA devices (0 = the library cannot compute). */
 RMB200_API int rmb200_device_count(void);
 /* RMB200_VERSION of the loaded library. */

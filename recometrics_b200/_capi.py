@@ -22,6 +22,7 @@ TOPK_METRICS = METRIC_ORDER[:8]
 EXPORTS = (
     "rmb200_calc_metrics_f32", "rmb200_calc_metrics_f64",
     "rmb200_calc_metrics_ex_f32", "rmb200_calc_metrics_ex_f64",
+    "rmb200_calc_metrics_exposure_f32", "rmb200_calc_metrics_exposure_f64", "rmb200_exposure_stats", "rmb200_sizeof_exposure",
     "rmb200_device_count", "rmb200_version", "rmb200_last_error",
     "rmb200_request_interrupt", "rmb200_measure_fma_peak", "rmb200_release_workspace",
     "rmb200_sizeof_extra", "rmb200_sizeof_timing",
@@ -60,6 +61,28 @@ class Extra(ctypes.Structure):
         ("has_nan_bits", ctypes.c_int32), ("filter_stats", ctypes.c_int32), ("nan_bits", ctypes.c_uint64),
         ("devices", ctypes.POINTER(ctypes.c_int32)), ("n_devices", ctypes.c_int32), ("reserved0", ctypes.c_int32),
     ]
+
+
+class Exposure(ctypes.Structure):
+    """rmb200_exposure_t (include/recometrics_b200.h): item exposure of a call's ranked lists."""
+    _fields_ = [
+        ("struct_size", ctypes.c_int32), ("reserved0", ctypes.c_int32), ("item_counts", ctypes.c_void_p),
+        ("users", ctypes.c_int64), ("entries", ctypes.c_int64), ("items_covered", ctypes.c_int64),
+        ("coverage", ctypes.c_double), ("gini", ctypes.c_double), ("entropy_bits", ctypes.c_double),
+    ]
+
+    def catalogue(self):
+        """The statistics as the front-ends return them (``EvalResult.catalogue``)."""
+        return {"Coverage@K": float(self.coverage), "Gini@K": float(self.gini), "Entropy@K": float(self.entropy_bits),
+                "users": int(self.users), "entries": int(self.entries), "items_covered": int(self.items_covered)}
+
+
+def make_exposure(item_counts=None):
+    """rmb200_exposure_t asking for the exposure of a call; `item_counts`: int64 numpy array [n], device address or None."""
+    e = Exposure()
+    e.struct_size = ctypes.sizeof(Exposure)
+    e.item_counts = _vp(item_counts)
+    return e
 
 
 class Csr(ctypes.Structure):
@@ -107,16 +130,18 @@ def load():
     lib.rmb200_sizeof_extra.restype = ctypes.c_int
     lib.rmb200_sizeof_timing.restype = ctypes.c_int
     lib.rmb200_sizeof_split.restype = ctypes.c_int
+    lib.rmb200_sizeof_exposure.restype = ctypes.c_int
     if (lib.rmb200_sizeof_extra() != ctypes.sizeof(Extra) or lib.rmb200_sizeof_timing() != ctypes.sizeof(Timing)
-            or lib.rmb200_sizeof_split() != ctypes.sizeof(Split)):
+            or lib.rmb200_sizeof_split() != ctypes.sizeof(Split) or lib.rmb200_sizeof_exposure() != ctypes.sizeof(Exposure)):
         raise NativeLibraryError("recometrics_b200: %s was built from a different include/recometrics_b200.h (struct sizes differ); rebuild it" % LIB_PATH)
     lib.rmb200_last_error.restype = ctypes.c_char_p
     lib.rmb200_request_interrupt.restype = None
     lib.rmb200_release_workspace.restype = None
     lib.rmb200_measure_fma_peak.restype = ctypes.c_double
     lib.rmb200_measure_fma_peak.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)]
-    for name in EXPORTS[:4]:
+    for name in EXPORTS[:7]:
         getattr(lib, name).restype = ctypes.c_int
+    lib.rmb200_exposure_stats.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(Exposure)]
     for name in EXPORTS:
         if name.startswith("rmb200_split_") and name != "rmb200_split_free":
             getattr(lib, name).restype = ctypes.c_int
@@ -181,12 +206,13 @@ def _vp(x):
 
 def calc_metrics(dtype, A, lda, B, ldb, m, n, k, trp, tri, tep, tei, tev, k_metrics, cumulative,
                  break_ties_with_noise, outs, consider_cold_start, min_items_pool, min_pos_test,
-                 nthreads=1, seed=1, item_biases=None, extra=None):
-    """Thin call into rmb200_calc_metrics_ex_{f32,f64}.  Array arguments are numpy arrays (host
-    memory), raw integer addresses (device memory, with extra.inputs_on_device=1) or None.
-    `outs` maps metric name -> array/address/None in METRIC_ORDER.  Returns the status code."""
+                 nthreads=1, seed=1, item_biases=None, extra=None, exposure=None):
+    """Thin call into rmb200_calc_metrics_ex_{f32,f64} (rmb200_calc_metrics_exposure_{f32,f64} with an `exposure` struct).
+    Array arguments are numpy arrays (host memory), raw integer addresses (device memory, with extra.inputs_on_device=1) or
+    None.  `outs` maps metric name -> array/address/None in METRIC_ORDER.  Returns the status code."""
     lib = load()
-    fn = lib.rmb200_calc_metrics_ex_f32 if np.dtype(dtype) == np.float32 else lib.rmb200_calc_metrics_ex_f64
+    kind = "ex" if exposure is None else "exposure"
+    fn = getattr(lib, "rmb200_calc_metrics_%s_%s" % (kind, "f32" if np.dtype(dtype) == np.float32 else "f64"))
     args = [
         _vp(A), ctypes.c_size_t(int(lda)), _vp(B), ctypes.c_size_t(int(ldb)),
         ctypes.c_int32(int(m)), ctypes.c_int32(int(n)), ctypes.c_int32(int(k)),
@@ -199,7 +225,19 @@ def calc_metrics(dtype, A, lda, B, ldb, m, n, k, trp, tri, tep, tei, tev, k_metr
         ctypes.c_int32(int(nthreads)), ctypes.c_uint64(int(seed)),
         _vp(item_biases), ctypes.byref(extra) if extra is not None else ctypes.c_void_p(None),
     ]
+    if exposure is not None:
+        args.append(ctypes.byref(exposure))
     return int(fn(*args))
+
+
+def exposure_stats(counts, users=0):
+    """rmb200_exposure_stats (host only, no GPU): the catalogue statistics of int64 item counts [n], as
+    ``Exposure.catalogue()`` returns them; `users` is passed through (the counts do not tell it)."""
+    counts = np.ascontiguousarray(counts, dtype=np.int64)
+    e = make_exposure()
+    raise_for_status(load().rmb200_exposure_stats(_vp(counts), ctypes.c_int32(int(counts.size)), ctypes.byref(e)))
+    e.users = int(users)
+    return e.catalogue()
 
 
 def make_extra(device=-1, user_begin=0, user_end=0, inputs_on_device=False, strict_min_pos_test=False,

@@ -26,6 +26,7 @@
 #include "prep.cuh"
 #include "score_select.cuh"
 #include "filter_select.cuh"
+#include "exposure.cuh"
 #include "full_order.h"
 
 namespace {
@@ -226,6 +227,7 @@ struct CallArgs {
     uint64_t seed;
     const T* bias;
     const rmb200_extra_t* ex;
+    rmb200_exposure_t* expo = nullptr;   // item exposure of the ranked lists (exposure.cuh); null: not requested
 };
 
 template <typename T, int C, bool AUC>
@@ -621,6 +623,25 @@ int user_range(const rmb200_extra_t* ex, int m, int* ub, int* ue)
     return RMB200_OK;
 }
 
+// The statistics of item counts (exposure.cuh) into *out: what every call that asks for them and rmb200_exposure_stats do
+int exposure_stats(const int64_t* counts, int n, rmb200_exposure_t* out)
+{
+    if (!rmb::exposure_stats_host(counts, n, out)) { set_err("bad argument", "item counts: n <= 0, a negative count or a total beyond int64"); return RMB200_ERR_BAD_ARG; }
+    return RMB200_OK;
+}
+
+// The exposure of a call that evaluates nobody (an empty user block): zero counts, no user
+int exposure_of_nobody(rmb200_exposure_t* expo, int n, bool counts_on_device)
+{
+    std::vector<int64_t> zero((size_t)n, 0);
+    if (expo->item_counts) {
+        if (counts_on_device) CK(cudaMemset(expo->item_counts, 0, (size_t)n * sizeof(int64_t)));
+        else std::memset(expo->item_counts, 0, (size_t)n * sizeof(int64_t));
+    }
+    expo->users = 0;
+    return exposure_stats(zero.data(), n, expo);
+}
+
 // One evaluation call on one device.  plan() makes every decision that needs only the arguments and the device; the resident
 // steps (csr_slices .. batch_buffers) put on the device what every batch reads; run_batch() evaluates one batch of UB users.
 // All of it runs on the legacy default stream `st`, but the uploads of host inputs (PrefetchStream) and result copies (ResultStream).
@@ -644,7 +665,7 @@ struct Call {
     int mip = 0, mpt = 0, C = 0, p_pad = 0, n_pad = 0, n_pad128 = 0, KB = 0, f_stages = 0, nsm = 148, UB = 0, fma_slices = 1, mean_W = 1;
     size_t rs = 1;
     T nan_value = std::numeric_limits<T>::quiet_NaN();
-    bool want_roc = false, want_pr = false, count_ranks = false, want_means = false, want_filter_stats = false;
+    bool want_roc = false, want_pr = false, count_ranks = false, want_means = false, want_filter_stats = false, want_exposure = false;
     bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
     int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
     int fo_chunk = 0; size_t fo_bytes = 0;
@@ -662,6 +683,7 @@ struct Call {
     DevBuf d_At, d_cs, d_ci, d_cc, d_out[2][10], d_tki[2], d_tks[2], d_stat_out[2], d_Ab, d_anorm;
     DevBuf d_capx, d_overflow, d_fb_list, d_At_fb;
     DevBuf d_psum, d_pcnt, d_means, d_mcounts;
+    DevBuf d_expo_hist, d_list_len, d_expo_counts;
     PrefetchStream pf;                          // (declared after the buffers they fill or read: destroyed, i.e. drained, before them)
     ResultStream rsx;
     Call(const CallArgs<T>& args, int device, int user_begin, int users) : a(args), ex(args.ex), on_dev(args.ex->inputs_on_device != 0),
@@ -687,6 +709,7 @@ struct Call {
         count_ranks = want_roc || want_pr || ex->pos_rank;
         want_means = ex->metric_means || ex->metric_counts;
         want_filter_stats = ex->filter_stats != 0;
+        want_exposure = a.expo != nullptr;
         p_pad = round_up(a.k, KPAD);
         n_pad = round_up(a.n, BN);
         rs = a.cumulative ? (size_t)K : 1;
@@ -1001,6 +1024,12 @@ struct Call {
             CK(d_psum.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(double)));
             CK(d_pcnt.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(int)));
         }
+        // item exposure: one uint32 count per item for the whole call (at most mr users each), [n] = users counted
+        if (want_exposure) {
+            CK(d_expo_hist.alloc(((size_t)a.n + 1) * sizeof(unsigned)));
+            CK(cudaMemsetAsync(d_expo_hist.p, 0, ((size_t)a.n + 1) * sizeof(unsigned), st));
+            CK(d_list_len.alloc((size_t)UB * sizeof(int)));
+        }
         return RMB200_OK;
     }
     // upload of users [b0, b0 + UB) into staging buffer `slot`, on the prefetch stream
@@ -1271,9 +1300,15 @@ struct Call {
         mp.topk_items = !ex->topk_items ? nullptr : on_dev ? ex->topk_items + row * K : d_tki[slot].as<int>();
         mp.topk_scores = !ex->topk_scores ? nullptr : on_dev ? reinterpret_cast<T*>(ex->topk_scores) + row * K : d_tks[slot].as<T>();
         mp.pos_rank = pos_rank_d;
+        mp.list_len = want_exposure ? d_list_len.as<int>() : nullptr;
         TRY(wait_test_rows());
         user_metrics_kernel<T><<<(b.nb + METRICS_WARPS - 1) / METRICS_WARPS, METRICS_WARPS * 32, 0, st>>>(mp);
         TRY(launched());
+        if (want_exposure) {
+            exposure_count_kernel<<<(b.nb + EXPOSURE_THREADS - 1) / EXPOSURE_THREADS, EXPOSURE_THREADS, 0, st>>>(
+                d_ci.as<int>(), C, d_list_len.as<int>(), b.nb, d_expo_hist.as<unsigned>(), a.n);
+            TRY(launched());
+        }
         if (want_means) {
             MeanParams<T> qp;
             for (int q = 0; q < 10; q++) qp.out[q] = outs[q];
@@ -1339,6 +1374,7 @@ struct Call {
                 if (ex->metric_counts) { CK(cudaMemcpyAsync(ex->metric_counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
             }
         }
+        if (want_exposure && !g_interrupt.load()) TRY(exposure_out());
         if (use_tensor && want_filter_stats) {
             float ratio = 0.f;
             CK(cudaMemcpyAsync(&ratio, d_maxbn.as<unsigned>() + 1, sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -1347,6 +1383,29 @@ struct Call {
         }
         CK(cudaStreamSynchronize(st));
         return RMB200_OK;
+    }
+    // the call's item counts, widened to int64, into the caller's array (device-resident calls: on the device, then a copy for
+    // the statistics) or an internal one; the statistics from them on the host
+    int exposure_out()
+    {
+        int64_t* dst_d = on_dev ? a.expo->item_counts : nullptr;
+        if (!dst_d) { CK(d_expo_counts.alloc((size_t)a.n * sizeof(int64_t))); dst_d = d_expo_counts.as<int64_t>(); }
+        pt.start();
+        rmb::exposure_widen_kernel<<<(a.n + 255) / 256 < 4 * nsm ? (a.n + 255) / 256 : 4 * nsm, 256, 0, st>>>(
+            d_expo_hist.as<unsigned>(), a.n, reinterpret_cast<long long*>(dst_d));
+        TRY(launched());
+        pt.stop(tm.metrics_ms);
+        std::vector<int64_t> own;
+        int64_t* dst_h = on_dev ? nullptr : a.expo->item_counts;
+        if (!dst_h) { own.resize((size_t)a.n); dst_h = own.data(); }
+        unsigned users = 0;
+        pt.start();
+        CK(cudaMemcpyAsync(dst_h, dst_d, (size_t)a.n * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(&users, d_expo_hist.as<unsigned>() + a.n, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
+        tm.d2h_bytes += (int64_t)a.n * (int64_t)sizeof(int64_t) + (int64_t)sizeof(unsigned);
+        pt.stop(tm.d2h_ms);   // (synchronises)
+        a.expo->users = (int64_t)users;
+        return exposure_stats(dst_h, a.n, a.expo);
     }
 };
 
@@ -1362,12 +1421,12 @@ int run_call(const CallArgs<T>& a)
     if (a.lda < (size_t)a.k || a.ldb < (size_t)a.k) { set_err("bad argument", "lda/ldb smaller than k"); return RMB200_ERR_BAD_ARG; }
     if (a.out[5] && !a.tev) { set_err("bad argument", "NDCG requested but Xtest_csr (values) is NULL"); return RMB200_ERR_BAD_ARG; }
     if (ex->struct_size != (int32_t)sizeof(rmb200_extra_t)) { set_err("bad argument", "rmb200_extra_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
-    bool any_out = ex->metric_means || ex->metric_counts || ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status;
+    bool any_out = ex->metric_means || ex->metric_counts || ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status || a.expo;
     for (int q = 0; q < 10; q++) any_out |= (a.out[q] != nullptr);
     if (!any_out) return RMB200_OK;
     int ub = 0, ue = 0;
     TRY(user_range(ex, a.m, &ub, &ue));
-    if (ue == ub) return RMB200_OK;
+    if (ue == ub && !a.expo) return RMB200_OK;
 
     // ---- device ----
     int ndev = 0;
@@ -1382,6 +1441,7 @@ int run_call(const CallArgs<T>& a)
     if (dev < 0) CK(cudaGetDevice(&dev));
     if (dev >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
     CK(cudaSetDevice(dev));
+    if (ue == ub) return exposure_of_nobody(a.expo, a.n, ex->inputs_on_device != 0);
 
     const bool nested = a.mc != nullptr;                   // run_multi() holds the mutex and the latch
     std::unique_lock<std::mutex> lock(g_call_mutex, std::defer_lock);
@@ -1481,7 +1541,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
         }
     }
     const int G = (int)devs.size();
-    if (G == 0) return RMB200_OK;
+    if (G == 0) return a0.expo ? exposure_of_nobody(a0.expo, a0.n, false) : RMB200_OK;
 
     std::unique_lock<std::mutex> lock(g_call_mutex);
     SignalLatch latch;
@@ -1494,6 +1554,8 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     std::vector<rmb200_timing_t> tms((size_t)G);
     std::vector<std::vector<double>> means((size_t)G);
     std::vector<std::vector<long long>> counts((size_t)G);
+    std::vector<rmb200_exposure_t> expos((size_t)G);
+    std::vector<std::vector<int64_t>> item_counts(a0.expo ? (size_t)G : 0);
     std::vector<int> rcs((size_t)G, RMB200_OK);
     std::vector<std::string> errs((size_t)G);
     std::vector<std::thread> workers;
@@ -1506,6 +1568,12 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
         if (want_means) {
             means[g].assign(cells, 0.0); counts[g].assign(cells, 0);
             e.metric_means = means[g].data(); e.metric_counts = reinterpret_cast<int64_t*>(counts[g].data());
+        }
+        if (a0.expo) {
+            item_counts[g].assign((size_t)a0.n, 0);
+            std::memset(&expos[g], 0, sizeof(rmb200_exposure_t));
+            expos[g].struct_size = (int32_t)sizeof(rmb200_exposure_t);
+            expos[g].item_counts = item_counts[g].data();
         }
         workers.emplace_back([&, g]() {
             g_err.clear();
@@ -1521,6 +1589,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
                     }
                 CallArgs<T> a = a0;
                 a.ex = &exs[g]; a.mc = &mc; a.mc_rank = g;
+                if (a0.expo) a.expo = &expos[g];
                 rc = run_call<T>(a);
             } catch (const std::bad_alloc&) {
                 set_err("host allocation failed"); rc = RMB200_ERR_OOM;
@@ -1552,6 +1621,20 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
             if (ex->metric_counts) ex->metric_counts[c] = cnt;
         }
     }
+    if (a0.expo) {          // the devices' counts added up (integers: exact), the statistics of the sum
+        std::vector<int64_t> own;
+        int64_t* sum = a0.expo->item_counts;
+        if (!sum) { own.resize((size_t)a0.n); sum = own.data(); }
+        int64_t users = 0;
+        for (int j = 0; j < a0.n; j++) {
+            int64_t c = 0;
+            for (int g = 0; g < G; g++) c += item_counts[g][j];
+            sum[j] = c;
+        }
+        for (int g = 0; g < G; g++) users += expos[g].users;
+        a0.expo->users = users;
+        TRY(exposure_stats(sum, a0.n, a0.expo));
+    }
     if (ex->timing) {
         rmb200_timing_t t = tms[0];
         for (int g = 1; g < G; g++) {
@@ -1576,9 +1659,10 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
           const int32_t* trp, const int32_t* tri, const int32_t* tep, const int32_t* tei, const T* tev,
           int32_t K, int cumulative, int noise,
           T* p, T* tp, T* r, T* ap, T* tap, T* ndcg, T* hit, T* rr, T* roc, T* pr,
-          int ccs, int32_t mip, int32_t mpt, uint64_t seed, const T* bias, const rmb200_extra_t* ex)
+          int ccs, int32_t mip, int32_t mpt, uint64_t seed, const T* bias, const rmb200_extra_t* ex, rmb200_exposure_t* expo = nullptr)
 {
     g_err.clear();
+    if (expo && expo->struct_size != (int32_t)sizeof(rmb200_exposure_t)) { set_err("bad argument", "rmb200_exposure_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     CallArgs<T> a;
     a.A = A; a.lda = lda; a.B = B; a.ldb = ldb; a.m = m; a.n = n; a.k = k;
     a.trp = trp; a.tri = tri; a.tep = tep; a.tei = tei; a.tev = tev;
@@ -1586,7 +1670,7 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
     T* outs[10] = {p, tp, r, ap, tap, ndcg, hit, rr, roc, pr};
     for (int q = 0; q < 10; q++) a.out[q] = outs[q];
     a.consider_cold_start = ccs ? 1 : 0; a.min_items_pool = mip; a.min_pos_test = mpt; a.seed = seed;
-    a.bias = bias; a.ex = ex_or_default(ex);
+    a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo;
     try {
         std::vector<int> devs;
         TRY(resolve_devices(a.ex, devs));
@@ -1676,6 +1760,49 @@ int rmb200_calc_metrics_ex_f64(
                          ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
                          min_pos_test, seed, item_biases, extra);
 }
+
+int rmb200_calc_metrics_exposure_f32(
+    const float* A, size_t lda, const float* B, size_t ldb, int32_t m, int32_t n, int32_t k,
+    const int32_t* Xtrain_csr_p, const int32_t* Xtrain_csr_i,
+    const int32_t* Xtest_csr_p, const int32_t* Xtest_csr_i, const float* Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    float* p_at_k, float* tp_at_k, float* r_at_k, float* ap_at_k, float* tap_at_k,
+    float* ndcg_at_k, float* hit_at_k, float* rr_at_k, float* roc_auc, float* pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, int32_t nthreads, uint64_t seed,
+    const float* item_biases, const rmb200_extra_t* extra, rmb200_exposure_t* exposure)
+{
+    (void)nthreads;
+    return entry<float>(A, lda, B, ldb, m, n, k, Xtrain_csr_p, Xtrain_csr_i, Xtest_csr_p, Xtest_csr_i, Xtest_csr,
+                        k_metrics, cumulative, break_ties_with_noise, p_at_k, tp_at_k, r_at_k, ap_at_k, tap_at_k,
+                        ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
+                        min_pos_test, seed, item_biases, extra, exposure);
+}
+
+int rmb200_calc_metrics_exposure_f64(
+    const double* A, size_t lda, const double* B, size_t ldb, int32_t m, int32_t n, int32_t k,
+    const int32_t* Xtrain_csr_p, const int32_t* Xtrain_csr_i,
+    const int32_t* Xtest_csr_p, const int32_t* Xtest_csr_i, const double* Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    double* p_at_k, double* tp_at_k, double* r_at_k, double* ap_at_k, double* tap_at_k,
+    double* ndcg_at_k, double* hit_at_k, double* rr_at_k, double* roc_auc, double* pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, int32_t nthreads, uint64_t seed,
+    const double* item_biases, const rmb200_extra_t* extra, rmb200_exposure_t* exposure)
+{
+    (void)nthreads;
+    return entry<double>(A, lda, B, ldb, m, n, k, Xtrain_csr_p, Xtrain_csr_i, Xtest_csr_p, Xtest_csr_i, Xtest_csr,
+                         k_metrics, cumulative, break_ties_with_noise, p_at_k, tp_at_k, r_at_k, ap_at_k, tap_at_k,
+                         ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
+                         min_pos_test, seed, item_biases, extra, exposure);
+}
+
+int rmb200_exposure_stats(const int64_t* counts, int32_t n, rmb200_exposure_t* out)
+{
+    g_err.clear();
+    if (!out || out->struct_size != (int32_t)sizeof(rmb200_exposure_t)) { set_err("bad argument", "rmb200_exposure_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
+    return exposure_stats(counts, n, out);
+}
+
+int rmb200_sizeof_exposure(void) { return (int)sizeof(rmb200_exposure_t); }
 
 int rmb200_device_count(void)
 {

@@ -30,6 +30,7 @@ struct MetricsParams {
     int* status_out;                      // optional, offset to the batch
     int* topk_items; T* topk_scores;      // optional [mb][K], offset to the batch
     long long* pos_rank;                  // optional [nnz_test] (absolute)
+    int* list_len;                        // optional [mb]: length of the user's ranked list, 0 where it is undefined (exposure.cuh)
 };
 
 constexpr int METRICS_WARPS = 8;           // users (warps) per block of user_metrics_kernel
@@ -95,6 +96,7 @@ __global__ void __launch_bounds__(METRICS_WARPS * 32) user_metrics_kernel(const 
     if (st != 0) {
         all_nan(P, ul, lane);
         if (P.status_out && lane == 0) P.status_out[uli] = st;
+        if (P.list_len && lane == 0) P.list_len[uli] = 0;
         return;
     }
     const int ntrain = P.trp[u + 1] - P.trp[u];
@@ -126,10 +128,12 @@ __global__ void __launch_bounds__(METRICS_WARPS * 32) user_metrics_kernel(const 
         if (bad) {
             all_nan(P, ul, lane);
             if (P.status_out && lane == 0) P.status_out[uli] = 3;
+            if (P.list_len && lane == 0) P.list_len[uli] = 0;
             return;
         }
     }
     if (P.status_out && lane == 0) P.status_out[uli] = 0;
+    if (P.list_len && lane == 0) P.list_len[uli] = walk;
     if (P.topk_items) for (int c = lane; c < walk; c += 32) P.topk_items[ul * K + c] = ci[c];
     if (P.topk_scores) for (int c = lane; c < walk; c += 32) P.topk_scores[ul * K + c] = cs[c];
 

@@ -99,10 +99,10 @@ def calc_reco_metrics_device(
         all_metrics=False, break_ties_with_noise=True, min_pos_test=1, min_items_pool=2,
         consider_cold_start=True, cumulative=False, seed=1,
         user_range=None, strict_min_pos_test=False, return_topk=False, return_status=False, scoring_path="auto",
-        return_means=False, means_only=False):
+        return_means=False, means_only=False, return_exposure=False):
     """``calc_reco_metrics_ex`` for inputs that live on the GPU (see the module docstring).  Returns an
-    :class:`EvalResult` whose ``metrics`` / ``status`` / ``topk_*`` entries are torch CUDA tensors on the device of
-    ``A`` (``means`` / ``counts`` are small and come back as Python numbers / numpy vectors)."""
+    :class:`EvalResult` whose ``metrics`` / ``status`` / ``topk_*`` / ``exposure`` entries are torch CUDA tensors on the
+    device of ``A`` (``means`` / ``counts`` / ``catalogue`` are small and come back as Python numbers / numpy vectors)."""
     torch = _torch()
     if A is None or B is None:
         raise ValueError("'A' and 'B' must be passed (device-resident factor matrices).")
@@ -205,11 +205,13 @@ def calc_reco_metrics_device(
                              strict_min_pos_test=strict_min_pos_test, topk_items=ptr(topk_items), topk_scores=ptr(topk_scores),
                              status=ptr(status), timing=timing, scoring_path=scoring_path, metric_means=ptr(means),
                              metric_counts=ptr(counts), skip_row_copy=bool(means_only))
+    item_counts = torch.zeros(n, dtype=torch.int64, device=dev) if return_exposure else None
+    expo = _capi.make_exposure(ptr(item_counts)) if return_exposure else None
     torch.cuda.synchronize(dev)            # the library runs on its own stream: the caller's pending writes must have landed
     rc = _capi.calc_metrics(dtype, dA.ptr, dA.ld, dB.ptr, dB.ld, m, n, dA.shape[1],
                             ptr(X_train.indptr), ptr(X_train.indices) if X_train.indices.numel() else None,
                             ptr(X_test.indptr), ptr(X_test.indices), ptr(tev), K, cumulative, bool(break_ties_with_noise), outs,
-                            bool(consider_cold_start), min_items_pool, min_pos_test, 1, seed, bias_ptr, extra)
+                            bool(consider_cold_start), min_items_pool, min_pos_test, 1, seed, bias_ptr, extra, exposure=expo)
     _capi.raise_for_status(rc)
 
     metrics, mean_d, count_d = {}, None, None
@@ -229,4 +231,5 @@ def calc_reco_metrics_device(
             count_d[key] = ch[i * W:(i + 1) * W].copy() if wide else int(ch[i * W])
     return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
                       topk_items=None if topk_items is None else topk_items.view(m, K),
-                      topk_scores=None if topk_scores is None else topk_scores.view(m, K))
+                      topk_scores=None if topk_scores is None else topk_scores.view(m, K),
+                      exposure=item_counts, catalogue=None if expo is None else expo.catalogue())

@@ -9,7 +9,7 @@ import numpy as np
 
 from .frontend import calc_reco_metrics_ex
 
-__all__ = ["shard_bounds", "gather_metric_rows", "calc_reco_metrics_sharded"]
+__all__ = ["shard_bounds", "gather_metric_rows", "reduce_exposure", "calc_reco_metrics_sharded"]
 
 
 def shard_bounds(m, world_size, rank):
@@ -60,21 +60,47 @@ def gather_metric_rows(local, m, group=None, dst=0):
     return out
 
 
-def calc_reco_metrics_sharded(X_train, X_test, A, B, k=5, group=None, dst=0, **kwargs):
+def reduce_exposure(local_counts, group=None, dst=0, local_users=0):
+    """Sum the ranks' item counts (``EvalResult.exposure`` of each rank's block; int64 [n], the same n everywhere) to rank
+    `dst`.  Counts are additive, so the sum is exactly what one call over all users counts; the catalogue statistics are
+    computed from it by the library's own host function.  `local_users`: this rank's counted users
+    (``EvalResult.catalogue["users"]``).  Returns ``(counts, catalogue)`` on `dst`, None elsewhere."""
+    import torch
+    import torch.distributed as dist
+
+    from . import _capi
+
+    rank = dist.get_rank(group)
+    dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend(group) == "nccl" else torch.device("cpu")
+    counts = np.ascontiguousarray(local_counts, dtype=np.int64)
+    t = torch.from_numpy(np.append(counts, np.int64(local_users))).to(dev)       # one collective: counts, then users
+    dist.reduce(t, dst=dst, op=dist.ReduceOp.SUM, group=group)
+    if rank != dst:
+        return None
+    total = t.cpu().numpy()
+    return total[:-1].copy(), _capi.exposure_stats(total[:-1], users=int(total[-1]))
+
+
+def calc_reco_metrics_sharded(X_train, X_test, A, B, k=5, group=None, dst=0, return_exposure=False, **kwargs):
     """Evaluate with every rank of `group` taking its block of users on its current CUDA device.
 
     Every rank passes the same (full) inputs; only the block's rows of A and of the CSR matrices are
-    copied to that rank's GPU, B entirely.  Returns the reference-style dict on `dst` (None elsewhere)."""
+    copied to that rank's GPU, B entirely.  Returns the reference-style dict on `dst` (None elsewhere).
+    ``return_exposure``: returns ``(dict, item_counts, catalogue)`` on `dst` instead, the ranks' item exposure summed by
+    :func:`reduce_exposure`."""
     import torch.distributed as dist
 
     world = dist.get_world_size(group)
     rank = dist.get_rank(group)
     m = X_test.shape[0]
     b, e = shard_bounds(m, world, rank)
-    res = calc_reco_metrics_ex(X_train, X_test, A, B, k=k, user_range=(b, e), **kwargs)
+    res = calc_reco_metrics_ex(X_train, X_test, A, B, k=k, user_range=(b, e), return_exposure=return_exposure, **kwargs)
     K = res.metrics["K"]
     local = {name: v[b:e] for name, v in res.metrics.items() if name != "K"}
     full = gather_metric_rows(local, m, group=group, dst=dst)
     if full is not None:
         full["K"] = K
-    return full
+    if not return_exposure:
+        return full
+    expo = reduce_exposure(res.exposure, group=group, dst=dst, local_users=res.catalogue["users"])
+    return None if expo is None else (full,) + expo

@@ -42,6 +42,8 @@ class EvalResult:
     pos_rank: np.ndarray = None
     means: dict = None       # return_means: reference-style keys -> mean over the evaluated users (NaN rows left out)
     counts: dict = None      # ... -> how many users entered each mean
+    exposure: np.ndarray = None   # return_exposure: int64 [n], how many evaluated users have item j in their ranked top-K list
+    catalogue: dict = None   # ... and its statistics: "Coverage@K", "Gini@K", "Entropy@K", "users", "entries", "items_covered"
 
 
 def _rows_c_layout(X):
@@ -177,7 +179,7 @@ def calc_reco_metrics_ex(
         consider_cold_start=True, cumulative=False, nthreads=-1, seed=1,
         device=-1, user_range=None, strict_min_pos_test=False,
         return_topk=False, return_ranks=False, return_status=False, scoring_path="auto",
-        return_means=False, means_only=False, filter_stats=False, nan_bits=None, devices=None):
+        return_means=False, means_only=False, filter_stats=False, nan_bits=None, devices=None, return_exposure=False):
     """Same evaluation as :func:`calc_reco_metrics`, returning an :class:`EvalResult` with the
     reference-style dict plus timing and the optional extras (top-K ids/scores, held-out ranks,
     per-user status).  ``user_range=(begin, end)`` evaluates only those rows (the sharding unit);
@@ -188,7 +190,10 @@ def calc_reco_metrics_ex(
     when ``cumulative``) -- ``result.means`` / ``result.counts``; with ``means_only`` the per-user rows are not copied
     back at all (``result.metrics`` then only holds ``"K"``).  ``devices``: list of CUDA ordinals to spread the users of
     this one call over (one host thread per GPU inside the native call).  ``nan_bits``: bit pattern written wherever a
-    metric is undefined (R's ``NA_REAL``) instead of a plain NaN.  ``filter_stats``: fill ``timing["filter_err_ratio_max"]``."""
+    metric is undefined (R's ``NA_REAL``) instead of a plain NaN.  ``filter_stats``: fill ``timing["filter_err_ratio_max"]``.
+    ``return_exposure``: count, on the device, how many evaluated users have each item in their ranked top-K list
+    (``result.exposure``, int64 ``[n]``: ``numpy.bincount`` of the defined ``topk_items``) and derive the catalogue's coverage,
+    Gini index and entropy from the counts (``result.catalogue``); the lists themselves stay on the device."""
     flags = dict(p=precision, tp=trunc_precision, r=recall, ap=average_precision, tap=trunc_average_precision,
                  ndcg=ndcg, hit=hit, rr=rr, roc=roc_auc, pr=pr_auc)
     flags = {q: bool(v) or bool(all_metrics) for q, v in flags.items()}
@@ -220,10 +225,12 @@ def calc_reco_metrics_ex(
                              topk_items=topk_items, topk_scores=topk_scores, pos_rank=pos_rank, status=status,
                              timing=timing, scoring_path=scoring_path, metric_means=means, metric_counts=counts,
                              skip_row_copy=bool(means_only), filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
+    item_counts = np.zeros(prep["n"], dtype=np.int64) if return_exposure else None
+    expo = _capi.make_exposure(item_counts) if return_exposure else None
     rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, prep["n"], prep["p"],
                             prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
                             bool(break_ties_with_noise), outs, prep["consider_cold_start"], prep["min_items_pool"],
-                            prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"], extra)
+                            prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"], extra, exposure=expo)
     _capi.raise_for_status(rc)
 
     metrics, mean_d, count_d = {}, None, None
@@ -243,7 +250,8 @@ def calc_reco_metrics_ex(
     return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
                       topk_items=None if topk_items is None else topk_items.reshape(m, K),
                       topk_scores=None if topk_scores is None else topk_scores.reshape(m, K),
-                      pos_rank=None if pos_rank is None else pos_rank[: int(prep["tep"][-1])])
+                      pos_rank=None if pos_rank is None else pos_rank[: int(prep["tep"][-1])],
+                      exposure=item_counts, catalogue=None if expo is None else expo.catalogue())
 
 
 def calc_reco_metrics(
