@@ -233,6 +233,66 @@ RMB200_API int rmb200_calc_metrics_exposure_f64(
 RMB200_API int rmb200_exposure_stats(const int64_t *counts, int32_t n, rmb200_exposure_t *out);
 RMB200_API int rmb200_sizeof_exposure(void);
 
+/* Per-user beyond-accuracy metrics of the ranked top-K lists (zero-initialise, then set struct_size = sizeof(rmb200_beyond_t)).
+ * A user's list is j_1..j_L with L = min(k_metrics, candidates) (the eligibility rules make it k_metrics); the user is defined
+ * when L > 0 -- exactly the users whose topk_items row the call writes.  Every other user gets the NaN value (nan_bits is
+ * honoured) in all three outputs.  pop_j = item_popularity[j] (e.g. rmb200_item_popularity over the first m rows of X_train),
+ * U = popularity_users (e.g. m).  Column i of a cumulative row (i = L otherwise):
+ *   Novelty@i = (1/i) sum_{r<=i} -log2((pop_{j_r} + 1) / (U + 1))            AvgPop@i = (1/i) sum_{r<=i} pop_{j_r}
+ *   ILD@i     = 1 - 2 P_i / (i (i - 1)): the mean pairwise cosine distance of the first i items, over the unit rows
+ *               u_r = b_{j_r} / ||b_{j_r}|| of B (item factors only, no bias; a zero row gives u_r = 0, distance 1), with
+ *               P_r = P_{r-1} + u_r . (u_1 + ... + u_{r-1}).  ILD@1 is NaN.
+ * Sums are accumulated in double in rank order and cast once: column k_metrics of a cumulative row is bit-identical to the
+ * non-cumulative value, and a user's values do not depend on user_range, the batch size or the devices.  ILD needs
+ * k <= 1024 (float) / 512 (double) factors (RMB200_ERR_UNSUPPORTED beyond).  RMB200_ERR_BAD_ARG, before any work: a wrong
+ * struct_size; Novelty or AvgPop without item_popularity; popularity_users < 1; a count outside [0, popularity_users]. */
+typedef struct rmb200_beyond {
+    int32_t struct_size;          /* = sizeof(rmb200_beyond_t)                                                            */
+    int32_t reserved0;            /* padding                                                                              */
+    const int64_t *item_popularity;    /* [n]; needed for Novelty / AvgPop; a device pointer when extra->inputs_on_device */
+    int64_t popularity_users;     /* U                                                                                    */
+    void *novelty, *avg_popularity, *ild;   /* optional out: [m] or [m * k_metrics] (cumulative) of T, rows written at       */
+                                  /* [user_begin, user_end); NULL = not requested; device pointers when inputs_on_device   */
+    double  *means;               /* optional out [3 * W], W = cumulative ? k_metrics : 1: numpy.nanmean of every requested */
+                                  /* row over the call's users (Novelty, AvgPop, ILD); NaN for a metric not requested      */
+    int64_t *counts;              /* optional out [3 * W]: users that entered each mean                                     */
+} rmb200_beyond_t;
+
+/* rmb200_calc_metrics_exposure_f32 / _f64 plus the beyond-accuracy metrics; beyond == NULL is exactly the exposure call.
+ * Requesting one of the three rows counts as an output.  An interrupted call writes no means. */
+RMB200_API int rmb200_calc_metrics_beyond_f32(
+    const float *A, size_t lda, const float *B, size_t ldb,
+    int32_t m, int32_t n, int32_t k,
+    const int32_t *Xtrain_csr_p, const int32_t *Xtrain_csr_i,
+    const int32_t *Xtest_csr_p, const int32_t *Xtest_csr_i, const float *Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    float *p_at_k, float *tp_at_k, float *r_at_k, float *ap_at_k, float *tap_at_k,
+    float *ndcg_at_k, float *hit_at_k, float *rr_at_k, float *roc_auc, float *pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test,
+    int32_t nthreads, uint64_t seed,
+    const float *item_biases, const rmb200_extra_t *extra, rmb200_exposure_t *exposure, rmb200_beyond_t *beyond);
+
+RMB200_API int rmb200_calc_metrics_beyond_f64(
+    const double *A, size_t lda, const double *B, size_t ldb,
+    int32_t m, int32_t n, int32_t k,
+    const int32_t *Xtrain_csr_p, const int32_t *Xtrain_csr_i,
+    const int32_t *Xtest_csr_p, const int32_t *Xtest_csr_i, const double *Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    double *p_at_k, double *tp_at_k, double *r_at_k, double *ap_at_k, double *tap_at_k,
+    double *ndcg_at_k, double *hit_at_k, double *rr_at_k, double *roc_auc, double *pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test,
+    int32_t nthreads, uint64_t seed,
+    const double *item_biases, const rmb200_extra_t *extra, rmb200_exposure_t *exposure, rmb200_beyond_t *beyond);
+
+RMB200_API int rmb200_sizeof_beyond(void);
+
+/* Item popularity on the GPU: counts[j] = number of entries of item j in rows [row_begin, row_end) of a CSR matrix
+ * (numpy.bincount of those rows' indices, minlength n).  indptr / indices / counts are device pointers on `device` when
+ * inputs_on_device, else host pointers (the indices go up through the library's upload pipeline).  device < 0: env
+ * RMB200_DEVICE or the current device. */
+RMB200_API int rmb200_item_popularity(const int32_t *indptr, const int32_t *indices, int32_t row_begin, int32_t row_end,
+    int32_t n, int32_t device, int32_t inputs_on_device, int64_t *counts);
+
 /* Number of usable CUDA devices (0 = the library cannot compute). */
 RMB200_API int rmb200_device_count(void);
 /* RMB200_VERSION of the loaded library. */

@@ -1,7 +1,8 @@
 """recometrics_b200 -- B200-native (sm_100a) per-user evaluation path of david-cortes/recometrics.
 
 Public surface: :func:`calc_reco_metrics` (drop-in for ``recometrics.calc_reco_metrics``),
-:func:`calc_reco_metrics_ex` (same call, plus timing / top-K ids / held-out ranks) and
+:func:`calc_reco_metrics_ex` (same call, plus timing / top-K ids / held-out ranks / beyond-accuracy metrics, with
+:func:`item_popularity` for the popularity they use) and
 :func:`calc_reco_metrics_device` (factors and, optionally, the CSR matrices already resident on the GPU:
 ``__cuda_array_interface__`` in, torch CUDA tensors out); and, for the step before the evaluation,
 :func:`split_reco_train_test` (drop-in for ``recometrics.split_reco_train_test``).
@@ -10,11 +11,11 @@ The native library is ``recometrics_b200/librecometrics_b200.so`` (C-ABI in
 """
 from . import _capi
 from .device import DeviceCSR, calc_reco_metrics_device
-from .frontend import EvalResult, calc_reco_metrics, calc_reco_metrics_ex
+from .frontend import EvalResult, calc_reco_metrics, calc_reco_metrics_ex, item_popularity
 from .splitting import split_reco_train_test
 
 __all__ = ["calc_reco_metrics", "calc_reco_metrics_ex", "calc_reco_metrics_device", "DeviceCSR", "EvalResult", "split_reco_train_test", "device_count",
-           "native_library_path"]
+           "native_library_path", "item_popularity"]
 __version__ = "0.1.0"
 
 

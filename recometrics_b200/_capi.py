@@ -23,6 +23,7 @@ EXPORTS = (
     "rmb200_calc_metrics_f32", "rmb200_calc_metrics_f64",
     "rmb200_calc_metrics_ex_f32", "rmb200_calc_metrics_ex_f64",
     "rmb200_calc_metrics_exposure_f32", "rmb200_calc_metrics_exposure_f64", "rmb200_exposure_stats", "rmb200_sizeof_exposure",
+    "rmb200_calc_metrics_beyond_f32", "rmb200_calc_metrics_beyond_f64", "rmb200_sizeof_beyond", "rmb200_item_popularity",
     "rmb200_device_count", "rmb200_version", "rmb200_last_error",
     "rmb200_request_interrupt", "rmb200_measure_fma_peak", "rmb200_release_workspace",
     "rmb200_sizeof_extra", "rmb200_sizeof_timing",
@@ -85,6 +86,34 @@ def make_exposure(item_counts=None):
     return e
 
 
+# order of the three beyond-accuracy rows in rmb200_beyond_t (and of its means / counts) and their result keys
+BEYOND_KEYS = (("novelty", "Novelty@K"), ("avg_popularity", "AvgPop@K"), ("ild", "ILD@K"))
+
+
+class Beyond(ctypes.Structure):
+    """rmb200_beyond_t (include/recometrics_b200.h): Novelty / AvgPop / ILD rows of a call's ranked lists."""
+    _fields_ = [
+        ("struct_size", ctypes.c_int32), ("reserved0", ctypes.c_int32),
+        ("item_popularity", ctypes.c_void_p), ("popularity_users", ctypes.c_int64),
+        ("novelty", ctypes.c_void_p), ("avg_popularity", ctypes.c_void_p), ("ild", ctypes.c_void_p),
+        ("means", ctypes.c_void_p), ("counts", ctypes.c_void_p),
+    ]
+
+
+def make_beyond(rows, item_popularity=None, popularity_users=0, means=None, counts=None):
+    """rmb200_beyond_t; `rows` maps "novelty" / "avg_popularity" / "ild" -> array, device address or None; the other
+    arguments are int64 [n] counts, U, and the optional [3 * W] means / counts (arrays or device addresses)."""
+    b = Beyond()
+    b.struct_size = ctypes.sizeof(Beyond)
+    b.item_popularity = _vp(item_popularity)
+    b.popularity_users = int(popularity_users)
+    for name, _ in BEYOND_KEYS:
+        setattr(b, name, _vp(rows.get(name)))
+    b.means = _vp(means)
+    b.counts = _vp(counts)
+    return b
+
+
 class Csr(ctypes.Structure):
     _fields_ = [("rows", ctypes.c_int32), ("cols", ctypes.c_int32), ("nnz", ctypes.c_int64),
                 ("indptr", ctypes.c_void_p), ("indices", ctypes.c_void_p), ("values", ctypes.c_void_p)]
@@ -131,8 +160,10 @@ def load():
     lib.rmb200_sizeof_timing.restype = ctypes.c_int
     lib.rmb200_sizeof_split.restype = ctypes.c_int
     lib.rmb200_sizeof_exposure.restype = ctypes.c_int
+    lib.rmb200_sizeof_beyond.restype = ctypes.c_int
     if (lib.rmb200_sizeof_extra() != ctypes.sizeof(Extra) or lib.rmb200_sizeof_timing() != ctypes.sizeof(Timing)
-            or lib.rmb200_sizeof_split() != ctypes.sizeof(Split) or lib.rmb200_sizeof_exposure() != ctypes.sizeof(Exposure)):
+            or lib.rmb200_sizeof_split() != ctypes.sizeof(Split) or lib.rmb200_sizeof_exposure() != ctypes.sizeof(Exposure)
+            or lib.rmb200_sizeof_beyond() != ctypes.sizeof(Beyond)):
         raise NativeLibraryError("recometrics_b200: %s was built from a different include/recometrics_b200.h (struct sizes differ); rebuild it" % LIB_PATH)
     lib.rmb200_last_error.restype = ctypes.c_char_p
     lib.rmb200_request_interrupt.restype = None
@@ -142,6 +173,10 @@ def load():
     for name in EXPORTS[:7]:
         getattr(lib, name).restype = ctypes.c_int
     lib.rmb200_exposure_stats.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(Exposure)]
+    for name in ("rmb200_calc_metrics_beyond_f32", "rmb200_calc_metrics_beyond_f64", "rmb200_item_popularity"):
+        getattr(lib, name).restype = ctypes.c_int
+    lib.rmb200_item_popularity.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                           ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]
     for name in EXPORTS:
         if name.startswith("rmb200_split_") and name != "rmb200_split_free":
             getattr(lib, name).restype = ctypes.c_int
@@ -206,12 +241,13 @@ def _vp(x):
 
 def calc_metrics(dtype, A, lda, B, ldb, m, n, k, trp, tri, tep, tei, tev, k_metrics, cumulative,
                  break_ties_with_noise, outs, consider_cold_start, min_items_pool, min_pos_test,
-                 nthreads=1, seed=1, item_biases=None, extra=None, exposure=None):
-    """Thin call into rmb200_calc_metrics_ex_{f32,f64} (rmb200_calc_metrics_exposure_{f32,f64} with an `exposure` struct).
-    Array arguments are numpy arrays (host memory), raw integer addresses (device memory, with extra.inputs_on_device=1) or
-    None.  `outs` maps metric name -> array/address/None in METRIC_ORDER.  Returns the status code."""
+                 nthreads=1, seed=1, item_biases=None, extra=None, exposure=None, beyond=None):
+    """Thin call into rmb200_calc_metrics_ex_{f32,f64} (rmb200_calc_metrics_exposure_{f32,f64} with an `exposure` struct,
+    rmb200_calc_metrics_beyond_{f32,f64} with a `beyond` struct).  Array arguments are numpy arrays (host memory), raw integer
+    addresses (device memory, with extra.inputs_on_device=1) or None.  `outs` maps metric name -> array/address/None in
+    METRIC_ORDER.  Returns the status code."""
     lib = load()
-    kind = "ex" if exposure is None else "exposure"
+    kind = "ex" if exposure is None and beyond is None else ("exposure" if beyond is None else "beyond")
     fn = getattr(lib, "rmb200_calc_metrics_%s_%s" % (kind, "f32" if np.dtype(dtype) == np.float32 else "f64"))
     args = [
         _vp(A), ctypes.c_size_t(int(lda)), _vp(B), ctypes.c_size_t(int(ldb)),
@@ -225,9 +261,19 @@ def calc_metrics(dtype, A, lda, B, ldb, m, n, k, trp, tri, tep, tei, tev, k_metr
         ctypes.c_int32(int(nthreads)), ctypes.c_uint64(int(seed)),
         _vp(item_biases), ctypes.byref(extra) if extra is not None else ctypes.c_void_p(None),
     ]
-    if exposure is not None:
-        args.append(ctypes.byref(exposure))
+    if kind != "ex":
+        args.append(ctypes.byref(exposure) if exposure is not None else ctypes.c_void_p(None))
+    if beyond is not None:
+        args.append(ctypes.byref(beyond))
     return int(fn(*args))
+
+
+def item_popularity(indptr, indices, row_begin, row_end, n, counts, device=-1, inputs_on_device=False):
+    """rmb200_item_popularity: counts[j] = entries of item j in CSR rows [row_begin, row_end), counted on the GPU.  The arrays
+    are numpy arrays (host) or device addresses (inputs_on_device).  Raises on failure."""
+    rc = load().rmb200_item_popularity(_vp(indptr), _vp(indices), int(row_begin), int(row_end), int(n), int(device),
+                                       int(bool(inputs_on_device)), _vp(counts))
+    raise_for_status(rc)
 
 
 def exposure_stats(counts, users=0):

@@ -27,6 +27,7 @@
 #include "score_select.cuh"
 #include "filter_select.cuh"
 #include "exposure.cuh"
+#include "beyond.cuh"
 #include "full_order.h"
 
 namespace {
@@ -228,6 +229,7 @@ struct CallArgs {
     const T* bias;
     const rmb200_extra_t* ex;
     rmb200_exposure_t* expo = nullptr;   // item exposure of the ranked lists (exposure.cuh); null: not requested
+    rmb200_beyond_t* bey = nullptr;      // Novelty / AvgPop / ILD of the ranked lists (beyond.cuh); null: not requested
 };
 
 template <typename T, int C, bool AUC>
@@ -666,6 +668,9 @@ struct Call {
     size_t rs = 1;
     T nan_value = std::numeric_limits<T>::quiet_NaN();
     bool want_roc = false, want_pr = false, count_ranks = false, want_means = false, want_filter_stats = false, want_exposure = false;
+    bool want_pop = false, want_ild = false, want_beyond = false, want_beyond_means = false;   // beyond.cuh
+    int unit_pitch = 0, unit_nch = 0;           // ILD: row pitch of the unit-row image (elements), 16-byte chunks per lane
+    T* bey_out[3] = {nullptr, nullptr, nullptr};   // caller's Novelty / AvgPop / ILD rows (null: not requested)
     bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
     int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
     int fo_chunk = 0; size_t fo_bytes = 0;
@@ -684,6 +689,8 @@ struct Call {
     DevBuf d_capx, d_overflow, d_fb_list, d_At_fb;
     DevBuf d_psum, d_pcnt, d_means, d_mcounts;
     DevBuf d_expo_hist, d_list_len, d_expo_counts;
+    DevBuf d_pop, d_poptab, d_pop_bad, d_unit, d_bout[2][3], d_bpsum, d_bpcnt, d_bmeans, d_bcounts;
+    const long long* pop_d = nullptr;           // the caller's popularity counts on the device
     PrefetchStream pf;                          // (declared after the buffers they fill or read: destroyed, i.e. drained, before them)
     ResultStream rsx;
     Call(const CallArgs<T>& args, int device, int user_begin, int users) : a(args), ex(args.ex), on_dev(args.ex->inputs_on_device != 0),
@@ -710,6 +717,20 @@ struct Call {
         want_means = ex->metric_means || ex->metric_counts;
         want_filter_stats = ex->filter_stats != 0;
         want_exposure = a.expo != nullptr;
+        if (a.bey) {
+            bey_out[0] = static_cast<T*>(a.bey->novelty); bey_out[1] = static_cast<T*>(a.bey->avg_popularity); bey_out[2] = static_cast<T*>(a.bey->ild);
+            want_pop = bey_out[0] || bey_out[1];
+            want_ild = bey_out[2] != nullptr;
+            want_beyond = want_pop || want_ild;
+            want_beyond_means = want_beyond && (a.bey->means || a.bey->counts);
+        }
+        if (want_ild) {            // lane l of beyond_accuracy_kernel holds 16-byte chunks l, l + 32, ... of a unit row: 1, 2, 4 or 8
+            constexpr int V = 16 / (int)sizeof(T);
+            unit_pitch = round_up(a.k, V);
+            const int chunks = unit_pitch / V;
+            unit_nch = chunks <= 32 ? 1 : chunks <= 64 ? 2 : chunks <= 128 ? 4 : chunks <= 256 ? 8 : 0;
+            if (!unit_nch) { set_err("unsupported", "ILD needs k <= 1024 (float) / 512 (double) factors"); return RMB200_ERR_UNSUPPORTED; }
+        }
         p_pad = round_up(a.k, KPAD);
         n_pad = round_up(a.n, BN);
         rs = a.cumulative ? (size_t)K : 1;
@@ -858,8 +879,46 @@ struct Call {
             pt.stop(tm.h2d_ms);
             Bsrc = d_Brow.as<T>(); Bld = (size_t)a.k;
         } else { Bsrc = a.B; Bld = a.ldb; }
+        if (want_ild) TRY(unit_rows());                 // (from the complete rows: after the peer fetch, before d_Brow goes)
         if (!use_tensor || fma_counts_first) TRY(ensure_Bt());
         if (!use_tensor) { d_Brow.release(); if (!on_dev) Bsrc = nullptr; }     // the FMA path reads only the tiled copy
+        return RMB200_OK;
+    }
+    // ILD: the unit-row image of B, once per call
+    int unit_rows()
+    {
+        CK(d_unit.alloc((size_t)a.n * unit_pitch * sizeof(T)));
+        pt.start();
+        constexpr int WARPS = 8;
+        rmb::unit_rows_kernel<T><<<(a.n + WARPS - 1) / WARPS, WARPS * 32, 0, st>>>(Bsrc, Bld, a.n, a.k, d_unit.as<T>(), unit_pitch);
+        TRY(launched());
+        pt.stop(tm.prep_ms);
+        return RMB200_OK;
+    }
+    // Novelty / AvgPop: the caller's popularity counts on the device, checked against [0, U] there, and the per-item table
+    int popularity_table()
+    {
+        if (!want_pop) return RMB200_OK;
+        pop_d = reinterpret_cast<const long long*>(a.bey->item_popularity);
+        if (!on_dev) {
+            CK(d_pop.alloc((size_t)a.n * sizeof(long long)));
+            pt.start();
+            CK(cudaMemcpyAsync(d_pop.p, a.bey->item_popularity, (size_t)a.n * sizeof(long long), cudaMemcpyHostToDevice, st));
+            tm.h2d_bytes += (int64_t)a.n * (int64_t)sizeof(long long);
+            pt.stop(tm.h2d_ms);
+            pop_d = d_pop.as<long long>();
+        }
+        CK(d_poptab.alloc((size_t)a.n * sizeof(double2)));
+        CK(d_pop_bad.alloc(sizeof(int)));
+        pt.start();
+        CK(cudaMemsetAsync(d_pop_bad.p, 0, sizeof(int), st));
+        rmb::popularity_table_kernel<<<(a.n + 255) / 256 < 4 * nsm ? (a.n + 255) / 256 : 4 * nsm, 256, 0, st>>>(
+            pop_d, a.n, (long long)a.bey->popularity_users, d_poptab.as<double2>(), d_pop_bad.as<int>());
+        TRY(launched());
+        int bad = 0;
+        CK(cudaMemcpyAsync(&bad, d_pop_bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+        pt.stop(tm.prep_ms);   // (synchronises)
+        if (bad) { set_err("bad argument", "item_popularity: a count outside [0, popularity_users]"); return RMB200_ERR_BAD_ARG; }
         return RMB200_OK;
     }
     long long item_slice(int h) const { return (long long)a.n * h / (nested ? a.mc->G : 1); }
@@ -1028,7 +1087,17 @@ struct Call {
         if (want_exposure) {
             CK(d_expo_hist.alloc(((size_t)a.n + 1) * sizeof(unsigned)));
             CK(cudaMemsetAsync(d_expo_hist.p, 0, ((size_t)a.n + 1) * sizeof(unsigned), st));
-            CK(d_list_len.alloc((size_t)UB * sizeof(int)));
+        }
+        if (want_exposure || want_beyond) CK(d_list_len.alloc((size_t)UB * sizeof(int)));
+        // beyond-accuracy rows: result sets of their own (host outputs), partial sums of their means
+        for (int set = 0; !on_dev && set < (UB < mr ? 2 : 1); set++)
+            for (int q = 0; q < 3; q++)
+                if (bey_out[q]) CK(d_bout[set][q].alloc((size_t)UB * rs * sizeof(T)));
+        if (want_beyond_means) {
+            int mean_blocks_total = 0;
+            for (int b0 = 0; b0 < mr; b0 += UB) mean_blocks_total += (((mr - b0) < UB ? (mr - b0) : UB) + rmb::MEAN_CHUNK - 1) / rmb::MEAN_CHUNK;
+            CK(d_bpsum.alloc((size_t)mean_blocks_total * 3 * mean_W * sizeof(double)));
+            CK(d_bpcnt.alloc((size_t)mean_blocks_total * 3 * mean_W * sizeof(int)));
         }
         return RMB200_OK;
     }
@@ -1300,7 +1369,7 @@ struct Call {
         mp.topk_items = !ex->topk_items ? nullptr : on_dev ? ex->topk_items + row * K : d_tki[slot].as<int>();
         mp.topk_scores = !ex->topk_scores ? nullptr : on_dev ? reinterpret_cast<T*>(ex->topk_scores) + row * K : d_tks[slot].as<T>();
         mp.pos_rank = pos_rank_d;
-        mp.list_len = want_exposure ? d_list_len.as<int>() : nullptr;
+        mp.list_len = (want_exposure || want_beyond) ? d_list_len.as<int>() : nullptr;
         TRY(wait_test_rows());
         user_metrics_kernel<T><<<(b.nb + METRICS_WARPS - 1) / METRICS_WARPS, METRICS_WARPS * 32, 0, st>>>(mp);
         TRY(launched());
@@ -1309,17 +1378,48 @@ struct Call {
                 d_ci.as<int>(), C, d_list_len.as<int>(), b.nb, d_expo_hist.as<unsigned>(), a.n);
             TRY(launched());
         }
+        T* bouts[3] = {nullptr, nullptr, nullptr};
+        if (want_beyond) {
+            BeyondParams<T> bp;
+            bp.items = d_ci.as<int>(); bp.C = C; bp.list_len = d_list_len.as<int>(); bp.nb = b.nb; bp.K = K; bp.cumulative = a.cumulative;
+            bp.pop = want_pop ? d_poptab.as<double2>() : nullptr;
+            bp.unit = want_ild ? d_unit.as<T>() : nullptr; bp.pitch = unit_pitch;
+            for (int q = 0; q < 3; q++)
+                bouts[q] = !bey_out[q] ? nullptr : on_dev ? bey_out[q] + row * rs : d_bout[slot][q].as<T>();
+            bp.nov = bouts[0]; bp.avgpop = bouts[1]; bp.ild = bouts[2];
+            bp.nan_value = nan_value;
+            TRY(launch_beyond(bp));
+        }
+        const int mblocks = (b.nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
         if (want_means) {
             MeanParams<T> qp;
             for (int q = 0; q < 10; q++) qp.out[q] = outs[q];
-            qp.nb = b.nb; qp.W = mean_W; qp.part_sum = d_psum.as<double>(); qp.part_cnt = d_pcnt.as<int>(); qp.block0 = mean_block0;
-            const int blocks = (b.nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
-            metric_partial_kernel<T><<<dim3(blocks, 10), MEAN_CHUNK, 0, st>>>(qp);
+            qp.nb = b.nb; qp.W = mean_W; qp.slots = 10; qp.wide = 8;
+            qp.part_sum = d_psum.as<double>(); qp.part_cnt = d_pcnt.as<int>(); qp.block0 = mean_block0;
+            metric_partial_kernel<T><<<dim3(mblocks, 10), MEAN_CHUNK, 0, st>>>(qp);
             TRY(launched());
-            mean_block0 += blocks;
         }
+        if (want_beyond_means) {
+            MeanParams<T> qp;
+            for (int q = 0; q < 10; q++) qp.out[q] = q < 3 ? bouts[q] : nullptr;
+            qp.nb = b.nb; qp.W = mean_W; qp.slots = 3; qp.wide = 3;
+            qp.part_sum = d_bpsum.as<double>(); qp.part_cnt = d_bpcnt.as<int>(); qp.block0 = mean_block0;
+            metric_partial_kernel<T><<<dim3(mblocks, 3), MEAN_CHUNK, 0, st>>>(qp);
+            TRY(launched());
+        }
+        mean_block0 += mblocks;
         pt.stop(tm.metrics_ms);
         return RMB200_OK;
+    }
+    int launch_beyond(const rmb::BeyondParams<T>& bp)
+    {
+        using namespace rmb;
+        const int blocks = (bp.nb + BEYOND_WARPS - 1) / BEYOND_WARPS, threads = BEYOND_WARPS * 32;
+        if (unit_nch <= 1) beyond_accuracy_kernel<T, 1><<<blocks, threads, 0, st>>>(bp);      // (also: no ILD)
+        else if (unit_nch == 2) beyond_accuracy_kernel<T, 2><<<blocks, threads, 0, st>>>(bp);
+        else if (unit_nch == 4) beyond_accuracy_kernel<T, 4><<<blocks, threads, 0, st>>>(bp);
+        else beyond_accuracy_kernel<T, 8><<<blocks, threads, 0, st>>>(bp);
+        return launched();
     }
     // results of the batch -> caller's arrays at the shard's row offset (no gather collective: every shard writes its own
     // disjoint rows)
@@ -1339,6 +1439,12 @@ struct Call {
         if (ex->status) { CK(cudaMemcpyAsync(ex->status + row, d_stat_out[b.slot].p, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * 4; }
         if (ex->topk_items) { CK(cudaMemcpyAsync(ex->topk_items + row * K, d_tki[b.slot].p, (size_t)nb * K * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * 4; }
         if (ex->topk_scores) { CK(cudaMemcpyAsync(reinterpret_cast<T*>(ex->topk_scores) + row * K, d_tks[b.slot].p, (size_t)nb * K * sizeof(T), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * (int64_t)sizeof(T); }
+        for (int q = 0; q < 3; q++) {
+            if (!bey_out[q] || ex->skip_row_copy) continue;
+            const size_t bytes = nb * rs * sizeof(T);
+            CK(cudaMemcpyAsync(bey_out[q] + row * rs, d_bout[b.slot][q].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
+            tm.d2h_bytes += (int64_t)bytes;
+        }
         CK(cudaEventRecord(rsx.copied[b.slot], rsx.s));
         rsx.copied_valid[b.slot] = true;
         return RMB200_OK;
@@ -1366,7 +1472,7 @@ struct Call {
                 if (ex->metric_counts) { CK(d_mcounts.alloc(cells * sizeof(long long))); counts_d = d_mcounts.as<long long>(); }
             }
             pt.start();
-            rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_psum.as<double>(), d_pcnt.as<int>(), mean_block0, mean_W, means_d, counts_d);
+            rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_psum.as<double>(), d_pcnt.as<int>(), mean_block0, 10, mean_W, means_d, counts_d);
             TRY(launched());
             pt.stop(tm.metrics_ms);
             if (!on_dev) {
@@ -1374,6 +1480,7 @@ struct Call {
                 if (ex->metric_counts) { CK(cudaMemcpyAsync(ex->metric_counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
             }
         }
+        if (want_beyond_means && !g_interrupt.load()) TRY(beyond_means_out());
         if (want_exposure && !g_interrupt.load()) TRY(exposure_out());
         if (use_tensor && want_filter_stats) {
             float ratio = 0.f;
@@ -1382,6 +1489,26 @@ struct Call {
             tm.filter_err_ratio_max = (double)ratio;
         }
         CK(cudaStreamSynchronize(st));
+        return RMB200_OK;
+    }
+    // means / counts of the Novelty, AvgPop and ILD rows: the accuracy metrics' reduction over a table of three
+    int beyond_means_out()
+    {
+        const size_t cells = (size_t)3 * mean_W;
+        double* means_d = nullptr; long long* counts_d = nullptr;
+        if (on_dev) { means_d = a.bey->means; counts_d = reinterpret_cast<long long*>(a.bey->counts); }
+        else {
+            if (a.bey->means) { CK(d_bmeans.alloc(cells * sizeof(double))); means_d = d_bmeans.as<double>(); }
+            if (a.bey->counts) { CK(d_bcounts.alloc(cells * sizeof(long long))); counts_d = d_bcounts.as<long long>(); }
+        }
+        pt.start();
+        rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_bpsum.as<double>(), d_bpcnt.as<int>(), mean_block0, 3, mean_W, means_d, counts_d);
+        TRY(launched());
+        pt.stop(tm.metrics_ms);
+        if (!on_dev) {
+            if (a.bey->means) { CK(cudaMemcpyAsync(a.bey->means, means_d, cells * sizeof(double), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(double)); }
+            if (a.bey->counts) { CK(cudaMemcpyAsync(a.bey->counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
+        }
         return RMB200_OK;
     }
     // the call's item counts, widened to int64, into the caller's array (device-resident calls: on the device, then a copy for
@@ -1421,7 +1548,16 @@ int run_call(const CallArgs<T>& a)
     if (a.lda < (size_t)a.k || a.ldb < (size_t)a.k) { set_err("bad argument", "lda/ldb smaller than k"); return RMB200_ERR_BAD_ARG; }
     if (a.out[5] && !a.tev) { set_err("bad argument", "NDCG requested but Xtest_csr (values) is NULL"); return RMB200_ERR_BAD_ARG; }
     if (ex->struct_size != (int32_t)sizeof(rmb200_extra_t)) { set_err("bad argument", "rmb200_extra_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
+    if (a.bey && (a.bey->novelty || a.bey->avg_popularity)) {
+        const int64_t U = a.bey->popularity_users;
+        if (!a.bey->item_popularity) { set_err("bad argument", "Novelty / AvgPop requested but item_popularity is NULL"); return RMB200_ERR_BAD_ARG; }
+        if (U < 1) { set_err("bad argument", "popularity_users must be >= 1"); return RMB200_ERR_BAD_ARG; }
+        if (!ex->inputs_on_device)            // (device-resident counts are checked on the device, before the first batch)
+            for (int j = 0; j < a.n; j++)
+                if (a.bey->item_popularity[j] < 0 || a.bey->item_popularity[j] > U) { set_err("bad argument", "item_popularity: a count outside [0, popularity_users]"); return RMB200_ERR_BAD_ARG; }
+    }
     bool any_out = ex->metric_means || ex->metric_counts || ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status || a.expo;
+    if (a.bey) any_out |= a.bey->novelty || a.bey->avg_popularity || a.bey->ild;
     for (int q = 0; q < 10; q++) any_out |= (a.out[q] != nullptr);
     if (!any_out) return RMB200_OK;
     int ub = 0, ue = 0;
@@ -1452,6 +1588,7 @@ int run_call(const CallArgs<T>& a)
     TRY(c.csr_slices());
     TRY(c.item_factors());
     TRY(c.item_bias());
+    TRY(c.popularity_table());
     TRY(c.item_image());
     TRY(c.user_state());
     TRY(c.batch_buffers());
@@ -1556,6 +1693,11 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     std::vector<std::vector<long long>> counts((size_t)G);
     std::vector<rmb200_exposure_t> expos((size_t)G);
     std::vector<std::vector<int64_t>> item_counts(a0.expo ? (size_t)G : 0);
+    const bool want_bmeans = a0.bey && (a0.bey->means || a0.bey->counts);
+    const size_t bcells = (size_t)3 * (size_t)(W > 0 ? W : 1);
+    std::vector<rmb200_beyond_t> beys((size_t)G);
+    std::vector<std::vector<double>> bmeans((size_t)G);
+    std::vector<std::vector<long long>> bcounts((size_t)G);
     std::vector<int> rcs((size_t)G, RMB200_OK);
     std::vector<std::string> errs((size_t)G);
     std::vector<std::thread> workers;
@@ -1575,6 +1717,13 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
             expos[g].struct_size = (int32_t)sizeof(rmb200_exposure_t);
             expos[g].item_counts = item_counts[g].data();
         }
+        if (a0.bey) {           // rows straight into the caller's arrays (every device writes its own); means per device
+            beys[g] = *a0.bey;
+            if (want_bmeans) {
+                bmeans[g].assign(bcells, 0.0); bcounts[g].assign(bcells, 0);
+                beys[g].means = bmeans[g].data(); beys[g].counts = reinterpret_cast<int64_t*>(bcounts[g].data());
+            }
+        }
         workers.emplace_back([&, g]() {
             g_err.clear();
             g_upload_share = G;
@@ -1590,6 +1739,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
                 CallArgs<T> a = a0;
                 a.ex = &exs[g]; a.mc = &mc; a.mc_rank = g;
                 if (a0.expo) a.expo = &expos[g];
+                if (a0.bey) a.bey = &beys[g];
                 rc = run_call<T>(a);
             } catch (const std::bad_alloc&) {
                 set_err("host allocation failed"); rc = RMB200_ERR_OOM;
@@ -1619,6 +1769,14 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
             for (int g = 0; g < G; g++) if (counts[g][c] > 0) { s += means[g][c] * (double)counts[g][c]; cnt += counts[g][c]; }
             if (ex->metric_means) ex->metric_means[c] = cnt ? s / (double)cnt : std::numeric_limits<double>::quiet_NaN();
             if (ex->metric_counts) ex->metric_counts[c] = cnt;
+        }
+    }
+    if (want_bmeans) {      // the same for the beyond-accuracy means
+        for (size_t c = 0; c < bcells; c++) {
+            double s = 0.0; long long cnt = 0;
+            for (int g = 0; g < G; g++) if (bcounts[g][c] > 0) { s += bmeans[g][c] * (double)bcounts[g][c]; cnt += bcounts[g][c]; }
+            if (a0.bey->means) a0.bey->means[c] = cnt ? s / (double)cnt : std::numeric_limits<double>::quiet_NaN();
+            if (a0.bey->counts) a0.bey->counts[c] = cnt;
         }
     }
     if (a0.expo) {          // the devices' counts added up (integers: exact), the statistics of the sum
@@ -1659,10 +1817,12 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
           const int32_t* trp, const int32_t* tri, const int32_t* tep, const int32_t* tei, const T* tev,
           int32_t K, int cumulative, int noise,
           T* p, T* tp, T* r, T* ap, T* tap, T* ndcg, T* hit, T* rr, T* roc, T* pr,
-          int ccs, int32_t mip, int32_t mpt, uint64_t seed, const T* bias, const rmb200_extra_t* ex, rmb200_exposure_t* expo = nullptr)
+          int ccs, int32_t mip, int32_t mpt, uint64_t seed, const T* bias, const rmb200_extra_t* ex, rmb200_exposure_t* expo = nullptr,
+          rmb200_beyond_t* bey = nullptr)
 {
     g_err.clear();
     if (expo && expo->struct_size != (int32_t)sizeof(rmb200_exposure_t)) { set_err("bad argument", "rmb200_exposure_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
+    if (bey && bey->struct_size != (int32_t)sizeof(rmb200_beyond_t)) { set_err("bad argument", "rmb200_beyond_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     CallArgs<T> a;
     a.A = A; a.lda = lda; a.B = B; a.ldb = ldb; a.m = m; a.n = n; a.k = k;
     a.trp = trp; a.tri = tri; a.tep = tep; a.tei = tei; a.tev = tev;
@@ -1670,7 +1830,7 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
     T* outs[10] = {p, tp, r, ap, tap, ndcg, hit, rr, roc, pr};
     for (int q = 0; q < 10; q++) a.out[q] = outs[q];
     a.consider_cold_start = ccs ? 1 : 0; a.min_items_pool = mip; a.min_pos_test = mpt; a.seed = seed;
-    a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo;
+    a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo; a.bey = bey;
     try {
         std::vector<int> devs;
         TRY(resolve_devices(a.ex, devs));
@@ -1689,6 +1849,56 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
         set_err("unexpected C++ exception");
         return RMB200_ERR_CUDA;
     }
+}
+
+// rmb200_item_popularity: the column count of CSR rows [rb, re) on the device, widened to int64 into `counts`
+int item_popularity(const int32_t* indptr, const int32_t* indices, int rb, int re, int n, int device, bool on_dev, int64_t* counts)
+{
+    if (n <= 0 || !indptr || !counts || rb < 0 || re < rb) { set_err("bad argument", "item_popularity: n <= 0, a NULL array or a bad row range"); return RMB200_ERR_BAD_ARG; }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+        cudaGetLastError();
+        set_err("no CUDA device", "librecometrics_b200 has no CPU fallback");
+        return RMB200_ERR_NO_DEVICE;
+    }
+    int dev = device;
+    if (dev < 0) if (const char* env = std::getenv("RMB200_DEVICE")) dev = std::atoi(env);
+    if (dev < 0) CK(cudaGetDevice(&dev));
+    if (dev >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
+    CK(cudaSetDevice(dev));
+    std::lock_guard<std::mutex> lock(g_call_mutex);       // (the upload lanes belong to the holder)
+    cudaStream_t st = nullptr;                             // legacy default stream, as the evaluation call
+    int lo = 0, hi = 0;
+    if (on_dev) {
+        CK(cudaMemcpy(&lo, indptr + rb, sizeof(int), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(&hi, indptr + re, sizeof(int), cudaMemcpyDeviceToHost));
+    } else { lo = indptr[rb]; hi = indptr[re]; }
+    if (hi < lo) { set_err("bad argument", "CSR index pointers decrease"); return RMB200_ERR_BAD_ARG; }
+    const long long nnz = (long long)hi - lo;
+    if (nnz && !indices) { set_err("bad argument", "CSR indices missing"); return RMB200_ERR_BAD_ARG; }
+    DevBuf d_idx, d_hist, d_counts;
+    const int* idx_d = on_dev ? indices + lo : nullptr;
+    if (!on_dev) {
+        CK(d_idx.alloc((size_t)nnz * sizeof(int)));
+        if (nnz) CK(upload_rows(d_idx.p, indices + lo, (size_t)nnz * sizeof(int), (size_t)nnz * sizeof(int), 1, st));
+        idx_d = d_idx.as<int>();
+    }
+    CK(d_hist.alloc((size_t)n * sizeof(unsigned)));
+    CK(cudaMemsetAsync(d_hist.p, 0, (size_t)n * sizeof(unsigned), st));
+    int nsm = 148;
+    cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    if (nnz) {
+        const long long want = (nnz + rmb::POPULARITY_THREADS - 1) / rmb::POPULARITY_THREADS;
+        rmb::item_popularity_kernel<<<(int)(want < 8ll * nsm ? want : 8ll * nsm), rmb::POPULARITY_THREADS, 0, st>>>(idx_d, nnz, d_hist.as<unsigned>(), n);
+        CK(cudaGetLastError());
+    }
+    long long* dst = on_dev ? reinterpret_cast<long long*>(counts) : nullptr;
+    if (!dst) { CK(d_counts.alloc((size_t)n * sizeof(long long))); dst = d_counts.as<long long>(); }
+    rmb::exposure_widen_kernel<<<(n + 255) / 256 < 4 * nsm ? (n + 255) / 256 : 4 * nsm, 256, 0, st>>>(d_hist.as<unsigned>(), n, dst);
+    CK(cudaGetLastError());
+    if (!on_dev) CK(cudaMemcpyAsync(counts, dst, (size_t)n * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return RMB200_OK;
 }
 
 }  // namespace
@@ -1803,6 +2013,57 @@ int rmb200_exposure_stats(const int64_t* counts, int32_t n, rmb200_exposure_t* o
 }
 
 int rmb200_sizeof_exposure(void) { return (int)sizeof(rmb200_exposure_t); }
+
+int rmb200_calc_metrics_beyond_f32(
+    const float* A, size_t lda, const float* B, size_t ldb, int32_t m, int32_t n, int32_t k,
+    const int32_t* Xtrain_csr_p, const int32_t* Xtrain_csr_i,
+    const int32_t* Xtest_csr_p, const int32_t* Xtest_csr_i, const float* Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    float* p_at_k, float* tp_at_k, float* r_at_k, float* ap_at_k, float* tap_at_k,
+    float* ndcg_at_k, float* hit_at_k, float* rr_at_k, float* roc_auc, float* pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, int32_t nthreads, uint64_t seed,
+    const float* item_biases, const rmb200_extra_t* extra, rmb200_exposure_t* exposure, rmb200_beyond_t* beyond)
+{
+    (void)nthreads;
+    return entry<float>(A, lda, B, ldb, m, n, k, Xtrain_csr_p, Xtrain_csr_i, Xtest_csr_p, Xtest_csr_i, Xtest_csr,
+                        k_metrics, cumulative, break_ties_with_noise, p_at_k, tp_at_k, r_at_k, ap_at_k, tap_at_k,
+                        ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
+                        min_pos_test, seed, item_biases, extra, exposure, beyond);
+}
+
+int rmb200_calc_metrics_beyond_f64(
+    const double* A, size_t lda, const double* B, size_t ldb, int32_t m, int32_t n, int32_t k,
+    const int32_t* Xtrain_csr_p, const int32_t* Xtrain_csr_i,
+    const int32_t* Xtest_csr_p, const int32_t* Xtest_csr_i, const double* Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    double* p_at_k, double* tp_at_k, double* r_at_k, double* ap_at_k, double* tap_at_k,
+    double* ndcg_at_k, double* hit_at_k, double* rr_at_k, double* roc_auc, double* pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, int32_t nthreads, uint64_t seed,
+    const double* item_biases, const rmb200_extra_t* extra, rmb200_exposure_t* exposure, rmb200_beyond_t* beyond)
+{
+    (void)nthreads;
+    return entry<double>(A, lda, B, ldb, m, n, k, Xtrain_csr_p, Xtrain_csr_i, Xtest_csr_p, Xtest_csr_i, Xtest_csr,
+                         k_metrics, cumulative, break_ties_with_noise, p_at_k, tp_at_k, r_at_k, ap_at_k, tap_at_k,
+                         ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
+                         min_pos_test, seed, item_biases, extra, exposure, beyond);
+}
+
+int rmb200_sizeof_beyond(void) { return (int)sizeof(rmb200_beyond_t); }
+
+int rmb200_item_popularity(const int32_t* indptr, const int32_t* indices, int32_t row_begin, int32_t row_end, int32_t n,
+                           int32_t device, int32_t inputs_on_device, int64_t* counts)
+{
+    g_err.clear();
+    try {
+        return item_popularity(indptr, indices, row_begin, row_end, n, device, inputs_on_device != 0, counts);
+    } catch (const std::bad_alloc&) {
+        set_err("host allocation failed");
+        return RMB200_ERR_OOM;
+    } catch (...) {
+        set_err("unexpected C++ exception");
+        return RMB200_ERR_CUDA;
+    }
+}
 
 int rmb200_device_count(void)
 {

@@ -30,7 +30,7 @@ struct MetricsParams {
     int* status_out;                      // optional, offset to the batch
     int* topk_items; T* topk_scores;      // optional [mb][K], offset to the batch
     long long* pos_rank;                  // optional [nnz_test] (absolute)
-    int* list_len;                        // optional [mb]: length of the user's ranked list, 0 where it is undefined (exposure.cuh)
+    int* list_len;                        // optional [mb]: length of the user's ranked list, 0 where it is undefined (exposure.cuh, beyond.cuh)
 };
 
 constexpr int METRICS_WARPS = 8;           // users (warps) per block of user_metrics_kernel
@@ -409,13 +409,16 @@ __global__ void all_equal_check_kernel(const T* __restrict__ cand_score, const i
 //   metric_partial_kernel  one block per 256 users of a batch and metric (blockIdx.y): sum and count of the non-NaN
 //                          entries of every column (W = K if cumulative else 1), users in ascending order
 //   metric_final_kernel    one thread per (metric, column): adds the blocks' partials in ascending order, divides
+// A table has `slots` metrics: the ten accuracy metrics (the first eight have W columns, ROC/PR-AUC one), or the three of
+// beyond.cuh (all W columns), each with partial buffers of its own.
 constexpr int MEAN_CHUNK = 256;
 
 template <typename T>
 struct MeanParams {
-    const T* out[10];        // metric rows of the batch (nullptr: not requested), row stride W (roc/pr: 1)
+    const T* out[10];        // metric rows of the batch (nullptr: not requested), row stride W (slots >= wide: 1)
     int nb, W;
-    double* part_sum;        // [blocks_total][10][W]
+    int slots, wide;         // metrics in the table; the first `wide` have W columns
+    double* part_sum;        // [blocks_total][slots][W]
     int* part_cnt;
     int block0;              // first partial block of this batch
 };
@@ -425,11 +428,11 @@ __global__ void metric_partial_kernel(const __grid_constant__ MeanParams<T> P)
 {
     const int q = blockIdx.y;
     const T* src = P.out[q];
-    const int W = P.W, Wq = q < 8 ? W : 1;
+    const int W = P.W, Wq = q < P.wide ? W : 1;
     const int u0 = blockIdx.x * MEAN_CHUNK;
     const int u1 = min(u0 + MEAN_CHUNK, P.nb);
-    double* ps = P.part_sum + ((size_t)(P.block0 + blockIdx.x) * 10 + q) * W;
-    int* pc = P.part_cnt + ((size_t)(P.block0 + blockIdx.x) * 10 + q) * W;
+    double* ps = P.part_sum + ((size_t)(P.block0 + blockIdx.x) * P.slots + q) * W;
+    int* pc = P.part_cnt + ((size_t)(P.block0 + blockIdx.x) * P.slots + q) * W;
     if (Wq > 1) {
         // a thread per column walks the chunk's users in order (consecutive threads read consecutive columns)
         for (int c = threadIdx.x; c < W; c += blockDim.x) {
@@ -462,13 +465,16 @@ __global__ void metric_partial_kernel(const __grid_constant__ MeanParams<T> P)
 }
 
 __global__ void metric_final_kernel(const double* __restrict__ part_sum, const int* __restrict__ part_cnt, const int blocks,
-                                    const int W, double* __restrict__ means, long long* __restrict__ counts)
+                                    const int slots, const int W, double* __restrict__ means, long long* __restrict__ counts)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;     // (metric, column)
-    if (i >= 10 * W) return;
+    const int cells = slots * W;
+    if (i >= cells) return;
     double s = 0.;
     long long c = 0;
-    for (int b = 0; b < blocks; b++) { s += part_sum[(size_t)b * 10 * W + i]; c += part_cnt[(size_t)b * 10 * W + i]; }
+    const double* ps = part_sum + i;
+    const int* pc = part_cnt + i;
+    for (int b = 0; b < blocks; b++, ps += cells, pc += cells) { s += *ps; c += *pc; }
     if (means) means[i] = c > 0 ? s / (double)c : CUDART_NAN;
     if (counts) counts[i] = c;
 }

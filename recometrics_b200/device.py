@@ -24,7 +24,7 @@ import numpy as np
 from scipy.sparse import issparse
 
 from . import _capi
-from .frontend import _KEYS, EvalResult, _canonical_csr
+from .frontend import _KEYS, EvalResult, _canonical_csr, _popularity_array, item_popularity as _item_popularity
 
 __all__ = ["DeviceCSR", "calc_reco_metrics_device"]
 
@@ -99,10 +99,13 @@ def calc_reco_metrics_device(
         all_metrics=False, break_ties_with_noise=True, min_pos_test=1, min_items_pool=2,
         consider_cold_start=True, cumulative=False, seed=1,
         user_range=None, strict_min_pos_test=False, return_topk=False, return_status=False, scoring_path="auto",
-        return_means=False, means_only=False, return_exposure=False):
+        return_means=False, means_only=False, return_exposure=False,
+        novelty=False, avg_popularity=False, diversity=False, item_popularity=None):
     """``calc_reco_metrics_ex`` for inputs that live on the GPU (see the module docstring).  Returns an
     :class:`EvalResult` whose ``metrics`` / ``status`` / ``topk_*`` / ``exposure`` entries are torch CUDA tensors on the
-    device of ``A`` (``means`` / ``counts`` / ``catalogue`` are small and come back as Python numbers / numpy vectors)."""
+    device of ``A`` (``means`` / ``counts`` / ``catalogue`` are small and come back as Python numbers / numpy vectors).
+    ``item_popularity`` (for ``novelty`` / ``avg_popularity``) may be a numpy array or a torch tensor; without it the counts
+    of ``X_train``'s first m rows are taken on the device."""
     torch = _torch()
     if A is None or B is None:
         raise ValueError("'A' and 'B' must be passed (device-resident factor matrices).")
@@ -207,11 +210,37 @@ def calc_reco_metrics_device(
                              metric_counts=ptr(counts), skip_row_copy=bool(means_only))
     item_counts = torch.zeros(n, dtype=torch.int64, device=dev) if return_exposure else None
     expo = _capi.make_exposure(ptr(item_counts)) if return_exposure else None
+    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
+    brows_t, bmeans, bcounts, bey = {}, None, None, None
+    if any(bflags.values()):
+        pop = None
+        if bflags["novelty"] or bflags["avg_popularity"]:
+            if item_popularity is None:
+                pop = _item_popularity(X_train, m=m)
+            elif isinstance(item_popularity, torch.Tensor):
+                if item_popularity.dim() != 1 or item_popularity.shape[0] != n:
+                    raise ValueError("'item_popularity' must be a 1-d array with one count per item (%d)." % n)
+                if item_popularity.dtype.is_floating_point or item_popularity.dtype.is_complex or item_popularity.dtype == torch.bool:
+                    raise TypeError("'item_popularity' must hold integer counts.")
+                pop = item_popularity.to(device=dev, dtype=torch.int64).contiguous()
+                if n and bool(((pop < 0) | (pop > m)).any()):
+                    raise ValueError("'item_popularity' counts must lie in [0, %d] (the number of users)." % m)
+            else:
+                pop = torch.from_numpy(_popularity_array(item_popularity, n, m)).to(dev)
+        for name, on in bflags.items():
+            if on:
+                brows_t[name] = torch.empty(m * W, dtype=tdt, device=dev)
+                if user_range is not None:
+                    brows_t[name].fill_(float("nan"))
+        bmeans = torch.full((3 * W,), float("nan"), dtype=torch.float64, device=dev) if return_means else None
+        bcounts = torch.zeros(3 * W, dtype=torch.int64, device=dev) if return_means else None
+        bey = _capi.make_beyond({name: t.data_ptr() for name, t in brows_t.items()}, ptr(pop), m, ptr(bmeans), ptr(bcounts))
     torch.cuda.synchronize(dev)            # the library runs on its own stream: the caller's pending writes must have landed
     rc = _capi.calc_metrics(dtype, dA.ptr, dA.ld, dB.ptr, dB.ld, m, n, dA.shape[1],
                             ptr(X_train.indptr), ptr(X_train.indices) if X_train.indices.numel() else None,
                             ptr(X_test.indptr), ptr(X_test.indices), ptr(tev), K, cumulative, bool(break_ties_with_noise), outs,
-                            bool(consider_cold_start), min_items_pool, min_pos_test, 1, seed, bias_ptr, extra, exposure=expo)
+                            bool(consider_cold_start), min_items_pool, min_pos_test, 1, seed, bias_ptr, extra, exposure=expo,
+                            beyond=bey)
     _capi.raise_for_status(rc)
 
     metrics, mean_d, count_d = {}, None, None
@@ -229,6 +258,16 @@ def calc_reco_metrics_device(
             wide = cumulative and q in _capi.TOPK_METRICS
             mean_d[key] = mh[i * W:(i + 1) * W].copy() if wide else float(mh[i * W])
             count_d[key] = ch[i * W:(i + 1) * W].copy() if wide else int(ch[i * W])
+    bmh, bch = (bmeans.cpu().numpy(), bcounts.cpu().numpy()) if bmeans is not None else (None, None)
+    for i, (name, key) in enumerate(_capi.BEYOND_KEYS):
+        if name not in brows_t:
+            continue
+        if not means_only:
+            metrics[key] = brows_t[name].view(m, K) if cumulative else brows_t[name]
+        if return_means:
+            mean_d[key] = bmh[i * W:(i + 1) * W].copy() if cumulative else float(bmh[i * W])
+            count_d[key] = bch[i * W:(i + 1) * W].copy() if cumulative else int(bch[i * W])
+    metrics["K"] = metrics.pop("K")
     return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
                       topk_items=None if topk_items is None else topk_items.view(m, K),
                       topk_scores=None if topk_scores is None else topk_scores.view(m, K),

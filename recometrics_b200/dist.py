@@ -7,9 +7,9 @@ plumbing for that gather only.
 """
 import numpy as np
 
-from .frontend import calc_reco_metrics_ex
+from .frontend import calc_reco_metrics_ex, item_popularity
 
-__all__ = ["shard_bounds", "gather_metric_rows", "reduce_exposure", "calc_reco_metrics_sharded"]
+__all__ = ["shard_bounds", "gather_metric_rows", "reduce_exposure", "reduce_popularity", "calc_reco_metrics_sharded"]
 
 
 def shard_bounds(m, world_size, rank):
@@ -81,19 +81,36 @@ def reduce_exposure(local_counts, group=None, dst=0, local_users=0):
     return total[:-1].copy(), _capi.exposure_stats(total[:-1], users=int(total[-1]))
 
 
+def reduce_popularity(local_counts, group=None):
+    """Sum the ranks' item popularity counts (:func:`recometrics_b200.item_popularity` of each rank's block of ``X_train``
+    rows; int64 [n], the same n everywhere) on every rank: one ``all_reduce``.  The sum is the popularity over all users,
+    exactly, so every rank's Novelty@K / AvgPop@K rows are those of one call over all users.  Returns numpy int64 [n]."""
+    import torch
+    import torch.distributed as dist
+
+    dev = torch.device("cuda", torch.cuda.current_device()) if dist.get_backend(group) == "nccl" else torch.device("cpu")
+    t = torch.from_numpy(np.ascontiguousarray(local_counts, dtype=np.int64).copy()).to(dev)
+    dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    return t.cpu().numpy()
+
+
 def calc_reco_metrics_sharded(X_train, X_test, A, B, k=5, group=None, dst=0, return_exposure=False, **kwargs):
     """Evaluate with every rank of `group` taking its block of users on its current CUDA device.
 
     Every rank passes the same (full) inputs; only the block's rows of A and of the CSR matrices are
     copied to that rank's GPU, B entirely.  Returns the reference-style dict on `dst` (None elsewhere).
     ``return_exposure``: returns ``(dict, item_counts, catalogue)`` on `dst` instead, the ranks' item exposure summed by
-    :func:`reduce_exposure`."""
+    :func:`reduce_exposure`.  ``novelty`` / ``avg_popularity`` without ``item_popularity``: every rank counts its block's
+    ``X_train`` rows and :func:`reduce_popularity` adds them up, so the rows equal those of one call over all users."""
     import torch.distributed as dist
 
     world = dist.get_world_size(group)
     rank = dist.get_rank(group)
     m = X_test.shape[0]
     b, e = shard_bounds(m, world, rank)
+    if (kwargs.get("novelty") or kwargs.get("avg_popularity")) and kwargs.get("item_popularity") is None:
+        local = item_popularity(X_train, user_range=(b, e)) if X_train is not None else np.zeros(X_test.shape[1], dtype=np.int64)
+        kwargs["item_popularity"] = reduce_popularity(local, group=group)
     res = calc_reco_metrics_ex(X_train, X_test, A, B, k=k, user_range=(b, e), return_exposure=return_exposure, **kwargs)
     K = res.metrics["K"]
     local = {name: v[b:e] for name, v in res.metrics.items() if name != "K"}

@@ -25,7 +25,7 @@ from scipy.sparse import csr_array, issparse
 
 from . import _capi
 
-__all__ = ["calc_reco_metrics", "calc_reco_metrics_ex", "EvalResult"]
+__all__ = ["calc_reco_metrics", "calc_reco_metrics_ex", "EvalResult", "item_popularity"]
 
 # reference dict keys, in the order the reference inserts them (__init__.py:591-610)
 _KEYS = (("p", "P@K"), ("tp", "TP@K"), ("r", "R@K"), ("ap", "AP@K"), ("tap", "TAP@K"),
@@ -67,6 +67,53 @@ def _canonical_csr(X):
     indptr = X.indptr if X.indptr.dtype == np.int32 else X.indptr.astype(np.int32)
     indices = X.indices if X.indices.dtype == np.int32 else X.indices.astype(np.int32)
     return X, np.ascontiguousarray(indptr), np.ascontiguousarray(indices)
+
+
+def _popularity_array(item_popularity, n, m):
+    """A caller's item popularity for Novelty@K / AvgPop@K: integer counts, one per item, each in [0, m]; int64 numpy."""
+    p = np.asarray(item_popularity)
+    if p.ndim != 1 or p.shape[0] != n:
+        raise ValueError("'item_popularity' must be a 1-d array with one count per item (%d)." % n)
+    if p.dtype.kind not in "iu":
+        raise TypeError("'item_popularity' must hold integer counts.")
+    if p.size and (p.min() < 0 or p.max() > m):
+        raise ValueError("'item_popularity' counts must lie in [0, %d] (the number of users)." % m)
+    return np.ascontiguousarray(p, dtype=np.int64)
+
+
+def _popularity_rows(rows, m, user_range):
+    """Rows [begin, end) of an item_popularity count: user_range, else the first m rows (default: all)."""
+    b, e = (0, rows if m is None else int(m)) if user_range is None else (int(user_range[0]), int(user_range[1]))
+    if not (0 <= b <= e <= rows):
+        raise ValueError("rows to count must lie within [0, %d] (the rows of 'X_train')." % rows)
+    return b, e
+
+
+def item_popularity(X_train, m=None, user_range=None, device=-1):
+    """How many users have each item in their ``X_train`` row -- the column count of rows ``[0, m)`` (default: every row) or
+    of rows ``user_range=(begin, end)`` -- counted on the GPU.  This is the popularity of ``novelty`` / ``avg_popularity``
+    (with ``U = m``); the evaluation calls compute it when they are not given one, so a caller who evaluates several models
+    against one split computes it once and passes it as ``item_popularity``.  ``X_train``: a scipy sparse matrix (returns a
+    numpy int64 ``[n]``; ``device``: the CUDA ordinal, -1 = default) or a :class:`DeviceCSR` (returns a torch int64 ``[n]``
+    on its device)."""
+    from .device import DeviceCSR
+    if isinstance(X_train, DeviceCSR):
+        import torch
+        rows, n = int(X_train.shape[0]), int(X_train.shape[1])
+        b, e = _popularity_rows(rows, m, user_range)
+        dev = X_train.indptr.device
+        counts = torch.zeros(n, dtype=torch.int64, device=dev)
+        torch.cuda.synchronize(dev)            # the library runs on its own stream: the caller's pending writes must have landed
+        _capi.item_popularity(X_train.indptr.data_ptr(), X_train.indices.data_ptr() if X_train.indices.numel() else None,
+                              b, e, n, counts.data_ptr(), device=dev.index, inputs_on_device=True)
+        return counts
+    if not issparse(X_train):
+        raise TypeError("'X_train' must be a sparse matrix or a DeviceCSR.")
+    X_train, indptr, indices = _canonical_csr(X_train)
+    b, e = _popularity_rows(X_train.shape[0], m, user_range)
+    counts = np.zeros(X_train.shape[1], dtype=np.int64)
+    _capi.item_popularity(indptr, indices, b, e, X_train.shape[1], counts, device=device)
+    return counts
 
 
 def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ties_with_noise,
@@ -179,7 +226,8 @@ def calc_reco_metrics_ex(
         consider_cold_start=True, cumulative=False, nthreads=-1, seed=1,
         device=-1, user_range=None, strict_min_pos_test=False,
         return_topk=False, return_ranks=False, return_status=False, scoring_path="auto",
-        return_means=False, means_only=False, filter_stats=False, nan_bits=None, devices=None, return_exposure=False):
+        return_means=False, means_only=False, filter_stats=False, nan_bits=None, devices=None, return_exposure=False,
+        novelty=False, avg_popularity=False, diversity=False, item_popularity=None):
     """Same evaluation as :func:`calc_reco_metrics`, returning an :class:`EvalResult` with the
     reference-style dict plus timing and the optional extras (top-K ids/scores, held-out ranks,
     per-user status).  ``user_range=(begin, end)`` evaluates only those rows (the sharding unit);
@@ -193,7 +241,13 @@ def calc_reco_metrics_ex(
     metric is undefined (R's ``NA_REAL``) instead of a plain NaN.  ``filter_stats``: fill ``timing["filter_err_ratio_max"]``.
     ``return_exposure``: count, on the device, how many evaluated users have each item in their ranked top-K list
     (``result.exposure``, int64 ``[n]``: ``numpy.bincount`` of the defined ``topk_items``) and derive the catalogue's coverage,
-    Gini index and entropy from the counts (``result.catalogue``); the lists themselves stay on the device."""
+    Gini index and entropy from the counts (``result.catalogue``); the lists themselves stay on the device.
+    ``novelty`` / ``avg_popularity`` / ``diversity``: per-user Novelty@K, AvgPop@K and ILD@K (intra-list diversity: the mean
+    pairwise cosine distance of the listed items' rows of ``B``) of the ranked lists, computed on the device -- rows
+    ``result.metrics["Novelty@K"]``, ``["AvgPop@K"]``, ``["ILD@K"]`` (``(m,)``, ``(m, k)`` when ``cumulative``) and, with
+    ``return_means``, their means and counts under the same keys; NaN for users without a list.  ``item_popularity``: int64
+    ``[n]`` counts of how many of the m users have each item in ``X_train`` (see :func:`item_popularity`, which computes it
+    when it is not given).  ``all_metrics`` does not turn these on."""
     flags = dict(p=precision, tp=trunc_precision, r=recall, ap=average_precision, tap=trunc_average_precision,
                  ndcg=ndcg, hit=hit, rr=rr, roc=roc_auc, pr=pr_auc)
     flags = {q: bool(v) or bool(all_metrics) for q, v in flags.items()}
@@ -227,10 +281,30 @@ def calc_reco_metrics_ex(
                              skip_row_copy=bool(means_only), filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
     item_counts = np.zeros(prep["n"], dtype=np.int64) if return_exposure else None
     expo = _capi.make_exposure(item_counts) if return_exposure else None
+    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
+    brows, bmeans, bcounts, bey = {}, None, None, None
+    if any(bflags.values()):
+        pop = None
+        if bflags["novelty"] or bflags["avg_popularity"]:
+            if item_popularity is not None:
+                pop = _popularity_array(item_popularity, prep["n"], m)
+            else:
+                pop = np.zeros(prep["n"], dtype=np.int64)
+                _capi.item_popularity(prep["trp"], prep["tri"], 0, m, prep["n"], pop,
+                                      device=device if device >= 0 else (devices[0] if devices else -1))
+        for name, on in bflags.items():
+            if on:
+                brows[name] = np.empty(m * W, dtype=dtype)
+                if user_range is not None:
+                    brows[name].fill(np.nan)
+        bmeans = np.full(3 * W, np.nan, dtype=np.float64) if return_means else None
+        bcounts = np.zeros(3 * W, dtype=np.int64) if return_means else None
+        bey = _capi.make_beyond(brows, pop, m, bmeans, bcounts)
     rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, prep["n"], prep["p"],
                             prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
                             bool(break_ties_with_noise), outs, prep["consider_cold_start"], prep["min_items_pool"],
-                            prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"], extra, exposure=expo)
+                            prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"], extra, exposure=expo,
+                            beyond=bey)
     _capi.raise_for_status(rc)
 
     metrics, mean_d, count_d = {}, None, None
@@ -247,6 +321,15 @@ def calc_reco_metrics_ex(
             wide = cumulative and q in _capi.TOPK_METRICS
             mean_d[key] = means[i * W:(i + 1) * W].copy() if wide else float(means[i * W])
             count_d[key] = counts[i * W:(i + 1) * W].copy() if wide else int(counts[i * W])
+    for i, (name, key) in enumerate(_capi.BEYOND_KEYS):
+        if name not in brows:
+            continue
+        if not means_only:
+            metrics[key] = brows[name].reshape(m, K) if cumulative else brows[name]
+        if return_means:
+            mean_d[key] = bmeans[i * W:(i + 1) * W].copy() if cumulative else float(bmeans[i * W])
+            count_d[key] = bcounts[i * W:(i + 1) * W].copy() if cumulative else int(bcounts[i * W])
+    metrics["K"] = metrics.pop("K")
     return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
                       topk_items=None if topk_items is None else topk_items.reshape(m, K),
                       topk_scores=None if topk_scores is None else topk_scores.reshape(m, K),
