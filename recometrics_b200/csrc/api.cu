@@ -644,6 +644,27 @@ int exposure_of_nobody(rmb200_exposure_t* expo, int n, bool counts_on_device)
     return exposure_stats(zero.data(), n, expo);
 }
 
+// One per-user output of a call: the caller's rows (host or device; null: not requested) at row_bytes per user; a host
+// output is written into one of two result sets and copied out behind its batch (Call::send_results)
+struct RowOut {
+    void* base = nullptr;
+    size_t row_bytes = 0;
+    bool skippable = false;                     // left on the device by rmb200_extra_t::skip_row_copy (metric and beyond rows)
+    DevBuf staged[2];
+    void set(void* p, size_t bytes, bool skip) { base = p; row_bytes = bytes; skippable = skip; }
+};
+
+// One [slots][W] table of means / counts over the users of a call (the first `wide` slots have W columns, the others one):
+// slot q reduces row output first_row + q into the caller's means / counts (host or device; both null: not requested)
+struct MeanTable {
+    int slots = 0, wide = 0, first_row = 0;
+    double* means = nullptr; long long* counts = nullptr;
+    DevBuf part_sum, part_cnt;                  // per 256 users of every batch (metric_partial_kernel), added up in order at the end
+    DevBuf d_means, d_counts;                   // the final values of host outputs
+    bool on() const { return means || counts; }
+    void set(int s, int w, int row0, double* m, int64_t* c) { slots = s; wide = w; first_row = row0; means = m; counts = reinterpret_cast<long long*>(c); }
+};
+
 // One evaluation call on one device.  plan() makes every decision that needs only the arguments and the device; the resident
 // steps (csr_slices .. batch_buffers) put on the device what every batch reads; run_batch() evaluates one batch of UB users.
 // All of it runs on the legacy default stream `st`, but the uploads of host inputs (PrefetchStream) and result copies (ResultStream).
@@ -663,14 +684,18 @@ struct Call {
     cudaStream_t st = nullptr;                  // legacy default stream: ordered after the caller's default-stream work
     PhaseTimer pt{st}, pk{st};                  // phases; the dominant scoring kernel alone
     rmb200_timing_t tm;
+    // the row outputs, in the order their copies leave: the 10 metrics (MetricsParams order), status, top-K items and scores,
+    // Novelty / AvgPop / ILD
+    static constexpr int RO_STATUS = 10, RO_TOPK_ITEMS = 11, RO_TOPK_SCORES = 12, RO_BEYOND = 13, ROW_OUTS = 16;
     // ---- the plan ----
     int mip = 0, mpt = 0, C = 0, p_pad = 0, n_pad = 0, n_pad128 = 0, KB = 0, f_stages = 0, nsm = 148, UB = 0, fma_slices = 1, mean_W = 1;
     size_t rs = 1;
     T nan_value = std::numeric_limits<T>::quiet_NaN();
-    bool want_roc = false, want_pr = false, count_ranks = false, want_means = false, want_filter_stats = false, want_exposure = false;
-    bool want_pop = false, want_ild = false, want_beyond = false, want_beyond_means = false;   // beyond.cuh
+    bool want_roc = false, want_pr = false, count_ranks = false, want_filter_stats = false, want_exposure = false;
+    bool want_pop = false, want_ild = false, want_beyond = false;   // beyond.cuh
     int unit_pitch = 0, unit_nch = 0;           // ILD: row pitch of the unit-row image (elements), 16-byte chunks per lane
-    T* bey_out[3] = {nullptr, nullptr, nullptr};   // caller's Novelty / AvgPop / ILD rows (null: not requested)
+    RowOut row_outs[ROW_OUTS];
+    MeanTable mean_tables[2];                   // the 10 metrics {10, 8}; Novelty / AvgPop / ILD {3, 3}
     bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
     int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
     int fo_chunk = 0; size_t fo_bytes = 0;
@@ -685,11 +710,10 @@ struct Call {
     DevBuf d_Bt, d_bias, d_Brow, d_Bb, d_maxbn, d_chunkn;
     DevBuf d_status, d_flags, d_umin, d_pos_raw, d_pos_sorted, d_pos_perm, d_pos_item, d_auc, d_log2, d_pos_rank;
     DevBuf d_fo, d_near, d_nz_mark, d_nz_list, d_nz_cnt, d_At_nz;
-    DevBuf d_At, d_cs, d_ci, d_cc, d_out[2][10], d_tki[2], d_tks[2], d_stat_out[2], d_Ab, d_anorm;
+    DevBuf d_At, d_cs, d_ci, d_cc, d_Ab, d_anorm;
     DevBuf d_capx, d_overflow, d_fb_list, d_At_fb;
-    DevBuf d_psum, d_pcnt, d_means, d_mcounts;
     DevBuf d_expo_hist, d_list_len, d_expo_counts;
-    DevBuf d_pop, d_poptab, d_pop_bad, d_unit, d_bout[2][3], d_bpsum, d_bpcnt, d_bmeans, d_bcounts;
+    DevBuf d_pop, d_poptab, d_pop_bad, d_unit;
     const long long* pop_d = nullptr;           // the caller's popularity counts on the device
     PrefetchStream pf;                          // (declared after the buffers they fill or read: destroyed, i.e. drained, before them)
     ResultStream rsx;
@@ -714,15 +738,22 @@ struct Call {
         C = (K <= 64) ? 256 : (K <= 192 ? 512 : 1024);
         want_roc = a.out[8] != nullptr; want_pr = a.out[9] != nullptr;
         count_ranks = want_roc || want_pr || ex->pos_rank;
-        want_means = ex->metric_means || ex->metric_counts;
         want_filter_stats = ex->filter_stats != 0;
         want_exposure = a.expo != nullptr;
+        rs = a.cumulative ? (size_t)K : 1;
+        mean_W = a.cumulative ? K : 1;
+        for (int q = 0; q < 10; q++) row_outs[q].set(a.out[q], (q < 8 ? rs : 1) * sizeof(T), true);
+        row_outs[RO_STATUS].set(ex->status, sizeof(int), false);
+        row_outs[RO_TOPK_ITEMS].set(ex->topk_items, (size_t)K * sizeof(int), false);
+        row_outs[RO_TOPK_SCORES].set(ex->topk_scores, (size_t)K * sizeof(T), false);
+        mean_tables[0].set(10, 8, 0, ex->metric_means, ex->metric_counts);
         if (a.bey) {
-            bey_out[0] = static_cast<T*>(a.bey->novelty); bey_out[1] = static_cast<T*>(a.bey->avg_popularity); bey_out[2] = static_cast<T*>(a.bey->ild);
-            want_pop = bey_out[0] || bey_out[1];
-            want_ild = bey_out[2] != nullptr;
+            void* const bey[3] = {a.bey->novelty, a.bey->avg_popularity, a.bey->ild};
+            for (int q = 0; q < 3; q++) row_outs[RO_BEYOND + q].set(bey[q], rs * sizeof(T), true);
+            want_pop = bey[0] || bey[1];
+            want_ild = bey[2] != nullptr;
             want_beyond = want_pop || want_ild;
-            want_beyond_means = want_beyond && (a.bey->means || a.bey->counts);
+            if (want_beyond) mean_tables[1].set(3, 3, RO_BEYOND, a.bey->means, a.bey->counts);
         }
         if (want_ild) {            // lane l of beyond_accuracy_kernel holds 16-byte chunks l, l + 32, ... of a unit row: 1, 2, 4 or 8
             constexpr int V = 16 / (int)sizeof(T);
@@ -733,8 +764,6 @@ struct Call {
         }
         p_pad = round_up(a.k, KPAD);
         n_pad = round_up(a.n, BN);
-        rs = a.cumulative ? (size_t)K : 1;
-        mean_W = a.cumulative ? K : 1;
         // ---- which scoring path: tensor-core filter + exact re-scoring (top-K only), or FMA tiles ----
         int path_req = ex->scoring_path;                                 // 0 auto, 1 fma, 2 tensor
         if (path_req == 0) if (const char* env = std::getenv("RMB200_PATH")) {
@@ -1069,19 +1098,15 @@ struct Call {
         CK(d_cs.alloc((size_t)UB * fma_slices * C * sizeof(T)));
         CK(d_ci.alloc((size_t)UB * fma_slices * C * sizeof(int)));
         CK(d_cc.alloc((size_t)UB * fma_slices * sizeof(int)));
-        for (int set = 0; !on_dev && set < (UB < mr ? 2 : 1); set++) {
-            for (int q = 0; q < 10; q++)
-                if (a.out[q]) CK(d_out[set][q].alloc((size_t)UB * (q < 8 ? rs : 1) * sizeof(T)));
-            if (ex->topk_items) CK(d_tki[set].alloc((size_t)UB * K * sizeof(int)));
-            if (ex->topk_scores) CK(d_tks[set].alloc((size_t)UB * K * sizeof(T)));
-            if (ex->status) CK(d_stat_out[set].alloc((size_t)UB * sizeof(int)));
-        }
-        // per-metric means over the users of the call (extension): partial sums per 256 users, added up in order at the end
-        if (want_means) {
-            int mean_blocks_total = 0;
-            for (int b0 = 0; b0 < mr; b0 += UB) mean_blocks_total += (((mr - b0) < UB ? (mr - b0) : UB) + rmb::MEAN_CHUNK - 1) / rmb::MEAN_CHUNK;
-            CK(d_psum.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(double)));
-            CK(d_pcnt.alloc((size_t)mean_blocks_total * 10 * mean_W * sizeof(int)));
+        for (int set = 0; !on_dev && set < (UB < mr ? 2 : 1); set++)
+            for (RowOut& r : row_outs)
+                if (r.base) CK(r.staged[set].alloc((size_t)UB * r.row_bytes));
+        int mean_blocks_total = 0;
+        for (int b0 = 0; b0 < mr; b0 += UB) mean_blocks_total += (((mr - b0) < UB ? (mr - b0) : UB) + rmb::MEAN_CHUNK - 1) / rmb::MEAN_CHUNK;
+        for (MeanTable& t : mean_tables) {
+            if (!t.on()) continue;
+            CK(t.part_sum.alloc((size_t)mean_blocks_total * t.slots * mean_W * sizeof(double)));
+            CK(t.part_cnt.alloc((size_t)mean_blocks_total * t.slots * mean_W * sizeof(int)));
         }
         // item exposure: one uint32 count per item for the whole call (at most mr users each), [n] = users counted
         if (want_exposure) {
@@ -1089,16 +1114,6 @@ struct Call {
             CK(cudaMemsetAsync(d_expo_hist.p, 0, ((size_t)a.n + 1) * sizeof(unsigned), st));
         }
         if (want_exposure || want_beyond) CK(d_list_len.alloc((size_t)UB * sizeof(int)));
-        // beyond-accuracy rows: result sets of their own (host outputs), partial sums of their means
-        for (int set = 0; !on_dev && set < (UB < mr ? 2 : 1); set++)
-            for (int q = 0; q < 3; q++)
-                if (bey_out[q]) CK(d_bout[set][q].alloc((size_t)UB * rs * sizeof(T)));
-        if (want_beyond_means) {
-            int mean_blocks_total = 0;
-            for (int b0 = 0; b0 < mr; b0 += UB) mean_blocks_total += (((mr - b0) < UB ? (mr - b0) : UB) + rmb::MEAN_CHUNK - 1) / rmb::MEAN_CHUNK;
-            CK(d_bpsum.alloc((size_t)mean_blocks_total * 3 * mean_W * sizeof(double)));
-            CK(d_bpcnt.alloc((size_t)mean_blocks_total * 3 * mean_W * sizeof(int)));
-        }
         return RMB200_OK;
     }
     // upload of users [b0, b0 + UB) into staging buffer `slot`, on the prefetch stream
@@ -1339,6 +1354,14 @@ struct Call {
         }
         return RMB200_OK;
     }
+    // where batch b writes row output i: the caller's rows on device-resident calls, else the batch's result set
+    template <typename U> U* rows_of(int i, const Batch& b) const
+    {
+        const RowOut& r = row_outs[i];
+        if (!r.base) return nullptr;
+        if (!on_dev) return static_cast<U*>(r.staged[b.slot].p);
+        return reinterpret_cast<U*>(static_cast<unsigned char*>(r.base) + (size_t)(ub + b.b0) * r.row_bytes);
+    }
     // per-user metrics (and the partial sums of their means) into the caller's rows, or into the batch's result set
     int metrics(Batch& b)
     {
@@ -1353,21 +1376,12 @@ struct Call {
         mp.auc_cnt = d_auc.as<unsigned int>(); mp.umin = d_umin.as<unsigned long long>();
         mp.pos_perm = d_pos_perm.as<int>(); mp.log2tab = d_log2.as<double>();
         mp.nan_value = nan_value;
-        T* outs[10];
         if (!on_dev && rsx.copied_valid[b.slot]) CK(cudaStreamWaitEvent(st, rsx.copied[b.slot], 0));      // the set's previous rows have left
-        const size_t row = (size_t)(ub + b.b0);
-        const int slot = b.slot;
-        for (int q = 0; q < 10; q++) {
-            const size_t stride = q < 8 ? rs : 1;
-            if (!a.out[q]) outs[q] = nullptr;
-            else if (on_dev) outs[q] = a.out[q] + row * stride;
-            else outs[q] = d_out[slot][q].as<T>();
-        }
-        mp.p = outs[0]; mp.tp = outs[1]; mp.r = outs[2]; mp.ap = outs[3]; mp.tap = outs[4];
-        mp.ndcg = outs[5]; mp.hit = outs[6]; mp.rr = outs[7]; mp.roc = outs[8]; mp.pr = outs[9];
-        mp.status_out = !ex->status ? nullptr : on_dev ? ex->status + row : d_stat_out[slot].as<int>();
-        mp.topk_items = !ex->topk_items ? nullptr : on_dev ? ex->topk_items + row * K : d_tki[slot].as<int>();
-        mp.topk_scores = !ex->topk_scores ? nullptr : on_dev ? reinterpret_cast<T*>(ex->topk_scores) + row * K : d_tks[slot].as<T>();
+        mp.p = rows_of<T>(0, b); mp.tp = rows_of<T>(1, b); mp.r = rows_of<T>(2, b); mp.ap = rows_of<T>(3, b); mp.tap = rows_of<T>(4, b);
+        mp.ndcg = rows_of<T>(5, b); mp.hit = rows_of<T>(6, b); mp.rr = rows_of<T>(7, b); mp.roc = rows_of<T>(8, b); mp.pr = rows_of<T>(9, b);
+        mp.status_out = rows_of<int>(RO_STATUS, b);
+        mp.topk_items = rows_of<int>(RO_TOPK_ITEMS, b);
+        mp.topk_scores = rows_of<T>(RO_TOPK_SCORES, b);
         mp.pos_rank = pos_rank_d;
         mp.list_len = (want_exposure || want_beyond) ? d_list_len.as<int>() : nullptr;
         TRY(wait_test_rows());
@@ -1378,33 +1392,23 @@ struct Call {
                 d_ci.as<int>(), C, d_list_len.as<int>(), b.nb, d_expo_hist.as<unsigned>(), a.n);
             TRY(launched());
         }
-        T* bouts[3] = {nullptr, nullptr, nullptr};
         if (want_beyond) {
             BeyondParams<T> bp;
             bp.items = d_ci.as<int>(); bp.C = C; bp.list_len = d_list_len.as<int>(); bp.nb = b.nb; bp.K = K; bp.cumulative = a.cumulative;
             bp.pop = want_pop ? d_poptab.as<double2>() : nullptr;
             bp.unit = want_ild ? d_unit.as<T>() : nullptr; bp.pitch = unit_pitch;
-            for (int q = 0; q < 3; q++)
-                bouts[q] = !bey_out[q] ? nullptr : on_dev ? bey_out[q] + row * rs : d_bout[slot][q].as<T>();
-            bp.nov = bouts[0]; bp.avgpop = bouts[1]; bp.ild = bouts[2];
+            bp.nov = rows_of<T>(RO_BEYOND, b); bp.avgpop = rows_of<T>(RO_BEYOND + 1, b); bp.ild = rows_of<T>(RO_BEYOND + 2, b);
             bp.nan_value = nan_value;
             TRY(launch_beyond(bp));
         }
         const int mblocks = (b.nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
-        if (want_means) {
+        for (const MeanTable& t : mean_tables) {
+            if (!t.on()) continue;
             MeanParams<T> qp;
-            for (int q = 0; q < 10; q++) qp.out[q] = outs[q];
-            qp.nb = b.nb; qp.W = mean_W; qp.slots = 10; qp.wide = 8;
-            qp.part_sum = d_psum.as<double>(); qp.part_cnt = d_pcnt.as<int>(); qp.block0 = mean_block0;
-            metric_partial_kernel<T><<<dim3(mblocks, 10), MEAN_CHUNK, 0, st>>>(qp);
-            TRY(launched());
-        }
-        if (want_beyond_means) {
-            MeanParams<T> qp;
-            for (int q = 0; q < 10; q++) qp.out[q] = q < 3 ? bouts[q] : nullptr;
-            qp.nb = b.nb; qp.W = mean_W; qp.slots = 3; qp.wide = 3;
-            qp.part_sum = d_bpsum.as<double>(); qp.part_cnt = d_bpcnt.as<int>(); qp.block0 = mean_block0;
-            metric_partial_kernel<T><<<dim3(mblocks, 3), MEAN_CHUNK, 0, st>>>(qp);
+            for (int q = 0; q < 10; q++) qp.out[q] = q < t.slots ? rows_of<T>(t.first_row + q, b) : nullptr;
+            qp.nb = b.nb; qp.W = mean_W; qp.slots = t.slots; qp.wide = t.wide;
+            qp.part_sum = t.part_sum.as<double>(); qp.part_cnt = t.part_cnt.as<int>(); qp.block0 = mean_block0;
+            metric_partial_kernel<T><<<dim3(mblocks, t.slots), MEAN_CHUNK, 0, st>>>(qp);
             TRY(launched());
         }
         mean_block0 += mblocks;
@@ -1429,20 +1433,10 @@ struct Call {
         const size_t row = (size_t)(ub + b.b0), nb = (size_t)b.nb;
         CK(cudaEventRecord(rsx.ready[b.slot], st));
         CK(cudaStreamWaitEvent(rsx.s, rsx.ready[b.slot], 0));
-        for (int q = 0; q < 10; q++) {
-            if (!a.out[q] || ex->skip_row_copy) continue;
-            const size_t stride = q < 8 ? rs : 1;
-            const size_t bytes = (size_t)nb * stride * sizeof(T);
-            CK(cudaMemcpyAsync(a.out[q] + row * stride, d_out[b.slot][q].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
-            tm.d2h_bytes += (int64_t)bytes;
-        }
-        if (ex->status) { CK(cudaMemcpyAsync(ex->status + row, d_stat_out[b.slot].p, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * 4; }
-        if (ex->topk_items) { CK(cudaMemcpyAsync(ex->topk_items + row * K, d_tki[b.slot].p, (size_t)nb * K * sizeof(int), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * 4; }
-        if (ex->topk_scores) { CK(cudaMemcpyAsync(reinterpret_cast<T*>(ex->topk_scores) + row * K, d_tks[b.slot].p, (size_t)nb * K * sizeof(T), cudaMemcpyDeviceToHost, rsx.s)); tm.d2h_bytes += (int64_t)nb * K * (int64_t)sizeof(T); }
-        for (int q = 0; q < 3; q++) {
-            if (!bey_out[q] || ex->skip_row_copy) continue;
-            const size_t bytes = nb * rs * sizeof(T);
-            CK(cudaMemcpyAsync(bey_out[q] + row * rs, d_bout[b.slot][q].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
+        for (const RowOut& r : row_outs) {
+            if (!r.base || (r.skippable && ex->skip_row_copy)) continue;
+            const size_t bytes = nb * r.row_bytes;
+            CK(cudaMemcpyAsync(static_cast<unsigned char*>(r.base) + row * r.row_bytes, r.staged[b.slot].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
             tm.d2h_bytes += (int64_t)bytes;
         }
         CK(cudaEventRecord(rsx.copied[b.slot], rsx.s));
@@ -1463,24 +1457,8 @@ struct Call {
             tm.d2h_bytes += (int64_t)(nnz_te * sizeof(long long));
             pt.stop(tm.d2h_ms);
         }
-        if (want_means && !g_interrupt.load()) {
-            double* means_d = nullptr; long long* counts_d = nullptr;
-            const size_t cells = (size_t)10 * mean_W;
-            if (on_dev) { means_d = ex->metric_means; counts_d = reinterpret_cast<long long*>(ex->metric_counts); }
-            else {
-                if (ex->metric_means) { CK(d_means.alloc(cells * sizeof(double))); means_d = d_means.as<double>(); }
-                if (ex->metric_counts) { CK(d_mcounts.alloc(cells * sizeof(long long))); counts_d = d_mcounts.as<long long>(); }
-            }
-            pt.start();
-            rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_psum.as<double>(), d_pcnt.as<int>(), mean_block0, 10, mean_W, means_d, counts_d);
-            TRY(launched());
-            pt.stop(tm.metrics_ms);
-            if (!on_dev) {
-                if (ex->metric_means) { CK(cudaMemcpyAsync(ex->metric_means, means_d, cells * sizeof(double), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(double)); }
-                if (ex->metric_counts) { CK(cudaMemcpyAsync(ex->metric_counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
-            }
-        }
-        if (want_beyond_means && !g_interrupt.load()) TRY(beyond_means_out());
+        for (MeanTable& t : mean_tables)
+            if (t.on() && !g_interrupt.load()) TRY(means_out(t));
         if (want_exposure && !g_interrupt.load()) TRY(exposure_out());
         if (use_tensor && want_filter_stats) {
             float ratio = 0.f;
@@ -1491,23 +1469,22 @@ struct Call {
         CK(cudaStreamSynchronize(st));
         return RMB200_OK;
     }
-    // means / counts of the Novelty, AvgPop and ILD rows: the accuracy metrics' reduction over a table of three
-    int beyond_means_out()
+    // a table's means / counts from its partial sums, into the caller's memory (device-resident calls) or copied out
+    int means_out(MeanTable& t)
     {
-        const size_t cells = (size_t)3 * mean_W;
-        double* means_d = nullptr; long long* counts_d = nullptr;
-        if (on_dev) { means_d = a.bey->means; counts_d = reinterpret_cast<long long*>(a.bey->counts); }
-        else {
-            if (a.bey->means) { CK(d_bmeans.alloc(cells * sizeof(double))); means_d = d_bmeans.as<double>(); }
-            if (a.bey->counts) { CK(d_bcounts.alloc(cells * sizeof(long long))); counts_d = d_bcounts.as<long long>(); }
+        const size_t cells = (size_t)t.slots * mean_W;
+        double* means_d = t.means; long long* counts_d = t.counts;
+        if (!on_dev) {
+            if (t.means) { CK(t.d_means.alloc(cells * sizeof(double))); means_d = t.d_means.as<double>(); }
+            if (t.counts) { CK(t.d_counts.alloc(cells * sizeof(long long))); counts_d = t.d_counts.as<long long>(); }
         }
         pt.start();
-        rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(d_bpsum.as<double>(), d_bpcnt.as<int>(), mean_block0, 3, mean_W, means_d, counts_d);
+        rmb::metric_final_kernel<<<(int)((cells + 127) / 128), 128, 0, st>>>(t.part_sum.as<double>(), t.part_cnt.as<int>(), mean_block0, t.slots, mean_W, means_d, counts_d);
         TRY(launched());
         pt.stop(tm.metrics_ms);
         if (!on_dev) {
-            if (a.bey->means) { CK(cudaMemcpyAsync(a.bey->means, means_d, cells * sizeof(double), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(double)); }
-            if (a.bey->counts) { CK(cudaMemcpyAsync(a.bey->counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
+            if (t.means) { CK(cudaMemcpyAsync(t.means, means_d, cells * sizeof(double), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(double)); }
+            if (t.counts) { CK(cudaMemcpyAsync(t.counts, counts_d, cells * sizeof(long long), cudaMemcpyDeviceToHost, st)); tm.d2h_bytes += (int64_t)(cells * sizeof(long long)); }
         }
         return RMB200_OK;
     }
@@ -1654,6 +1631,31 @@ int resolve_devices(const rmb200_extra_t* ex, std::vector<int>& devs)
     return RMB200_OK;
 }
 
+// One means / counts table of a multi-GPU call (the caller's; both null: not requested): every device reduces its users into
+// a table of its own, the call's means are the devices' means weighted by their user counts
+struct DeviceMeans {
+    double* means; int64_t* counts; size_t cells;
+    std::vector<std::vector<double>> dev_means;
+    std::vector<std::vector<long long>> dev_counts;
+    DeviceMeans(double* m, int64_t* c, size_t n, int G) : means(m), counts(c), cells(n),
+        dev_means(m || c ? G : 0, std::vector<double>(n, 0.0)), dev_counts(m || c ? G : 0, std::vector<long long>(n, 0)) {}
+    void attach(int g, double*& m, int64_t*& c)          // device g's call reduces into its own table
+    {
+        if (dev_means.empty()) return;
+        m = dev_means[g].data(); c = reinterpret_cast<int64_t*>(dev_counts[g].data());
+    }
+    void merge() const
+    {
+        for (size_t i = 0; !dev_means.empty() && i < cells; i++) {
+            double s = 0.0; long long cnt = 0;
+            for (size_t g = 0; g < dev_means.size(); g++)
+                if (dev_counts[g][i] > 0) { s += dev_means[g][i] * (double)dev_counts[g][i]; cnt += dev_counts[g][i]; }
+            if (means) means[i] = cnt ? s / (double)cnt : std::numeric_limits<double>::quiet_NaN();
+            if (counts) counts[i] = cnt;
+        }
+    }
+};
+
 // /root/reference/src/recometrics.hpp:428-437: the reference's one call spreads the users over every core
 // (`#pragma omp parallel for schedule(dynamic) num_threads(nthreads)`); this spreads them over every listed GPU.
 template <typename T>
@@ -1684,20 +1686,14 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     SignalLatch latch;
     MultiCtx mc;
     mc.G = G;
-    const bool want_means = ex->metric_means || ex->metric_counts;
-    const int W = a0.cumulative ? a0.K : 1;
-    const size_t cells = (size_t)10 * (size_t)(W > 0 ? W : 1);
+    const size_t W = (size_t)(a0.cumulative && a0.K > 0 ? a0.K : 1);
+    DeviceMeans metric_means(ex->metric_means, ex->metric_counts, 10 * W, G);
+    DeviceMeans beyond_means(a0.bey ? a0.bey->means : nullptr, a0.bey ? a0.bey->counts : nullptr, 3 * W, G);
     std::vector<rmb200_extra_t> exs((size_t)G, *ex);
     std::vector<rmb200_timing_t> tms((size_t)G);
-    std::vector<std::vector<double>> means((size_t)G);
-    std::vector<std::vector<long long>> counts((size_t)G);
     std::vector<rmb200_exposure_t> expos((size_t)G);
     std::vector<std::vector<int64_t>> item_counts(a0.expo ? (size_t)G : 0);
-    const bool want_bmeans = a0.bey && (a0.bey->means || a0.bey->counts);
-    const size_t bcells = (size_t)3 * (size_t)(W > 0 ? W : 1);
     std::vector<rmb200_beyond_t> beys((size_t)G);
-    std::vector<std::vector<double>> bmeans((size_t)G);
-    std::vector<std::vector<long long>> bcounts((size_t)G);
     std::vector<int> rcs((size_t)G, RMB200_OK);
     std::vector<std::string> errs((size_t)G);
     std::vector<std::thread> workers;
@@ -1707,10 +1703,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
         e.device = devs[g]; e.devices = nullptr; e.n_devices = 0;
         e.user_begin = lo[g]; e.user_end = hi[g];
         e.timing = &tms[g];
-        if (want_means) {
-            means[g].assign(cells, 0.0); counts[g].assign(cells, 0);
-            e.metric_means = means[g].data(); e.metric_counts = reinterpret_cast<int64_t*>(counts[g].data());
-        }
+        metric_means.attach(g, e.metric_means, e.metric_counts);
         if (a0.expo) {
             item_counts[g].assign((size_t)a0.n, 0);
             std::memset(&expos[g], 0, sizeof(rmb200_exposure_t));
@@ -1719,10 +1712,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
         }
         if (a0.bey) {           // rows straight into the caller's arrays (every device writes its own); means per device
             beys[g] = *a0.bey;
-            if (want_bmeans) {
-                bmeans[g].assign(bcells, 0.0); bcounts[g].assign(bcells, 0);
-                beys[g].means = bmeans[g].data(); beys[g].counts = reinterpret_cast<int64_t*>(bcounts[g].data());
-            }
+            beyond_means.attach(g, beys[g].means, beys[g].counts);
         }
         workers.emplace_back([&, g]() {
             g_err.clear();
@@ -1763,22 +1753,8 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     }
     if (rc != RMB200_OK) return rc;
 
-    if (want_means) {       // means of the call = the devices' means weighted by their user counts
-        for (size_t c = 0; c < cells; c++) {
-            double s = 0.0; long long cnt = 0;
-            for (int g = 0; g < G; g++) if (counts[g][c] > 0) { s += means[g][c] * (double)counts[g][c]; cnt += counts[g][c]; }
-            if (ex->metric_means) ex->metric_means[c] = cnt ? s / (double)cnt : std::numeric_limits<double>::quiet_NaN();
-            if (ex->metric_counts) ex->metric_counts[c] = cnt;
-        }
-    }
-    if (want_bmeans) {      // the same for the beyond-accuracy means
-        for (size_t c = 0; c < bcells; c++) {
-            double s = 0.0; long long cnt = 0;
-            for (int g = 0; g < G; g++) if (bcounts[g][c] > 0) { s += bmeans[g][c] * (double)bcounts[g][c]; cnt += bcounts[g][c]; }
-            if (a0.bey->means) a0.bey->means[c] = cnt ? s / (double)cnt : std::numeric_limits<double>::quiet_NaN();
-            if (a0.bey->counts) a0.bey->counts[c] = cnt;
-        }
-    }
+    metric_means.merge();
+    beyond_means.merge();
     if (a0.expo) {          // the devices' counts added up (integers: exact), the statistics of the sum
         std::vector<int64_t> own;
         int64_t* sum = a0.expo->item_counts;

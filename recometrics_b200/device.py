@@ -24,7 +24,7 @@ import numpy as np
 from scipy.sparse import issparse
 
 from . import _capi
-from .frontend import _KEYS, EvalResult, _canonical_csr, _popularity_array, item_popularity as _item_popularity
+from .frontend import EvalResult, _ResultRows, _canonical_csr, _popularity_array, item_popularity as _item_popularity
 
 __all__ = ["DeviceCSR", "calc_reco_metrics_device"]
 
@@ -185,34 +185,27 @@ def calc_reco_metrics_device(
         bias_ptr = int(bias_keep.__cuda_array_interface__["data"][0])
 
     K = k
-    W = K if cumulative else 1
-    outs_t, outs = {}, {}
-    for q in _capi.METRIC_ORDER:
-        if flags[q]:
-            outs_t[q] = torch.empty(m * (W if q in _capi.TOPK_METRICS else 1), dtype=tdt, device=dev)
-            if user_range is not None:
-                outs_t[q].fill_(float("nan"))
-            outs[q] = outs_t[q].data_ptr()
+    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
+    tdts = {np.float32: torch.float32, np.float64: torch.float64, np.int64: torch.int64}
+    res = _ResultRows(lambda size, dt, fill: torch.empty(size, dtype=tdts[dt], device=dev) if fill is None
+                      else torch.full((size,), fill, dtype=tdts[dt], device=dev),
+                      dtype, m, K, cumulative, flags, bflags, user_range, bool(return_means) or bool(means_only))
     timing = _capi.Timing()
     status = torch.zeros(m, dtype=torch.int32, device=dev) if return_status else None
     topk_items = torch.full((m * K,), -1, dtype=torch.int32, device=dev) if return_topk else None
     topk_scores = torch.full((m * K,), float("nan"), dtype=tdt, device=dev) if return_topk else None
-    return_means = bool(return_means) or bool(means_only)
-    means = torch.full((10 * W,), float("nan"), dtype=torch.float64, device=dev) if return_means else None
-    counts = torch.zeros(10 * W, dtype=torch.int64, device=dev) if return_means else None
     ub, ue = (0, 0) if user_range is None else (int(user_range[0]), int(user_range[1]))
     if user_range is not None and ub == ue:
         ub, ue = 0, -1          # an EMPTY block; 0,0 would mean "all users" in the C-ABI
     ptr = lambda t: None if t is None else t.data_ptr()
     extra = _capi.make_extra(device=device, user_begin=ub, user_end=ue, inputs_on_device=True,
                              strict_min_pos_test=strict_min_pos_test, topk_items=ptr(topk_items), topk_scores=ptr(topk_scores),
-                             status=ptr(status), timing=timing, scoring_path=scoring_path, metric_means=ptr(means),
-                             metric_counts=ptr(counts), skip_row_copy=bool(means_only))
+                             status=ptr(status), timing=timing, scoring_path=scoring_path, metric_means=ptr(res.means),
+                             metric_counts=ptr(res.counts), skip_row_copy=bool(means_only))
     item_counts = torch.zeros(n, dtype=torch.int64, device=dev) if return_exposure else None
     expo = _capi.make_exposure(ptr(item_counts)) if return_exposure else None
-    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
-    brows_t, bmeans, bcounts, bey = {}, None, None, None
-    if any(bflags.values()):
+    bey = None
+    if res.brows:
         pop = None
         if bflags["novelty"] or bflags["avg_popularity"]:
             if item_popularity is None:
@@ -227,47 +220,16 @@ def calc_reco_metrics_device(
                     raise ValueError("'item_popularity' counts must lie in [0, %d] (the number of users)." % m)
             else:
                 pop = torch.from_numpy(_popularity_array(item_popularity, n, m)).to(dev)
-        for name, on in bflags.items():
-            if on:
-                brows_t[name] = torch.empty(m * W, dtype=tdt, device=dev)
-                if user_range is not None:
-                    brows_t[name].fill_(float("nan"))
-        bmeans = torch.full((3 * W,), float("nan"), dtype=torch.float64, device=dev) if return_means else None
-        bcounts = torch.zeros(3 * W, dtype=torch.int64, device=dev) if return_means else None
-        bey = _capi.make_beyond({name: t.data_ptr() for name, t in brows_t.items()}, ptr(pop), m, ptr(bmeans), ptr(bcounts))
+        bey = _capi.make_beyond({name: t.data_ptr() for name, t in res.brows.items()}, ptr(pop), m, ptr(res.bmeans), ptr(res.bcounts))
     torch.cuda.synchronize(dev)            # the library runs on its own stream: the caller's pending writes must have landed
     rc = _capi.calc_metrics(dtype, dA.ptr, dA.ld, dB.ptr, dB.ld, m, n, dA.shape[1],
                             ptr(X_train.indptr), ptr(X_train.indices) if X_train.indices.numel() else None,
-                            ptr(X_test.indptr), ptr(X_test.indices), ptr(tev), K, cumulative, bool(break_ties_with_noise), outs,
-                            bool(consider_cold_start), min_items_pool, min_pos_test, 1, seed, bias_ptr, extra, exposure=expo,
-                            beyond=bey)
+                            ptr(X_test.indptr), ptr(X_test.indices), ptr(tev), K, cumulative, bool(break_ties_with_noise),
+                            {q: t.data_ptr() for q, t in res.outs.items()}, bool(consider_cold_start), min_items_pool,
+                            min_pos_test, 1, seed, bias_ptr, extra, exposure=expo, beyond=bey)
     _capi.raise_for_status(rc)
 
-    metrics, mean_d, count_d = {}, None, None
-    for q, key in _KEYS:
-        if q in outs_t and not means_only:
-            metrics[key] = outs_t[q].view(m, K) if (cumulative and q in _capi.TOPK_METRICS) else outs_t[q]
-    metrics["K"] = K
-    if return_means:
-        mh, ch = means.cpu().numpy(), counts.cpu().numpy()
-        mean_d, count_d = {}, {}
-        for i, q in enumerate(_capi.METRIC_ORDER):
-            if q not in outs_t:
-                continue
-            key = dict(_KEYS)[q]
-            wide = cumulative and q in _capi.TOPK_METRICS
-            mean_d[key] = mh[i * W:(i + 1) * W].copy() if wide else float(mh[i * W])
-            count_d[key] = ch[i * W:(i + 1) * W].copy() if wide else int(ch[i * W])
-    bmh, bch = (bmeans.cpu().numpy(), bcounts.cpu().numpy()) if bmeans is not None else (None, None)
-    for i, (name, key) in enumerate(_capi.BEYOND_KEYS):
-        if name not in brows_t:
-            continue
-        if not means_only:
-            metrics[key] = brows_t[name].view(m, K) if cumulative else brows_t[name]
-        if return_means:
-            mean_d[key] = bmh[i * W:(i + 1) * W].copy() if cumulative else float(bmh[i * W])
-            count_d[key] = bch[i * W:(i + 1) * W].copy() if cumulative else int(bch[i * W])
-    metrics["K"] = metrics.pop("K")
+    metrics, mean_d, count_d = res.unpack(means_only, lambda t: t.cpu().numpy())
     return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
                       topk_items=None if topk_items is None else topk_items.view(m, K),
                       topk_scores=None if topk_scores is None else topk_scores.view(m, K),

@@ -116,6 +116,45 @@ def item_popularity(X_train, m=None, user_range=None, device=-1):
     return counts
 
 
+class _ResultRows:
+    """The per-user rows of one call -- the requested metrics and Novelty / AvgPop / ILD rows, NaN outside ``user_range`` --
+    and their means / counts tables, allocated with ``alloc(size, dtype, fill)`` (numpy or torch; ``fill=None``: left
+    uninitialised).  A table is ``[slot][W]``, ``W = K`` when ``cumulative`` else 1, over its rows in order: the ten metrics
+    (the first eight W wide, ROC / PR-AUC one value each), and the three beyond-accuracy rows (all W wide)."""
+
+    def __init__(self, alloc, dtype, m, K, cumulative, flags, bflags, user_range, return_means):
+        self.m, self.K, self.W, self.cumulative = m, K, (K if cumulative else 1), cumulative
+        fill = None if user_range is None else np.nan
+
+        def table(slots, on):       # means, counts
+            return (alloc(slots * self.W, np.float64, np.nan), alloc(slots * self.W, np.int64, 0)) if on else (None, None)
+        self.outs = {q: alloc(m * (self.W if q in _capi.TOPK_METRICS else 1), dtype, fill) for q in _capi.METRIC_ORDER if flags[q]}
+        self.means, self.counts = table(10, return_means)
+        self.brows = {name: alloc(m * self.W, dtype, fill) for name, _ in _capi.BEYOND_KEYS if bflags[name]}
+        self.bmeans, self.bcounts = table(3, return_means and bool(self.brows))
+
+    def unpack(self, means_only, to_numpy=lambda x: x):
+        """``metrics`` (W wide rows as ``(m, K)``, ``"K"`` last), ``means`` and ``counts`` of the call's EvalResult;
+        ``to_numpy`` brings a means / counts table to the host."""
+        metrics, W = {}, self.W
+        mean_d, count_d = ({}, {}) if self.means is not None else (None, None)
+        for rows, keys, wide_slots, means, counts in ((self.outs, _KEYS, 8, self.means, self.counts),
+                                                      (self.brows, _capi.BEYOND_KEYS, 3, self.bmeans, self.bcounts)):
+            if means is not None:
+                means, counts = to_numpy(means), to_numpy(counts)
+            for i, (name, key) in enumerate(keys):
+                if name not in rows:
+                    continue
+                wide = self.cumulative and i < wide_slots
+                if not means_only:
+                    metrics[key] = rows[name].reshape(self.m, self.K) if wide else rows[name]
+                if means is not None:
+                    mean_d[key] = means[i * W:(i + 1) * W].copy() if wide else float(means[i * W])
+                    count_d[key] = counts[i * W:(i + 1) * W].copy() if wide else int(counts[i * W])
+        metrics["K"] = self.K
+        return metrics, mean_d, count_d
+
+
 def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ties_with_noise,
                           min_pos_test, min_items_pool, consider_cold_start, cumulative, nthreads, seed):
     if (A is None) != (B is None):
@@ -255,14 +294,9 @@ def calc_reco_metrics_ex(
     prep = _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ties_with_noise,
                                  min_pos_test, min_items_pool, consider_cold_start, cumulative, nthreads, seed)
     dtype, m, K = prep["dtype"], prep["m"], prep["k"]
-
-    outs = {}
-    for q in _capi.METRIC_ORDER:
-        if flags[q]:
-            size = m * K if (cumulative and q in _capi.TOPK_METRICS) else m
-            outs[q] = np.empty(size, dtype=dtype)
-            if user_range is not None:
-                outs[q].fill(np.nan)
+    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
+    res = _ResultRows(lambda size, dt, fill: np.empty(size, dt) if fill is None else np.full(size, fill, dt),
+                      dtype, m, K, cumulative, flags, bflags, user_range, bool(return_means) or bool(means_only))
     timing = _capi.Timing()
     status = np.zeros(m, dtype=np.int32) if return_status else None
     topk_items = np.full(m * K, -1, dtype=np.int32) if return_topk else None
@@ -271,19 +305,14 @@ def calc_reco_metrics_ex(
     ub, ue = (0, 0) if user_range is None else (int(user_range[0]), int(user_range[1]))
     if user_range is not None and ub == ue:
         ub, ue = 0, -1          # an EMPTY block (a rank with no users); 0,0 would mean "all users" in the C-ABI
-    return_means = bool(return_means) or bool(means_only)
-    W = K if cumulative else 1
-    means = np.full(10 * W, np.nan, dtype=np.float64) if return_means else None
-    counts = np.zeros(10 * W, dtype=np.int64) if return_means else None
     extra = _capi.make_extra(device=device, user_begin=ub, user_end=ue, strict_min_pos_test=strict_min_pos_test,
                              topk_items=topk_items, topk_scores=topk_scores, pos_rank=pos_rank, status=status,
-                             timing=timing, scoring_path=scoring_path, metric_means=means, metric_counts=counts,
+                             timing=timing, scoring_path=scoring_path, metric_means=res.means, metric_counts=res.counts,
                              skip_row_copy=bool(means_only), filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
     item_counts = np.zeros(prep["n"], dtype=np.int64) if return_exposure else None
     expo = _capi.make_exposure(item_counts) if return_exposure else None
-    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
-    brows, bmeans, bcounts, bey = {}, None, None, None
-    if any(bflags.values()):
+    bey = None
+    if res.brows:
         pop = None
         if bflags["novelty"] or bflags["avg_popularity"]:
             if item_popularity is not None:
@@ -292,44 +321,15 @@ def calc_reco_metrics_ex(
                 pop = np.zeros(prep["n"], dtype=np.int64)
                 _capi.item_popularity(prep["trp"], prep["tri"], 0, m, prep["n"], pop,
                                       device=device if device >= 0 else (devices[0] if devices else -1))
-        for name, on in bflags.items():
-            if on:
-                brows[name] = np.empty(m * W, dtype=dtype)
-                if user_range is not None:
-                    brows[name].fill(np.nan)
-        bmeans = np.full(3 * W, np.nan, dtype=np.float64) if return_means else None
-        bcounts = np.zeros(3 * W, dtype=np.int64) if return_means else None
-        bey = _capi.make_beyond(brows, pop, m, bmeans, bcounts)
+        bey = _capi.make_beyond(res.brows, pop, m, res.bmeans, res.bcounts)
     rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, prep["n"], prep["p"],
                             prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
-                            bool(break_ties_with_noise), outs, prep["consider_cold_start"], prep["min_items_pool"],
+                            bool(break_ties_with_noise), res.outs, prep["consider_cold_start"], prep["min_items_pool"],
                             prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"], extra, exposure=expo,
                             beyond=bey)
     _capi.raise_for_status(rc)
 
-    metrics, mean_d, count_d = {}, None, None
-    for q, key in _KEYS:
-        if q in outs and not means_only:
-            metrics[key] = outs[q].reshape(m, K) if (cumulative and q in _capi.TOPK_METRICS) else outs[q]
-    metrics["K"] = K
-    if return_means:
-        mean_d, count_d = {}, {}
-        for i, q in enumerate(_capi.METRIC_ORDER):
-            if q not in outs:
-                continue
-            key = dict(_KEYS)[q]
-            wide = cumulative and q in _capi.TOPK_METRICS
-            mean_d[key] = means[i * W:(i + 1) * W].copy() if wide else float(means[i * W])
-            count_d[key] = counts[i * W:(i + 1) * W].copy() if wide else int(counts[i * W])
-    for i, (name, key) in enumerate(_capi.BEYOND_KEYS):
-        if name not in brows:
-            continue
-        if not means_only:
-            metrics[key] = brows[name].reshape(m, K) if cumulative else brows[name]
-        if return_means:
-            mean_d[key] = bmeans[i * W:(i + 1) * W].copy() if cumulative else float(bmeans[i * W])
-            count_d[key] = bcounts[i * W:(i + 1) * W].copy() if cumulative else int(bcounts[i * W])
-    metrics["K"] = metrics.pop("K")
+    metrics, mean_d, count_d = res.unpack(means_only)
     return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
                       topk_items=None if topk_items is None else topk_items.reshape(m, K),
                       topk_scores=None if topk_scores is None else topk_scores.reshape(m, K),
