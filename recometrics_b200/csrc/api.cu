@@ -17,7 +17,6 @@
 #include <cstring>
 #include <limits>
 #include <mutex>
-#include <new>
 #include <string>
 #include <thread>
 #include <vector>
@@ -29,25 +28,15 @@
 #include "exposure.cuh"
 #include "beyond.cuh"
 #include "full_order.h"
+#include "runtime.h"
 
 namespace {
 
-thread_local std::string g_err;
+using rmb::DevBuf;
+using rmb::set_err;
+using rmb::upload_rows;
+
 std::atomic<int> g_interrupt{0};
-std::mutex g_call_mutex;   // one call at a time per process (the SIGINT latch is process-wide)
-constexpr int MAX_DEVICES = 16;   // GPUs one call can be spread over
-
-void set_err(const char* what, const char* detail = nullptr)
-{
-    g_err = what;
-    if (detail) { g_err += ": "; g_err += detail; }
-}
-
-}  // namespace
-namespace rmb {
-void set_last_error(const char* what, const char* detail) { set_err(what, detail); }   // for the library's other translation units (split.cu)
-}
-namespace {
 
 extern "C" void rmb200_sigint_handler(int) { g_interrupt.store(1); }
 
@@ -69,97 +58,6 @@ struct SignalLatch {
     }
     ~SignalLatch() { restore(); }
 };
-
-// Device workspace cache: a call needs a few GB of scratch (operand images, candidate buffers); cudaMalloc / cudaFree
-// of those cost tens of milliseconds per call and synchronise the device, so released blocks are kept for the next
-// call (rmb200_release_workspace() or RMB200_NO_POOL=1 gives them back).
-struct PoolEntry { void* p; size_t bytes; int dev; bool in_use; };
-std::vector<PoolEntry> g_pool;
-std::mutex g_pool_mutex;
-
-bool pool_enabled()
-{
-    static const bool on = []() { const char* e = std::getenv("RMB200_NO_POOL"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
-void pool_trim_locked(int dev_only)
-{
-    for (size_t i = 0; i < g_pool.size();) {
-        if (!g_pool[i].in_use && (dev_only < 0 || g_pool[i].dev == dev_only)) {
-            cudaFree(g_pool[i].p);
-            g_pool[i] = g_pool.back();
-            g_pool.pop_back();
-        } else i++;
-    }
-}
-
-cudaError_t pool_alloc(void** out, size_t bytes)
-{
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::lock_guard<std::mutex> lk(g_pool_mutex);
-    if (pool_enabled()) {
-        int best = -1;
-        for (size_t i = 0; i < g_pool.size(); i++) {
-            const PoolEntry& e = g_pool[i];
-            if (e.in_use || e.dev != dev || e.bytes < bytes || e.bytes > bytes + bytes / 4 + (1u << 20)) continue;
-            if (best < 0 || e.bytes < g_pool[best].bytes) best = (int)i;
-        }
-        if (best >= 0) { g_pool[best].in_use = true; *out = g_pool[best].p; return cudaSuccess; }
-    }
-    cudaError_t e = cudaMalloc(out, bytes);
-    if (e == cudaErrorMemoryAllocation) {           // give cached blocks back and try once more
-        cudaGetLastError();
-        pool_trim_locked(dev);
-        e = cudaMalloc(out, bytes);
-    }
-    if (e == cudaSuccess && pool_enabled()) g_pool.push_back(PoolEntry{*out, bytes, dev, true});
-    return e;
-}
-
-void pool_free(void* p)
-{
-    std::lock_guard<std::mutex> lk(g_pool_mutex);
-    for (auto& e : g_pool)
-        if (e.p == p) { e.in_use = false; return; }
-    cudaFree(p);
-}
-
-}  // namespace
-namespace rmb {   // the same cache for the library's other translation units (split.cu)
-cudaError_t workspace_alloc(void** out, size_t bytes) { return pool_alloc(out, bytes); }
-void workspace_free(void* p) { pool_free(p); }
-}
-namespace {
-
-struct DevBuf {
-    void* p = nullptr;
-    DevBuf() = default;
-    DevBuf(const DevBuf&) = delete;
-    DevBuf& operator=(const DevBuf&) = delete;
-    ~DevBuf() { release(); }
-    void release() { if (p) { pool_free(p); p = nullptr; } }
-    cudaError_t alloc(size_t bytes)
-    {
-        release();
-        if (bytes == 0) bytes = 16;
-        return pool_alloc(&p, bytes);
-    }
-    template <typename U> U* as() const { return reinterpret_cast<U*>(p); }
-};
-
-#define CK(call)                                                                         \
-    do {                                                                                 \
-        cudaError_t e_ = (call);                                                         \
-        if (e_ != cudaSuccess) {                                                         \
-            set_err(#call, cudaGetErrorString(e_));                                      \
-            cudaGetLastError();                                                          \
-            return (e_ == cudaErrorMemoryAllocation) ? RMB200_ERR_OOM : RMB200_ERR_CUDA; \
-        }                                                                                \
-    } while (0)
-
-#define TRY(expr) do { const int rc_ = (expr); if (rc_ != RMB200_OK) return rc_; } while (0)   // int return codes
 
 inline int round_up(int x, int q) { return (x + q - 1) / q * q; }
 
@@ -196,8 +94,8 @@ struct MultiCtx {
     int arrived[2] = {0, 0};
     int departed = 0;
     bool failed = false;
-    void* Bptr[MAX_DEVICES] = {};
-    int Bdev[MAX_DEVICES] = {};
+    void* Bptr[rmb::MAX_DEVICES] = {};
+    int Bdev[rmb::MAX_DEVICES] = {};
     // false: a peer failed (the caller gives up as well)
     bool meet(int phase)
     {
@@ -321,239 +219,6 @@ cudaError_t launch_rank_topk(T* cs, int* ci, const int* cc, int C, int nb, int K
     return cudaGetLastError();
 }
 
-// Copy a row-major host/device matrix slab [rows][cols] (leading dimension ld) into a compact
-// device buffer when it lives on the host; on-device inputs are used in place.
-
-// ---------------------------------------------------------------- host -> device uploads
-// The reference's callers hand over ordinary (pageable) numpy / R memory (wrapper.pyx:208-224).  cudaMemcpy from
-// pageable memory goes through the driver's single staging buffer at ~11 GB/s (measured: 62 ms for the 0.67 GB of a
-// 151K-user cfg4 call); a PCIe 5 x16 link takes 55 GB/s from pinned memory.  Large pageable sources therefore go through
-// our own pipeline: UP_THREADS host threads each copy their share of the rows into pinned bounce buffers (two per
-// thread, UP_CHUNK bytes) and queue the DMA from there on their own stream -- the memcpy of one chunk overlaps the DMA
-// of the previous one and the threads overlap each other.  Pinned (or registered) sources and small copies take the
-// plain cudaMemcpyAsync path.  RMB200_UPLOAD_THREADS=0 switches the pipeline off.
-constexpr size_t UP_CHUNK = 8u << 20;
-constexpr int UP_MAX_THREADS = 16;
-struct UploadLane {
-    cudaStream_t st = nullptr;
-    void* buf[2] = {nullptr, nullptr};
-    cudaEvent_t ev[2] = {nullptr, nullptr};      // recorded behind the DMA that reads buf[i]
-    bool recorded[2] = {false, false};           // ... at least once: the buffer may still be in flight from an earlier upload
-};
-struct UploadPool {
-    int dev = -1;
-    UploadLane lane[UP_MAX_THREADS];
-    cudaEvent_t done[UP_MAX_THREADS] = {};
-    cudaEvent_t start = nullptr;
-    int lanes = 0;
-    bool ok = false;
-};
-UploadPool g_ups[MAX_DEVICES];   // one per device: calls are serialised by the library's mutex, and inside a multi-GPU call
-                                 // every device has its own host thread
-thread_local int g_upload_share = 1;   // a multi-GPU call divides the host's copy threads among its devices
-
-int upload_threads()
-{
-    int v = (int)std::thread::hardware_concurrency() / 2;      // measured on a 16-core box: 60 ms plain, 32 ms with 4 threads, 25 ms with 8
-    if (v < 1) v = 1;
-    if (const char* e = std::getenv("RMB200_UPLOAD_THREADS")) v = std::atoi(e);
-    if (v > 1 && g_upload_share > 1) { v /= g_upload_share; if (v < 1) v = 1; }
-    return v < 0 ? 0 : (v > UP_MAX_THREADS ? UP_MAX_THREADS : v);
-}
-
-void upload_pool_release(UploadPool& g_up)
-{
-    if (g_up.dev < 0) return;
-    int cur = 0;
-    cudaGetDevice(&cur);
-    cudaSetDevice(g_up.dev);
-    for (int t = 0; t < UP_MAX_THREADS; t++) {
-        UploadLane& L = g_up.lane[t];
-        for (int b = 0; b < 2; b++) { if (L.buf[b]) cudaFreeHost(L.buf[b]); if (L.ev[b]) cudaEventDestroy(L.ev[b]); L.buf[b] = nullptr; L.ev[b] = nullptr; L.recorded[b] = false; }
-        if (L.st) cudaStreamDestroy(L.st);
-        L.st = nullptr;
-        if (g_up.done[t]) cudaEventDestroy(g_up.done[t]);
-        g_up.done[t] = nullptr;
-    }
-    if (g_up.start) cudaEventDestroy(g_up.start);
-    g_up.start = nullptr;
-    g_up.dev = -1; g_up.ok = false; g_up.lanes = 0;
-    cudaSetDevice(cur);
-}
-
-void upload_pool_release_all()
-{
-    for (int d = 0; d < MAX_DEVICES; d++) upload_pool_release(g_ups[d]);
-}
-
-bool upload_pool_ready(int dev, int nthreads)
-{
-    if (dev < 0 || dev >= MAX_DEVICES) return false;
-    UploadPool& g_up = g_ups[dev];
-    if (g_up.ok && g_up.dev == dev && g_up.lanes >= nthreads) return true;
-    upload_pool_release(g_up);
-    g_up.dev = dev;
-    g_up.lanes = nthreads;
-    for (int t = 0; t < nthreads; t++) {
-        UploadLane& L = g_up.lane[t];
-        if (cudaStreamCreateWithFlags(&L.st, cudaStreamNonBlocking) != cudaSuccess) { cudaGetLastError(); upload_pool_release(g_up); return false; }
-        for (int b = 0; b < 2; b++) {
-            if (cudaHostAlloc(&L.buf[b], UP_CHUNK, cudaHostAllocDefault) != cudaSuccess ||
-                cudaEventCreateWithFlags(&L.ev[b], cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); upload_pool_release(g_up); return false; }
-        }
-        if (cudaEventCreateWithFlags(&g_up.done[t], cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); upload_pool_release(g_up); return false; }
-    }
-    if (cudaEventCreateWithFlags(&g_up.start, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); upload_pool_release(g_up); return false; }
-    g_up.ok = true;
-    return true;
-}
-
-bool host_pointer_is_pageable(const void* p)
-{
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return true; }
-    return at.type == cudaMemoryTypeUnregistered;
-}
-
-// rows x row_bytes from host memory (row pitch src_pitch) to a packed device buffer, ordered on stream `st`
-cudaError_t upload_rows(void* dst, const void* src, size_t src_pitch, size_t row_bytes, size_t rows, cudaStream_t st)
-{
-    const size_t total = row_bytes * rows;
-    const int nt = upload_threads();
-    int dev = 0;
-    cudaGetDevice(&dev);
-    // a contiguous source is a byte stream (chunks of UP_CHUNK bytes); a pitched one is cut at row boundaries
-    const bool contiguous = (src_pitch == row_bytes) || rows == 1;
-    size_t min_bytes = 32u << 20;
-    if (const char* env = std::getenv("RMB200_UPLOAD_MIN_BYTES")) min_bytes = (size_t)std::atoll(env);      // developer / tests
-    if (total < min_bytes || total == 0 || nt == 0 || (!contiguous && row_bytes > UP_CHUNK) || !host_pointer_is_pageable(src) ||
-        !upload_pool_ready(dev, nt)) {
-        if (src_pitch == row_bytes) return cudaMemcpyAsync(dst, src, total, cudaMemcpyHostToDevice, st);
-        return cudaMemcpy2DAsync(dst, row_bytes, src, src_pitch, row_bytes, rows, cudaMemcpyHostToDevice, st);
-    }
-    UploadPool& g_up = g_ups[dev];
-    // what is already queued on `st` (e.g. kernels still reading dst's previous contents) comes first
-    cudaEvent_t start = g_up.start;
-    cudaError_t e = cudaEventRecord(start, st);
-    if (e != cudaSuccess) return e;
-    const size_t unit = contiguous ? 1 : row_bytes;                              // bytes per indivisible piece
-    const size_t units = contiguous ? total : rows;
-    const size_t rows_per_chunk = contiguous ? UP_CHUNK : UP_CHUNK / row_bytes;   // pieces per chunk
-    const size_t nchunks = (units + rows_per_chunk - 1) / rows_per_chunk;
-    cudaError_t errs[UP_MAX_THREADS];
-    std::vector<std::thread> workers;
-    for (int t = 0; t < nt; t++) {
-        errs[t] = cudaSuccess;
-        workers.emplace_back([&, t]() {
-            cudaError_t er = cudaSetDevice(dev);
-            UploadLane& L = g_up.lane[t];
-            if (er == cudaSuccess) er = cudaStreamWaitEvent(L.st, start, 0);
-            int b = 0;
-            for (size_t c = (size_t)t; c < nchunks && er == cudaSuccess; c += (size_t)nt, b ^= 1) {
-                const size_t r0 = c * rows_per_chunk, nr = (units - r0) < rows_per_chunk ? (units - r0) : rows_per_chunk;
-                if (L.recorded[b]) er = cudaEventSynchronize(L.ev[b]);     // the DMA that last read this bounce buffer (this upload's or an earlier one's)
-                if (er != cudaSuccess) break;
-                const unsigned char* sp = static_cast<const unsigned char*>(src) + r0 * (contiguous ? 1 : src_pitch);
-                if (contiguous) std::memcpy(L.buf[b], sp, nr);
-                else for (size_t r = 0; r < nr; r++) std::memcpy(static_cast<unsigned char*>(L.buf[b]) + r * row_bytes, sp + r * src_pitch, row_bytes);
-                er = cudaMemcpyAsync(static_cast<unsigned char*>(dst) + r0 * unit, L.buf[b], nr * unit, cudaMemcpyHostToDevice, L.st);
-                if (er == cudaSuccess) { er = cudaEventRecord(L.ev[b], L.st); L.recorded[b] = true; }
-            }
-            errs[t] = er;
-        });
-    }
-    for (auto& w : workers) w.join();
-    for (int t = 0; t < nt; t++) if (errs[t] != cudaSuccess) return errs[t];
-    // `st` continues once every lane's copies have landed (the bounce buffers are reused only after their own events)
-    for (int t = 0; t < nt; t++) {
-        e = cudaEventRecord(g_up.done[t], g_up.lane[t].st);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(st, g_up.done[t], 0);
-        if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
-}
-
-// The mirror image of upload_rows for one contiguous block: device memory to ordinary (pageable) host memory through the
-// lanes' pinned bounce buffers, every lane alternating between the DMA into one buffer and the memcpy out of the other.  The
-// driver's own path stages through one buffer and copies out on one thread (12 GB/s measured); this reaches what the host's
-// memory system gives several threads.  Work queued on `st` before the call is waited for; returns when the bytes are in dst.
-cudaError_t download_bytes(void* dst, const void* src, size_t total, cudaStream_t st)
-{
-    const int nt = upload_threads();
-    int dev = 0;
-    cudaGetDevice(&dev);
-    size_t min_bytes = 32u << 20;
-    if (const char* env = std::getenv("RMB200_UPLOAD_MIN_BYTES")) min_bytes = (size_t)std::atoll(env);      // developer / tests
-    if (total < min_bytes || nt == 0 || !host_pointer_is_pageable(dst) || !upload_pool_ready(dev, nt)) {
-        const cudaError_t e = cudaMemcpyAsync(dst, src, total, cudaMemcpyDeviceToHost, st);
-        return e != cudaSuccess ? e : cudaStreamSynchronize(st);
-    }
-    UploadPool& g_up = g_ups[dev];
-    cudaEvent_t start = g_up.start;
-    cudaError_t e = cudaEventRecord(start, st);
-    if (e != cudaSuccess) return e;
-    const size_t nchunks = (total + UP_CHUNK - 1) / UP_CHUNK;
-    cudaError_t errs[UP_MAX_THREADS];
-    std::vector<std::thread> workers;
-    for (int t = 0; t < nt; t++) {
-        errs[t] = cudaSuccess;
-        workers.emplace_back([&, t]() {
-            cudaError_t er = cudaSetDevice(dev);
-            UploadLane& L = g_up.lane[t];
-            if (er == cudaSuccess) er = cudaStreamWaitEvent(L.st, start, 0);
-            // (an earlier UPLOAD may still be reading the bounce buffers: its events come first)
-            for (int b = 0; b < 2 && er == cudaSuccess; b++) if (L.recorded[b]) er = cudaEventSynchronize(L.ev[b]);
-            auto span = [&](size_t c, size_t* off) { *off = c * UP_CHUNK; return (total - *off) < UP_CHUNK ? (total - *off) : UP_CHUNK; };
-            auto fetch = [&](size_t c, int b) {
-                size_t off; const size_t nb = span(c, &off);
-                cudaError_t x = cudaMemcpyAsync(L.buf[b], static_cast<const unsigned char*>(src) + off, nb, cudaMemcpyDeviceToHost, L.st);
-                if (x == cudaSuccess) { x = cudaEventRecord(L.ev[b], L.st); L.recorded[b] = true; }
-                return x;
-            };
-            int b = 0;
-            if (er == cudaSuccess && (size_t)t < nchunks) er = fetch((size_t)t, 0);
-            for (size_t c = (size_t)t; c < nchunks && er == cudaSuccess; c += (size_t)nt, b ^= 1) {
-                if (c + (size_t)nt < nchunks) er = fetch(c + (size_t)nt, b ^ 1);       // the next chunk's DMA runs under this chunk's memcpy
-                if (er == cudaSuccess) er = cudaEventSynchronize(L.ev[b]);
-                if (er != cudaSuccess) break;
-                size_t off; const size_t nb = span(c, &off);
-                std::memcpy(static_cast<unsigned char*>(dst) + off, L.buf[b], nb);
-            }
-            errs[t] = er;
-        });
-    }
-    for (auto& w : workers) w.join();
-    for (int t = 0; t < nt; t++) if (errs[t] != cudaSuccess) return errs[t];
-    return cudaSuccess;
-}
-
-}  // namespace
-namespace rmb {   // the pageable-memory copy pipelines for the library's other translation units (split.cu).  The lanes belong
-                  // to whoever holds the call mutex: a split that runs beside an evaluation call takes the driver's plain path.
-cudaError_t upload_bytes_pageable(void* dst, const void* src, size_t bytes, cudaStream_t st, int share)
-{
-    std::unique_lock<std::mutex> lk(g_call_mutex, std::try_to_lock);
-    if (!lk.owns_lock()) return bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess;
-    g_upload_share = share > 1 ? share : 1;
-    const cudaError_t e = bytes ? upload_rows(dst, src, bytes, bytes, 1, st) : cudaSuccess;
-    g_upload_share = 1;
-    return e;
-}
-cudaError_t download_bytes_pageable(void* dst, const void* src, size_t bytes, cudaStream_t st, int share)
-{
-    if (!bytes) return cudaSuccess;
-    std::unique_lock<std::mutex> lk(g_call_mutex, std::try_to_lock);
-    if (!lk.owns_lock()) {
-        const cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
-        return e != cudaSuccess ? e : cudaStreamSynchronize(st);
-    }
-    g_upload_share = share > 1 ? share : 1;
-    const cudaError_t e = download_bytes(dst, src, bytes, st);
-    g_upload_share = 1;
-    return e;
-}
-}
-namespace {
 
 // The user factors are uploaded one user batch ahead, on a stream of their own, into two alternating staging buffers:
 // the upload of batch b+1 runs while the scoring kernel of batch b does.  ready[s]: the upload into buffer s has landed;
@@ -1513,6 +1178,13 @@ struct Call {
     }
 };
 
+// The device a call asks for: `device`, else env RMB200_DEVICE, else (-1) the calling thread's current device
+int requested_device(int device)
+{
+    const char* env = std::getenv("RMB200_DEVICE");
+    return device >= 0 ? device : (env ? std::atoi(env) : -1);
+}
+
 template <typename T>
 int run_call(const CallArgs<T>& a)
 {
@@ -1541,23 +1213,12 @@ int run_call(const CallArgs<T>& a)
     TRY(user_range(ex, a.m, &ub, &ue));
     if (ue == ub && !a.expo) return RMB200_OK;
 
-    // ---- device ----
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        set_err("no CUDA device", "librecometrics_b200 has no CPU fallback");
-        return RMB200_ERR_NO_DEVICE;
-    }
-    int dev = -1;
-    if (ex->device >= 0) dev = ex->device;
-    else if (const char* env = std::getenv("RMB200_DEVICE")) dev = std::atoi(env);
-    if (dev < 0) CK(cudaGetDevice(&dev));
-    if (dev >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
-    CK(cudaSetDevice(dev));
+    int dev = 0;
+    TRY(rmb::use_device(requested_device(ex->device), &dev));
     if (ue == ub) return exposure_of_nobody(a.expo, a.n, ex->inputs_on_device != 0);
 
     const bool nested = a.mc != nullptr;                   // run_multi() holds the mutex and the latch
-    std::unique_lock<std::mutex> lock(g_call_mutex, std::defer_lock);
+    std::unique_lock<std::mutex> lock(rmb::g_call_mutex, std::defer_lock);
     if (!nested) lock.lock();
     SignalLatch latch(!nested);
     Call<T> c(a, dev, ub, ue - ub);
@@ -1600,9 +1261,8 @@ int resolve_devices(const rmb200_extra_t* ex, std::vector<int>& devs)
         const char* env = std::getenv("RMB200_DEVICES");
         if (!env || !env[0]) return RMB200_OK;
         if (!std::strcmp(env, "all")) {
-            int ndev = 0;
-            if (cudaGetDeviceCount(&ndev) != cudaSuccess) { cudaGetLastError(); ndev = 0; }
-            for (int d = 0; d < ndev && d < MAX_DEVICES; d++) devs.push_back(d);
+            const int ndev = rmb200_device_count();
+            for (int d = 0; d < ndev && d < rmb::MAX_DEVICES; d++) devs.push_back(d);
         } else {
             for (const char* c = env; *c;) {
                 char* end = nullptr;
@@ -1615,13 +1275,9 @@ int resolve_devices(const rmb200_extra_t* ex, std::vector<int>& devs)
         }
     }
     if (devs.empty()) return RMB200_OK;
-    if ((int)devs.size() > MAX_DEVICES) { set_err("bad argument", "more than 16 devices"); return RMB200_ERR_BAD_ARG; }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        set_err("no CUDA device", "librecometrics_b200 has no CPU fallback");
-        return RMB200_ERR_NO_DEVICE;
-    }
+    if ((int)devs.size() > rmb::MAX_DEVICES) { set_err("bad argument", "more than 16 devices"); return RMB200_ERR_BAD_ARG; }
+    int ndev = rmb200_device_count();
+    if (ndev == 0) return rmb::use_device(-1, &ndev);      // (RMB200_ERR_NO_DEVICE, as for every call without a device)
     for (size_t i = 0; i < devs.size(); i++) {
         if (devs[i] < 0 || devs[i] >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
         for (size_t j = 0; j < i; j++)
@@ -1682,7 +1338,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     const int G = (int)devs.size();
     if (G == 0) return a0.expo ? exposure_of_nobody(a0.expo, a0.n, false) : RMB200_OK;
 
-    std::unique_lock<std::mutex> lock(g_call_mutex);
+    std::unique_lock<std::mutex> lock(rmb::g_call_mutex);
     SignalLatch latch;
     MultiCtx mc;
     mc.G = G;
@@ -1715,10 +1371,9 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
             beyond_means.attach(g, beys[g].means, beys[g].counts);
         }
         workers.emplace_back([&, g]() {
-            g_err.clear();
-            g_upload_share = G;
-            int rc;
-            try {
+            rmb::g_err.clear();
+            rmb::g_upload_share = G;
+            const int rc = rmb::guard([&] {
                 // peers' memory directly over NVLink where the hardware allows it (else the copies are staged by the driver)
                 if (cudaSetDevice(devs[g]) == cudaSuccess)
                     for (int h = 0; h < G; h++) {
@@ -1730,13 +1385,9 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
                 a.ex = &exs[g]; a.mc = &mc; a.mc_rank = g;
                 if (a0.expo) a.expo = &expos[g];
                 if (a0.bey) a.bey = &beys[g];
-                rc = run_call<T>(a);
-            } catch (const std::bad_alloc&) {
-                set_err("host allocation failed"); rc = RMB200_ERR_OOM;
-            } catch (...) {
-                set_err("unexpected C++ exception"); rc = RMB200_ERR_CUDA;
-            }
-            rcs[g] = rc; errs[g] = g_err;
+                return run_call<T>(a);
+            });
+            rcs[g] = rc; errs[g] = rmb::g_err;
             mc.depart(rc != RMB200_OK);
         });
     }
@@ -1744,7 +1395,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
 
     int rc = RMB200_OK;
     for (int g = 0; g < G && rc == RMB200_OK; g++)
-        if (rcs[g] != RMB200_OK && rcs[g] != RMB200_ERR_INTERRUPTED) { rc = rcs[g]; g_err = errs[g]; }
+        if (rcs[g] != RMB200_OK && rcs[g] != RMB200_ERR_INTERRUPTED) { rc = rcs[g]; rmb::g_err = errs[g]; }
     if (rc == RMB200_OK && g_interrupt.load()) {
         latch.restore();
         std::raise(SIGINT);
@@ -1796,7 +1447,7 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
           int ccs, int32_t mip, int32_t mpt, uint64_t seed, const T* bias, const rmb200_extra_t* ex, rmb200_exposure_t* expo = nullptr,
           rmb200_beyond_t* bey = nullptr)
 {
-    g_err.clear();
+    rmb::g_err.clear();
     if (expo && expo->struct_size != (int32_t)sizeof(rmb200_exposure_t)) { set_err("bad argument", "rmb200_exposure_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     if (bey && bey->struct_size != (int32_t)sizeof(rmb200_beyond_t)) { set_err("bad argument", "rmb200_beyond_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     CallArgs<T> a;
@@ -1807,7 +1458,7 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
     for (int q = 0; q < 10; q++) a.out[q] = outs[q];
     a.consider_cold_start = ccs ? 1 : 0; a.min_items_pool = mip; a.min_pos_test = mpt; a.seed = seed;
     a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo; a.bey = bey;
-    try {
+    return rmb::guard([&] {
         std::vector<int> devs;
         TRY(resolve_devices(a.ex, devs));
         if (devs.size() > 1) return run_multi<T>(a, devs);
@@ -1818,31 +1469,16 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
             return run_call<T>(a);
         }
         return run_call<T>(a);
-    } catch (const std::bad_alloc&) {
-        set_err("host allocation failed");
-        return RMB200_ERR_OOM;
-    } catch (...) {
-        set_err("unexpected C++ exception");
-        return RMB200_ERR_CUDA;
-    }
+    });
 }
 
 // rmb200_item_popularity: the column count of CSR rows [rb, re) on the device, widened to int64 into `counts`
 int item_popularity(const int32_t* indptr, const int32_t* indices, int rb, int re, int n, int device, bool on_dev, int64_t* counts)
 {
     if (n <= 0 || !indptr || !counts || rb < 0 || re < rb) { set_err("bad argument", "item_popularity: n <= 0, a NULL array or a bad row range"); return RMB200_ERR_BAD_ARG; }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        set_err("no CUDA device", "librecometrics_b200 has no CPU fallback");
-        return RMB200_ERR_NO_DEVICE;
-    }
-    int dev = device;
-    if (dev < 0) if (const char* env = std::getenv("RMB200_DEVICE")) dev = std::atoi(env);
-    if (dev < 0) CK(cudaGetDevice(&dev));
-    if (dev >= ndev) { set_err("bad argument", "device ordinal out of range"); return RMB200_ERR_BAD_ARG; }
-    CK(cudaSetDevice(dev));
-    std::lock_guard<std::mutex> lock(g_call_mutex);       // (the upload lanes belong to the holder)
+    int dev = 0;
+    TRY(rmb::use_device(requested_device(device), &dev));
+    std::lock_guard<std::mutex> lock(rmb::g_call_mutex);       // (the upload lanes belong to the holder)
     cudaStream_t st = nullptr;                             // legacy default stream, as the evaluation call
     int lo = 0, hi = 0;
     if (on_dev) {
@@ -1983,7 +1619,7 @@ int rmb200_calc_metrics_exposure_f64(
 
 int rmb200_exposure_stats(const int64_t* counts, int32_t n, rmb200_exposure_t* out)
 {
-    g_err.clear();
+    rmb::g_err.clear();
     if (!out || out->struct_size != (int32_t)sizeof(rmb200_exposure_t)) { set_err("bad argument", "rmb200_exposure_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     return exposure_stats(counts, n, out);
 }
@@ -2029,16 +1665,8 @@ int rmb200_sizeof_beyond(void) { return (int)sizeof(rmb200_beyond_t); }
 int rmb200_item_popularity(const int32_t* indptr, const int32_t* indices, int32_t row_begin, int32_t row_end, int32_t n,
                            int32_t device, int32_t inputs_on_device, int64_t* counts)
 {
-    g_err.clear();
-    try {
-        return item_popularity(indptr, indices, row_begin, row_end, n, device, inputs_on_device != 0, counts);
-    } catch (const std::bad_alloc&) {
-        set_err("host allocation failed");
-        return RMB200_ERR_OOM;
-    } catch (...) {
-        set_err("unexpected C++ exception");
-        return RMB200_ERR_CUDA;
-    }
+    rmb::g_err.clear();
+    return rmb::guard([&] { return item_popularity(indptr, indices, row_begin, row_end, n, device, inputs_on_device != 0, counts); });
 }
 
 int rmb200_device_count(void)
@@ -2054,25 +1682,12 @@ int rmb200_sizeof_extra(void) { return (int)sizeof(rmb200_extra_t); }
 
 int rmb200_sizeof_timing(void) { return (int)sizeof(rmb200_timing_t); }
 
-const char* rmb200_last_error(void) { return g_err.c_str(); }
-
 void rmb200_request_interrupt(void) { g_interrupt.store(1); }
-
-void rmb200_release_workspace(void)
-{
-    std::lock_guard<std::mutex> call(g_call_mutex);      // not while a call is using them
-    upload_pool_release_all();
-    std::lock_guard<std::mutex> lk(g_pool_mutex);
-    pool_trim_locked(-1);
-}
 
 double rmb200_measure_fma_peak(int device, int dtype_bytes, double* elapsed_ms)
 {
-    g_err.clear();
-    int ndev = rmb200_device_count();
-    if (ndev <= 0) { set_err("no CUDA device"); return -1.0; }
-    if (device < 0) cudaGetDevice(&device);
-    if (device >= ndev || cudaSetDevice(device) != cudaSuccess) { set_err("bad device"); return -1.0; }
+    rmb::g_err.clear();
+    if (rmb::use_device(device, &device) != RMB200_OK) return -1.0;
     int nsm = 148;
     cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
     const int threads = 256, blocks = nsm * 8;

@@ -38,7 +38,6 @@
 #include <locale>
 #include <memory>
 #include <mutex>
-#include <exception>
 #include <new>
 #include <cstdlib>
 #include <cstring>
@@ -55,15 +54,7 @@
 #include <cub/device/device_segmented_radix_sort.cuh>
 #include <thrust/iterator/transform_iterator.h>
 
-namespace rmb {   // api.cu
-void set_last_error(const char* what, const char* detail);
-cudaError_t workspace_alloc(void** out, size_t bytes);      // device blocks cached between calls (rmb200_release_workspace() frees them)
-void workspace_free(void* p);
-// pageable host memory <-> device through several copy threads and pinned bounce buffers (the evaluation path's upload pipeline
-// and its mirror image); `share`: divide the host's copy threads by this much.  The download returns when the bytes are there.
-cudaError_t upload_bytes_pageable(void* dst, const void* src, size_t bytes, cudaStream_t st, int share);
-cudaError_t download_bytes_pageable(void* dst, const void* src, size_t bytes, cudaStream_t st, int share);
-}
+#include "runtime.h"
 
 namespace {
 
@@ -562,26 +553,6 @@ struct ByteToInt {
     __host__ __device__ __forceinline__ int operator()(const uint8_t& b) const { return (int)b; }
 };
 
-thread_local double* t_alloc_ms = nullptr;     // (diagnostics) where the current thread's device allocation time is added up
-
-// a device block from the library's workspace cache: cudaMalloc / cudaFree of a call's ~600 MB cost anything between 10 and
-// 200 ms on a busy box (measured, profiles/r02_split_gpu_run.log) -- more than everything else the call does
-struct DevMem {
-    void* p = nullptr;
-    DevMem() = default;
-    DevMem(const DevMem&) = delete;
-    DevMem& operator=(const DevMem&) = delete;
-    cudaError_t alloc(size_t bytes)
-    {
-        const auto t0 = clk::now();
-        const cudaError_t e = rmb::workspace_alloc(&p, bytes ? bytes : 16);
-        if (t_alloc_ms) *t_alloc_ms += ms_since(t0);
-        return e;
-    }
-    ~DevMem() { if (p) rmb::workspace_free(p); }
-    template <typename U> U* as() const { return (U*)p; }
-};
-
 // one block per call, carved into the call's arrays (256-byte aligned)
 struct Slot { void* p = nullptr; template <typename U> U* as() const { return (U*)p; } };
 struct Carver {
@@ -626,7 +597,7 @@ void touch_pages(const SplitOwner* own)
 
 int fail(int code, const char* what, const char* detail = nullptr)
 {
-    rmb::set_last_error(what, detail);
+    rmb::set_err(what, detail);
     return code;
 }
 
@@ -723,7 +694,7 @@ struct DeviceJob {
         return true;
     }
 
-    double dbg_setup = 0, dbg_alloc = 0, dbg_wait = 0, dbg_body = 0;
+    double dbg_setup = 0, dbg_wait = 0, dbg_body = 0;
     clk::time_point dbg_end;
 
     void run()
@@ -732,8 +703,8 @@ struct DeviceJob {
         dbg_end = t0;
         body();
         if (std::getenv("RMB200_SPLIT_DBG"))
-            std::fprintf(stderr, "split device thread: %.1f ms = setup %.1f + h2d %.1f (cudaMalloc %.1f) + kernels %.2f + d2h %.1f + waiting %.1f + rest, "
-                         "teardown %.1f\n", ms_since(t0), dbg_setup, h2d_ms, dbg_alloc, kernel_ms, d2h_ms, dbg_wait,
+            std::fprintf(stderr, "split device thread: %.1f ms = setup %.1f + h2d %.1f + kernels %.2f + d2h %.1f + waiting %.1f + rest, "
+                         "teardown %.1f\n", ms_since(t0), dbg_setup, h2d_ms, kernel_ms, d2h_ms, dbg_wait,
                          std::chrono::duration<double, std::milli>(clk::now() - dbg_end).count());
     }
 
@@ -746,7 +717,6 @@ struct DeviceJob {
         const int64_t kept_nnz = sel_nnz - test_nnz;
         const int64_t train_nnz = kept_nnz + (kind == SPLIT_JOINED ? rem_nnz : 0);
         const auto t_setup = clk::now();
-        t_alloc_ms = &dbg_alloc;
         JOB_CUDA(cudaSetDevice(device));
         struct Stream { cudaStream_t s = nullptr; ~Stream() { if (s) cudaStreamDestroy(s); } } stream;
         struct Event { cudaEvent_t e = nullptr; ~Event() { if (e) cudaEventDestroy(e); } } ev0, ev1;
@@ -785,7 +755,8 @@ struct DeviceJob {
             return e;
         };
 
-        // ---- one device block for the call (from the library's workspace cache), X and the plan's index arrays up ----
+        // ---- one device block for the call, X and the plan's index arrays up.  The block comes from the library's workspace
+        //      cache: cudaMalloc / cudaFree of a call's ~600 MB cost 10-200 ms on a busy box, more than the rest of the call ----
         const auto t_up = clk::now();
         int64_t longest_chunk = 0;
         for (size_t c = 0, rb = 0; c < Q.chunk_end.size(); rb = (size_t)Q.chunk_end[c++])
@@ -809,7 +780,7 @@ struct DeviceJob {
         Carver carve;
         size_t offsets[sizeof(layout) / sizeof(layout[0])];
         for (size_t k = 0; k < sizeof(layout) / sizeof(layout[0]); k++) offsets[k] = carve.reserve(layout[k].second);
-        DevMem block;
+        rmb::DevBuf block;
         JOB_CUDA(block.alloc(carve.total));
         carve.base = block.as<char>();
         for (size_t k = 0; k < sizeof(layout) / sizeof(layout[0]); k++) layout[k].first->p = carve.at<char>(offsets[k]);
@@ -841,7 +812,7 @@ struct DeviceJob {
         V.ns = ns; V.j0 = 0; V.j1 = (int)sel_nnz;
 
         // ---- what does not wait for the replay: the order of unsorted rows, and the rows the split leaves alone ----
-        DevMem d_keys0, d_keys1, d_vals0, d_perm, d_sort_temp, d_flags;     // (the rare unsorted input: blocks of their own)
+        rmb::DevBuf d_keys0, d_keys1, d_vals0, d_perm, d_sort_temp, d_flags;     // (the rare unsorted input: blocks of their own)
         const int* perm = nullptr;
         if (sel_nnz) {
             JOB_CUDA(kernels_begin());
@@ -944,7 +915,7 @@ int run_split_impl(SplitKind kind, const int32_t* Xp, const int32_t* Xi, const T
                    int32_t n_users_test, double test_fraction, bool consider_cold_start, int32_t min_items_pool,
                    int32_t min_pos_test, uint64_t seed, int32_t device, rmb200_split_t* out)
 {
-    rmb::set_last_error("", nullptr);
+    rmb::g_err.clear();
     if (!out) return fail(RMB200_ERR_BAD_ARG, "rmb200_split: out is NULL");
     std::memset(out, 0, sizeof(*out));
     out->value_bytes = (int32_t)sizeof(T);
@@ -964,13 +935,7 @@ int run_split_impl(SplitKind kind, const int32_t* Xp, const int32_t* Xi, const T
     if (Xp[0] != 0) return fail(RMB200_ERR_BAD_ARG, "rmb200_split: X_csr_p[0] must be 0");
     if (nnz < 0 || (nnz > 0 && (!Xi || !Xv))) return fail(RMB200_ERR_BAD_ARG, "rmb200_split: X_csr_i / X_csr missing");
 
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return fail(RMB200_ERR_NO_DEVICE, "no usable CUDA device (the splitters have no CPU path)");
-    }
-    if (device < 0) { if (cudaGetDevice(&device) != cudaSuccess) device = 0; }
-    if (device >= ndev) return fail(RMB200_ERR_BAD_ARG, "rmb200_split: no such device");
+    TRY(rmb::use_device(device, &device));
     out->device = device;
 
     // ---- which rows, and how many entries of each are held out: everything the result's shape depends on ----
@@ -1050,19 +1015,13 @@ int run_split_impl(SplitKind kind, const int32_t* Xp, const int32_t* Xi, const T
     return RMB200_OK;
 }
 
-// nothing may unwind through the C boundary (std::vector / std::thread can throw)
+// a failed split hands back no matrices
 template <typename T, typename... Args>
 int run_split(rmb200_split_t* out, Args... args)
 {
-    try {
-        return run_split_impl<T>(args..., out);
-    } catch (const std::bad_alloc&) {
-        if (out) rmb200_split_free(out);
-        return fail(RMB200_ERR_OOM, "host allocation failed during the split");
-    } catch (const std::exception& e) {
-        if (out) rmb200_split_free(out);
-        return fail(RMB200_ERR_CUDA, "rmb200_split", e.what());
-    }
+    const int rc = rmb::guard([&] { return run_split_impl<T>(args..., out); });
+    if (rc != RMB200_OK && out) rmb200_split_free(out);
+    return rc;
 }
 
 }  // namespace
@@ -1117,9 +1076,9 @@ int rmb200_split_plan(const int32_t* Xp, int32_t m, int32_t n, int32_t sample_us
                       int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, uint64_t seed,
                       int32_t* users_test, int32_t* n_users_out, uint8_t* held, int64_t* n_entries_out)
 {
-    rmb::set_last_error("", nullptr);
+    rmb::g_err.clear();
     if (!Xp || m <= 0 || !held || !n_entries_out) return fail(RMB200_ERR_BAD_ARG, "rmb200_split_plan: bad arguments");
-    try {
+    return rmb::guard([&] {
         SplitPlan P;
         if (sample_users) {
             if (!users_test || !n_users_out) return fail(RMB200_ERR_BAD_ARG, "rmb200_split_plan: users_test missing");
@@ -1143,10 +1102,8 @@ int rmb200_split_plan(const int32_t* Xp, int32_t m, int32_t n, int32_t sample_us
         } else if (n_users_out) *n_users_out = m;
         std::memcpy(held, P.held.data(), P.held.size());
         *n_entries_out = (int64_t)P.held.size();
-    } catch (const std::bad_alloc&) {
-        return fail(RMB200_ERR_OOM, "host allocation failed during the split plan");
-    }
-    return RMB200_OK;
+        return (int)RMB200_OK;
+    });
 }
 
 void rmb200_split_free(rmb200_split_t* split)

@@ -441,7 +441,7 @@ def test_cpp_shim_computes_on_the_gpu(rb, tmp_path):
 
 def test_pageable_upload_pipeline_equals_plain_copies(rb, monkeypatch):
     """Host inputs in ordinary (pageable) numpy memory go up through copy threads and pinned bounce buffers once they are
-    large (api.cu upload_rows); forced on for every array here -- pitched factor matrices, the contiguous CSR arrays,
+    large (runtime.cu upload_rows); forced on for every array here -- pitched factor matrices, the contiguous CSR arrays,
     several user batches (two alternating staging buffers on the prefetch stream) -- the results must be those of the
     plain cudaMemcpy path, bit for bit."""
     d = synth.make(3, m=5000, n=6000, p=40)

@@ -51,7 +51,7 @@ def test_split_in_many_chunks_and_with_a_threaded_replay(rb, monkeypatch, knobs)
 
 def test_split_through_the_pageable_copy_pipelines(rb, oracle_mod, monkeypatch):
     """X goes up and the untouched users' rows come down through the library's copy pipelines for pageable memory (several
-    copy threads + pinned bounce buffers, recometrics_b200/csrc/api.cu upload_rows / download_bytes) once a block reaches
+    copy threads + pinned bounce buffers, recometrics_b200/csrc/runtime.cu upload_rows / download_bytes) once a block reaches
     32 MB.  Forced here on small blocks (RMB200_UPLOAD_MIN_BYTES=1), and run on blocks of several bounce buffers each
     (2 M entries: 8 MB per index array and per lane buffer), against the oracle."""
     monkeypatch.setenv("RMB200_UPLOAD_MIN_BYTES", "1")
