@@ -370,7 +370,11 @@ static int32_t FN(one_user)(
 
         const REAL vmax = user_v[ind[0]];
         const REAL vmin = user_v[ind[L-1]];
-        if (isnan(vmax) || isinf(vmax) || isnan(vmin) || isinf(vmin) || vmax <= 0) {   /* :875-887 */
+        /* A NaN gain makes NDCG NaN wherever it sits (quirk Q9): the reference checks only the two values partial_sort
+         * leaves at ranks 0 and L-1, and where a NaN lands under its '>' comparator is unspecified. */
+        int nan_gain = 0;
+        for (int32_t ix = 0; ix < (int32_t)npos; ix++) nan_gain |= isnan(user_v[ix]);
+        if (nan_gain || isnan(vmax) || isinf(vmax) || isnan(vmin) || isinf(vmin) || vmax <= 0) {   /* :875-887 */
             if (!cumulative) o->ndcg[user] = (REAL)NAN;
             else for (int32_t c = 0; c < K; c++) ndcg_u[c] = (REAL)NAN;
             return 0;

@@ -10,6 +10,7 @@
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
+#include <cfloat>
 #include <cmath>
 #include <csignal>
 #include <cstdio>
@@ -958,6 +959,7 @@ struct Call {
         fp.sample_tiles = f_sample_tiles; fp.sample_stride = f_sample_stride; fp.sample_rank = f_sample_rank;
         fp.retries = d_overflow.as<int>() + 1;
         fp.noise_band = a.noise ? 2.02e-12f : 0.f;
+        fp.score_max = sizeof(T) == 4 ? 0.5f * FLT_MAX : HUGE_VALF;
         cudaEventRecord(pk.a, st);
         CK(launch_filter_select(fp, C, b.nb_pad / BM, st));
         cudaEventRecord(pk.b, st);
@@ -989,8 +991,11 @@ struct Call {
         pt.start();
         // a few users of a large catalogue go to the full-order path (every candidate scored by item-parallel blocks, one
         // segmented sort) -- on the FMA tiles ONE CTA walked the whole catalogue for them (78 ms at 1M items for a
-        // single user, profiles/r02v: two of four ranks of a strong-scaling run ran at half speed for it)
-        return hand_back(b, d_At_fb, d_fb_list.as<int>(), n_over, d_cc.as<int>(), d_overflow.as<int>() + 6, n_over > 2048 || a.n < 32768);
+        // single user, profiles/r02v: two of four ranks of a strong-scaling run ran at half speed for it).  Under the noise
+        // every hand-back goes there: the FMA tiles neither add the noise nor check the noise branch's validity rule
+        // (any infinite candidate => NaN row), which is what a user with a -inf score below its top K needs.
+        const bool on_fma = !a.noise && (n_over > 2048 || a.n < 32768);
+        return hand_back(b, d_At_fb, d_fb_list.as<int>(), n_over, d_cc.as<int>(), d_overflow.as<int>() + 6, on_fma);
     }
     // the selected candidates ranked; the noise hand-back; the all-equal check of the FMA tiles under the noise
     int rank_fixups(Batch& b)

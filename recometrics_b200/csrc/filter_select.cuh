@@ -71,6 +71,8 @@ struct FilterParams {
     int KB;                                 // fp16 factors per row, multiple of 16
     float c_rel, c_abs, c_const;            // error bound of an approximate score (host: filter_err_coefs)
     float noise_band;                       // break_ties_with_noise: how far the noise can move two scores apart (2e-12), else 0
+    float score_max;                        // largest ||a|| * max ||b|| whose scores cannot overflow the input type (float:
+                                            // FLT_MAX / 2; double: +inf, as both norms are below 6e29 here)
     int stages;                             // depth of the B ring
     int n, mb, user0;
     const float* __restrict__ anorm;        // [mb] ||a_u|| (with the 1.0 bias component), rounded up; 0 = all-zero row
@@ -416,6 +418,10 @@ filter_select_kernel(const __grid_constant__ FilterParams P)
                         const float an = P.anorm[ul], bn = __uint_as_float(*P.maxbn);
                         if (an == 0.f) ranked = false;                           // all-zero user factors: every score equal, NaN row (hpp:541-548, :524-527)
                         else if (!(filter_scalable(an) && filter_scalable(bn))) { fl = 8; ranked = false; }
+                        // |score| <= ||a|| ||b|| (the bias is one more factor of both norms): a user whose scores can
+                        // overflow to +-inf goes back too, so that the path it lands on sees every infinite candidate
+                        // (under the noise one anywhere makes the row NaN, hpp:524-527; the exact stage sees survivors only)
+                        else if (!(an * bn <= P.score_max)) { fl = 8; ranked = false; }
                         else {
                             const float sa = pow2_scale_for(an), sb = pow2_scale_for(bn);
                             const float ap = an * sa;                                            // ||a'|| in [0.5, 1.002)

@@ -807,7 +807,10 @@ __device__ __noinline__ void auc_count_role(const ScoreSelectParams<T>& P, RowSt
                 bool on = t < run;
                 if (on && near_g != nullptr && noise_reach(thr[t]) > (T)0) { banded |= 1u << t; on = false; }
                 if (!on) col[t] = 0;
-                eff[t] = !on ? NumTraits<T>::inf() : (col[t] >= BN ? next_below<T>(thr[t]) : thr[t]);
+                // "s >= -inf" has no strict form (next_below(-inf) is a NaN): a tile before a -inf entry counts "s > -inf"
+                // and then its -inf scores one by one, like the columns before the entry in its own tile
+                const bool before_tile = col[t] >= BN && thr[t] != -NumTraits<T>::inf();
+                eff[t] = !on ? NumTraits<T>::inf() : (before_tile ? next_below<T>(thr[t]) : thr[t]);
             }
             unsigned c[UN];
             count_above<UN>(src, eff, c);
@@ -815,8 +818,8 @@ __device__ __noinline__ void auc_count_role(const ScoreSelectParams<T>& P, RowSt
             for (int t = 0; t < UN; t++) {
                 if (t < run && !((banded >> t) & 1u)) {
                     unsigned ct = c[t];
-                    if (col[t] > 0 && col[t] < BN)
-                        for (int x = 0; x < col[t]; x++) ct += (src[x] == thr[t]);
+                    const int eq = col[t] >= BN ? (thr[t] == -NumTraits<T>::inf() ? BN : 0) : col[t];
+                    for (int x = 0; x < eq; x++) ct += (src[x] == thr[t]);
                     if (!sliced) cnt_g[e0 + t] = before[t] + ct;
                     else if (ct) atomicAdd(&cnt_g[e0 + t], ct);
                 }

@@ -41,13 +41,16 @@ def ambiguity(S64, X_train, X_test, K):
         s = S64[u].copy()
         tr = X_train.indices[X_train.indptr[u]:X_train.indptr[u + 1]]
         te = X_test.indices[X_test.indptr[u]:X_test.indptr[u + 1]]
-        s[tr] = -np.inf
         cand = n - tr.shape[0]
-        if cand < 2 or not np.all(np.isfinite(np.delete(s, tr))):
-            continue
+        if cand < 2 or np.isnan(np.delete(s, tr)).any():
+            continue                                  # (a NaN candidate score: NaN row)
+        s[tr] = np.nan                                # train items sort after every candidate, -inf ones included
         order = np.argsort(-s, kind="stable")[:cand]
         so = s[order]
-        S_u = max(abs(so[0]), abs(so[-1]))            # the user's score scale
+        fin = so[np.isfinite(so)]
+        if fin.size == 0:
+            continue
+        S_u = max(abs(fin[0]), abs(fin[-1]))          # the user's score scale (over its finite scores)
         top = so[: min(K + 1, cand)]
         gaps = np.abs(np.diff(top))
         topk_amb[u] = bool(np.any(gaps <= REL_GAP * S_u))
@@ -99,13 +102,20 @@ def run_oracle(oracle, data, metrics, k, cumulative=False, dtype=None, **kw):
                               nthreads=8, fix_quirks=True, extras=True, dtype=dt, **kw)
 
 
-def compare(res, orc, data, metrics, k, cumulative=False, check_ranks=True, max_amb_frac=0.25, label=""):
-    """Assert parity between a product EvalResult and the oracle's dict.  Returns a report dict."""
+def near_ties(data, k):
+    """The float64 scores and ambiguity() of `data` at `k`: what compare() needs from the inputs alone, to be reused by
+    several compare() calls on the same inputs (pre=)."""
+    S64 = scores_f64(data["A"], data["B"], data.get("item_biases"))
+    return (S64,) + ambiguity(S64, data["X_train"], data["X_test"], k)
+
+
+def compare(res, orc, data, metrics, k, cumulative=False, check_ranks=True, max_amb_frac=0.25, label="", pre=None):
+    """Assert parity between a product EvalResult and the oracle's dict.  Returns a report dict.
+    pre: near_ties(data, k), when the caller compares several results on the same inputs."""
     A, B, bias = data["A"], data["B"], data.get("item_biases")
     X_train, X_test = data["X_train"], data["X_test"]
     m = X_test.shape[0]
-    S64 = scores_f64(A, B, bias)
-    topk_amb, rank_amb, band = ambiguity(S64, X_train, X_test, k)
+    S64, topk_amb, rank_amb, band = near_ties(data, k) if pre is None else pre
     # exact ties inside the oracle's own float scores (reference order unspecified there too)
     tie = orc["tie_flags"]
     topk_amb = topk_amb | ((tie & 1) != 0)
@@ -138,7 +148,7 @@ def compare(res, orc, data, metrics, k, cumulative=False, check_ranks=True, max_
     # ---- top-K scores: GPU fp accumulation order differs from the CPU's SIMD order -> tolerance
     sg, so = res.topk_scores, orc["topk_scores"]
     eps = 2e-5 if sg.dtype == np.float32 else 1e-12
-    scale = np.maximum(1.0, np.nanmax(np.abs(S64), axis=1, keepdims=True))
+    scale = np.maximum(1.0, np.where(np.isfinite(S64), np.abs(S64), 0).max(axis=1, keepdims=True))
     ok = nan_equal_close(sg / scale, so / scale, eps) | ~row_equal[:, None]
     assert ok.all(), f"{label}: top-K scores differ beyond accumulation-order tolerance"
 

@@ -1,7 +1,8 @@
 """Randomised differential test of the three scoring paths (GPU): random shapes, metric sets and flags; the FMA tiles, the
 tensor-core filter (where it applies) and the full-order path must return identical status, ranked top-K ids / scores, held-out
 ranks and metric rows (break_ties_with_noise off: all three rank equal scores by item id).  With the noise on, the automatic
-path (filter + noise-reach hand-back) must equal the full-order path.  Usage: python tools/fuzz_paths.py [seconds] [seed]"""
+path (filter + noise-reach hand-back) must equal the full-order path.  One case in ten carries NaN / inf factors or biases,
+or factors whose scores overflow, in a few rows.  Usage: python tools/fuzz_paths.py [seconds] [seed]"""
 import os
 import sys
 import time
@@ -43,6 +44,27 @@ while time.time() - t0 < budget:
     if rng.random() < 0.2:
         A[rng.random(m) < 0.1] = 0               # users unseen in training
     bias = (0.5 * rng.standard_normal(n)).astype(dtype) if rng.random() < 0.3 else None
+    bad = 0
+    if rng.random() < 0.1:                       # non-finite or overflowing scores (tests/test_gpu_nonfinite.py N1-N5), a few rows
+        bad = int(rng.integers(1, 6))
+        items, users = rng.random(n) < 0.01, rng.random(m) < 0.03
+        if bad == 1:
+            B[items] = np.nan
+        elif bad == 2:
+            B[items, int(rng.integers(p))] = rng.choice([np.inf, -np.inf])
+        elif bad == 3:
+            bias = np.zeros(n, dtype=dtype) if bias is None else bias
+            bias[items] = rng.choice([-np.inf, np.inf, np.nan], p=[0.8, 0.1, 0.1])
+        elif bad == 4:
+            A[users, int(rng.integers(p))] = rng.choice([np.nan, np.inf, -np.inf])
+        elif dtype == np.float64:                # one product of a scaled user and a scaled item leaves the range
+            A[users, -1] = 1e160 * rng.choice([-1.0, 1.0], int(users.sum()))
+            B[items, -1] = 1e160
+        else:                                    # ... with norms within ~1000x of each other (B * 1e18, ||a|| ~ 1e19, items ~4e21),
+            B *= 1e18                            # which the filter could rank: every other score stays below ||a|| ||b|| < 1.7e38
+            A[users] *= 5e17 / np.maximum(1.0, np.abs(A[users]).max(axis=1, keepdims=True))
+            A[users, -1] = 1e19 * rng.choice([-1.0, 1.0], int(users.sum()))
+            B[items, -1] = 4e21
     flags = {f: bool(rng.random() < 0.4) for f in FLAGS}
     if not any(flags[f] for f in ("precision", "average_precision", "ndcg")):      # (the reference's "at least one metric" guard, quirk Q7)
         flags["precision"] = True
@@ -51,8 +73,8 @@ while time.time() - t0 < budget:
     kw = dict(k=K, item_biases=bias, cumulative=cumulative, break_ties_with_noise=noise, seed=int(rng.integers(1, 1000)),
               return_topk=True, return_status=True, return_ranks=flags["roc_auc"] or flags["pr_auc"],
               min_pos_test=int(rng.integers(1, 3)), consider_cold_start=bool(rng.random() < 0.8), **flags)
-    what = "m=%d n=%d p=%d K=%d %s cum=%d noise=%d bias=%d flags=%s" % (m, n, p, K, np.dtype(dtype).name, cumulative, noise, bias is not None,
-                                                                         [f for f in FLAGS if flags[f]])
+    what = "m=%d n=%d p=%d K=%d %s cum=%d noise=%d bias=%d nonfinite=N%d flags=%s" % (
+        m, n, p, K, np.dtype(dtype).name, cumulative, noise, bias is not None, bad, [f for f in FLAGS if flags[f]])
     try:
         full = rb.calc_reco_metrics_ex(d["X_train"], d["X_test"], A, B, scoring_path="full", **kw)
         auto = rb.calc_reco_metrics_ex(d["X_train"], d["X_test"], A, B, scoring_path="auto", **kw)
