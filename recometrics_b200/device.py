@@ -18,13 +18,12 @@ used for device allocations only.  Argument meaning, defaults, validation messag
 ``calc_reco_metrics_ex``.
 """
 from dataclasses import dataclass
-from warnings import warn
 
 import numpy as np
 from scipy.sparse import issparse
 
-from . import _capi
-from .frontend import EvalResult, _ResultRows, _canonical_csr, _popularity_array, item_popularity as _item_popularity
+from .frontend import (_canonical_csr, _check_bias_items, _check_csr_kind, _check_factor_shapes, _check_train_shape,
+                       _counts, _evaluate, _metric_flags, _popularity, item_popularity as _item_popularity)
 
 __all__ = ["DeviceCSR", "calc_reco_metrics_device"]
 
@@ -119,46 +118,22 @@ def calc_reco_metrics_device(
         raise ValueError("'A' and 'B' must be on the same device.")
     dev = torch.device("cuda", device)
 
-    flags = dict(p=precision, tp=trunc_precision, r=recall, ap=average_precision, tap=trunc_average_precision,
-                 ndcg=ndcg, hit=hit, rr=rr, roc=roc_auc, pr=pr_auc)
-    flags = {q: bool(v) or bool(all_metrics) for q, v in flags.items()}
-    if not (flags["p"] or flags["ap"] or flags["ndcg"] or flags["hit"] or flags["rr"] or flags["roc"]):
-        raise ValueError("Must pass at least one metric to calculate.")
-    cumulative = bool(cumulative)
+    flags = _metric_flags(all_metrics, precision, trunc_precision, recall, average_precision, trunc_average_precision, ndcg,
+                          hit, rr, roc_auc, pr_auc)
 
+    _check_csr_kind(X_test, "X_test")
     if issparse(X_test):
         X_test = DeviceCSR.from_scipy(X_test, device, dtype)
-    if not isinstance(X_test, DeviceCSR):
-        raise TypeError("'X_test' must be a sparse matrix or a DeviceCSR.")
     m, n = X_test.shape
     if X_train is None:
         X_train = DeviceCSR(torch.zeros(m + 1, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.int32, device=dev), None, (m, n))
         consider_cold_start = True
-    elif issparse(X_train):
+    _check_csr_kind(X_train, "X_train")
+    if issparse(X_train):
         X_train = DeviceCSR.from_scipy(X_train, device, dtype, with_data=False)
-    if not isinstance(X_train, DeviceCSR):
-        raise TypeError("'X_train' must be a sparse matrix or a DeviceCSR.")
-    if X_train.shape[1] != n:
-        raise ValueError("'X_train' and 'X_test' should have the same number of columns.")
-    if X_train.shape[0] < m:
-        raise ValueError("'X_train' and 'X_test' should have the same number of rows.")
-    if dA.shape[1] != dB.shape[1]:
-        raise ValueError("'A' and 'B' must have the same number of columns.")
-    if 0 in (dA.shape[0], dA.shape[1], m, n):
-        raise ValueError("Input matrices cannot be empty.")
-    if dA.shape[0] < m:
-        raise ValueError("Number of users in 'A' and 'X_test' does not match.")
-    if dB.shape[0] < n:
-        raise ValueError("Number of items in 'B' and 'X_test' does not match.")
-    if dA.shape[0] > m:
-        warn("'A' has more users than 'X_test'.")
-    if dB.shape[0] > n:
-        warn("'B' has more items than 'X_test'.")
-    seed, k, min_pos_test, min_items_pool = int(seed), int(k), int(min_pos_test), int(min_items_pool)
-    if seed < 1 or k < 1 or min_pos_test < 1 or min_items_pool < 1:
-        raise ValueError("'seed', 'k', 'min_pos_test' and 'min_items_pool' must be >= 1.")
-    if k > n:
-        raise ValueError("'k' should be smaller than the number of items.")
+    _check_train_shape(X_train.shape, m, n)
+    _check_factor_shapes(dA.shape, dB.shape, m, n)
+    seed, k, min_pos_test, min_items_pool = _counts(seed, k, min_pos_test, min_items_pool, n)
     for name, X in (("X_train", X_train), ("X_test", X_test)):
         for part in ("indptr", "indices"):
             t = getattr(X, part)
@@ -179,58 +154,23 @@ def calc_reco_metrics_device(
             if db.dtype != dA.dtype:
                 raise TypeError("'item_biases' must have the dtype of the factors.")
             bias_keep = item_biases
-        nb = int(bias_keep.shape[0])
-        if nb < n:
-            raise ValueError("Number of items in 'item_biases' must match with 'X_test'.")
+        _check_bias_items(int(bias_keep.shape[0]), n)
         bias_ptr = int(bias_keep.__cuda_array_interface__["data"][0])
 
-    K = k
-    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
-    tdts = {np.float32: torch.float32, np.float64: torch.float64, np.int64: torch.int64}
-    res = _ResultRows(lambda size, dt, fill: torch.empty(size, dtype=tdts[dt], device=dev) if fill is None
-                      else torch.full((size,), fill, dtype=tdts[dt], device=dev),
-                      dtype, m, K, cumulative, flags, bflags, user_range, bool(return_means) or bool(means_only))
-    timing = _capi.Timing()
-    status = torch.zeros(m, dtype=torch.int32, device=dev) if return_status else None
-    topk_items = torch.full((m * K,), -1, dtype=torch.int32, device=dev) if return_topk else None
-    topk_scores = torch.full((m * K,), float("nan"), dtype=tdt, device=dev) if return_topk else None
-    ub, ue = (0, 0) if user_range is None else (int(user_range[0]), int(user_range[1]))
-    if user_range is not None and ub == ue:
-        ub, ue = 0, -1          # an EMPTY block; 0,0 would mean "all users" in the C-ABI
-    ptr = lambda t: None if t is None else t.data_ptr()
-    extra = _capi.make_extra(device=device, user_begin=ub, user_end=ue, inputs_on_device=True,
-                             strict_min_pos_test=strict_min_pos_test, topk_items=ptr(topk_items), topk_scores=ptr(topk_scores),
-                             status=ptr(status), timing=timing, scoring_path=scoring_path, metric_means=ptr(res.means),
-                             metric_counts=ptr(res.counts), skip_row_copy=bool(means_only))
-    item_counts = torch.zeros(n, dtype=torch.int64, device=dev) if return_exposure else None
-    expo = _capi.make_exposure(ptr(item_counts)) if return_exposure else None
-    bey = None
-    if res.brows:
-        pop = None
-        if bflags["novelty"] or bflags["avg_popularity"]:
-            if item_popularity is None:
-                pop = _item_popularity(X_train, m=m)
-            elif isinstance(item_popularity, torch.Tensor):
-                if item_popularity.dim() != 1 or item_popularity.shape[0] != n:
-                    raise ValueError("'item_popularity' must be a 1-d array with one count per item (%d)." % n)
-                if item_popularity.dtype.is_floating_point or item_popularity.dtype.is_complex or item_popularity.dtype == torch.bool:
-                    raise TypeError("'item_popularity' must hold integer counts.")
-                pop = item_popularity.to(device=dev, dtype=torch.int64).contiguous()
-                if n and bool(((pop < 0) | (pop > m)).any()):
-                    raise ValueError("'item_popularity' counts must lie in [0, %d] (the number of users)." % m)
-            else:
-                pop = torch.from_numpy(_popularity_array(item_popularity, n, m)).to(dev)
-        bey = _capi.make_beyond({name: t.data_ptr() for name, t in res.brows.items()}, ptr(pop), m, ptr(res.bmeans), ptr(res.bcounts))
-    torch.cuda.synchronize(dev)            # the library runs on its own stream: the caller's pending writes must have landed
-    rc = _capi.calc_metrics(dtype, dA.ptr, dA.ld, dB.ptr, dB.ld, m, n, dA.shape[1],
-                            ptr(X_train.indptr), ptr(X_train.indices) if X_train.indices.numel() else None,
-                            ptr(X_test.indptr), ptr(X_test.indices), ptr(tev), K, cumulative, bool(break_ties_with_noise),
-                            {q: t.data_ptr() for q, t in res.outs.items()}, bool(consider_cold_start), min_items_pool,
-                            min_pos_test, 1, seed, bias_ptr, extra, exposure=expo, beyond=bey)
-    _capi.raise_for_status(rc)
+    # the addresses stay valid while X_train, X_test, tev and bias_keep live: until this function returns
+    prep = dict(A=dA.ptr, lda=dA.ld, B=dB.ptr, ldb=dB.ld, dtype=dtype, m=m, n=n, p=dA.shape[1],
+                trp=X_train.indptr.data_ptr(), tri=X_train.indices.data_ptr() if X_train.indices.numel() else None,
+                tep=X_test.indptr.data_ptr(), tei=X_test.indices.data_ptr(), tev=None if tev is None else tev.data_ptr(),
+                k=k, item_biases=bias_ptr, min_pos_test=min_pos_test, min_items_pool=min_items_pool,
+                consider_cold_start=bool(consider_cold_start), nthreads=1, seed=seed, flags=flags)
+    tdts = {np.float32: torch.float32, np.float64: torch.float64, np.int32: torch.int32, np.int64: torch.int64}
 
-    metrics, mean_d, count_d = res.unpack(means_only, lambda t: t.cpu().numpy())
-    return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
-                      topk_items=None if topk_items is None else topk_items.view(m, K),
-                      topk_scores=None if topk_scores is None else topk_scores.view(m, K),
-                      exposure=item_counts, catalogue=None if expo is None else expo.catalogue())
+    def popularity():
+        return _item_popularity(X_train, m=m) if item_popularity is None else _popularity(item_popularity, n, m, dev)
+    return _evaluate(lambda size, dt, fill: torch.empty(size, dtype=tdts[dt], device=dev) if fill is None
+                     else torch.full((size,), fill, dtype=tdts[dt], device=dev), lambda t: t.data_ptr(), prep, popularity,
+                     cumulative, break_ties_with_noise, user_range, return_topk, return_status, return_means, means_only,
+                     return_exposure, novelty, avg_popularity, diversity, to_numpy=lambda t: t.cpu().numpy(),
+                     # the library runs on its own stream: the caller's pending writes and the fills above must have landed
+                     sync=lambda: torch.cuda.synchronize(dev),
+                     device=device, inputs_on_device=True, strict_min_pos_test=strict_min_pos_test, scoring_path=scoring_path)

@@ -69,16 +69,28 @@ def _canonical_csr(X):
     return X, np.ascontiguousarray(indptr), np.ascontiguousarray(indices)
 
 
-def _popularity_array(item_popularity, n, m):
-    """A caller's item popularity for Novelty@K / AvgPop@K: integer counts, one per item, each in [0, m]; int64 numpy."""
-    p = np.asarray(item_popularity)
+def _popularity(item_popularity, n, m, device=None):
+    """A caller's item popularity for Novelty@K / AvgPop@K: integer counts, one per item, each in [0, m]; int64 numpy --
+    or, with a torch ``device`` (the device front-end, which also takes a torch tensor), an int64 tensor on it."""
+    if device is not None:
+        import torch
+    p = item_popularity
+    if device is not None and isinstance(p, torch.Tensor):
+        integer = not (p.dtype.is_floating_point or p.dtype.is_complex or p.dtype == torch.bool)
+    else:
+        p = np.asarray(p)
+        integer = p.dtype.kind in "iu"
     if p.ndim != 1 or p.shape[0] != n:
         raise ValueError("'item_popularity' must be a 1-d array with one count per item (%d)." % n)
-    if p.dtype.kind not in "iu":
+    if not integer:
         raise TypeError("'item_popularity' must hold integer counts.")
-    if p.size and (p.min() < 0 or p.max() > m):
+    if isinstance(p, np.ndarray):
+        p = np.ascontiguousarray(p, dtype=np.int64)
+    if device is not None:
+        p = torch.as_tensor(p).to(device=device, dtype=torch.int64).contiguous()
+    if bool(((p < 0) | (p > m)).any()):
         raise ValueError("'item_popularity' counts must lie in [0, %d] (the number of users)." % m)
-    return np.ascontiguousarray(p, dtype=np.int64)
+    return p
 
 
 def _popularity_rows(rows, m, user_range):
@@ -97,6 +109,7 @@ def item_popularity(X_train, m=None, user_range=None, device=-1):
     numpy int64 ``[n]``; ``device``: the CUDA ordinal, -1 = default) or a :class:`DeviceCSR` (returns a torch int64 ``[n]``
     on its device)."""
     from .device import DeviceCSR
+    _check_csr_kind(X_train, "X_train")
     if isinstance(X_train, DeviceCSR):
         import torch
         rows, n = int(X_train.shape[0]), int(X_train.shape[1])
@@ -107,8 +120,6 @@ def item_popularity(X_train, m=None, user_range=None, device=-1):
         _capi.item_popularity(X_train.indptr.data_ptr(), X_train.indices.data_ptr() if X_train.indices.numel() else None,
                               b, e, n, counts.data_ptr(), device=dev.index, inputs_on_device=True)
         return counts
-    if not issparse(X_train):
-        raise TypeError("'X_train' must be a sparse matrix or a DeviceCSR.")
     X_train, indptr, indices = _canonical_csr(X_train)
     b, e = _popularity_rows(X_train.shape[0], m, user_range)
     counts = np.zeros(X_train.shape[1], dtype=np.int64)
@@ -155,8 +166,63 @@ class _ResultRows:
         return metrics, mean_d, count_d
 
 
-def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ties_with_noise,
-                          min_pos_test, min_items_pool, consider_cold_start, cumulative, nthreads, seed):
+# Argument checks that both front-ends make, each front-end in its own order (the reference's for the host one).
+def _metric_flags(all_metrics, *switches):
+    """The ten metric switches, in METRIC_ORDER, as flags (``all_metrics`` sets them all)."""
+    flags = {q: bool(v) or bool(all_metrics) for q, v in zip(_capi.METRIC_ORDER, switches, strict=True)}
+    # the reference's guard ignores recall / trunc_* / pr_auc (quirk Q7, :499-500) -- kept as is
+    if not (flags["p"] or flags["ap"] or flags["ndcg"] or flags["hit"] or flags["rr"] or flags["roc"]):
+        raise ValueError("Must pass at least one metric to calculate.")
+    return flags
+
+
+def _check_factor_shapes(a_shape, b_shape, m, n):
+    """A [users, p] and B [items, p] against X_test [m, n]; the rows past m / n are not read."""
+    if a_shape[1] != b_shape[1]:
+        raise ValueError("'A' and 'B' must have the same number of columns.")
+    if 0 in (a_shape[0], a_shape[1], m, n):
+        raise ValueError("Input matrices cannot be empty.")
+    if a_shape[0] < m:
+        raise ValueError("Number of users in 'A' and 'X_test' does not match.")
+    if b_shape[0] < n:
+        raise ValueError("Number of items in 'B' and 'X_test' does not match.")
+    if a_shape[0] > m:
+        warn("'A' has more users than 'X_test'.")
+    if b_shape[0] > n:
+        warn("'B' has more items than 'X_test'.")
+
+
+def _check_csr_kind(X, name):
+    from .device import DeviceCSR
+    if not (issparse(X) or isinstance(X, DeviceCSR)):
+        raise TypeError("'%s' must be a sparse matrix or a DeviceCSR." % name)
+
+
+def _check_train_shape(train_shape, m, n):
+    if train_shape[1] != n:
+        raise ValueError("'X_train' and 'X_test' should have the same number of columns.")
+    if train_shape[0] < m:
+        raise ValueError("'X_train' and 'X_test' should have the same number of rows.")
+
+
+def _counts(seed, k, min_pos_test, min_items_pool, n):
+    """The call's integer arguments as ints: each at least 1, ``k`` at most the ``n`` items."""
+    seed, k, min_pos_test, min_items_pool = int(seed), int(k), int(min_pos_test), int(min_items_pool)
+    if seed < 1 or k < 1 or min_pos_test < 1 or min_items_pool < 1:
+        raise ValueError("'seed', 'k', 'min_pos_test' and 'min_items_pool' must be >= 1.")
+    if k > n:
+        raise ValueError("'k' should be smaller than the number of items.")
+    return seed, k, min_pos_test, min_items_pool
+
+
+def _check_bias_items(items, n):
+    if items < n:
+        raise ValueError("Number of items in 'item_biases' must match with 'X_test'.")
+
+
+def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, min_pos_test, min_items_pool, consider_cold_start,
+                          nthreads, seed, *metric_switches):
+    """The host front-end's checks and conversions (``metric_switches``: as :func:`_metric_flags` takes them)."""
     if (A is None) != (B is None):
         raise ValueError("'A' and 'B' must either be passed together or passed as 'None' together.")
     if item_biases is not None and hasattr(item_biases, "to_numpy"):
@@ -184,20 +250,8 @@ def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ti
         raise ValueError("'A' must be a 2-dimensional array.")
     if B.ndim != 2:
         raise ValueError("'B' must be a 2-dimensional array.")
-    if A.shape[1] != B.shape[1]:
-        raise ValueError("'A' and 'B' must have the same number of columns.")
-    if 0 in (A.shape[0], A.shape[1], B.shape[1], X_test.shape[0], X_test.shape[1]):
-        raise ValueError("Input matrices cannot be empty.")
-    if A.shape[0] < X_test.shape[0]:
-        raise ValueError("Number of users in 'A' and 'X_test' does not match.")
-    if B.shape[0] < X_test.shape[1]:
-        raise ValueError("Number of items in 'B' and 'X_test' does not match.")
-    if A.shape[0] > X_test.shape[0]:
-        warn("'A' has more users than 'X_test'.")
-        A = A[:X_test.shape[0], :]
-    if B.shape[0] > X_test.shape[1]:
-        warn("'B' has more items than 'X_test'.")
-        B = B[:X_test.shape[1], :]
+    _check_factor_shapes(A.shape, B.shape, X_test.shape[0], X_test.shape[1])
+    A, B = A[:X_test.shape[0], :], B[:X_test.shape[1], :]
 
     # float32 only if both factor matrices are float32 (reference :469)
     dtype = np.float32 if (A.dtype == np.float32 and B.dtype == np.float32) else np.float64
@@ -207,27 +261,18 @@ def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ti
         consider_cold_start = True
     if not issparse(X_train):
         raise TypeError("'X_train' must be a sparse matrix.")
-    if X_train.shape[1] != X_test.shape[1]:
-        raise ValueError("'X_train' and 'X_test' should have the same number of columns.")
-    if X_train.shape[0] < X_test.shape[0]:
-        raise ValueError("'X_train' and 'X_test' should have the same number of rows.")
+    _check_train_shape(X_train.shape, X_test.shape[0], X_test.shape[1])
     if X_train.shape[0] > X_test.shape[0]:
         warn("'X_train' mas more rows than 'X_test'.")
 
-    # the reference's guard ignores recall / trunc_* / pr_auc (quirk Q7, :499-500) -- kept as is
-    if not (flags["p"] or flags["ap"] or flags["ndcg"] or flags["hit"] or flags["rr"] or flags["roc"]):
-        raise ValueError("Must pass at least one metric to calculate.")
+    flags = _metric_flags(*metric_switches)
 
     if isinstance(seed, np.random.RandomState):
         seed = int(seed.randint(imax))
     elif isinstance(seed, np.random.Generator):
         seed = int(seed.integers(imax))
     nthreads = 1 if nthreads is None else int(nthreads)
-    seed, k, min_pos_test, min_items_pool = int(seed), int(k), int(min_pos_test), int(min_items_pool)
-    if seed < 1 or k < 1 or min_pos_test < 1 or min_items_pool < 1:
-        raise ValueError("'seed', 'k', 'min_pos_test' and 'min_items_pool' must be >= 1.")
-    if k > X_test.shape[1]:
-        raise ValueError("'k' should be smaller than the number of items.")
+    seed, k, min_pos_test, min_items_pool = _counts(seed, k, min_pos_test, min_items_pool, X_test.shape[1])
 
     if item_biases is not None:
         if not isinstance(item_biases, np.ndarray):
@@ -237,8 +282,7 @@ def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ti
         item_biases = item_biases.reshape(-1)
         if not item_biases.shape[0]:
             raise ValueError("'item_biases' is empty.")
-        if item_biases.shape[0] < X_test.shape[1]:
-            raise ValueError("Number of items in 'item_biases' must match with 'X_test'.")
+        _check_bias_items(item_biases.shape[0], X_test.shape[1])
         if item_biases.shape[0] > X_test.shape[1]:
             warn("'item_biases' has more items than 'X_test'.")
             item_biases = item_biases[:X_test.shape[1]]
@@ -254,7 +298,51 @@ def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ti
     return dict(A=A, lda=lda, B=B, ldb=ldb, dtype=dtype, m=X_test.shape[0], n=X_test.shape[1], p=A.shape[1],
                 trp=trp, tri=tri, tep=tep, tei=tei, tev=tev, k=k, item_biases=item_biases,
                 min_pos_test=min_pos_test, min_items_pool=min_items_pool,
-                consider_cold_start=bool(consider_cold_start), nthreads=nthreads, seed=seed)
+                consider_cold_start=bool(consider_cold_start), nthreads=nthreads, seed=seed, flags=flags)
+
+
+def _evaluate(alloc, addr, prep, popularity, cumulative, break_ties_with_noise, user_range, return_topk, return_status,
+              return_means, means_only, return_exposure, novelty, avg_popularity, diversity, return_ranks=False,
+              to_numpy=lambda x: x, sync=lambda: None, **extra):
+    """The evaluation call both front-ends end in, on the inputs ``prep`` they validated (``_validate_and_prepare``'s keys:
+    host arrays or device addresses, as ``_capi.calc_metrics`` takes them).  The result rows and the asked-for extras are
+    allocated with ``alloc(size, dtype, fill)`` (see :class:`_ResultRows`) and handed to the library as ``addr(array)``;
+    ``popularity()`` gives the item popularity when Novelty / AvgPop is asked for, ``sync()`` runs right before the call,
+    ``to_numpy`` brings a means / counts table to the host and ``extra`` goes to ``_capi.make_extra``."""
+    dtype, m, n, K, cumulative = prep["dtype"], prep["m"], prep["n"], prep["k"], bool(cumulative)
+    ptr = lambda x: None if x is None else addr(x)
+    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
+    res = _ResultRows(alloc, dtype, m, K, cumulative, prep["flags"], bflags, user_range, bool(return_means) or bool(means_only))
+    timing = _capi.Timing()
+    status = alloc(m, np.int32, 0) if return_status else None
+    topk_items = alloc(m * K, np.int32, -1) if return_topk else None
+    topk_scores = alloc(m * K, dtype, np.nan) if return_topk else None
+    pos_rank = alloc(max(int(prep["tep"][-1]), 1), np.int64, 0) if return_ranks else None
+    ub, ue = (0, 0) if user_range is None else (int(user_range[0]), int(user_range[1]))
+    if user_range is not None and ub == ue:
+        ub, ue = 0, -1          # an EMPTY block (a rank with no users); 0,0 would mean "all users" in the C-ABI
+    ex = _capi.make_extra(user_begin=ub, user_end=ue, topk_items=ptr(topk_items), topk_scores=ptr(topk_scores),
+                          pos_rank=ptr(pos_rank), status=ptr(status), timing=timing, metric_means=ptr(res.means),
+                          metric_counts=ptr(res.counts), skip_row_copy=bool(means_only), **extra)
+    item_counts = alloc(n, np.int64, 0) if return_exposure else None
+    expo = _capi.make_exposure(ptr(item_counts)) if return_exposure else None
+    pop = popularity() if bflags["novelty"] or bflags["avg_popularity"] else None
+    bey = _capi.make_beyond({name: addr(r) for name, r in res.brows.items()}, ptr(pop), m, ptr(res.bmeans),
+                            ptr(res.bcounts)) if res.brows else None
+    sync()
+    rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, n, prep["p"],
+                            prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
+                            bool(break_ties_with_noise), {q: addr(r) for q, r in res.outs.items()}, prep["consider_cold_start"],
+                            prep["min_items_pool"], prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"],
+                            ex, exposure=expo, beyond=bey)
+    _capi.raise_for_status(rc)
+
+    metrics, mean_d, count_d = res.unpack(means_only, to_numpy)
+    return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
+                      topk_items=None if topk_items is None else topk_items.reshape(m, K),
+                      topk_scores=None if topk_scores is None else topk_scores.reshape(m, K),
+                      pos_rank=None if pos_rank is None else pos_rank[: int(prep["tep"][-1])],
+                      exposure=item_counts, catalogue=None if expo is None else expo.catalogue())
 
 
 def calc_reco_metrics_ex(
@@ -287,54 +375,22 @@ def calc_reco_metrics_ex(
     ``return_means``, their means and counts under the same keys; NaN for users without a list.  ``item_popularity``: int64
     ``[n]`` counts of how many of the m users have each item in ``X_train`` (see :func:`item_popularity`, which computes it
     when it is not given).  ``all_metrics`` does not turn these on."""
-    flags = dict(p=precision, tp=trunc_precision, r=recall, ap=average_precision, tap=trunc_average_precision,
-                 ndcg=ndcg, hit=hit, rr=rr, roc=roc_auc, pr=pr_auc)
-    flags = {q: bool(v) or bool(all_metrics) for q, v in flags.items()}
-    cumulative = bool(cumulative)
-    prep = _validate_and_prepare(X_train, X_test, A, B, k, item_biases, flags, break_ties_with_noise,
-                                 min_pos_test, min_items_pool, consider_cold_start, cumulative, nthreads, seed)
-    dtype, m, K = prep["dtype"], prep["m"], prep["k"]
-    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
-    res = _ResultRows(lambda size, dt, fill: np.empty(size, dt) if fill is None else np.full(size, fill, dt),
-                      dtype, m, K, cumulative, flags, bflags, user_range, bool(return_means) or bool(means_only))
-    timing = _capi.Timing()
-    status = np.zeros(m, dtype=np.int32) if return_status else None
-    topk_items = np.full(m * K, -1, dtype=np.int32) if return_topk else None
-    topk_scores = np.full(m * K, np.nan, dtype=dtype) if return_topk else None
-    pos_rank = np.zeros(max(int(prep["tep"][-1]), 1), dtype=np.int64) if return_ranks else None
-    ub, ue = (0, 0) if user_range is None else (int(user_range[0]), int(user_range[1]))
-    if user_range is not None and ub == ue:
-        ub, ue = 0, -1          # an EMPTY block (a rank with no users); 0,0 would mean "all users" in the C-ABI
-    extra = _capi.make_extra(device=device, user_begin=ub, user_end=ue, strict_min_pos_test=strict_min_pos_test,
-                             topk_items=topk_items, topk_scores=topk_scores, pos_rank=pos_rank, status=status,
-                             timing=timing, scoring_path=scoring_path, metric_means=res.means, metric_counts=res.counts,
-                             skip_row_copy=bool(means_only), filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
-    item_counts = np.zeros(prep["n"], dtype=np.int64) if return_exposure else None
-    expo = _capi.make_exposure(item_counts) if return_exposure else None
-    bey = None
-    if res.brows:
-        pop = None
-        if bflags["novelty"] or bflags["avg_popularity"]:
-            if item_popularity is not None:
-                pop = _popularity_array(item_popularity, prep["n"], m)
-            else:
-                pop = np.zeros(prep["n"], dtype=np.int64)
-                _capi.item_popularity(prep["trp"], prep["tri"], 0, m, prep["n"], pop,
-                                      device=device if device >= 0 else (devices[0] if devices else -1))
-        bey = _capi.make_beyond(res.brows, pop, m, res.bmeans, res.bcounts)
-    rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, prep["n"], prep["p"],
-                            prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
-                            bool(break_ties_with_noise), res.outs, prep["consider_cold_start"], prep["min_items_pool"],
-                            prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"], extra, exposure=expo,
-                            beyond=bey)
-    _capi.raise_for_status(rc)
+    prep = _validate_and_prepare(X_train, X_test, A, B, k, item_biases, min_pos_test, min_items_pool, consider_cold_start,
+                                 nthreads, seed, all_metrics, precision, trunc_precision, recall, average_precision,
+                                 trunc_average_precision, ndcg, hit, rr, roc_auc, pr_auc)
 
-    metrics, mean_d, count_d = res.unpack(means_only)
-    return EvalResult(metrics=metrics, timing=timing.as_dict(), status=status, means=mean_d, counts=count_d,
-                      topk_items=None if topk_items is None else topk_items.reshape(m, K),
-                      topk_scores=None if topk_scores is None else topk_scores.reshape(m, K),
-                      pos_rank=None if pos_rank is None else pos_rank[: int(prep["tep"][-1])],
-                      exposure=item_counts, catalogue=None if expo is None else expo.catalogue())
+    def popularity():
+        if item_popularity is not None:
+            return _popularity(item_popularity, prep["n"], prep["m"])
+        pop = np.zeros(prep["n"], dtype=np.int64)
+        _capi.item_popularity(prep["trp"], prep["tri"], 0, prep["m"], prep["n"], pop,
+                              device=device if device >= 0 else (devices[0] if devices else -1))
+        return pop
+    return _evaluate(lambda size, dt, fill: np.empty(size, dt) if fill is None else np.full(size, fill, dt), lambda x: x,
+                     prep, popularity, cumulative, break_ties_with_noise, user_range, return_topk, return_status,
+                     return_means, means_only, return_exposure, novelty, avg_popularity, diversity, return_ranks=return_ranks,
+                     device=device, strict_min_pos_test=strict_min_pos_test, scoring_path=scoring_path,
+                     filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
 
 
 def calc_reco_metrics(

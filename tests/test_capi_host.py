@@ -113,31 +113,71 @@ def test_product_never_imports_the_oracle():
             assert "librmoracle" not in txt and "librecometrics_ref" not in txt, path
 
 
+def _exact(msg):
+    return "^%s$" % re.escape(msg)
+
+
 def test_frontend_validation_mirrors_reference(rb):
-    """Argument errors are raised on the host before anything touches the GPU
-    (reference: recometrics/__init__.py:426-467, :499-500, :531-532)."""
-    from scipy.sparse import csr_array
+    """Argument errors and warnings are raised on the host before anything touches the GPU, each with its full text, and of
+    several faults the first in the reference's order is reported (reference: recometrics/__init__.py:426-467, :499-500,
+    :531-532; then the checks of item_popularity)."""
+    from scipy.sparse import coo_array, csr_array, vstack
     from tools import synth
     d = synth.make(1, m=30, n=50, p=4, k=3)
     Xtr, Xte, A, B = d["X_train"], d["X_test"], d["A"], d["B"]
-    with pytest.raises(ValueError, match="passed together"):
-        rb.calc_reco_metrics(Xtr, Xte, A, None)
-    with pytest.raises(ValueError, match="same number of columns"):
-        rb.calc_reco_metrics(Xtr, Xte, A, B[:, :3])
-    with pytest.raises(ValueError, match="Number of users"):
-        rb.calc_reco_metrics(Xtr, Xte, A[:10], B)
-    with pytest.raises(ValueError, match="Number of items"):
-        rb.calc_reco_metrics(Xtr, Xte, A, B[:10])
-    with pytest.raises(ValueError, match="at least one metric"):
-        rb.calc_reco_metrics(Xtr, Xte, A, B, precision=False, average_precision=False, ndcg=False, recall=True)
-    with pytest.raises(ValueError, match="smaller than the number of items"):
-        rb.calc_reco_metrics(Xtr, Xte, A, B, k=51)
-    with pytest.raises(ValueError, match="empty"):
-        rb.calc_reco_metrics(Xtr, csr_array(Xte.shape, dtype=np.float32), A, B)
-    with pytest.raises(ValueError, match="item biases"):
-        rb.calc_reco_metrics(Xtr, Xte, None, None)
-    with pytest.raises(ValueError, match="item_biases"):
-        rb.calc_reco_metrics(Xtr, Xte, A, B, item_biases=np.ones(10, dtype=np.float32))
+    imax = np.iinfo(np.int32).max
+
+    def call(**kw):
+        return rb.calc_reco_metrics_ex(**{**dict(X_train=Xtr, X_test=Xte, A=A, B=B, k=3, break_ties_with_noise=False), **kw})
+
+    no_metric = dict(precision=False, average_precision=False, ndcg=False, recall=True)
+    counts_rule = "'seed', 'k', 'min_pos_test' and 'min_items_pool' must be >= 1."
+    pop_len = "'item_popularity' must be a 1-d array with one count per item (50)."
+    pop_range = "'item_popularity' counts must lie in [0, 30] (the number of users)."
+    for kw, exc, msg in (
+            (dict(B=None), ValueError, "'A' and 'B' must either be passed together or passed as 'None' together."),
+            (dict(A=None, B=None), ValueError, "Must pass item biases if not passing factors."),
+            (dict(A=A.tolist()), TypeError, "'A' and 'B' must be numpy arrays."),
+            (dict(X_test=Xte.toarray()), TypeError, "'X_test' must be a sparse matrix."),
+            (dict(X_test=coo_array((imax, 50))), ValueError, "Number of test user is larger than maximum supported."),
+            (dict(X_test=coo_array((30, imax))), ValueError, "Number of items is larger than maximum supported."),
+            (dict(X_test=csr_array(Xte.shape, dtype=np.float32)), ValueError, "'X_test' is empty."),
+            (dict(A=A[:, 0]), ValueError, "'A' must be a 2-dimensional array."),
+            (dict(B=B[:, 0]), ValueError, "'B' must be a 2-dimensional array."),
+            (dict(B=B[:, :3]), ValueError, "'A' and 'B' must have the same number of columns."),
+            (dict(A=A[:, :0], B=B[:, :0]), ValueError, "Input matrices cannot be empty."),
+            (dict(A=A[:10]), ValueError, "Number of users in 'A' and 'X_test' does not match."),
+            (dict(B=B[:10]), ValueError, "Number of items in 'B' and 'X_test' does not match."),
+            (dict(X_train=Xtr.toarray()), TypeError, "'X_train' must be a sparse matrix."),
+            (dict(X_train=Xtr[:, :49]), ValueError, "'X_train' and 'X_test' should have the same number of columns."),
+            (dict(X_train=Xtr[:29]), ValueError, "'X_train' and 'X_test' should have the same number of rows."),
+            (no_metric, ValueError, "Must pass at least one metric to calculate."),
+            (dict(seed=0), ValueError, counts_rule),
+            (dict(k=0), ValueError, counts_rule),
+            (dict(min_pos_test=0), ValueError, counts_rule),
+            (dict(min_items_pool=0), ValueError, counts_rule),
+            (dict(k=51), ValueError, "'k' should be smaller than the number of items."),
+            (dict(item_biases=[0.0] * 50), TypeError, "'item_biases' must be a numpy array."),
+            (dict(item_biases=np.ones((50, 1, 1), dtype=np.float32)), ValueError, "'item_biases' should be a 1-d array."),
+            (dict(item_biases=np.ones(0, dtype=np.float32)), ValueError, "'item_biases' is empty."),
+            (dict(item_biases=np.ones(10, dtype=np.float32)), ValueError, "Number of items in 'item_biases' must match with 'X_test'."),
+            (dict(novelty=True, item_popularity=np.zeros(49, dtype=np.int64)), ValueError, pop_len),
+            (dict(avg_popularity=True, item_popularity=np.zeros((50, 1), dtype=np.int64)), ValueError, pop_len),
+            (dict(novelty=True, item_popularity=np.zeros(50)), TypeError, "'item_popularity' must hold integer counts."),
+            (dict(novelty=True, item_popularity=np.full(50, 31, dtype=np.int64)), ValueError, pop_range),
+            (dict(avg_popularity=True, item_popularity=np.full(50, -1, dtype=np.int32)), ValueError, pop_range),
+            # several faults: the column count comes first here (the device front-end reports the metric guard first)
+            (dict(B=B[:, :3], **no_metric), ValueError, "'A' and 'B' must have the same number of columns.")):
+        with pytest.raises(exc, match=_exact(msg)):
+            call(**kw)
+
+    # the warnings: the call goes on past each, up to a bad item_popularity, which is checked after all of them
+    for kw, msg in ((dict(A=np.vstack([A, A[:1]])), "'A' has more users than 'X_test'."),
+                    (dict(B=np.vstack([B, B[:1]])), "'B' has more items than 'X_test'."),
+                    (dict(X_train=vstack([Xtr, Xtr[:1]]).tocsr()), "'X_train' mas more rows than 'X_test'."),
+                    (dict(item_biases=np.ones(51, dtype=np.float32)), "'item_biases' has more items than 'X_test'.")):
+        with pytest.warns(UserWarning, match=_exact(msg)), pytest.raises(ValueError, match=_exact(pop_len)):
+            call(novelty=True, item_popularity=np.zeros(49, dtype=np.int64), **kw)
 
 
 def test_shard_bounds_partition():
