@@ -286,6 +286,61 @@ RMB200_API int rmb200_calc_metrics_beyond_f64(
 
 RMB200_API int rmb200_sizeof_beyond(void);
 
+/* Per-user unexpectedness and serendipity of the ranked top-K lists against each user's training history (zero-initialise,
+ * then set struct_size = sizeof(rmb200_serendipity_t)).  A user's list is j_1..j_L as for rmb200_beyond_t; H_u is the set of
+ * stored entries of the user's X_train row (values are ignored: the entries the candidate exclusion removes) and
+ * T_u = |H_u|.  u_j = b_j / ||b_j|| are ILD's unit rows of B (item factors only, no bias; a zero row gives u_j = 0).
+ *   c_u   = sum_{t in H_u} u_t, summed in the row's order;   sim_r = (u_{j_r} . c_u) / T_u, the mean cosine similarity of the
+ *           r-th listed item to the history;   rel_r = 1 when j_r is stored in the user's X_test row (any value), else 0 --
+ *           the membership P@K and Hit@K count.  Column i of a cumulative row (i = L otherwise):
+ *   Unexpectedness@i = (1/i) sum_{r<=i} (1 - sim_r)          Serendipity@i = (1/i) sum_{r<=i} rel_r (1 - sim_r)
+ * (Serendipity is Microsoft Recommenders' user_serendipity with cosine similarity over B's rows and held-out membership as the
+ * relevance; Unexpectedness is its relevance-free form.)  A user is defined when L > 0 and T_u > 0; every other user --
+ * including cold-start users, who have a list but no history, and every user of a call without X_train entries -- gets the
+ * NaN value (nan_bits is honoured) in both outputs.  Sums are accumulated in double in a fixed order and cast once: column
+ * k_metrics of a cumulative row is bit-identical to the non-cumulative value, and a user's values do not depend on
+ * user_range, the batch size or the devices.  Needs k <= 1024 (float) / 512 (double) factors (RMB200_ERR_UNSUPPORTED
+ * beyond).  RMB200_ERR_BAD_ARG, before any work: a wrong struct_size. */
+typedef struct rmb200_serendipity {
+    int32_t struct_size;          /* = sizeof(rmb200_serendipity_t)                                                       */
+    int32_t reserved0;            /* padding                                                                              */
+    void *unexpectedness, *serendipity;   /* optional out: [m] or [m * k_metrics] (cumulative) of T, rows written at         */
+                                  /* [user_begin, user_end); NULL = not requested; device pointers when inputs_on_device   */
+    double  *means;               /* optional out [2 * W], W = cumulative ? k_metrics : 1: numpy.nanmean of every requested */
+                                  /* row over the call's users (Unexpectedness, Serendipity); NaN for a row not requested  */
+    int64_t *counts;              /* optional out [2 * W]: users that entered each mean                                     */
+} rmb200_serendipity_t;
+
+/* rmb200_calc_metrics_beyond_f32 / _f64 plus unexpectedness and serendipity; serendipity == NULL is exactly the beyond call.
+ * Requesting one of the two rows counts as an output.  An interrupted call writes no means. */
+RMB200_API int rmb200_calc_metrics_serendipity_f32(
+    const float *A, size_t lda, const float *B, size_t ldb,
+    int32_t m, int32_t n, int32_t k,
+    const int32_t *Xtrain_csr_p, const int32_t *Xtrain_csr_i,
+    const int32_t *Xtest_csr_p, const int32_t *Xtest_csr_i, const float *Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    float *p_at_k, float *tp_at_k, float *r_at_k, float *ap_at_k, float *tap_at_k,
+    float *ndcg_at_k, float *hit_at_k, float *rr_at_k, float *roc_auc, float *pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test,
+    int32_t nthreads, uint64_t seed,
+    const float *item_biases, const rmb200_extra_t *extra, rmb200_exposure_t *exposure, rmb200_beyond_t *beyond,
+    rmb200_serendipity_t *serendipity);
+
+RMB200_API int rmb200_calc_metrics_serendipity_f64(
+    const double *A, size_t lda, const double *B, size_t ldb,
+    int32_t m, int32_t n, int32_t k,
+    const int32_t *Xtrain_csr_p, const int32_t *Xtrain_csr_i,
+    const int32_t *Xtest_csr_p, const int32_t *Xtest_csr_i, const double *Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    double *p_at_k, double *tp_at_k, double *r_at_k, double *ap_at_k, double *tap_at_k,
+    double *ndcg_at_k, double *hit_at_k, double *rr_at_k, double *roc_auc, double *pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test,
+    int32_t nthreads, uint64_t seed,
+    const double *item_biases, const rmb200_extra_t *extra, rmb200_exposure_t *exposure, rmb200_beyond_t *beyond,
+    rmb200_serendipity_t *serendipity);
+
+RMB200_API int rmb200_sizeof_serendipity(void);
+
 /* Item popularity on the GPU: counts[j] = number of entries of item j in rows [row_begin, row_end) of a CSR matrix
  * (numpy.bincount of those rows' indices, minlength n).  indptr / indices / counts are device pointers on `device` when
  * inputs_on_device, else host pointers (the indices go up through the library's upload pipeline).  device < 0: env

@@ -24,6 +24,7 @@ EXPORTS = (
     "rmb200_calc_metrics_ex_f32", "rmb200_calc_metrics_ex_f64",
     "rmb200_calc_metrics_exposure_f32", "rmb200_calc_metrics_exposure_f64", "rmb200_exposure_stats", "rmb200_sizeof_exposure",
     "rmb200_calc_metrics_beyond_f32", "rmb200_calc_metrics_beyond_f64", "rmb200_sizeof_beyond", "rmb200_item_popularity",
+    "rmb200_calc_metrics_serendipity_f32", "rmb200_calc_metrics_serendipity_f64", "rmb200_sizeof_serendipity",
     "rmb200_device_count", "rmb200_version", "rmb200_last_error",
     "rmb200_request_interrupt", "rmb200_measure_fma_peak", "rmb200_release_workspace",
     "rmb200_sizeof_extra", "rmb200_sizeof_timing",
@@ -114,6 +115,31 @@ def make_beyond(rows, item_popularity=None, popularity_users=0, means=None, coun
     return b
 
 
+# order of the two history rows in rmb200_serendipity_t (and of its means / counts) and their result keys
+SERENDIPITY_KEYS = (("unexpectedness", "Unexpectedness@K"), ("serendipity", "Serendipity@K"))
+
+
+class Serendipity(ctypes.Structure):
+    """rmb200_serendipity_t (include/recometrics_b200.h): Unexpectedness / Serendipity rows of a call's ranked lists."""
+    _fields_ = [
+        ("struct_size", ctypes.c_int32), ("reserved0", ctypes.c_int32),
+        ("unexpectedness", ctypes.c_void_p), ("serendipity", ctypes.c_void_p),
+        ("means", ctypes.c_void_p), ("counts", ctypes.c_void_p),
+    ]
+
+
+def make_serendipity(rows, means=None, counts=None):
+    """rmb200_serendipity_t; `rows` maps "unexpectedness" / "serendipity" -> array, device address or None; `means` /
+    `counts` are the optional [2 * W] tables (arrays or device addresses)."""
+    s = Serendipity()
+    s.struct_size = ctypes.sizeof(Serendipity)
+    for name, _ in SERENDIPITY_KEYS:
+        setattr(s, name, _vp(rows.get(name)))
+    s.means = _vp(means)
+    s.counts = _vp(counts)
+    return s
+
+
 class Csr(ctypes.Structure):
     _fields_ = [("rows", ctypes.c_int32), ("cols", ctypes.c_int32), ("nnz", ctypes.c_int64),
                 ("indptr", ctypes.c_void_p), ("indices", ctypes.c_void_p), ("values", ctypes.c_void_p)]
@@ -161,9 +187,10 @@ def load():
     lib.rmb200_sizeof_split.restype = ctypes.c_int
     lib.rmb200_sizeof_exposure.restype = ctypes.c_int
     lib.rmb200_sizeof_beyond.restype = ctypes.c_int
+    lib.rmb200_sizeof_serendipity.restype = ctypes.c_int
     if (lib.rmb200_sizeof_extra() != ctypes.sizeof(Extra) or lib.rmb200_sizeof_timing() != ctypes.sizeof(Timing)
             or lib.rmb200_sizeof_split() != ctypes.sizeof(Split) or lib.rmb200_sizeof_exposure() != ctypes.sizeof(Exposure)
-            or lib.rmb200_sizeof_beyond() != ctypes.sizeof(Beyond)):
+            or lib.rmb200_sizeof_beyond() != ctypes.sizeof(Beyond) or lib.rmb200_sizeof_serendipity() != ctypes.sizeof(Serendipity)):
         raise NativeLibraryError("recometrics_b200: %s was built from a different include/recometrics_b200.h (struct sizes differ); rebuild it" % LIB_PATH)
     lib.rmb200_last_error.restype = ctypes.c_char_p
     lib.rmb200_request_interrupt.restype = None
@@ -173,7 +200,8 @@ def load():
     for name in EXPORTS[:7]:
         getattr(lib, name).restype = ctypes.c_int
     lib.rmb200_exposure_stats.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(Exposure)]
-    for name in ("rmb200_calc_metrics_beyond_f32", "rmb200_calc_metrics_beyond_f64", "rmb200_item_popularity"):
+    for name in ("rmb200_calc_metrics_beyond_f32", "rmb200_calc_metrics_beyond_f64", "rmb200_item_popularity",
+                 "rmb200_calc_metrics_serendipity_f32", "rmb200_calc_metrics_serendipity_f64"):
         getattr(lib, name).restype = ctypes.c_int
     lib.rmb200_item_popularity.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                            ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]
@@ -241,13 +269,17 @@ def _vp(x):
 
 def calc_metrics(dtype, A, lda, B, ldb, m, n, k, trp, tri, tep, tei, tev, k_metrics, cumulative,
                  break_ties_with_noise, outs, consider_cold_start, min_items_pool, min_pos_test,
-                 nthreads=1, seed=1, item_biases=None, extra=None, exposure=None, beyond=None):
+                 nthreads=1, seed=1, item_biases=None, extra=None, exposure=None, beyond=None, serendipity=None):
     """Thin call into rmb200_calc_metrics_ex_{f32,f64} (rmb200_calc_metrics_exposure_{f32,f64} with an `exposure` struct,
-    rmb200_calc_metrics_beyond_{f32,f64} with a `beyond` struct).  Array arguments are numpy arrays (host memory), raw integer
-    addresses (device memory, with extra.inputs_on_device=1) or None.  `outs` maps metric name -> array/address/None in
-    METRIC_ORDER.  Returns the status code."""
+    rmb200_calc_metrics_beyond_{f32,f64} with a `beyond` struct, rmb200_calc_metrics_serendipity_{f32,f64} with a
+    `serendipity` struct).  Array arguments are numpy arrays (host memory), raw integer addresses (device memory, with
+    extra.inputs_on_device=1) or None.  `outs` maps metric name -> array/address/None in METRIC_ORDER.  Returns the status
+    code."""
     lib = load()
-    kind = "ex" if exposure is None and beyond is None else ("exposure" if beyond is None else "beyond")
+    if serendipity is not None:
+        kind = "serendipity"
+    else:
+        kind = "ex" if exposure is None and beyond is None else ("exposure" if beyond is None else "beyond")
     fn = getattr(lib, "rmb200_calc_metrics_%s_%s" % (kind, "f32" if np.dtype(dtype) == np.float32 else "f64"))
     args = [
         _vp(A), ctypes.c_size_t(int(lda)), _vp(B), ctypes.c_size_t(int(ldb)),
@@ -263,8 +295,10 @@ def calc_metrics(dtype, A, lda, B, ldb, m, n, k, trp, tri, tep, tei, tev, k_metr
     ]
     if kind != "ex":
         args.append(ctypes.byref(exposure) if exposure is not None else ctypes.c_void_p(None))
-    if beyond is not None:
-        args.append(ctypes.byref(beyond))
+    if kind in ("beyond", "serendipity"):
+        args.append(ctypes.byref(beyond) if beyond is not None else ctypes.c_void_p(None))
+    if serendipity is not None:
+        args.append(ctypes.byref(serendipity))
     return int(fn(*args))
 
 

@@ -28,6 +28,7 @@
 #include "filter_select.cuh"
 #include "exposure.cuh"
 #include "beyond.cuh"
+#include "history.cuh"
 #include "full_order.h"
 #include "runtime.h"
 
@@ -129,6 +130,7 @@ struct CallArgs {
     const rmb200_extra_t* ex;
     rmb200_exposure_t* expo = nullptr;   // item exposure of the ranked lists (exposure.cuh); null: not requested
     rmb200_beyond_t* bey = nullptr;      // Novelty / AvgPop / ILD of the ranked lists (beyond.cuh); null: not requested
+    rmb200_serendipity_t* ser = nullptr; // Unexpectedness / Serendipity of the ranked lists (history.cuh); null: not requested
 };
 
 template <typename T, int C, bool AUC>
@@ -351,17 +353,18 @@ struct Call {
     PhaseTimer pt{st}, pk{st};                  // phases; the dominant scoring kernel alone
     rmb200_timing_t tm;
     // the row outputs, in the order their copies leave: the 10 metrics (MetricsParams order), status, top-K items and scores,
-    // Novelty / AvgPop / ILD
-    static constexpr int RO_STATUS = 10, RO_TOPK_ITEMS = 11, RO_TOPK_SCORES = 12, RO_BEYOND = 13, ROW_OUTS = 16;
+    // Novelty / AvgPop / ILD, Unexpectedness / Serendipity
+    static constexpr int RO_STATUS = 10, RO_TOPK_ITEMS = 11, RO_TOPK_SCORES = 12, RO_BEYOND = 13, RO_HISTORY = 16, ROW_OUTS = 18;
     // ---- the plan ----
     int mip = 0, mpt = 0, C = 0, p_pad = 0, n_pad = 0, n_pad128 = 0, KB = 0, f_stages = 0, nsm = 148, UB = 0, fma_slices = 1, mean_W = 1;
     size_t rs = 1;
     T nan_value = std::numeric_limits<T>::quiet_NaN();
     bool want_roc = false, want_pr = false, count_ranks = false, want_filter_stats = false, want_exposure = false;
     bool want_pop = false, want_ild = false, want_beyond = false;   // beyond.cuh
-    int unit_pitch = 0, unit_nch = 0;           // ILD: row pitch of the unit-row image (elements), 16-byte chunks per lane
+    bool want_hist = false;                     // history.cuh
+    int unit_pitch = 0, unit_nch = 0;           // ILD / history: row pitch of the unit-row image (elements), 16-byte chunks per lane
     RowOut row_outs[ROW_OUTS];
-    MeanTable mean_tables[2];                   // the 10 metrics {10, 8}; Novelty / AvgPop / ILD {3, 3}
+    MeanTable mean_tables[3];                   // the 10 metrics {10, 8}; Novelty / AvgPop / ILD {3, 3}; Unexpectedness / Serendipity {2, 2}
     bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
     int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
     int fo_chunk = 0; size_t fo_bytes = 0;
@@ -421,12 +424,18 @@ struct Call {
             want_beyond = want_pop || want_ild;
             if (want_beyond) mean_tables[1].set(3, 3, RO_BEYOND, a.bey->means, a.bey->counts);
         }
-        if (want_ild) {            // lane l of beyond_accuracy_kernel holds 16-byte chunks l, l + 32, ... of a unit row: 1, 2, 4 or 8
+        if (a.ser) {
+            void* const ser[2] = {a.ser->unexpectedness, a.ser->serendipity};
+            for (int q = 0; q < 2; q++) row_outs[RO_HISTORY + q].set(ser[q], rs * sizeof(T), true);
+            want_hist = ser[0] || ser[1];
+            if (want_hist) mean_tables[2].set(2, 2, RO_HISTORY, a.ser->means, a.ser->counts);
+        }
+        if (want_ild || want_hist) {   // lane l of beyond_accuracy_kernel / history_distance_kernel holds 16-byte chunks l, l + 32, ... of a unit row: 1, 2, 4 or 8
             constexpr int V = 16 / (int)sizeof(T);
             unit_pitch = round_up(a.k, V);
             const int chunks = unit_pitch / V;
             unit_nch = chunks <= 32 ? 1 : chunks <= 64 ? 2 : chunks <= 128 ? 4 : chunks <= 256 ? 8 : 0;
-            if (!unit_nch) { set_err("unsupported", "ILD needs k <= 1024 (float) / 512 (double) factors"); return RMB200_ERR_UNSUPPORTED; }
+            if (!unit_nch) { set_err("unsupported", "ILD, Unexpectedness and Serendipity need k <= 1024 (float) / 512 (double) factors"); return RMB200_ERR_UNSUPPORTED; }
         }
         p_pad = round_up(a.k, KPAD);
         n_pad = round_up(a.n, BN);
@@ -574,12 +583,12 @@ struct Call {
             pt.stop(tm.h2d_ms);
             Bsrc = d_Brow.as<T>(); Bld = (size_t)a.k;
         } else { Bsrc = a.B; Bld = a.ldb; }
-        if (want_ild) TRY(unit_rows());                 // (from the complete rows: after the peer fetch, before d_Brow goes)
+        if (want_ild || want_hist) TRY(unit_rows());    // (from the complete rows: after the peer fetch, before d_Brow goes)
         if (!use_tensor || fma_counts_first) TRY(ensure_Bt());
         if (!use_tensor) { d_Brow.release(); if (!on_dev) Bsrc = nullptr; }     // the FMA path reads only the tiled copy
         return RMB200_OK;
     }
-    // ILD: the unit-row image of B, once per call
+    // ILD, Unexpectedness, Serendipity: the unit-row image of B, once per call
     int unit_rows()
     {
         CK(d_unit.alloc((size_t)a.n * unit_pitch * sizeof(T)));
@@ -779,7 +788,7 @@ struct Call {
             CK(d_expo_hist.alloc(((size_t)a.n + 1) * sizeof(unsigned)));
             CK(cudaMemsetAsync(d_expo_hist.p, 0, ((size_t)a.n + 1) * sizeof(unsigned), st));
         }
-        if (want_exposure || want_beyond) CK(d_list_len.alloc((size_t)UB * sizeof(int)));
+        if (want_exposure || want_beyond || want_hist) CK(d_list_len.alloc((size_t)UB * sizeof(int)));
         return RMB200_OK;
     }
     // upload of users [b0, b0 + UB) into staging buffer `slot`, on the prefetch stream
@@ -1053,7 +1062,7 @@ struct Call {
         mp.topk_items = rows_of<int>(RO_TOPK_ITEMS, b);
         mp.topk_scores = rows_of<T>(RO_TOPK_SCORES, b);
         mp.pos_rank = pos_rank_d;
-        mp.list_len = (want_exposure || want_beyond) ? d_list_len.as<int>() : nullptr;
+        mp.list_len = (want_exposure || want_beyond || want_hist) ? d_list_len.as<int>() : nullptr;
         TRY(wait_test_rows());
         user_metrics_kernel<T><<<(b.nb + METRICS_WARPS - 1) / METRICS_WARPS, METRICS_WARPS * 32, 0, st>>>(mp);
         TRY(launched());
@@ -1070,6 +1079,16 @@ struct Call {
             bp.nov = rows_of<T>(RO_BEYOND, b); bp.avgpop = rows_of<T>(RO_BEYOND + 1, b); bp.ild = rows_of<T>(RO_BEYOND + 2, b);
             bp.nan_value = nan_value;
             TRY(launch_beyond(bp));
+        }
+        if (want_hist) {
+            HistoryParams<T> hp;
+            hp.items = d_ci.as<int>(); hp.C = C; hp.list_len = d_list_len.as<int>();
+            hp.nb = b.nb; hp.user0 = b.b0; hp.n = a.n; hp.K = K; hp.cumulative = a.cumulative;
+            hp.trp = trp_d; hp.tri = tri_d; hp.tep = tep_d; hp.tei = tei_d;
+            hp.unit = d_unit.as<T>(); hp.pitch = unit_pitch;
+            hp.unexp = rows_of<T>(RO_HISTORY, b); hp.seren = rows_of<T>(RO_HISTORY + 1, b);
+            hp.nan_value = nan_value;
+            TRY(launch_history(hp));
         }
         const int mblocks = (b.nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
         for (const MeanTable& t : mean_tables) {
@@ -1093,6 +1112,16 @@ struct Call {
         else if (unit_nch == 2) beyond_accuracy_kernel<T, 2><<<blocks, threads, 0, st>>>(bp);
         else if (unit_nch == 4) beyond_accuracy_kernel<T, 4><<<blocks, threads, 0, st>>>(bp);
         else beyond_accuracy_kernel<T, 8><<<blocks, threads, 0, st>>>(bp);
+        return launched();
+    }
+    int launch_history(const rmb::HistoryParams<T>& hp)
+    {
+        using namespace rmb;
+        const int blocks = (hp.nb + HISTORY_WARPS - 1) / HISTORY_WARPS, threads = HISTORY_WARPS * 32;
+        if (unit_nch == 1) history_distance_kernel<T, 1><<<blocks, threads, 0, st>>>(hp);
+        else if (unit_nch == 2) history_distance_kernel<T, 2><<<blocks, threads, 0, st>>>(hp);
+        else if (unit_nch == 4) history_distance_kernel<T, 4><<<blocks, threads, 0, st>>>(hp);
+        else history_distance_kernel<T, 8><<<blocks, threads, 0, st>>>(hp);
         return launched();
     }
     // results of the batch -> caller's arrays at the shard's row offset (no gather collective: every shard writes its own
@@ -1212,6 +1241,7 @@ int run_call(const CallArgs<T>& a)
     }
     bool any_out = ex->metric_means || ex->metric_counts || ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status || a.expo;
     if (a.bey) any_out |= a.bey->novelty || a.bey->avg_popularity || a.bey->ild;
+    if (a.ser) any_out |= a.ser->unexpectedness || a.ser->serendipity;
     for (int q = 0; q < 10; q++) any_out |= (a.out[q] != nullptr);
     if (!any_out) return RMB200_OK;
     int ub = 0, ue = 0;
@@ -1350,11 +1380,13 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     const size_t W = (size_t)(a0.cumulative && a0.K > 0 ? a0.K : 1);
     DeviceMeans metric_means(ex->metric_means, ex->metric_counts, 10 * W, G);
     DeviceMeans beyond_means(a0.bey ? a0.bey->means : nullptr, a0.bey ? a0.bey->counts : nullptr, 3 * W, G);
+    DeviceMeans history_means(a0.ser ? a0.ser->means : nullptr, a0.ser ? a0.ser->counts : nullptr, 2 * W, G);
     std::vector<rmb200_extra_t> exs((size_t)G, *ex);
     std::vector<rmb200_timing_t> tms((size_t)G);
     std::vector<rmb200_exposure_t> expos((size_t)G);
     std::vector<std::vector<int64_t>> item_counts(a0.expo ? (size_t)G : 0);
     std::vector<rmb200_beyond_t> beys((size_t)G);
+    std::vector<rmb200_serendipity_t> sers((size_t)G);
     std::vector<int> rcs((size_t)G, RMB200_OK);
     std::vector<std::string> errs((size_t)G);
     std::vector<std::thread> workers;
@@ -1375,6 +1407,10 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
             beys[g] = *a0.bey;
             beyond_means.attach(g, beys[g].means, beys[g].counts);
         }
+        if (a0.ser) {
+            sers[g] = *a0.ser;
+            history_means.attach(g, sers[g].means, sers[g].counts);
+        }
         workers.emplace_back([&, g]() {
             rmb::g_err.clear();
             rmb::g_upload_share = G;
@@ -1390,6 +1426,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
                 a.ex = &exs[g]; a.mc = &mc; a.mc_rank = g;
                 if (a0.expo) a.expo = &expos[g];
                 if (a0.bey) a.bey = &beys[g];
+                if (a0.ser) a.ser = &sers[g];
                 return run_call<T>(a);
             });
             rcs[g] = rc; errs[g] = rmb::g_err;
@@ -1411,6 +1448,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
 
     metric_means.merge();
     beyond_means.merge();
+    history_means.merge();
     if (a0.expo) {          // the devices' counts added up (integers: exact), the statistics of the sum
         std::vector<int64_t> own;
         int64_t* sum = a0.expo->item_counts;
@@ -1450,11 +1488,12 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
           int32_t K, int cumulative, int noise,
           T* p, T* tp, T* r, T* ap, T* tap, T* ndcg, T* hit, T* rr, T* roc, T* pr,
           int ccs, int32_t mip, int32_t mpt, uint64_t seed, const T* bias, const rmb200_extra_t* ex, rmb200_exposure_t* expo = nullptr,
-          rmb200_beyond_t* bey = nullptr)
+          rmb200_beyond_t* bey = nullptr, rmb200_serendipity_t* ser = nullptr)
 {
     rmb::g_err.clear();
     if (expo && expo->struct_size != (int32_t)sizeof(rmb200_exposure_t)) { set_err("bad argument", "rmb200_exposure_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     if (bey && bey->struct_size != (int32_t)sizeof(rmb200_beyond_t)) { set_err("bad argument", "rmb200_beyond_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
+    if (ser && ser->struct_size != (int32_t)sizeof(rmb200_serendipity_t)) { set_err("bad argument", "rmb200_serendipity_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
     CallArgs<T> a;
     a.A = A; a.lda = lda; a.B = B; a.ldb = ldb; a.m = m; a.n = n; a.k = k;
     a.trp = trp; a.tri = tri; a.tep = tep; a.tei = tei; a.tev = tev;
@@ -1462,7 +1501,7 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
     T* outs[10] = {p, tp, r, ap, tap, ndcg, hit, rr, roc, pr};
     for (int q = 0; q < 10; q++) a.out[q] = outs[q];
     a.consider_cold_start = ccs ? 1 : 0; a.min_items_pool = mip; a.min_pos_test = mpt; a.seed = seed;
-    a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo; a.bey = bey;
+    a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo; a.bey = bey; a.ser = ser;
     return rmb::guard([&] {
         std::vector<int> devs;
         TRY(resolve_devices(a.ex, devs));
@@ -1666,6 +1705,44 @@ int rmb200_calc_metrics_beyond_f64(
 }
 
 int rmb200_sizeof_beyond(void) { return (int)sizeof(rmb200_beyond_t); }
+
+int rmb200_calc_metrics_serendipity_f32(
+    const float* A, size_t lda, const float* B, size_t ldb, int32_t m, int32_t n, int32_t k,
+    const int32_t* Xtrain_csr_p, const int32_t* Xtrain_csr_i,
+    const int32_t* Xtest_csr_p, const int32_t* Xtest_csr_i, const float* Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    float* p_at_k, float* tp_at_k, float* r_at_k, float* ap_at_k, float* tap_at_k,
+    float* ndcg_at_k, float* hit_at_k, float* rr_at_k, float* roc_auc, float* pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, int32_t nthreads, uint64_t seed,
+    const float* item_biases, const rmb200_extra_t* extra, rmb200_exposure_t* exposure, rmb200_beyond_t* beyond,
+    rmb200_serendipity_t* serendipity)
+{
+    (void)nthreads;
+    return entry<float>(A, lda, B, ldb, m, n, k, Xtrain_csr_p, Xtrain_csr_i, Xtest_csr_p, Xtest_csr_i, Xtest_csr,
+                        k_metrics, cumulative, break_ties_with_noise, p_at_k, tp_at_k, r_at_k, ap_at_k, tap_at_k,
+                        ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
+                        min_pos_test, seed, item_biases, extra, exposure, beyond, serendipity);
+}
+
+int rmb200_calc_metrics_serendipity_f64(
+    const double* A, size_t lda, const double* B, size_t ldb, int32_t m, int32_t n, int32_t k,
+    const int32_t* Xtrain_csr_p, const int32_t* Xtrain_csr_i,
+    const int32_t* Xtest_csr_p, const int32_t* Xtest_csr_i, const double* Xtest_csr,
+    int32_t k_metrics, int cumulative, int break_ties_with_noise,
+    double* p_at_k, double* tp_at_k, double* r_at_k, double* ap_at_k, double* tap_at_k,
+    double* ndcg_at_k, double* hit_at_k, double* rr_at_k, double* roc_auc, double* pr_auc,
+    int consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, int32_t nthreads, uint64_t seed,
+    const double* item_biases, const rmb200_extra_t* extra, rmb200_exposure_t* exposure, rmb200_beyond_t* beyond,
+    rmb200_serendipity_t* serendipity)
+{
+    (void)nthreads;
+    return entry<double>(A, lda, B, ldb, m, n, k, Xtrain_csr_p, Xtrain_csr_i, Xtest_csr_p, Xtest_csr_i, Xtest_csr,
+                         k_metrics, cumulative, break_ties_with_noise, p_at_k, tp_at_k, r_at_k, ap_at_k, tap_at_k,
+                         ndcg_at_k, hit_at_k, rr_at_k, roc_auc, pr_auc, consider_cold_start, min_items_pool,
+                         min_pos_test, seed, item_biases, extra, exposure, beyond, serendipity);
+}
+
+int rmb200_sizeof_serendipity(void) { return (int)sizeof(rmb200_serendipity_t); }
 
 int rmb200_item_popularity(const int32_t* indptr, const int32_t* indices, int32_t row_begin, int32_t row_end, int32_t n,
                            int32_t device, int32_t inputs_on_device, int64_t* counts)

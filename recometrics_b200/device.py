@@ -99,7 +99,7 @@ def calc_reco_metrics_device(
         consider_cold_start=True, cumulative=False, seed=1,
         user_range=None, strict_min_pos_test=False, return_topk=False, return_status=False, scoring_path="auto",
         return_means=False, means_only=False, return_exposure=False,
-        novelty=False, avg_popularity=False, diversity=False, item_popularity=None):
+        novelty=False, avg_popularity=False, diversity=False, item_popularity=None, unexpectedness=False, serendipity=False):
     """``calc_reco_metrics_ex`` for inputs that live on the GPU (see the module docstring).  Returns an
     :class:`EvalResult` whose ``metrics`` / ``status`` / ``topk_*`` / ``exposure`` entries are torch CUDA tensors on the
     device of ``A`` (``means`` / ``counts`` / ``catalogue`` are small and come back as Python numbers / numpy vectors).
@@ -170,7 +170,8 @@ def calc_reco_metrics_device(
     return _evaluate(lambda size, dt, fill: torch.empty(size, dtype=tdts[dt], device=dev) if fill is None
                      else torch.full((size,), fill, dtype=tdts[dt], device=dev), lambda t: t.data_ptr(), prep, popularity,
                      cumulative, break_ties_with_noise, user_range, return_topk, return_status, return_means, means_only,
-                     return_exposure, novelty, avg_popularity, diversity, to_numpy=lambda t: t.cpu().numpy(),
+                     return_exposure, novelty, avg_popularity, diversity, unexpectedness=unexpectedness,
+                     serendipity=serendipity, to_numpy=lambda t: t.cpu().numpy(),
                      # the library runs on its own stream: the caller's pending writes and the fills above must have landed
                      sync=lambda: torch.cuda.synchronize(dev),
                      device=device, inputs_on_device=True, strict_min_pos_test=strict_min_pos_test, scoring_path=scoring_path)

@@ -101,7 +101,9 @@ def calc_reco_metrics_sharded(X_train, X_test, A, B, k=5, group=None, dst=0, ret
     copied to that rank's GPU, B entirely.  Returns the reference-style dict on `dst` (None elsewhere).
     ``return_exposure``: returns ``(dict, item_counts, catalogue)`` on `dst` instead, the ranks' item exposure summed by
     :func:`reduce_exposure`.  ``novelty`` / ``avg_popularity`` without ``item_popularity``: every rank counts its block's
-    ``X_train`` rows and :func:`reduce_popularity` adds them up, so the rows equal those of one call over all users."""
+    ``X_train`` rows and :func:`reduce_popularity` adds them up, so the rows equal those of one call over all users.
+    ``unexpectedness`` / ``serendipity`` (see :func:`calc_reco_metrics_ex`) pass through ``kwargs`` as they are: a user's
+    values read only that user's own ``X_train`` and ``X_test`` rows, so the ranks' rows need no reduction step."""
     import torch.distributed as dist
 
     world = dist.get_world_size(group)

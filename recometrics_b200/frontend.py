@@ -128,12 +128,13 @@ def item_popularity(X_train, m=None, user_range=None, device=-1):
 
 
 class _ResultRows:
-    """The per-user rows of one call -- the requested metrics and Novelty / AvgPop / ILD rows, NaN outside ``user_range`` --
-    and their means / counts tables, allocated with ``alloc(size, dtype, fill)`` (numpy or torch; ``fill=None``: left
-    uninitialised).  A table is ``[slot][W]``, ``W = K`` when ``cumulative`` else 1, over its rows in order: the ten metrics
-    (the first eight W wide, ROC / PR-AUC one value each), and the three beyond-accuracy rows (all W wide)."""
+    """The per-user rows of one call -- the requested metrics, Novelty / AvgPop / ILD and Unexpectedness / Serendipity rows,
+    NaN outside ``user_range`` -- and their means / counts tables, allocated with ``alloc(size, dtype, fill)`` (numpy or
+    torch; ``fill=None``: left uninitialised).  A table is ``[slot][W]``, ``W = K`` when ``cumulative`` else 1, over its rows
+    in order: the ten metrics (the first eight W wide, ROC / PR-AUC one value each), the three beyond-accuracy rows and the
+    two history rows (all W wide)."""
 
-    def __init__(self, alloc, dtype, m, K, cumulative, flags, bflags, user_range, return_means):
+    def __init__(self, alloc, dtype, m, K, cumulative, flags, bflags, sflags, user_range, return_means):
         self.m, self.K, self.W, self.cumulative = m, K, (K if cumulative else 1), cumulative
         fill = None if user_range is None else np.nan
 
@@ -143,6 +144,8 @@ class _ResultRows:
         self.means, self.counts = table(10, return_means)
         self.brows = {name: alloc(m * self.W, dtype, fill) for name, _ in _capi.BEYOND_KEYS if bflags[name]}
         self.bmeans, self.bcounts = table(3, return_means and bool(self.brows))
+        self.srows = {name: alloc(m * self.W, dtype, fill) for name, _ in _capi.SERENDIPITY_KEYS if sflags[name]}
+        self.smeans, self.scounts = table(2, return_means and bool(self.srows))
 
     def unpack(self, means_only, to_numpy=lambda x: x):
         """``metrics`` (W wide rows as ``(m, K)``, ``"K"`` last), ``means`` and ``counts`` of the call's EvalResult;
@@ -150,7 +153,8 @@ class _ResultRows:
         metrics, W = {}, self.W
         mean_d, count_d = ({}, {}) if self.means is not None else (None, None)
         for rows, keys, wide_slots, means, counts in ((self.outs, _KEYS, 8, self.means, self.counts),
-                                                      (self.brows, _capi.BEYOND_KEYS, 3, self.bmeans, self.bcounts)):
+                                                      (self.brows, _capi.BEYOND_KEYS, 3, self.bmeans, self.bcounts),
+                                                      (self.srows, _capi.SERENDIPITY_KEYS, 2, self.smeans, self.scounts)):
             if means is not None:
                 means, counts = to_numpy(means), to_numpy(counts)
             for i, (name, key) in enumerate(keys):
@@ -302,8 +306,8 @@ def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, min_pos_test, m
 
 
 def _evaluate(alloc, addr, prep, popularity, cumulative, break_ties_with_noise, user_range, return_topk, return_status,
-              return_means, means_only, return_exposure, novelty, avg_popularity, diversity, return_ranks=False,
-              to_numpy=lambda x: x, sync=lambda: None, **extra):
+              return_means, means_only, return_exposure, novelty, avg_popularity, diversity, unexpectedness=False,
+              serendipity=False, return_ranks=False, to_numpy=lambda x: x, sync=lambda: None, **extra):
     """The evaluation call both front-ends end in, on the inputs ``prep`` they validated (``_validate_and_prepare``'s keys:
     host arrays or device addresses, as ``_capi.calc_metrics`` takes them).  The result rows and the asked-for extras are
     allocated with ``alloc(size, dtype, fill)`` (see :class:`_ResultRows`) and handed to the library as ``addr(array)``;
@@ -312,7 +316,9 @@ def _evaluate(alloc, addr, prep, popularity, cumulative, break_ties_with_noise, 
     dtype, m, n, K, cumulative = prep["dtype"], prep["m"], prep["n"], prep["k"], bool(cumulative)
     ptr = lambda x: None if x is None else addr(x)
     bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
-    res = _ResultRows(alloc, dtype, m, K, cumulative, prep["flags"], bflags, user_range, bool(return_means) or bool(means_only))
+    sflags = dict(unexpectedness=bool(unexpectedness), serendipity=bool(serendipity))
+    res = _ResultRows(alloc, dtype, m, K, cumulative, prep["flags"], bflags, sflags, user_range,
+                      bool(return_means) or bool(means_only))
     timing = _capi.Timing()
     status = alloc(m, np.int32, 0) if return_status else None
     topk_items = alloc(m * K, np.int32, -1) if return_topk else None
@@ -329,12 +335,14 @@ def _evaluate(alloc, addr, prep, popularity, cumulative, break_ties_with_noise, 
     pop = popularity() if bflags["novelty"] or bflags["avg_popularity"] else None
     bey = _capi.make_beyond({name: addr(r) for name, r in res.brows.items()}, ptr(pop), m, ptr(res.bmeans),
                             ptr(res.bcounts)) if res.brows else None
+    ser = _capi.make_serendipity({name: addr(r) for name, r in res.srows.items()}, ptr(res.smeans),
+                                 ptr(res.scounts)) if res.srows else None
     sync()
     rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, n, prep["p"],
                             prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
                             bool(break_ties_with_noise), {q: addr(r) for q, r in res.outs.items()}, prep["consider_cold_start"],
                             prep["min_items_pool"], prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"],
-                            ex, exposure=expo, beyond=bey)
+                            ex, exposure=expo, beyond=bey, serendipity=ser)
     _capi.raise_for_status(rc)
 
     metrics, mean_d, count_d = res.unpack(means_only, to_numpy)
@@ -354,7 +362,7 @@ def calc_reco_metrics_ex(
         device=-1, user_range=None, strict_min_pos_test=False,
         return_topk=False, return_ranks=False, return_status=False, scoring_path="auto",
         return_means=False, means_only=False, filter_stats=False, nan_bits=None, devices=None, return_exposure=False,
-        novelty=False, avg_popularity=False, diversity=False, item_popularity=None):
+        novelty=False, avg_popularity=False, diversity=False, item_popularity=None, unexpectedness=False, serendipity=False):
     """Same evaluation as :func:`calc_reco_metrics`, returning an :class:`EvalResult` with the
     reference-style dict plus timing and the optional extras (top-K ids/scores, held-out ranks,
     per-user status).  ``user_range=(begin, end)`` evaluates only those rows (the sharding unit);
@@ -374,7 +382,14 @@ def calc_reco_metrics_ex(
     ``result.metrics["Novelty@K"]``, ``["AvgPop@K"]``, ``["ILD@K"]`` (``(m,)``, ``(m, k)`` when ``cumulative``) and, with
     ``return_means``, their means and counts under the same keys; NaN for users without a list.  ``item_popularity``: int64
     ``[n]`` counts of how many of the m users have each item in ``X_train`` (see :func:`item_popularity`, which computes it
-    when it is not given).  ``all_metrics`` does not turn these on."""
+    when it is not given).  ``unexpectedness`` / ``serendipity``: per-user Unexpectedness@K and Serendipity@K of the ranked
+    lists against each user's ``X_train`` row, computed on the device -- with ``sim_r`` the mean cosine similarity of the
+    r-th listed item's row of ``B`` to the rows of the user's training items, Unexpectedness@K is the mean of ``1 - sim_r``
+    over the list and Serendipity@K the mean of ``rel_r * (1 - sim_r)``, ``rel_r = 1`` when the item is in the user's
+    ``X_test`` row (Microsoft Recommenders' ``user_serendipity`` with held-out relevance); rows
+    ``result.metrics["Unexpectedness@K"]`` and ``["Serendipity@K"]``, shaped and reduced like the rows above; NaN for users
+    without a list or without a training item (cold-start users, and every user when ``X_train`` is None).  ``all_metrics``
+    does not turn these on."""
     prep = _validate_and_prepare(X_train, X_test, A, B, k, item_biases, min_pos_test, min_items_pool, consider_cold_start,
                                  nthreads, seed, all_metrics, precision, trunc_precision, recall, average_precision,
                                  trunc_average_precision, ndcg, hit, rr, roc_auc, pr_auc)
@@ -388,7 +403,8 @@ def calc_reco_metrics_ex(
         return pop
     return _evaluate(lambda size, dt, fill: np.empty(size, dt) if fill is None else np.full(size, fill, dt), lambda x: x,
                      prep, popularity, cumulative, break_ties_with_noise, user_range, return_topk, return_status,
-                     return_means, means_only, return_exposure, novelty, avg_popularity, diversity, return_ranks=return_ranks,
+                     return_means, means_only, return_exposure, novelty, avg_popularity, diversity,
+                     unexpectedness=unexpectedness, serendipity=serendipity, return_ranks=return_ranks,
                      device=device, strict_min_pos_test=strict_min_pos_test, scoring_path=scoring_path,
                      filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
 
