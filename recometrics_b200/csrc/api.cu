@@ -20,6 +20,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "metrics.cuh"
@@ -116,6 +117,28 @@ struct MultiCtx {
     }
 };
 
+// The per-user row outputs of a call, in the order their copies leave: the 10 metrics (MetricsParams order), status, top-K
+// items and scores, Novelty / AvgPop / ILD (beyond.cuh), Unexpectedness / Serendipity (history.cuh)
+constexpr int RO_STATUS = 10, RO_TOPK_ITEMS = 11, RO_TOPK_SCORES = 12, RO_BEYOND = 13, RO_HISTORY = 16, ROW_OUTS = 18, MEAN_TABLES = 3;
+// Per row output: columns (rs = K when cumulative else 1, 1 or K), element (T or int), left on the device by skip_row_copy
+enum RowCols { COLS_RS, COLS_1, COLS_K };
+struct RowShape { RowCols cols; bool is_int, skippable; };
+constexpr RowShape WIDE_T{COLS_RS, false, true}, ONE_T{COLS_1, false, true};
+constexpr RowShape ROW_SHAPES[ROW_OUTS] = {WIDE_T, WIDE_T, WIDE_T, WIDE_T, WIDE_T, WIDE_T, WIDE_T, WIDE_T, ONE_T, ONE_T,
+    {COLS_1, true, false}, {COLS_K, true, false}, {COLS_K, false, false}, WIDE_T, WIDE_T, WIDE_T, WIDE_T, WIDE_T};
+// The means / counts tables of a call (MeanTable): the 10 metrics, Novelty / AvgPop / ILD, Unexpectedness / Serendipity
+struct TableShape { int slots, wide, first_row; };
+constexpr TableShape MEAN_SHAPES[MEAN_TABLES] = {{10, 8, 0}, {3, 3, RO_BEYOND}, {2, 2, RO_HISTORY}};
+
+// What a call writes, decoded once by entry() from the metric arguments, rmb200_extra_t and the optional structs
+struct Outputs {
+    void* rows[ROW_OUTS] = {};                  // the caller's rows (host or device); null: not requested
+    double* means[MEAN_TABLES] = {}; int64_t* counts[MEAN_TABLES] = {};   // the caller's tables; both null: the table is off
+    int64_t* pos_rank = nullptr;                // [nnz_test]: rank of every held-out item; null: not requested
+    const int64_t* item_popularity = nullptr; int64_t popularity_users = 0;   // Novelty / AvgPop: the counts [n] and their U
+    rmb200_exposure_t* expo = nullptr;          // item exposure of the ranked lists (exposure.cuh); null: not requested
+};
+
 template <typename T>
 struct CallArgs {
     MultiCtx* mc = nullptr; int mc_rank = 0;
@@ -123,14 +146,11 @@ struct CallArgs {
     int m, n, k;
     const int32_t *trp, *tri, *tep, *tei; const T* tev;
     int K, cumulative, noise;
-    T* out[10];   // p tp r ap tap ndcg hit rr roc pr
     int consider_cold_start, min_items_pool, min_pos_test;
     uint64_t seed;
     const T* bias;
     const rmb200_extra_t* ex;
-    rmb200_exposure_t* expo = nullptr;   // item exposure of the ranked lists (exposure.cuh); null: not requested
-    rmb200_beyond_t* bey = nullptr;      // Novelty / AvgPop / ILD of the ranked lists (beyond.cuh); null: not requested
-    rmb200_serendipity_t* ser = nullptr; // Unexpectedness / Serendipity of the ranked lists (history.cuh); null: not requested
+    Outputs outs;
 };
 
 template <typename T, int C, bool AUC>
@@ -317,9 +337,7 @@ int exposure_of_nobody(rmb200_exposure_t* expo, int n, bool counts_on_device)
 struct RowOut {
     void* base = nullptr;
     size_t row_bytes = 0;
-    bool skippable = false;                     // left on the device by rmb200_extra_t::skip_row_copy (metric and beyond rows)
     DevBuf staged[2];
-    void set(void* p, size_t bytes, bool skip) { base = p; row_bytes = bytes; skippable = skip; }
 };
 
 // One [slots][W] table of means / counts over the users of a call (the first `wide` slots have W columns, the others one):
@@ -330,7 +348,7 @@ struct MeanTable {
     DevBuf part_sum, part_cnt;                  // per 256 users of every batch (metric_partial_kernel), added up in order at the end
     DevBuf d_means, d_counts;                   // the final values of host outputs
     bool on() const { return means || counts; }
-    void set(int s, int w, int row0, double* m, int64_t* c) { slots = s; wide = w; first_row = row0; means = m; counts = reinterpret_cast<long long*>(c); }
+    void set(const TableShape& s, double* m, int64_t* c) { slots = s.slots; wide = s.wide; first_row = s.first_row; means = m; counts = reinterpret_cast<long long*>(c); }
 };
 
 // One evaluation call on one device.  plan() makes every decision that needs only the arguments and the device; the resident
@@ -352,19 +370,15 @@ struct Call {
     cudaStream_t st = nullptr;                  // legacy default stream: ordered after the caller's default-stream work
     PhaseTimer pt{st}, pk{st};                  // phases; the dominant scoring kernel alone
     rmb200_timing_t tm;
-    // the row outputs, in the order their copies leave: the 10 metrics (MetricsParams order), status, top-K items and scores,
-    // Novelty / AvgPop / ILD, Unexpectedness / Serendipity
-    static constexpr int RO_STATUS = 10, RO_TOPK_ITEMS = 11, RO_TOPK_SCORES = 12, RO_BEYOND = 13, RO_HISTORY = 16, ROW_OUTS = 18;
     // ---- the plan ----
     int mip = 0, mpt = 0, C = 0, p_pad = 0, n_pad = 0, n_pad128 = 0, KB = 0, f_stages = 0, nsm = 148, UB = 0, fma_slices = 1, mean_W = 1;
     size_t rs = 1;
     T nan_value = std::numeric_limits<T>::quiet_NaN();
     bool want_roc = false, want_pr = false, count_ranks = false, want_filter_stats = false, want_exposure = false;
-    bool want_pop = false, want_ild = false, want_beyond = false;   // beyond.cuh
-    bool want_hist = false;                     // history.cuh
+    bool want_pop = false, want_ild = false, want_beyond = false, want_hist = false;   // beyond.cuh, history.cuh
     int unit_pitch = 0, unit_nch = 0;           // ILD / history: row pitch of the unit-row image (elements), 16-byte chunks per lane
     RowOut row_outs[ROW_OUTS];
-    MeanTable mean_tables[3];                   // the 10 metrics {10, 8}; Novelty / AvgPop / ILD {3, 3}; Unexpectedness / Serendipity {2, 2}
+    MeanTable mean_tables[MEAN_TABLES];
     bool use_full = false, use_tensor = false, fma_counts_first = false, noise_handback = false;
     int f_sample_tiles = 0, f_sample_stride = 1, f_sample_rank = 0;
     int fo_chunk = 0; size_t fo_bytes = 0;
@@ -405,31 +419,21 @@ struct Call {
         // candidate buffer: K kept + 128 appended per tile + head-room between two cuts (the tensor-core filter keeps
         // the slack band below the K-th best as well: about 2.5 K entries on Gaussian scores, so it gets more room)
         C = (K <= 64) ? 256 : (K <= 192 ? 512 : 1024);
-        want_roc = a.out[8] != nullptr; want_pr = a.out[9] != nullptr;
-        count_ranks = want_roc || want_pr || ex->pos_rank;
+        want_roc = a.outs.rows[8] != nullptr; want_pr = a.outs.rows[9] != nullptr;
+        count_ranks = want_roc || want_pr || a.outs.pos_rank;
         want_filter_stats = ex->filter_stats != 0;
-        want_exposure = a.expo != nullptr;
+        want_exposure = a.outs.expo != nullptr;
         rs = a.cumulative ? (size_t)K : 1;
         mean_W = a.cumulative ? K : 1;
-        for (int q = 0; q < 10; q++) row_outs[q].set(a.out[q], (q < 8 ? rs : 1) * sizeof(T), true);
-        row_outs[RO_STATUS].set(ex->status, sizeof(int), false);
-        row_outs[RO_TOPK_ITEMS].set(ex->topk_items, (size_t)K * sizeof(int), false);
-        row_outs[RO_TOPK_SCORES].set(ex->topk_scores, (size_t)K * sizeof(T), false);
-        mean_tables[0].set(10, 8, 0, ex->metric_means, ex->metric_counts);
-        if (a.bey) {
-            void* const bey[3] = {a.bey->novelty, a.bey->avg_popularity, a.bey->ild};
-            for (int q = 0; q < 3; q++) row_outs[RO_BEYOND + q].set(bey[q], rs * sizeof(T), true);
-            want_pop = bey[0] || bey[1];
-            want_ild = bey[2] != nullptr;
-            want_beyond = want_pop || want_ild;
-            if (want_beyond) mean_tables[1].set(3, 3, RO_BEYOND, a.bey->means, a.bey->counts);
+        for (int i = 0; i < ROW_OUTS; i++) {
+            const RowShape& s = ROW_SHAPES[i];
+            row_outs[i].base = a.outs.rows[i];
+            row_outs[i].row_bytes = (s.cols == COLS_RS ? rs : s.cols == COLS_K ? (size_t)K : 1) * (s.is_int ? sizeof(int) : sizeof(T));
         }
-        if (a.ser) {
-            void* const ser[2] = {a.ser->unexpectedness, a.ser->serendipity};
-            for (int q = 0; q < 2; q++) row_outs[RO_HISTORY + q].set(ser[q], rs * sizeof(T), true);
-            want_hist = ser[0] || ser[1];
-            if (want_hist) mean_tables[2].set(2, 2, RO_HISTORY, a.ser->means, a.ser->counts);
-        }
+        for (int t = 0; t < MEAN_TABLES; t++) mean_tables[t].set(MEAN_SHAPES[t], a.outs.means[t], a.outs.counts[t]);
+        want_pop = row_outs[RO_BEYOND].base || row_outs[RO_BEYOND + 1].base;
+        want_ild = row_outs[RO_BEYOND + 2].base != nullptr; want_beyond = want_pop || want_ild;
+        want_hist = row_outs[RO_HISTORY].base || row_outs[RO_HISTORY + 1].base;
         if (want_ild || want_hist) {   // lane l of beyond_accuracy_kernel / history_distance_kernel holds 16-byte chunks l, l + 32, ... of a unit row: 1, 2, 4 or 8
             constexpr int V = 16 / (int)sizeof(T);
             unit_pitch = round_up(a.k, V);
@@ -603,11 +607,11 @@ struct Call {
     int popularity_table()
     {
         if (!want_pop) return RMB200_OK;
-        pop_d = reinterpret_cast<const long long*>(a.bey->item_popularity);
+        pop_d = reinterpret_cast<const long long*>(a.outs.item_popularity);
         if (!on_dev) {
             CK(d_pop.alloc((size_t)a.n * sizeof(long long)));
             pt.start();
-            CK(cudaMemcpyAsync(d_pop.p, a.bey->item_popularity, (size_t)a.n * sizeof(long long), cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(d_pop.p, a.outs.item_popularity, (size_t)a.n * sizeof(long long), cudaMemcpyHostToDevice, st));
             tm.h2d_bytes += (int64_t)a.n * (int64_t)sizeof(long long);
             pt.stop(tm.h2d_ms);
             pop_d = d_pop.as<long long>();
@@ -617,7 +621,7 @@ struct Call {
         pt.start();
         CK(cudaMemsetAsync(d_pop_bad.p, 0, sizeof(int), st));
         rmb::popularity_table_kernel<<<(a.n + 255) / 256 < 4 * nsm ? (a.n + 255) / 256 : 4 * nsm, 256, 0, st>>>(
-            pop_d, a.n, (long long)a.bey->popularity_users, d_poptab.as<double2>(), d_pop_bad.as<int>());
+            pop_d, a.n, (long long)a.outs.popularity_users, d_poptab.as<double2>(), d_pop_bad.as<int>());
         TRY(launched());
         int bad = 0;
         CK(cudaMemcpyAsync(&bad, d_pop_bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -723,8 +727,8 @@ struct Call {
             CK(cudaMemsetAsync(d_pos_perm.p, 0, nnz_te * sizeof(int) + (nnz_te ? 0 : 16), st));
             CK(cudaMemsetAsync(d_pos_item.p, 0, nnz_te * sizeof(int) + (nnz_te ? 0 : 16), st));
         }
-        if (ex->pos_rank) {
-            if (on_dev) pos_rank_d = reinterpret_cast<long long*>(ex->pos_rank) + lo_hi[2];
+        if (a.outs.pos_rank) {
+            if (on_dev) pos_rank_d = reinterpret_cast<long long*>(a.outs.pos_rank) + lo_hi[2];
             else { CK(d_pos_rank.alloc(nnz_te * sizeof(long long))); pos_rank_d = d_pos_rank.as<long long>(); }
             CK(cudaMemsetAsync(pos_rank_d, 0, nnz_te * sizeof(long long), st));
         }
@@ -735,8 +739,8 @@ struct Call {
         pt.start();
         StatusParams sp;
         sp.trp = trp_d; sp.tep = tep_d; sp.n = a.n; sp.K = K; sp.user_begin = 0; sp.user_end = mr;
-        sp.has_ndcg = a.out[5] != nullptr;
-        sp.has_rescue = (a.out[8] || a.out[9] || a.out[3] || a.out[4] || a.out[7]) ? 1 : 0;   // hpp:485
+        sp.has_ndcg = a.outs.rows[5] != nullptr;
+        sp.has_rescue = (a.outs.rows[8] || a.outs.rows[9] || a.outs.rows[3] || a.outs.rows[4] || a.outs.rows[7]) ? 1 : 0;   // hpp:485
         sp.consider_cold_start = a.consider_cold_start; sp.min_items_pool = mip; sp.min_pos_test = mpt;
         sp.ustatus = d_status.as<int>(); sp.uflags = d_flags.as<int>();
         sp.umin = count_ranks ? d_umin.as<unsigned long long>() : nullptr;
@@ -1078,7 +1082,7 @@ struct Call {
             bp.unit = want_ild ? d_unit.as<T>() : nullptr; bp.pitch = unit_pitch;
             bp.nov = rows_of<T>(RO_BEYOND, b); bp.avgpop = rows_of<T>(RO_BEYOND + 1, b); bp.ild = rows_of<T>(RO_BEYOND + 2, b);
             bp.nan_value = nan_value;
-            TRY(launch_beyond(bp));
+            TRY(unit_launch([&](auto nch) { beyond_accuracy_kernel<T, nch><<<(b.nb + BEYOND_WARPS - 1) / BEYOND_WARPS, BEYOND_WARPS * 32, 0, st>>>(bp); }));
         }
         if (want_hist) {
             HistoryParams<T> hp;
@@ -1088,7 +1092,7 @@ struct Call {
             hp.unit = d_unit.as<T>(); hp.pitch = unit_pitch;
             hp.unexp = rows_of<T>(RO_HISTORY, b); hp.seren = rows_of<T>(RO_HISTORY + 1, b);
             hp.nan_value = nan_value;
-            TRY(launch_history(hp));
+            TRY(unit_launch([&](auto nch) { history_distance_kernel<T, nch><<<(b.nb + HISTORY_WARPS - 1) / HISTORY_WARPS, HISTORY_WARPS * 32, 0, st>>>(hp); }));
         }
         const int mblocks = (b.nb + MEAN_CHUNK - 1) / MEAN_CHUNK;
         for (const MeanTable& t : mean_tables) {
@@ -1104,24 +1108,13 @@ struct Call {
         pt.stop(tm.metrics_ms);
         return RMB200_OK;
     }
-    int launch_beyond(const rmb::BeyondParams<T>& bp)
+    // beyond_accuracy_kernel / history_distance_kernel<T, NCH>: NCH = unit_nch chunks per lane of a unit row (0, none: 1)
+    template <typename Launch> int unit_launch(Launch launch)
     {
-        using namespace rmb;
-        const int blocks = (bp.nb + BEYOND_WARPS - 1) / BEYOND_WARPS, threads = BEYOND_WARPS * 32;
-        if (unit_nch <= 1) beyond_accuracy_kernel<T, 1><<<blocks, threads, 0, st>>>(bp);      // (also: no ILD)
-        else if (unit_nch == 2) beyond_accuracy_kernel<T, 2><<<blocks, threads, 0, st>>>(bp);
-        else if (unit_nch == 4) beyond_accuracy_kernel<T, 4><<<blocks, threads, 0, st>>>(bp);
-        else beyond_accuracy_kernel<T, 8><<<blocks, threads, 0, st>>>(bp);
-        return launched();
-    }
-    int launch_history(const rmb::HistoryParams<T>& hp)
-    {
-        using namespace rmb;
-        const int blocks = (hp.nb + HISTORY_WARPS - 1) / HISTORY_WARPS, threads = HISTORY_WARPS * 32;
-        if (unit_nch == 1) history_distance_kernel<T, 1><<<blocks, threads, 0, st>>>(hp);
-        else if (unit_nch == 2) history_distance_kernel<T, 2><<<blocks, threads, 0, st>>>(hp);
-        else if (unit_nch == 4) history_distance_kernel<T, 4><<<blocks, threads, 0, st>>>(hp);
-        else history_distance_kernel<T, 8><<<blocks, threads, 0, st>>>(hp);
+        if (unit_nch <= 1) launch(std::integral_constant<int, 1>());
+        else if (unit_nch == 2) launch(std::integral_constant<int, 2>());
+        else if (unit_nch == 4) launch(std::integral_constant<int, 4>());
+        else launch(std::integral_constant<int, 8>());
         return launched();
     }
     // results of the batch -> caller's arrays at the shard's row offset (no gather collective: every shard writes its own
@@ -1132,8 +1125,9 @@ struct Call {
         const size_t row = (size_t)(ub + b.b0), nb = (size_t)b.nb;
         CK(cudaEventRecord(rsx.ready[b.slot], st));
         CK(cudaStreamWaitEvent(rsx.s, rsx.ready[b.slot], 0));
-        for (const RowOut& r : row_outs) {
-            if (!r.base || (r.skippable && ex->skip_row_copy)) continue;
+        for (int i = 0; i < ROW_OUTS; i++) {
+            const RowOut& r = row_outs[i];
+            if (!r.base || (ROW_SHAPES[i].skippable && ex->skip_row_copy)) continue;
             const size_t bytes = nb * r.row_bytes;
             CK(cudaMemcpyAsync(static_cast<unsigned char*>(r.base) + row * r.row_bytes, r.staged[b.slot].p, bytes, cudaMemcpyDeviceToHost, rsx.s));
             tm.d2h_bytes += (int64_t)bytes;
@@ -1150,9 +1144,9 @@ struct Call {
             CK(cudaStreamSynchronize(rsx.s));
             tm.d2h_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_d).count();
         }
-        if (!on_dev && ex->pos_rank && !g_interrupt.load()) {
+        if (!on_dev && a.outs.pos_rank && !g_interrupt.load()) {
             pt.start();
-            CK(cudaMemcpyAsync(ex->pos_rank + lo_hi[2], pos_rank_d, nnz_te * sizeof(long long), cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(a.outs.pos_rank + lo_hi[2], pos_rank_d, nnz_te * sizeof(long long), cudaMemcpyDeviceToHost, st));
             tm.d2h_bytes += (int64_t)(nnz_te * sizeof(long long));
             pt.stop(tm.d2h_ms);
         }
@@ -1191,7 +1185,7 @@ struct Call {
     // the statistics) or an internal one; the statistics from them on the host
     int exposure_out()
     {
-        int64_t* dst_d = on_dev ? a.expo->item_counts : nullptr;
+        int64_t* dst_d = on_dev ? a.outs.expo->item_counts : nullptr;
         if (!dst_d) { CK(d_expo_counts.alloc((size_t)a.n * sizeof(int64_t))); dst_d = d_expo_counts.as<int64_t>(); }
         pt.start();
         rmb::exposure_widen_kernel<<<(a.n + 255) / 256 < 4 * nsm ? (a.n + 255) / 256 : 4 * nsm, 256, 0, st>>>(
@@ -1199,7 +1193,7 @@ struct Call {
         TRY(launched());
         pt.stop(tm.metrics_ms);
         std::vector<int64_t> own;
-        int64_t* dst_h = on_dev ? nullptr : a.expo->item_counts;
+        int64_t* dst_h = on_dev ? nullptr : a.outs.expo->item_counts;
         if (!dst_h) { own.resize((size_t)a.n); dst_h = own.data(); }
         unsigned users = 0;
         pt.start();
@@ -1207,8 +1201,8 @@ struct Call {
         CK(cudaMemcpyAsync(&users, d_expo_hist.as<unsigned>() + a.n, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
         tm.d2h_bytes += (int64_t)a.n * (int64_t)sizeof(int64_t) + (int64_t)sizeof(unsigned);
         pt.stop(tm.d2h_ms);   // (synchronises)
-        a.expo->users = (int64_t)users;
-        return exposure_stats(dst_h, a.n, a.expo);
+        a.outs.expo->users = (int64_t)users;
+        return exposure_stats(dst_h, a.n, a.outs.expo);
     }
 };
 
@@ -1224,33 +1218,33 @@ int run_call(const CallArgs<T>& a)
 {
     const auto t_begin = std::chrono::steady_clock::now();
     const rmb200_extra_t* ex = a.ex;
+    const Outputs& o = a.outs;
     // ---- argument checks (shape errors are the binding's job in the reference,
     //      recometrics/wrapper.pyx:261-268; here they become RMB200_ERR_BAD_ARG) ----
     if (a.m <= 0 || a.n <= 0 || a.k <= 0 || a.K <= 0) { set_err("bad argument", "m, n, k and k_metrics must be positive"); return RMB200_ERR_BAD_ARG; }
     if (!a.A || !a.B || !a.trp || !a.tep) { set_err("bad argument", "A, B, Xtrain_csr_p and Xtest_csr_p are required"); return RMB200_ERR_BAD_ARG; }
     if (a.lda < (size_t)a.k || a.ldb < (size_t)a.k) { set_err("bad argument", "lda/ldb smaller than k"); return RMB200_ERR_BAD_ARG; }
-    if (a.out[5] && !a.tev) { set_err("bad argument", "NDCG requested but Xtest_csr (values) is NULL"); return RMB200_ERR_BAD_ARG; }
+    if (o.rows[5] && !a.tev) { set_err("bad argument", "NDCG requested but Xtest_csr (values) is NULL"); return RMB200_ERR_BAD_ARG; }
     if (ex->struct_size != (int32_t)sizeof(rmb200_extra_t)) { set_err("bad argument", "rmb200_extra_t::struct_size mismatch"); return RMB200_ERR_BAD_ARG; }
-    if (a.bey && (a.bey->novelty || a.bey->avg_popularity)) {
-        const int64_t U = a.bey->popularity_users;
-        if (!a.bey->item_popularity) { set_err("bad argument", "Novelty / AvgPop requested but item_popularity is NULL"); return RMB200_ERR_BAD_ARG; }
+    if (o.rows[RO_BEYOND] || o.rows[RO_BEYOND + 1]) {
+        const int64_t U = o.popularity_users;
+        if (!o.item_popularity) { set_err("bad argument", "Novelty / AvgPop requested but item_popularity is NULL"); return RMB200_ERR_BAD_ARG; }
         if (U < 1) { set_err("bad argument", "popularity_users must be >= 1"); return RMB200_ERR_BAD_ARG; }
         if (!ex->inputs_on_device)            // (device-resident counts are checked on the device, before the first batch)
             for (int j = 0; j < a.n; j++)
-                if (a.bey->item_popularity[j] < 0 || a.bey->item_popularity[j] > U) { set_err("bad argument", "item_popularity: a count outside [0, popularity_users]"); return RMB200_ERR_BAD_ARG; }
+                if (o.item_popularity[j] < 0 || o.item_popularity[j] > U) { set_err("bad argument", "item_popularity: a count outside [0, popularity_users]"); return RMB200_ERR_BAD_ARG; }
     }
-    bool any_out = ex->metric_means || ex->metric_counts || ex->topk_items || ex->topk_scores || ex->pos_rank || ex->status || a.expo;
-    if (a.bey) any_out |= a.bey->novelty || a.bey->avg_popularity || a.bey->ild;
-    if (a.ser) any_out |= a.ser->unexpectedness || a.ser->serendipity;
-    for (int q = 0; q < 10; q++) any_out |= (a.out[q] != nullptr);
+    bool any_out = o.pos_rank || o.expo;
+    for (void* r : o.rows) any_out |= r != nullptr;
+    for (int t = 0; t < MEAN_TABLES; t++) any_out |= o.means[t] || o.counts[t];
     if (!any_out) return RMB200_OK;
     int ub = 0, ue = 0;
     TRY(user_range(ex, a.m, &ub, &ue));
-    if (ue == ub && !a.expo) return RMB200_OK;
+    if (ue == ub && !o.expo) return RMB200_OK;
 
     int dev = 0;
     TRY(rmb::use_device(requested_device(ex->device), &dev));
-    if (ue == ub) return exposure_of_nobody(a.expo, a.n, ex->inputs_on_device != 0);
+    if (ue == ub) return exposure_of_nobody(o.expo, a.n, ex->inputs_on_device != 0);
 
     const bool nested = a.mc != nullptr;                   // run_multi() holds the mutex and the latch
     std::unique_lock<std::mutex> lock(rmb::g_call_mutex, std::defer_lock);
@@ -1371,22 +1365,21 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
         }
     }
     const int G = (int)devs.size();
-    if (G == 0) return a0.expo ? exposure_of_nobody(a0.expo, a0.n, false) : RMB200_OK;
+    if (G == 0) return a0.outs.expo ? exposure_of_nobody(a0.outs.expo, a0.n, false) : RMB200_OK;
 
     std::unique_lock<std::mutex> lock(rmb::g_call_mutex);
     SignalLatch latch;
     MultiCtx mc;
     mc.G = G;
     const size_t W = (size_t)(a0.cumulative && a0.K > 0 ? a0.K : 1);
-    DeviceMeans metric_means(ex->metric_means, ex->metric_counts, 10 * W, G);
-    DeviceMeans beyond_means(a0.bey ? a0.bey->means : nullptr, a0.bey ? a0.bey->counts : nullptr, 3 * W, G);
-    DeviceMeans history_means(a0.ser ? a0.ser->means : nullptr, a0.ser ? a0.ser->counts : nullptr, 2 * W, G);
+    std::vector<DeviceMeans> tables;
+    for (int t = 0; t < MEAN_TABLES; t++) tables.emplace_back(a0.outs.means[t], a0.outs.counts[t], MEAN_SHAPES[t].slots * W, G);
     std::vector<rmb200_extra_t> exs((size_t)G, *ex);
     std::vector<rmb200_timing_t> tms((size_t)G);
-    std::vector<rmb200_exposure_t> expos((size_t)G);
-    std::vector<std::vector<int64_t>> item_counts(a0.expo ? (size_t)G : 0);
-    std::vector<rmb200_beyond_t> beys((size_t)G);
-    std::vector<rmb200_serendipity_t> sers((size_t)G);
+    std::vector<rmb200_exposure_t> expos((size_t)G);                  // (zeroed)
+    std::vector<std::vector<int64_t>> item_counts(a0.outs.expo ? (size_t)G : 0);
+    // rows straight into the caller's arrays (every device writes its own); means, counts and exposure per device
+    std::vector<Outputs> outs((size_t)G, a0.outs);
     std::vector<int> rcs((size_t)G, RMB200_OK);
     std::vector<std::string> errs((size_t)G);
     std::vector<std::thread> workers;
@@ -1396,20 +1389,12 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
         e.device = devs[g]; e.devices = nullptr; e.n_devices = 0;
         e.user_begin = lo[g]; e.user_end = hi[g];
         e.timing = &tms[g];
-        metric_means.attach(g, e.metric_means, e.metric_counts);
-        if (a0.expo) {
+        for (int t = 0; t < MEAN_TABLES; t++) tables[t].attach(g, outs[g].means[t], outs[g].counts[t]);
+        if (a0.outs.expo) {
             item_counts[g].assign((size_t)a0.n, 0);
-            std::memset(&expos[g], 0, sizeof(rmb200_exposure_t));
             expos[g].struct_size = (int32_t)sizeof(rmb200_exposure_t);
             expos[g].item_counts = item_counts[g].data();
-        }
-        if (a0.bey) {           // rows straight into the caller's arrays (every device writes its own); means per device
-            beys[g] = *a0.bey;
-            beyond_means.attach(g, beys[g].means, beys[g].counts);
-        }
-        if (a0.ser) {
-            sers[g] = *a0.ser;
-            history_means.attach(g, sers[g].means, sers[g].counts);
+            outs[g].expo = &expos[g];
         }
         workers.emplace_back([&, g]() {
             rmb::g_err.clear();
@@ -1423,10 +1408,7 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
                         cudaGetLastError();
                     }
                 CallArgs<T> a = a0;
-                a.ex = &exs[g]; a.mc = &mc; a.mc_rank = g;
-                if (a0.expo) a.expo = &expos[g];
-                if (a0.bey) a.bey = &beys[g];
-                if (a0.ser) a.ser = &sers[g];
+                a.ex = &exs[g]; a.mc = &mc; a.mc_rank = g; a.outs = outs[g];
                 return run_call<T>(a);
             });
             rcs[g] = rc; errs[g] = rmb::g_err;
@@ -1446,12 +1428,10 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
     }
     if (rc != RMB200_OK) return rc;
 
-    metric_means.merge();
-    beyond_means.merge();
-    history_means.merge();
-    if (a0.expo) {          // the devices' counts added up (integers: exact), the statistics of the sum
+    for (const DeviceMeans& t : tables) t.merge();
+    if (a0.outs.expo) {          // the devices' counts added up (integers: exact), the statistics of the sum
         std::vector<int64_t> own;
-        int64_t* sum = a0.expo->item_counts;
+        int64_t* sum = a0.outs.expo->item_counts;
         if (!sum) { own.resize((size_t)a0.n); sum = own.data(); }
         int64_t users = 0;
         for (int j = 0; j < a0.n; j++) {
@@ -1460,8 +1440,8 @@ int run_multi(const CallArgs<T>& a0, const std::vector<int>& devs_in)
             sum[j] = c;
         }
         for (int g = 0; g < G; g++) users += expos[g].users;
-        a0.expo->users = users;
-        TRY(exposure_stats(sum, a0.n, a0.expo));
+        a0.outs.expo->users = users;
+        TRY(exposure_stats(sum, a0.n, a0.outs.expo));
     }
     if (ex->timing) {
         rmb200_timing_t t = tms[0];
@@ -1498,10 +1478,29 @@ int entry(const T* A, size_t lda, const T* B, size_t ldb, int32_t m, int32_t n, 
     a.A = A; a.lda = lda; a.B = B; a.ldb = ldb; a.m = m; a.n = n; a.k = k;
     a.trp = trp; a.tri = tri; a.tep = tep; a.tei = tei; a.tev = tev;
     a.K = K; a.cumulative = cumulative ? 1 : 0; a.noise = noise ? 1 : 0;
-    T* outs[10] = {p, tp, r, ap, tap, ndcg, hit, rr, roc, pr};
-    for (int q = 0; q < 10; q++) a.out[q] = outs[q];
     a.consider_cold_start = ccs ? 1 : 0; a.min_items_pool = mip; a.min_pos_test = mpt; a.seed = seed;
-    a.bias = bias; a.ex = ex_or_default(ex); a.expo = expo; a.bey = bey; a.ser = ser;
+    a.bias = bias; a.ex = ex_or_default(ex);
+    Outputs& o = a.outs;                            // ---- what the call writes ----
+    o = Outputs{{p, tp, r, ap, tap, ndcg, hit, rr, roc, pr}};
+    if (a.ex->struct_size == (int32_t)sizeof(rmb200_extra_t)) {     // (else run_call reports it before anything is written)
+        o.rows[RO_STATUS] = a.ex->status; o.rows[RO_TOPK_ITEMS] = a.ex->topk_items; o.rows[RO_TOPK_SCORES] = a.ex->topk_scores;
+        o.means[0] = a.ex->metric_means; o.counts[0] = a.ex->metric_counts; o.pos_rank = a.ex->pos_rank;
+    }
+    o.expo = expo;
+    if (bey) {
+        o.rows[RO_BEYOND] = bey->novelty; o.rows[RO_BEYOND + 1] = bey->avg_popularity; o.rows[RO_BEYOND + 2] = bey->ild;
+        o.means[1] = bey->means; o.counts[1] = bey->counts;
+        o.item_popularity = bey->item_popularity; o.popularity_users = bey->popularity_users;
+    }
+    if (ser) {
+        o.rows[RO_HISTORY] = ser->unexpectedness; o.rows[RO_HISTORY + 1] = ser->serendipity;
+        o.means[2] = ser->means; o.counts[2] = ser->counts;
+    }
+    for (int t = 1; t < MEAN_TABLES; t++) {     // a family's table is on only with one of its rows (the metrics': whenever given)
+        bool rows = false;
+        for (int q = 0; q < MEAN_SHAPES[t].slots; q++) rows |= o.rows[MEAN_SHAPES[t].first_row + q] != nullptr;
+        if (!rows) { o.means[t] = nullptr; o.counts[t] = nullptr; }
+    }
     return rmb::guard([&] {
         std::vector<int> devs;
         TRY(resolve_devices(a.ex, devs));

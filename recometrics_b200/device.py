@@ -170,8 +170,8 @@ def calc_reco_metrics_device(
     return _evaluate(lambda size, dt, fill: torch.empty(size, dtype=tdts[dt], device=dev) if fill is None
                      else torch.full((size,), fill, dtype=tdts[dt], device=dev), lambda t: t.data_ptr(), prep, popularity,
                      cumulative, break_ties_with_noise, user_range, return_topk, return_status, return_means, means_only,
-                     return_exposure, novelty, avg_popularity, diversity, unexpectedness=unexpectedness,
-                     serendipity=serendipity, to_numpy=lambda t: t.cpu().numpy(),
+                     return_exposure, dict(novelty=novelty, avg_popularity=avg_popularity, ild=diversity,
+                     unexpectedness=unexpectedness, serendipity=serendipity), to_numpy=lambda t: t.cpu().numpy(),
                      # the library runs on its own stream: the caller's pending writes and the fills above must have landed
                      sync=lambda: torch.cuda.synchronize(dev),
                      device=device, inputs_on_device=True, strict_min_pos_test=strict_min_pos_test, scoring_path=scoring_path)

@@ -17,6 +17,7 @@ There is no CPU fallback: without the built library or without a CUDA device the
 """
 import ctypes
 import re
+from collections import namedtuple
 from dataclasses import dataclass
 from warnings import warn
 
@@ -127,42 +128,41 @@ def item_popularity(X_train, m=None, user_range=None, device=-1):
     return counts
 
 
+# A family of per-user rows: its (name, result key) pairs in the order of its C struct and of its means / counts table, how
+# many of them are W wide when cumulative, the requested rows by name, and the table (None: not requested)
+_Family = namedtuple("_Family", "keys wide_slots rows means counts")
+
+
 class _ResultRows:
     """The per-user rows of one call -- the requested metrics, Novelty / AvgPop / ILD and Unexpectedness / Serendipity rows,
     NaN outside ``user_range`` -- and their means / counts tables, allocated with ``alloc(size, dtype, fill)`` (numpy or
-    torch; ``fill=None``: left uninitialised).  A table is ``[slot][W]``, ``W = K`` when ``cumulative`` else 1, over its rows
-    in order: the ten metrics (the first eight W wide, ROC / PR-AUC one value each), the three beyond-accuracy rows and the
-    two history rows (all W wide)."""
+    torch; ``fill=None``: left uninitialised).  ``flags`` maps every row name to whether it is requested.  The families are
+    the ten metrics (arguments of the C call, means in rmb200_extra_t), rmb200_beyond_t's and rmb200_serendipity_t's rows.  A
+    table is ``[slot][W]``, ``W = K`` when ``cumulative`` else 1, over its family's rows, and exists when one of them does."""
 
-    def __init__(self, alloc, dtype, m, K, cumulative, flags, bflags, sflags, user_range, return_means):
+    def __init__(self, alloc, dtype, m, K, cumulative, flags, user_range, return_means):
         self.m, self.K, self.W, self.cumulative = m, K, (K if cumulative else 1), cumulative
         fill = None if user_range is None else np.nan
-
-        def table(slots, on):       # means, counts
-            return (alloc(slots * self.W, np.float64, np.nan), alloc(slots * self.W, np.int64, 0)) if on else (None, None)
-        self.outs = {q: alloc(m * (self.W if q in _capi.TOPK_METRICS else 1), dtype, fill) for q in _capi.METRIC_ORDER if flags[q]}
-        self.means, self.counts = table(10, return_means)
-        self.brows = {name: alloc(m * self.W, dtype, fill) for name, _ in _capi.BEYOND_KEYS if bflags[name]}
-        self.bmeans, self.bcounts = table(3, return_means and bool(self.brows))
-        self.srows = {name: alloc(m * self.W, dtype, fill) for name, _ in _capi.SERENDIPITY_KEYS if sflags[name]}
-        self.smeans, self.scounts = table(2, return_means and bool(self.srows))
+        self.families = []
+        for keys, wide_slots in ((_KEYS, 8), (_capi.BEYOND_KEYS, 3), (_capi.SERENDIPITY_KEYS, 2)):
+            rows = {name: alloc(m * (self.W if i < wide_slots else 1), dtype, fill) for i, (name, _) in enumerate(keys) if flags[name]}
+            on, cells = return_means and bool(rows), len(keys) * self.W
+            self.families.append(_Family(keys, wide_slots, rows, alloc(cells, np.float64, np.nan) if on else None,
+                                         alloc(cells, np.int64, 0) if on else None))
 
     def unpack(self, means_only, to_numpy=lambda x: x):
         """``metrics`` (W wide rows as ``(m, K)``, ``"K"`` last), ``means`` and ``counts`` of the call's EvalResult;
         ``to_numpy`` brings a means / counts table to the host."""
         metrics, W = {}, self.W
-        mean_d, count_d = ({}, {}) if self.means is not None else (None, None)
-        for rows, keys, wide_slots, means, counts in ((self.outs, _KEYS, 8, self.means, self.counts),
-                                                      (self.brows, _capi.BEYOND_KEYS, 3, self.bmeans, self.bcounts),
-                                                      (self.srows, _capi.SERENDIPITY_KEYS, 2, self.smeans, self.scounts)):
-            if means is not None:
-                means, counts = to_numpy(means), to_numpy(counts)
-            for i, (name, key) in enumerate(keys):
-                if name not in rows:
+        mean_d, count_d = ({}, {}) if self.families[0].means is not None else (None, None)
+        for f in self.families:
+            means, counts = (None, None) if f.means is None else (to_numpy(f.means), to_numpy(f.counts))
+            for i, (name, key) in enumerate(f.keys):
+                if name not in f.rows:
                     continue
-                wide = self.cumulative and i < wide_slots
+                wide = self.cumulative and i < f.wide_slots
                 if not means_only:
-                    metrics[key] = rows[name].reshape(self.m, self.K) if wide else rows[name]
+                    metrics[key] = f.rows[name].reshape(self.m, self.K) if wide else f.rows[name]
                 if means is not None:
                     mean_d[key] = means[i * W:(i + 1) * W].copy() if wide else float(means[i * W])
                     count_d[key] = counts[i * W:(i + 1) * W].copy() if wide else int(counts[i * W])
@@ -306,19 +306,19 @@ def _validate_and_prepare(X_train, X_test, A, B, k, item_biases, min_pos_test, m
 
 
 def _evaluate(alloc, addr, prep, popularity, cumulative, break_ties_with_noise, user_range, return_topk, return_status,
-              return_means, means_only, return_exposure, novelty, avg_popularity, diversity, unexpectedness=False,
-              serendipity=False, return_ranks=False, to_numpy=lambda x: x, sync=lambda: None, **extra):
+              return_means, means_only, return_exposure, list_rows, return_ranks=False, to_numpy=lambda x: x,
+              sync=lambda: None, **extra):
     """The evaluation call both front-ends end in, on the inputs ``prep`` they validated (``_validate_and_prepare``'s keys:
     host arrays or device addresses, as ``_capi.calc_metrics`` takes them).  The result rows and the asked-for extras are
     allocated with ``alloc(size, dtype, fill)`` (see :class:`_ResultRows`) and handed to the library as ``addr(array)``;
-    ``popularity()`` gives the item popularity when Novelty / AvgPop is asked for, ``sync()`` runs right before the call,
-    ``to_numpy`` brings a means / counts table to the host and ``extra`` goes to ``_capi.make_extra``."""
+    ``list_rows`` switches the beyond-accuracy and history rows by name; ``popularity()`` gives the item popularity when
+    Novelty / AvgPop is asked for, ``sync()`` runs right before the call, ``to_numpy`` brings a means / counts table to the
+    host and ``extra`` goes to ``_capi.make_extra``."""
     dtype, m, n, K, cumulative = prep["dtype"], prep["m"], prep["n"], prep["k"], bool(cumulative)
     ptr = lambda x: None if x is None else addr(x)
-    bflags = dict(novelty=bool(novelty), avg_popularity=bool(avg_popularity), ild=bool(diversity))
-    sflags = dict(unexpectedness=bool(unexpectedness), serendipity=bool(serendipity))
-    res = _ResultRows(alloc, dtype, m, K, cumulative, prep["flags"], bflags, sflags, user_range,
-                      bool(return_means) or bool(means_only))
+    flags = {**prep["flags"], **{name: bool(on) for name, on in list_rows.items()}}
+    res = _ResultRows(alloc, dtype, m, K, cumulative, flags, user_range, bool(return_means) or bool(means_only))
+    metric, beyond, history = res.families
     timing = _capi.Timing()
     status = alloc(m, np.int32, 0) if return_status else None
     topk_items = alloc(m * K, np.int32, -1) if return_topk else None
@@ -328,19 +328,18 @@ def _evaluate(alloc, addr, prep, popularity, cumulative, break_ties_with_noise, 
     if user_range is not None and ub == ue:
         ub, ue = 0, -1          # an EMPTY block (a rank with no users); 0,0 would mean "all users" in the C-ABI
     ex = _capi.make_extra(user_begin=ub, user_end=ue, topk_items=ptr(topk_items), topk_scores=ptr(topk_scores),
-                          pos_rank=ptr(pos_rank), status=ptr(status), timing=timing, metric_means=ptr(res.means),
-                          metric_counts=ptr(res.counts), skip_row_copy=bool(means_only), **extra)
+                          pos_rank=ptr(pos_rank), status=ptr(status), timing=timing, metric_means=ptr(metric.means),
+                          metric_counts=ptr(metric.counts), skip_row_copy=bool(means_only), **extra)
     item_counts = alloc(n, np.int64, 0) if return_exposure else None
     expo = _capi.make_exposure(ptr(item_counts)) if return_exposure else None
-    pop = popularity() if bflags["novelty"] or bflags["avg_popularity"] else None
-    bey = _capi.make_beyond({name: addr(r) for name, r in res.brows.items()}, ptr(pop), m, ptr(res.bmeans),
-                            ptr(res.bcounts)) if res.brows else None
-    ser = _capi.make_serendipity({name: addr(r) for name, r in res.srows.items()}, ptr(res.smeans),
-                                 ptr(res.scounts)) if res.srows else None
+    addrs = [{name: addr(r) for name, r in f.rows.items()} for f in res.families]
+    pop = popularity() if "novelty" in beyond.rows or "avg_popularity" in beyond.rows else None
+    bey = _capi.make_beyond(addrs[1], ptr(pop), m, ptr(beyond.means), ptr(beyond.counts)) if beyond.rows else None
+    ser = _capi.make_serendipity(addrs[2], ptr(history.means), ptr(history.counts)) if history.rows else None
     sync()
     rc = _capi.calc_metrics(dtype, prep["A"], prep["lda"], prep["B"], prep["ldb"], m, n, prep["p"],
                             prep["trp"], prep["tri"], prep["tep"], prep["tei"], prep["tev"], K, cumulative,
-                            bool(break_ties_with_noise), {q: addr(r) for q, r in res.outs.items()}, prep["consider_cold_start"],
+                            bool(break_ties_with_noise), addrs[0], prep["consider_cold_start"],
                             prep["min_items_pool"], prep["min_pos_test"], prep["nthreads"], prep["seed"], prep["item_biases"],
                             ex, exposure=expo, beyond=bey, serendipity=ser)
     _capi.raise_for_status(rc)
@@ -403,8 +402,8 @@ def calc_reco_metrics_ex(
         return pop
     return _evaluate(lambda size, dt, fill: np.empty(size, dt) if fill is None else np.full(size, fill, dt), lambda x: x,
                      prep, popularity, cumulative, break_ties_with_noise, user_range, return_topk, return_status,
-                     return_means, means_only, return_exposure, novelty, avg_popularity, diversity,
-                     unexpectedness=unexpectedness, serendipity=serendipity, return_ranks=return_ranks,
+                     return_means, means_only, return_exposure, dict(novelty=novelty, avg_popularity=avg_popularity,
+                     ild=diversity, unexpectedness=unexpectedness, serendipity=serendipity), return_ranks=return_ranks,
                      device=device, strict_min_pos_test=strict_min_pos_test, scoring_path=scoring_path,
                      filter_stats=filter_stats, nan_bits=nan_bits, devices=devices)
 
