@@ -32,7 +32,6 @@
 #include <atomic>
 #include <chrono>
 #include <cmath>
-#include <cstdio>
 #include <condition_variable>
 #include <deque>
 #include <locale>
@@ -97,35 +96,6 @@ struct SplitPlan {
     int32_t ns = 0, nr = 0, longest = 0;
 };
 
-// /root/reference/src/recometrics.hpp:1037-1040: the held-out count of every split row, as index pointers
-void count_rows(const int32_t* Xp, const int32_t* rows, int32_t ns, double test_fraction, SplitPlan& P)
-{
-    P.ns = ns;
-    P.sel_p.resize((size_t)ns + 1);
-    P.test_p.resize((size_t)ns + 1);
-    P.train_p.resize((size_t)ns + 1);
-    P.sel_p[0] = P.test_p[0] = P.train_p[0] = 0;
-    P.longest = 0;
-    for (int32_t r = 0; r < ns; r++) {
-        const int32_t u = rows ? rows[r] : r;
-        const int32_t cnt = Xp[u + 1] - Xp[u];
-        P.sel_p[r + 1] = P.sel_p[r] + cnt;
-        P.test_p[r + 1] = P.test_p[r] + (int32_t)std::round(cnt * test_fraction);
-        P.train_p[r + 1] = P.sel_p[r + 1] - P.test_p[r + 1];
-        P.longest = std::max(P.longest, cnt);
-    }
-    // chunks of whole rows, about a sixteenth of the entries each but not below a million: what the device thread works on
-    const int64_t total = P.sel_p[ns];
-    int64_t floor_entries = 1 << 20;
-    if (const char* env = std::getenv("RMB200_SPLIT_CHUNK")) { const long long v = std::atoll(env); if (v >= 1) floor_entries = v; }   // (tests)
-    const int64_t per_chunk = std::max<int64_t>(floor_entries, (total + 15) / 16);
-    P.chunk_end.clear();
-    int64_t next = per_chunk;
-    for (int32_t r = 0; r < ns; r++)
-        if (P.sel_p[r + 1] >= next && r + 1 < ns) { P.chunk_end.push_back(r + 1); next = P.sel_p[r + 1] + per_chunk; }
-    P.chunk_end.push_back(ns);
-}
-
 // The threads of one call wait for each other here.  Blocking waits, not spinning: in a container with a CPU quota a handful of
 // spinning threads burns the quota and the kernel then stalls ALL of the call's threads for the rest of the period.
 struct Signal {
@@ -135,38 +105,29 @@ struct Signal {
     template <class Pred> void wait(Pred&& ready) { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, ready); }
 };
 
-// libstdc++'s std::shuffle consumes, for `cnt` elements, a number of raw mt19937 outputs that depends on the outputs
-// themselves (the rejection loop of its bounded draw, bits/uniform_int_dist.h _S_nd; two positions per draw while cnt*cnt fits
-// 32 bits, bits/stl_algo.h).  skip_shuffle() consumes exactly those outputs WITHOUT shuffling anything: about half the cost.
-// It is only ever used to run AHEAD of the real thing -- every state it predicts is checked against std::shuffle's own.
-inline void skip_bounded_draw(std::mt19937& g, uint32_t range)
-{
-    uint32_t low = (uint32_t)((uint64_t)g() * (uint64_t)range);
-    if (low < range) {
-        const uint32_t threshold = (uint32_t)(0u - range) % range;
-        while (low < threshold) low = (uint32_t)((uint64_t)g() * (uint64_t)range);
+// What the replay, the device thread and the page toucher of one call tell each other.
+struct Progress {
+    std::unique_ptr<std::atomic<int>[]> chunk_done;   // [chunks] set (release: the bytes are visible) when a chunk's bytes are final
+    std::atomic<int> stop{0};                         // the device thread failed or the replay threw: the others need not go on
+    std::atomic<int> touched{0};                      // the result arrays' pages have been touched: copies into them may start
+    Signal sig;
+    explicit Progress(size_t chunks) : chunk_done(new std::atomic<int>[chunks])
+    {
+        for (size_t c = 0; c < chunks; c++) chunk_done[c].store(0);
     }
-}
+};
 
-inline void skip_shuffle(std::mt19937& g, uint32_t cnt)
-{
-    if (cnt < 2) return;
-    if (0xffffffffull / cnt >= cnt) {
-        uint32_t i = 1;
-        if ((cnt & 1u) == 0) { skip_bounded_draw(g, 2); i++; }
-        for (; i != cnt; i += 2) skip_bounded_draw(g, (uint32_t)(((uint64_t)i + 1) * ((uint64_t)i + 2)));
-    } else {
-        for (uint32_t i = 1; i < cnt; i++) skip_bounded_draw(g, i + 1);
-    }
-}
-
-// The scout's faster form: the raw mt19937 outputs generated 624 at a time by the textbook in-place recurrence (the state array
-// is laid out exactly like libstdc++'s, so a std::mt19937 can be made from it through the engine's own operator>>), and the
-// draws of a whole row screened at once -- a bounded draw of range R can only be rejected when the low 32 bits of x * R fall
-// below R (bits/uniform_int_dist.h), which for the ranges of a shuffle happens about once in 10^4 draws; only then are the
-// row's draws walked one by one.  ~1.2 ns per draw against ~2.2 for std::mt19937 + the scalar rejection test.
-// usable(): the generator and the state hand-over are compared with std::mt19937 itself before the scout relies on them; and,
-// as for skip_shuffle(), every state it predicts is checked against std::shuffle's own generator afterwards.
+// The replay's scout.  libstdc++'s std::shuffle consumes, for `cnt` elements, a number of raw mt19937 outputs that depends on the
+// outputs themselves (the rejection loop of its bounded draw, bits/uniform_int_dist.h _S_nd; two positions per draw while
+// cnt*cnt fits 32 bits, bits/stl_algo.h).  skip_row() consumes exactly those outputs WITHOUT shuffling anything: the raw
+// outputs generated 624 at a time by the textbook in-place recurrence (the state array is laid out exactly like libstdc++'s, so
+// a std::mt19937 can be made from it through the engine's own operator>>), and the draws of a whole row screened at once -- a
+// bounded draw of range R can only be rejected when the low 32 bits of x * R fall below R (bits/uniform_int_dist.h), which for
+// the ranges of a shuffle happens about once in 10^4 draws; only then are the row's draws walked one by one.  ~1.2 ns per draw
+// against ~2.2 for std::mt19937 + the scalar rejection test.
+// It is only ever used to run AHEAD of the real thing: usable() compares the generator and the state hand-over with
+// std::mt19937 itself before the replay relies on them, and every state it predicts is checked against std::shuffle's own
+// generator afterwards.
 class RawScout {
     uint32_t x[624];
     uint32_t out[624];
@@ -271,11 +232,11 @@ public:
 };
 
 // /root/reference/src/recometrics.hpp:1041-1060 without the data movement: for rows with something on both sides, the
-// positions std::shuffle puts first.  chunk_done[c] is set (release: the bytes are visible) when chunk c's bytes are final.
+// positions std::shuffle puts first.  prog.chunk_done[c] is set when chunk c's bytes are final.
 //
 // sequential(): the reference's loop, one generator, row after row.
-// parallel():   the same stream, several threads.  One thread (the scout) runs ahead with skip_shuffle() and leaves a copy of
-//               the generator at every chunk boundary; the others pick chunks, start from the scout's copy, do the real
+// parallel():   the same stream, several threads.  One thread (the scout) runs ahead with RawScout::skip_row() and leaves a
+//               copy of the generator at every chunk boundary; the others pick chunks, start from the scout's copy, do the real
 //               std::shuffle of every row -- and publish a chunk only if their generator ends in exactly the state the scout
 //               left for the next chunk.  A mismatch (a libstdc++ whose shuffle draws differently) costs time, never the
 //               result: the chunk that disagreed is kept (its start was verified, its end state is std::shuffle's own) and the
@@ -283,9 +244,7 @@ public:
 struct Replay {
     SplitPlan& P;
     uint64_t seed;
-    std::atomic<int>* chunk_done;
-    const std::atomic<int>& stop;
-    Signal& sig;
+    Progress& prog;
     int fault_chunk = -1;        // (tests) the scout miscounts in this chunk
 
     int32_t chunk_begin(size_t c) const { return c ? P.chunk_end[c - 1] : 0; }
@@ -308,9 +267,9 @@ struct Replay {
     {
         std::vector<int32_t> order((size_t)P.longest);
         for (size_t c = from_chunk; c < P.chunk_end.size(); c++) {
-            if (stop.load(std::memory_order_relaxed)) return;
+            if (prog.stop.load(std::memory_order_relaxed)) return;
             rows(rng, order, chunk_begin(c), P.chunk_end[c]);
-            sig.update([&]() { chunk_done[c].store(1, std::memory_order_release); });
+            prog.sig.update([&]() { prog.chunk_done[c].store(1, std::memory_order_release); });
         }
     }
 
@@ -321,6 +280,8 @@ struct Replay {
         std::atomic<size_t> scouted{0};            // start[0 .. scouted) are known
         std::atomic<size_t> next{0};
         std::atomic<size_t> first_bad{nc};         // lowest chunk whose end state disagreed with the scout
+        const std::atomic<int>& stop = prog.stop;
+        Signal& sig = prog.sig;
         auto give_up = [&]() { return stop.load(std::memory_order_relaxed) || first_bad.load(std::memory_order_relaxed) < nc; };
         // a chunk ABOVE one that disagreed started from a state nobody vouches for; the chunks below it still have to be finished
         auto doomed = [&](size_t c) { return stop.load(std::memory_order_relaxed) || first_bad.load(std::memory_order_relaxed) < c; };
@@ -334,7 +295,7 @@ struct Replay {
                 // (the scout stops after a disagreement at chunk b, but it had passed b + 1 by then: no chunk below b waits in vain)
                 sig.wait([&]() { return scouted.load(std::memory_order_acquire) > c + 1 || doomed(c); });
                 if (doomed(c)) return;
-                if (rng == start[c + 1]) { sig.update([&]() { chunk_done[c].store(1, std::memory_order_release); }); continue; }
+                if (rng == start[c + 1]) { sig.update([&]() { prog.chunk_done[c].store(1, std::memory_order_release); }); continue; }
                 sig.update([&]() {
                     if (c < first_bad.load()) { first_bad.store(c); start[c + 1] = rng; }   // (only the lowest disagreeing chunk's state is used below)
                 });
@@ -345,21 +306,18 @@ struct Replay {
         struct JoinAll { std::vector<std::thread>& v; ~JoinAll() { for (auto& t : v) if (t.joinable()) t.join(); } } join_all{pool};
         for (int w = 0; w < workers; w++) pool.emplace_back(work);
         {   // the scout
-            const bool fast = RawScout::usable(seed) && !std::getenv("RMB200_SPLIT_PLAIN_SCOUT");
-            std::mt19937 g(seed);
             RawScout raw(seed);
-            start[0] = g;
+            start[0] = std::mt19937(seed);
             sig.update([&]() { scouted.store(1, std::memory_order_release); });
             for (size_t c = 0; c < nc && !give_up(); c++) {
                 for (int32_t r = chunk_begin(c); r < P.chunk_end[c]; r++) {
                     const int32_t cnt = P.sel_p[r + 1] - P.sel_p[r];
                     const int32_t out = P.test_p[r + 1] - P.test_p[r];
                     if (out <= 0 || out >= cnt) continue;
-                    if (fast) raw.skip_row((uint32_t)cnt);
-                    else skip_shuffle(g, (uint32_t)cnt);
+                    raw.skip_row((uint32_t)cnt);
                 }
-                if ((int)c == fault_chunk) { if (fast) raw.next(); else g(); }
-                if (fast) g = raw.engine();
+                if ((int)c == fault_chunk) raw.next();
+                const std::mt19937 g = raw.engine();
                 // (a worker that disagreed with this scout may already have put std::shuffle's own state into start[c + 1]: the
                 //  scout stops at the next give_up(); what it writes after a disagreement is never used)
                 sig.update([&]() { if (first_bad.load() >= nc) { start[c + 1] = g; } scouted.store(c + 2, std::memory_order_release); });
@@ -368,22 +326,22 @@ struct Replay {
         work();                                    // the scout's thread joins the others
         for (auto& t : pool) t.join();
         const size_t bad = first_bad.load();
-        if (std::getenv("RMB200_SPLIT_DBG")) std::fprintf(stderr, "replay: %zu chunks, first_bad %zu\n", nc, bad);
         if (bad >= nc || stop.load()) return;
         // chunks 0 .. bad-1 were verified and published; chunk `bad` started from a verified state and start[bad + 1] is where
         // std::shuffle itself left the generator.  Anything written further on started from the scout's wrong guess.
-        for (size_t c = bad + 1; c < nc; c++) chunk_done[c].store(0, std::memory_order_relaxed);
+        for (size_t c = bad + 1; c < nc; c++) prog.chunk_done[c].store(0, std::memory_order_relaxed);
         if (bad + 1 < nc) std::memset(P.held.data() + P.sel_p[P.chunk_end[bad]], 0, (size_t)(P.sel_p[P.ns] - P.sel_p[P.chunk_end[bad]]));
-        sig.update([&]() { chunk_done[bad].store(1, std::memory_order_release); });
+        sig.update([&]() { prog.chunk_done[bad].store(1, std::memory_order_release); });
         sequential(bad + 1, start[bad + 1]);
     }
 
+    // in parallel only where the scout is known to walk in step with this library's std::mt19937 (RawScout::usable)
     void run()
     {
         int workers = (int)std::min(4u, std::max(1u, std::thread::hardware_concurrency() / 4));
         if (const char* env = std::getenv("RMB200_SPLIT_THREADS")) workers = std::max(0, std::atoi(env));
         if (const char* env = std::getenv("RMB200_SPLIT_SCOUT_FAULT")) fault_chunk = std::atoi(env);
-        if (workers >= 1 && P.chunk_end.size() >= 4) parallel(workers);
+        if (workers >= 1 && P.chunk_end.size() >= 4 && RawScout::usable(seed)) parallel(workers);
         else sequential(0, std::mt19937(seed));
     }
 };
@@ -424,6 +382,45 @@ const char* pick_users(const int32_t* Xp, int32_t m, int32_t n, int32_t n_users_
     P.rem_p.resize((size_t)P.nr + 1);
     P.rem_p[0] = 0;
     for (int32_t r = 0; r < P.nr; r++) P.rem_p[r + 1] = P.rem_p[r] + (Xp[P.rem_rows[r] + 1] - Xp[P.rem_rows[r]]);
+    return nullptr;
+}
+
+// Everything the result's shape depends on: which rows are split (a sample of the users when `sample_users`, else every row of
+// X), how many entries of each are held out (/root/reference/src/recometrics.hpp:1037-1040), the chunks the device thread works
+// on, and the held-out bytes, all 0.  Returns the reference's error text or nullptr.
+const char* plan_split(const int32_t* Xp, int32_t m, int32_t n, bool sample_users, int32_t n_users_test, double test_fraction,
+                       bool consider_cold_start, int32_t min_items_pool, int32_t min_pos_test, uint64_t seed, SplitPlan& P)
+{
+    if (sample_users)
+        if (const char* refusal = pick_users(Xp, m, n, n_users_test, test_fraction, consider_cold_start, min_items_pool,
+                                             min_pos_test, seed, P))
+            return refusal;
+    const int32_t ns = P.whole ? m : (int32_t)P.sel_rows.size();
+    P.ns = ns;
+    P.sel_p.resize((size_t)ns + 1);
+    P.test_p.resize((size_t)ns + 1);
+    P.train_p.resize((size_t)ns + 1);
+    P.sel_p[0] = P.test_p[0] = P.train_p[0] = 0;
+    P.longest = 0;
+    for (int32_t r = 0; r < ns; r++) {
+        const int32_t u = P.whole ? r : P.sel_rows[r];
+        const int32_t cnt = Xp[u + 1] - Xp[u];
+        P.sel_p[r + 1] = P.sel_p[r] + cnt;
+        P.test_p[r + 1] = P.test_p[r] + (int32_t)std::round(cnt * test_fraction);
+        P.train_p[r + 1] = P.sel_p[r + 1] - P.test_p[r + 1];
+        P.longest = std::max(P.longest, cnt);
+    }
+    // chunks of whole rows, about a sixteenth of the entries each but not below a million: what the device thread works on
+    const int64_t total = P.sel_p[ns];
+    int64_t floor_entries = 1 << 20;
+    if (const char* env = std::getenv("RMB200_SPLIT_CHUNK")) { const long long v = std::atoll(env); if (v >= 1) floor_entries = v; }   // (tests)
+    const int64_t per_chunk = std::max<int64_t>(floor_entries, (total + 15) / 16);
+    P.chunk_end.clear();
+    int64_t next = per_chunk;
+    for (int32_t r = 0; r < ns; r++)
+        if (P.sel_p[r + 1] >= next && r + 1 < ns) { P.chunk_end.push_back(r + 1); next = P.sel_p[r + 1] + per_chunk; }
+    P.chunk_end.push_back(ns);
+    P.held.reset((size_t)total);
     return nullptr;
 }
 
@@ -616,14 +613,14 @@ struct Downloads {
     double copy_ms = 0.0;              // summed over the threads
     std::vector<std::thread> threads;
 
-    void start(int device, int n, Signal* sig, std::atomic<int>* touched)
+    void start(int device, int n, Progress& prog)
     {
         for (int t = 0; t < n; t++)
-            threads.emplace_back([this, device, sig, touched]() {
+            threads.emplace_back([this, device, &prog]() {
                 cudaStream_t st = nullptr;
                 cudaError_t e = cudaSetDevice(device);
                 if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
-                sig->wait([&]() { return touched->load(std::memory_order_acquire) != 0; });
+                prog.sig.wait([&]() { return prog.touched.load(std::memory_order_acquire) != 0; });
                 double ms = 0.0;
                 for (;;) {
                     Piece p;
@@ -663,25 +660,43 @@ struct Downloads {
     ~Downloads() { finish(); }
 };
 
-// The device side of one call, run on its own host thread.
+struct Stream { cudaStream_t s = nullptr; ~Stream() { if (s) cudaStreamDestroy(s); } };
+struct Event { cudaEvent_t e = nullptr; ~Event() { if (e) cudaEventDestroy(e); } };
+
+// The device side of one call, run on its own host thread: upload(), order_unsorted_rows(), gather_untouched_rows() and
+// partition_chunks(), in that order, sharing what they set up through the members below.  A step that fails records the
+// error, sets prog.stop and returns false.
+#define JOB_CUDA(call) do { if (bad((call), #call)) return false; } while (0)
 template <typename T>
 struct DeviceJob {
     SplitKind kind;
     int device;
     const int32_t *Xp, *Xi; const T* Xv;
     int32_t m; int64_t nnz;
-    const SplitPlan* P;
+    const SplitPlan& Q;
     rmb200_split_t* out;
-    std::atomic<int>* chunk_done;      // [chunks] set by the replay when a chunk's bytes are final
-    std::atomic<int>* stop;            // set by this thread on failure: the replay need not go on
-    std::atomic<int>* touched;         // the result arrays' pages have been touched: copies into them may start
-    Signal* sig;
+    Progress& prog;
     // results
     int status = RMB200_OK;
     std::string what, detail;
     double h2d_ms = 0, d2h_ms = 0, kernel_ms = 0;
     int64_t launches = 0, h2d_bytes = 0, d2h_bytes = 0;
     int sorted_on_device = 0;
+    // shared by the steps
+    int32_t ns = 0, nr = 0;
+    int64_t sel_nnz = 0, test_nnz = 0, rem_nnz = 0, kept_nnz = 0;
+    Stream stream;
+    Event ev0, ev1;
+    cudaStream_t st = nullptr;
+    int nsm = 148;
+    size_t scan_bytes = 0;
+    rmb::DevBuf block;
+    Slot dXp, dXi, dXv, d_selrows, d_selp, d_testp, d_remrows, d_remp, d_held, d_scan, d_tri, d_trv, d_tei, d_tev, d_unsorted,
+         d_scan_temp, d_rei, d_rev;
+    rmb::DevBuf d_keys0, d_keys1, d_vals0, d_perm, d_sort_temp, d_flags;     // (the rare unsorted input: blocks of their own)
+    const int* perm = nullptr;
+    SplitView V;
+    Downloads downloads;
 
     bool bad(cudaError_t e, const char* where)
     {
@@ -690,84 +705,71 @@ struct DeviceJob {
         status = (e == cudaErrorMemoryAllocation) ? RMB200_ERR_OOM : RMB200_ERR_CUDA;
         what = where;
         detail = cudaGetErrorString(e);
-        sig->update([&]() { stop->store(1); });
+        prog.sig.update([&]() { prog.stop.store(1); });
         return true;
     }
 
-    double dbg_setup = 0, dbg_wait = 0, dbg_body = 0;
-    clk::time_point dbg_end;
-
-    void run()
+    cudaError_t up(void* dst, const void* src, size_t bytes)
     {
-        const auto t0 = clk::now();
-        dbg_end = t0;
-        body();
-        if (std::getenv("RMB200_SPLIT_DBG"))
-            std::fprintf(stderr, "split device thread: %.1f ms = setup %.1f + h2d %.1f + kernels %.2f + d2h %.1f + waiting %.1f + rest, "
-                         "teardown %.1f\n", ms_since(t0), dbg_setup, h2d_ms, kernel_ms, d2h_ms, dbg_wait,
-                         std::chrono::duration<double, std::milli>(clk::now() - dbg_end).count());
+        h2d_bytes += (int64_t)bytes;
+        if (!bytes) return cudaSuccess;
+        return rmb::upload_bytes_pageable(dst, src, bytes, st, 2);
     }
 
-    void body()
+    cudaError_t down(void* dst, const void* src, size_t bytes)      // (pageable destination: returns when the bytes are there)
     {
-#define JOB_CUDA(call) do { if (bad((call), #call)) return; } while (0)
-        const SplitPlan& Q = *P;
-        const int32_t ns = Q.ns, nr = Q.nr;
-        const int64_t sel_nnz = Q.sel_p[ns], test_nnz = Q.test_p[ns], rem_nnz = nr ? Q.rem_p[nr] : 0;
-        const int64_t kept_nnz = sel_nnz - test_nnz;
+        if (!bytes) return cudaSuccess;
+        prog.sig.wait([&]() { return prog.touched.load(std::memory_order_acquire) != 0; });
+        const auto t0 = clk::now();
+        const cudaError_t e = rmb::download_bytes_pageable(dst, src, bytes, st, 2);
+        d2h_ms += ms_since(t0);
+        d2h_bytes += (int64_t)bytes;
+        return e;
+    }
+
+    cudaError_t down_later(void* dst, const void* src, size_t bytes)      // (on the copy threads, while this thread goes on)
+    {
+        d2h_bytes += (int64_t)bytes;
+        downloads.push(dst, src, bytes);
+        return cudaSuccess;
+    }
+
+    cudaError_t kernels_begin() { return cudaEventRecord(ev0.e, st); }
+
+    cudaError_t kernels_end()
+    {
+        float span = 0.f;
+        cudaError_t e = cudaEventRecord(ev1.e, st);
+        if (e == cudaSuccess) e = cudaEventSynchronize(ev1.e);
+        if (e == cudaSuccess) e = cudaEventElapsedTime(&span, ev0.e, ev1.e);
+        if (e == cudaSuccess) kernel_ms += span;
+        return e;
+    }
+
+    int grid_for(int64_t work) const { return (int)std::max<int64_t>(1, std::min<int64_t>((work + TPB - 1) / TPB, (int64_t)nsm * 16)); }
+
+    // The stream, one device block for the call, X and the plan's index arrays up.  The block comes from the library's workspace
+    // cache: cudaMalloc / cudaFree of a call's ~600 MB cost 10-200 ms on a busy box, more than the rest of the call.
+    bool upload()
+    {
+        ns = Q.ns; nr = Q.nr;
+        sel_nnz = Q.sel_p[ns]; test_nnz = Q.test_p[ns]; rem_nnz = nr ? Q.rem_p[nr] : 0;
+        kept_nnz = sel_nnz - test_nnz;
         const int64_t train_nnz = kept_nnz + (kind == SPLIT_JOINED ? rem_nnz : 0);
-        const auto t_setup = clk::now();
         JOB_CUDA(cudaSetDevice(device));
-        struct Stream { cudaStream_t s = nullptr; ~Stream() { if (s) cudaStreamDestroy(s); } } stream;
-        struct Event { cudaEvent_t e = nullptr; ~Event() { if (e) cudaEventDestroy(e); } } ev0, ev1;
         JOB_CUDA(cudaStreamCreateWithFlags(&stream.s, cudaStreamNonBlocking));
         JOB_CUDA(cudaEventCreate(&ev0.e));
         JOB_CUDA(cudaEventCreate(&ev1.e));
-        const cudaStream_t st = stream.s;
-        dbg_setup = ms_since(t_setup);
-        const bool plain_copies = []() { const char* e = std::getenv("RMB200_SPLIT_PLAIN_COPIES"); return e && e[0] == '1'; }();
-        auto up = [&](void* dst, const void* src, size_t bytes) {
-            h2d_bytes += (int64_t)bytes;
-            if (!bytes) return cudaSuccess;
-            return plain_copies ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st) : rmb::upload_bytes_pageable(dst, src, bytes, st, 2);
-        };
-        auto down = [&](void* dst, const void* src, size_t bytes) {     // (pageable destination: returns when the bytes are there)
-            if (!bytes) return cudaSuccess;
-            sig->wait([&]() { return touched->load(std::memory_order_acquire) != 0; });
-            const auto t0 = clk::now();
-            cudaError_t e;
-            if (plain_copies) {
-                e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
-                const cudaError_t e2 = cudaStreamSynchronize(st);
-                if (e == cudaSuccess) e = e2;
-            } else e = rmb::download_bytes_pageable(dst, src, bytes, st, 2);
-            d2h_ms += ms_since(t0);
-            d2h_bytes += (int64_t)bytes;
-            return e;
-        };
-        float span = 0.f;
-        auto kernels_begin = [&]() { return cudaEventRecord(ev0.e, st); };
-        auto kernels_end = [&]() {
-            cudaError_t e = cudaEventRecord(ev1.e, st);
-            if (e == cudaSuccess) e = cudaEventSynchronize(ev1.e);
-            if (e == cudaSuccess) e = cudaEventElapsedTime(&span, ev0.e, ev1.e);
-            if (e == cudaSuccess) kernel_ms += span;
-            return e;
-        };
+        st = stream.s;
 
-        // ---- one device block for the call, X and the plan's index arrays up.  The block comes from the library's workspace
-        //      cache: cudaMalloc / cudaFree of a call's ~600 MB cost 10-200 ms on a busy box, more than the rest of the call ----
         const auto t_up = clk::now();
         int64_t longest_chunk = 0;
         for (size_t c = 0, rb = 0; c < Q.chunk_end.size(); rb = (size_t)Q.chunk_end[c++])
             longest_chunk = std::max<int64_t>(longest_chunk, Q.sel_p[Q.chunk_end[c]] - Q.sel_p[rb]);
-        size_t scan_bytes = 0;
         if (longest_chunk) {
             auto probe = thrust::make_transform_iterator((const uint8_t*)nullptr, ByteToInt());
             JOB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, probe, (int*)nullptr, (int)longest_chunk, st));
         }
-        Slot dXp, dXi, dXv, d_selrows, d_selp, d_testp, d_remrows, d_remp, d_held, d_scan, d_tri, d_trv, d_tei, d_tev, d_unsorted,
-             d_scan_temp, d_rei, d_rev;
         const bool own_rem = (kind == SPLIT_SEPARATE) && rem_nnz;
         const std::pair<Slot*, size_t> layout[] = {
             {&dXp, sizeof(int32_t) * ((size_t)m + 1)}, {&dXi, sizeof(int32_t) * (size_t)nnz}, {&dXv, sizeof(T) * (size_t)nnz},
@@ -780,7 +782,6 @@ struct DeviceJob {
         Carver carve;
         size_t offsets[sizeof(layout) / sizeof(layout[0])];
         for (size_t k = 0; k < sizeof(layout) / sizeof(layout[0]); k++) offsets[k] = carve.reserve(layout[k].second);
-        rmb::DevBuf block;
         JOB_CUDA(block.alloc(carve.total));
         carve.base = block.as<char>();
         for (size_t k = 0; k < sizeof(layout) / sizeof(layout[0]); k++) layout[k].first->p = carve.at<char>(offsets[k]);
@@ -800,81 +801,79 @@ struct DeviceJob {
         JOB_CUDA(cudaStreamSynchronize(st));
         h2d_ms = ms_since(t_up);
 
-        int nsm = 148;
         cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
-        auto grid_for = [&](int64_t work) { return (int)std::max<int64_t>(1, std::min<int64_t>((work + TPB - 1) / TPB, (int64_t)nsm * 16)); };
-
-        SplitView V;
         V.Xp = dXp.as<int>(); V.Xi = dXi.as<int>();
         V.sel_rows = Q.whole ? nullptr : d_selrows.as<int>();
         V.sel_p = Q.whole ? dXp.as<int>() : d_selp.as<int>();
         V.test_p = d_testp.as<int>();
         V.ns = ns; V.j0 = 0; V.j1 = (int)sel_nnz;
+        return true;
+    }
 
-        // ---- what does not wait for the replay: the order of unsorted rows, and the rows the split leaves alone ----
-        rmb::DevBuf d_keys0, d_keys1, d_vals0, d_perm, d_sort_temp, d_flags;     // (the rare unsorted input: blocks of their own)
-        const int* perm = nullptr;
-        if (sel_nnz) {
-            JOB_CUDA(kernels_begin());
-            check_sorted_kernel<<<grid_for(sel_nnz), TPB, 0, st>>>(V, d_unsorted.as<int>());
-            launches++;
-            JOB_CUDA(kernels_end());
-            int unsorted = 0;
-            JOB_CUDA(cudaMemcpyAsync(&unsorted, d_unsorted.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-            JOB_CUDA(cudaStreamSynchronize(st));
-            if (unsorted) {
-                sorted_on_device = 1;
-                JOB_CUDA(d_keys0.alloc(sizeof(int) * (size_t)sel_nnz));
-                JOB_CUDA(d_keys1.alloc(sizeof(int) * (size_t)sel_nnz));
-                JOB_CUDA(d_vals0.alloc(sizeof(int) * (size_t)sel_nnz));
-                JOB_CUDA(d_perm.alloc(sizeof(int) * (size_t)sel_nnz));
-                JOB_CUDA(d_flags.alloc((size_t)sel_nnz));
-                size_t temp_bytes = 0;
-                JOB_CUDA(cub::DeviceSegmentedRadixSort::SortPairs(nullptr, temp_bytes, (const int*)d_keys0.as<int>(), d_keys1.as<int>(),
-                                                                  (const int*)d_vals0.as<int>(), d_perm.as<int>(), (int)sel_nnz, ns,
-                                                                  V.sel_p, V.sel_p + 1, 0, 32, st));
-                JOB_CUDA(d_sort_temp.alloc(temp_bytes));
-                JOB_CUDA(kernels_begin());
-                sort_input_kernel<<<grid_for(sel_nnz), TPB, 0, st>>>(V, d_keys0.as<int>(), d_vals0.as<int>());
-                JOB_CUDA(cub::DeviceSegmentedRadixSort::SortPairs(d_sort_temp.p, temp_bytes, (const int*)d_keys0.as<int>(), d_keys1.as<int>(),
-                                                                  (const int*)d_vals0.as<int>(), d_perm.as<int>(), (int)sel_nnz, ns,
-                                                                  V.sel_p, V.sel_p + 1, 0, 32, st));
-                launches += 3;     // (cub's segmented sort: at least its partition + sort kernels)
-                JOB_CUDA(kernels_end());
-                perm = d_perm.as<int>();
-            }
-        }
-        if (rem_nnz) {
-            int* dst_i; T* dst_v;
-            if (kind == SPLIT_JOINED) { dst_i = d_tri.as<int>() + kept_nnz; dst_v = d_trv.as<T>() + kept_nnz; }
-            else { dst_i = d_rei.as<int>(); dst_v = d_rev.as<T>(); }
-            JOB_CUDA(kernels_begin());
-            gather_rows_kernel<T><<<grid_for(rem_nnz), TPB, 0, st>>>(dXp.as<int>(), dXi.as<int>(), dXv.as<T>(), d_remrows.as<int>(),
-                                                                      d_remp.as<int>(), nr, (int)rem_nnz, dst_i, dst_v);
-            launches++;
-            JOB_CUDA(kernels_end());
-            rmb200_csr_t& M = (kind == SPLIT_JOINED) ? out->train : out->rem;
-            const int64_t at = (kind == SPLIT_JOINED) ? kept_nnz : 0;
-            JOB_CUDA(down(M.indices + at, dst_i, sizeof(int32_t) * (size_t)rem_nnz));
-            JOB_CUDA(down((T*)M.values + at, dst_v, sizeof(T) * (size_t)rem_nnz));
-        }
+    // Does not wait for the replay: check_sorted_kernel, and when a split row is out of order, the segmented sort of every split
+    // row's (item id, position) pairs into `perm`.
+    bool order_unsorted_rows()
+    {
+        if (!sel_nnz) return true;
+        JOB_CUDA(kernels_begin());
+        check_sorted_kernel<<<grid_for(sel_nnz), TPB, 0, st>>>(V, d_unsorted.as<int>());
+        launches++;
+        JOB_CUDA(kernels_end());
+        int unsorted = 0;
+        JOB_CUDA(cudaMemcpyAsync(&unsorted, d_unsorted.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+        JOB_CUDA(cudaStreamSynchronize(st));
+        if (!unsorted) return true;
+        sorted_on_device = 1;
+        JOB_CUDA(d_keys0.alloc(sizeof(int) * (size_t)sel_nnz));
+        JOB_CUDA(d_keys1.alloc(sizeof(int) * (size_t)sel_nnz));
+        JOB_CUDA(d_vals0.alloc(sizeof(int) * (size_t)sel_nnz));
+        JOB_CUDA(d_perm.alloc(sizeof(int) * (size_t)sel_nnz));
+        JOB_CUDA(d_flags.alloc((size_t)sel_nnz));
+        size_t temp_bytes = 0;
+        JOB_CUDA(cub::DeviceSegmentedRadixSort::SortPairs(nullptr, temp_bytes, (const int*)d_keys0.as<int>(), d_keys1.as<int>(),
+                                                          (const int*)d_vals0.as<int>(), d_perm.as<int>(), (int)sel_nnz, ns,
+                                                          V.sel_p, V.sel_p + 1, 0, 32, st));
+        JOB_CUDA(d_sort_temp.alloc(temp_bytes));
+        JOB_CUDA(kernels_begin());
+        sort_input_kernel<<<grid_for(sel_nnz), TPB, 0, st>>>(V, d_keys0.as<int>(), d_vals0.as<int>());
+        JOB_CUDA(cub::DeviceSegmentedRadixSort::SortPairs(d_sort_temp.p, temp_bytes, (const int*)d_keys0.as<int>(), d_keys1.as<int>(),
+                                                          (const int*)d_vals0.as<int>(), d_perm.as<int>(), (int)sel_nnz, ns,
+                                                          V.sel_p, V.sel_p + 1, 0, 32, st));
+        launches += 3;     // (cub's segmented sort: at least its partition + sort kernels)
+        JOB_CUDA(kernels_end());
+        perm = d_perm.as<int>();
+        return true;
+    }
 
-        // ---- the split rows, chunk by chunk behind the replay ----
-        Downloads downloads;
-        if (!plain_copies) downloads.start(device, 2, sig, touched);
-        auto down_later = [&](void* dst, const void* src, size_t bytes) {
-            if (plain_copies) return down(dst, src, bytes);
-            d2h_bytes += (int64_t)bytes;
-            downloads.push(dst, src, bytes);
-            return cudaSuccess;
-        };
+    // Does not wait for the replay either: the rows the split leaves alone, gathered below the training rows (joined) or into
+    // a matrix of their own (separated), and brought down.
+    bool gather_untouched_rows()
+    {
+        if (!rem_nnz) return true;
+        int* dst_i; T* dst_v;
+        if (kind == SPLIT_JOINED) { dst_i = d_tri.as<int>() + kept_nnz; dst_v = d_trv.as<T>() + kept_nnz; }
+        else { dst_i = d_rei.as<int>(); dst_v = d_rev.as<T>(); }
+        JOB_CUDA(kernels_begin());
+        gather_rows_kernel<T><<<grid_for(rem_nnz), TPB, 0, st>>>(dXp.as<int>(), dXi.as<int>(), dXv.as<T>(), d_remrows.as<int>(),
+                                                                  d_remp.as<int>(), nr, (int)rem_nnz, dst_i, dst_v);
+        launches++;
+        JOB_CUDA(kernels_end());
+        rmb200_csr_t& M = (kind == SPLIT_JOINED) ? out->train : out->rem;
+        const int64_t at = (kind == SPLIT_JOINED) ? kept_nnz : 0;
+        JOB_CUDA(down(M.indices + at, dst_i, sizeof(int32_t) * (size_t)rem_nnz));
+        JOB_CUDA(down((T*)M.values + at, dst_v, sizeof(T) * (size_t)rem_nnz));
+        return true;
+    }
+
+    // The split rows, chunk by chunk behind the replay: the chunk's bytes up, scan, partition, and its pieces to the copy threads.
+    bool partition_chunks()
+    {
+        downloads.start(device, 2, prog);
         int32_t r0 = 0;
         for (size_t c = 0; c < Q.chunk_end.size(); c++) {
             const int32_t r1 = Q.chunk_end[c];
-            const auto t_wait = clk::now();
-            sig->wait([&]() { return chunk_done[c].load(std::memory_order_acquire) != 0 || stop->load() != 0; });
-            dbg_wait += ms_since(t_wait);
-            if (stop->load()) return;
+            prog.sig.wait([&]() { return prog.chunk_done[c].load(std::memory_order_acquire) != 0 || prog.stop.load() != 0; });
+            if (prog.stop.load()) return false;
             const int j0 = Q.sel_p[r0], j1 = Q.sel_p[r1];
             const int t0 = Q.test_p[r0], t1 = Q.test_p[r1];
             if (j1 > j0) {
@@ -905,10 +904,10 @@ struct DeviceJob {
         }
         JOB_CUDA(downloads.finish());
         d2h_ms += downloads.copy_ms;          // (thread time: two copies run side by side)
-        dbg_end = clk::now();
-#undef JOB_CUDA
+        return true;
     }
 };
+#undef JOB_CUDA
 
 template <typename T>
 int run_split_impl(SplitKind kind, const int32_t* Xp, const int32_t* Xi, const T* Xv, int32_t m, int32_t n,
@@ -940,15 +939,12 @@ int run_split_impl(SplitKind kind, const int32_t* Xp, const int32_t* Xi, const T
 
     // ---- which rows, and how many entries of each are held out: everything the result's shape depends on ----
     SplitPlan P;
-    if (kind != SPLIT_WHOLE)
-        if (const char* refusal = pick_users(Xp, m, n, n_users_test, test_fraction, consider_cold_start, min_items_pool,
-                                             min_pos_test, seed, P))
-            return fail(RMB200_ERR_RUNTIME, refusal);
-    count_rows(Xp, P.whole ? nullptr : P.sel_rows.data(), P.whole ? m : (int32_t)P.sel_rows.size(), test_fraction, P);
+    if (const char* refusal = plan_split(Xp, m, n, kind != SPLIT_WHOLE, n_users_test, test_fraction, consider_cold_start,
+                                         min_items_pool, min_pos_test, seed, P))
+        return fail(RMB200_ERR_RUNTIME, refusal);
     const int32_t ns = P.ns, nr = P.nr;
     const int64_t sel_nnz = P.sel_p[ns], test_nnz = P.test_p[ns], rem_nnz = nr ? P.rem_p[nr] : 0;
     const int64_t train_nnz = sel_nnz - test_nnz + (kind == SPLIT_JOINED ? rem_nnz : 0);
-    P.held.reset((size_t)sel_nnz);
 
     // ---- the result (host side): pointer arrays come straight from the plan ----
     SplitOwner* own = new (std::nothrow) SplitOwner();
@@ -979,26 +975,24 @@ int run_split_impl(SplitKind kind, const int32_t* Xp, const int32_t* Xi, const T
     }
 
     // ---- three things at once: pages of the result touched, the GPU driven, the random stream replayed (this thread) ----
-    std::unique_ptr<std::atomic<int>[]> chunk_done(new std::atomic<int>[P.chunk_end.size()]);
-    for (size_t c = 0; c < P.chunk_end.size(); c++) chunk_done[c].store(0);
-    std::atomic<int> stop{0}, touched{0};
-    Signal sig;
-    DeviceJob<T> job;
-    job.kind = kind; job.device = device; job.Xp = Xp; job.Xi = Xi; job.Xv = Xv; job.m = m; job.nnz = nnz;
-    job.P = &P; job.out = out; job.chunk_done = chunk_done.get(); job.stop = &stop; job.touched = &touched; job.sig = &sig;
+    Progress prog(P.chunk_end.size());
+    DeviceJob<T> job{kind, device, Xp, Xi, Xv, m, nnz, P, out, prog};
     struct Joiner { std::thread t; ~Joiner() { if (t.joinable()) t.join(); } };
     double replay_ms = 0.0;
     {
-        Joiner toucher{std::thread([&]() { try { touch_pages(own); } catch (...) {} sig.update([&]() { touched.store(1, std::memory_order_release); }); })};
+        Joiner toucher{std::thread([&]() { try { touch_pages(own); } catch (...) {} prog.sig.update([&]() { prog.touched.store(1, std::memory_order_release); }); })};
         Joiner driver{std::thread([&]() {
-            try { job.run(); } catch (...) { job.status = RMB200_ERR_OOM; job.what = "device thread"; sig.update([&]() { stop.store(1); }); }
+            try {
+                if (job.upload() && job.order_unsorted_rows() && job.gather_untouched_rows()) job.partition_chunks();
+            } catch (...) { job.status = RMB200_ERR_OOM; job.what = "device thread"; prog.sig.update([&]() { prog.stop.store(1); }); }
+            job.downloads.finish();      // (after a failure too: the copy threads write into the result, which is freed below)
         })};
         const auto t_replay = clk::now();
         try {
-            Replay replay{P, seed, chunk_done.get(), stop, sig};
+            Replay replay{P, seed, prog};
             replay.run();
         } catch (...) {
-            sig.update([&]() { stop.store(1); });
+            prog.sig.update([&]() { prog.stop.store(1); });
             throw;                   // (Joiner joins the device thread first)
         }
         replay_ms = ms_since(t_replay);
@@ -1079,23 +1073,16 @@ int rmb200_split_plan(const int32_t* Xp, int32_t m, int32_t n, int32_t sample_us
     rmb::g_err.clear();
     if (!Xp || m <= 0 || !held || !n_entries_out) return fail(RMB200_ERR_BAD_ARG, "rmb200_split_plan: bad arguments");
     return rmb::guard([&] {
+        if (sample_users && (!users_test || !n_users_out)) return fail(RMB200_ERR_BAD_ARG, "rmb200_split_plan: users_test missing");
         SplitPlan P;
-        if (sample_users) {
-            if (!users_test || !n_users_out) return fail(RMB200_ERR_BAD_ARG, "rmb200_split_plan: users_test missing");
-            if (const char* refusal = pick_users(Xp, m, n, n_users_test, test_fraction, consider_cold_start != 0, min_items_pool,
-                                                 min_pos_test, seed, P))
-                return fail(RMB200_ERR_RUNTIME, refusal);
-        }
-        count_rows(Xp, P.whole ? nullptr : P.sel_rows.data(), P.whole ? m : (int32_t)P.sel_rows.size(), test_fraction, P);
-        P.held.reset((size_t)P.sel_p[P.ns]);
-        std::unique_ptr<std::atomic<int>[]> chunk_done(new std::atomic<int>[P.chunk_end.size()]);
-        for (size_t c = 0; c < P.chunk_end.size(); c++) chunk_done[c].store(0);
-        std::atomic<int> stop{0};
-        Signal sig;
-        Replay replay{P, seed, chunk_done.get(), stop, sig};
+        if (const char* refusal = plan_split(Xp, m, n, sample_users != 0, n_users_test, test_fraction, consider_cold_start != 0,
+                                             min_items_pool, min_pos_test, seed, P))
+            return fail(RMB200_ERR_RUNTIME, refusal);
+        Progress prog(P.chunk_end.size());
+        Replay replay{P, seed, prog};
         replay.run();
         for (size_t c = 0; c < P.chunk_end.size(); c++)
-            if (!chunk_done[c].load()) return fail(RMB200_ERR_CUDA, "rmb200_split_plan: a chunk was never published");
+            if (!prog.chunk_done[c].load()) return fail(RMB200_ERR_CUDA, "rmb200_split_plan: a chunk was never published");
         if (sample_users) {
             std::memcpy(users_test, P.sel_rows.data(), sizeof(int32_t) * P.sel_rows.size());
             *n_users_out = (int32_t)P.sel_rows.size();

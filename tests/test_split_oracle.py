@@ -200,8 +200,8 @@ def test_host_plan_threaded_replay(rb, oracle_mod, monkeypatch, knobs):
 
 
 def test_host_plan_threaded_replay_randomised(rb, monkeypatch):
-    """A few hundred calls with random worker counts, both forms of the scout, random injected miscounts and seeds beyond 32 bits,
-    on rows that reach the shuffle's second regime (65,536 entries and more): always the bytes of the sequential replay."""
+    """A few hundred calls with random worker counts, random injected miscounts and seeds beyond 32 bits, on rows that reach
+    the shuffle's second regime (65,536 entries and more): always the bytes of the sequential replay."""
     from recometrics_b200 import _capi
     rs = np.random.RandomState(11)
     p, i, v = split_cases.make_csr(m=1500, n=70001, seed=31, mean_len=12.0, heavy_rows=(66000, 65535, 2, 3, 4, 5))
@@ -212,10 +212,6 @@ def test_host_plan_threaded_replay_randomised(rb, monkeypatch):
         monkeypatch.setenv("RMB200_SPLIT_CHUNK", "9000")
         for _ in range(60):
             monkeypatch.setenv("RMB200_SPLIT_THREADS", str(rs.randint(1, 7)))
-            if rs.rand() < 0.5:
-                monkeypatch.setenv("RMB200_SPLIT_PLAIN_SCOUT", "1")
-            else:
-                monkeypatch.delenv("RMB200_SPLIT_PLAIN_SCOUT", raising=False)
             fault = int(rs.randint(-1, 20))
             if fault >= 0:
                 monkeypatch.setenv("RMB200_SPLIT_SCOUT_FAULT", str(fault))
